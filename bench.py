@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the B200 reference-matching stage (BASELINE.json metric: matching-stage images/s).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One process per GPU (the driver launches torchrun for N>1; RANK/LOCAL_RANK/WORLD_SIZE from the env).  Every run
 executes the reference's three stages through the repository's own host code:
@@ -55,7 +55,8 @@ WORKLOAD = dict(workload="coco80x10_sam2L_dinov2L_1024masks_1024x1024", n_masks=
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps of the resident measurement (`value`); the e2e "
+                    "legs time min(steps, 10) steps of their own, at least 2, and report that number")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--images-per-step", type=int, default=256, help="images per step per GPU")
@@ -71,7 +72,14 @@ def parse():
                     help="context tunable for A/B runs (MatchingStage.TUNABLES), e.g. upsample_stage_bytes=0")
     ap.add_argument("--value-only", action="store_true", help="A/B helper: fill + `value` only, short line "
                     "(no e2e legs, no roofline / cpu_baseline) - not the driver's contract line")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one returned as "
+                    "DIR/<name>.npy (rank 0's images; see dump_outputs) to compare two builds output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
+    return args
 
 
 def configure_workload(args, world):
@@ -194,6 +202,65 @@ def stage_floor(n_masks, us_per_image):
     peak, _ = measured_peak()
     floor_us = nbytes / (peak * 1e9) * 1e6
     return dict(compulsory_bytes=nbytes, floor_us=floor_us, achieved_us=us_per_image, frac=floor_us / us_per_image)
+
+
+DUMP_BYTES = 64 << 20  # what --dump-outputs may write in all: half for the per-image arrays, half for the mask sample
+DUMP_PIXELS = 4096     # sampled pixels per output mask (fewer when many stream slots share the half)
+
+
+def dump_outputs(out_dir, last_step, num_out, seed=0):
+    """Write what the last timed step returned to its caller as float `.npy` files, so that two builds can be
+    compared output for output on the same seeded inputs.
+
+    `last_step`: (image, stream slot, PendingResult) in launch order.  For every distinct image (its last result; a
+    seeded sample of the images if there are too many): `scores`, `labels`, `bboxes`, `index` [images, num_out(, 4)],
+    NaN past the image's n_out, `counts` [images, 3] = (n_keep, n_sel, n_out) and `image`, the image's index in the
+    synthetic dataset.  Masks share one buffer per stream slot, so only the last image of each slot still holds its
+    masks: for those images (`mask_image`), `mask_area` [.., num_out] and `mask_samples` [.., num_out, P], the masks
+    at the P flat pixel indices `mask_pixels` drawn with a fixed seed, NaN past n_out."""
+    import numpy as np
+    last = {img: r for r, (img, _, _) in enumerate(last_step)}
+    rows = sorted(last.values())
+    row_bytes = num_out * (4 + 8 + 32 + 8) + 32
+    if len(rows) * row_bytes > DUMP_BYTES // 2:
+        pick = np.random.default_rng(seed + 1).choice(len(rows), DUMP_BYTES // 2 // row_bytes, replace=False)
+        rows = [rows[i] for i in sorted(pick)]
+    mask_rows = sorted({slot: r for r, (_, slot, _) in enumerate(last_step)}.values())
+    res = {r: last_step[r][2].get() for r in set(rows) | set(mask_rows)}
+    ori_hw = last_step[0][2].ori_hw
+
+    def padded(values, shape, dtype):
+        out = np.full(shape, np.nan, dtype)
+        for i, v in enumerate(values):
+            out[i, :len(v)] = v
+        return out
+
+    n = len(rows)
+    arrays = dict(
+        image=np.array([last_step[r][0] for r in rows], np.float64),
+        counts=np.array([[res[r]["counts"][k] for k in ("n_keep", "n_sel", "n_out")] for r in rows], np.float64),
+        scores=padded([res[r]["scores"].cpu().numpy() for r in rows], (n, num_out), np.float32),
+        labels=padded([res[r]["labels"].cpu().numpy() for r in rows], (n, num_out), np.float64),
+        bboxes=padded([res[r]["bboxes"].cpu().numpy() for r in rows], (n, num_out, 4), np.float64),
+        index=padded([res[r]["index"].cpu().numpy() for r in rows], (n, num_out), np.float64))
+    hw, m_img = ori_hw[0] * ori_hw[1], len(mask_rows)
+    n_pix = min(DUMP_PIXELS, hw, (DUMP_BYTES // 2 - 8 * m_img * (num_out + 1)) // (4 * m_img * num_out + 8))
+    pixels = np.sort(np.random.default_rng(seed).choice(hw, n_pix, replace=False))
+    idx = torch.from_numpy(pixels).to(res[mask_rows[0]]["bboxes"].device)
+    areas, samples = [], []
+    for r in mask_rows:
+        m = res[r]["binary_masks"]
+        m = m.reshape(m.shape[0], hw)
+        areas.append(m.sum(1).cpu().numpy())
+        samples.append(m[:, idx].cpu().numpy())
+    arrays.update(mask_image=np.array([last_step[r][0] for r in mask_rows], np.float64),
+                  mask_area=padded(areas, (len(mask_rows), num_out), np.float64),
+                  mask_samples=padded(samples, (len(mask_rows), num_out, n_pix), np.float32),
+                  mask_pixels=pixels.astype(np.float64))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return arrays
 
 
 def cpu_synthetic(args):
@@ -421,8 +488,10 @@ def main():
             g.lr_masks, g.pred_ious, g.tar_feat = resident[i]
             graphs[(i, pos % S)] = g.capture()
 
+    last_step = []  # (image, slot, result) of every image of the most recent step, for --dump-outputs
+
     def resident_step():
-        pend = None
+        last_step.clear()
         for b in range(B):
             pos = b % len(shard)
             k = pos % S
@@ -431,7 +500,7 @@ def main():
                     pend = graphs[(shard[pos], k)].replay()
                 else:
                     pend = stage.match_async(*resident[shard[pos]], ori_hw, slot=k, persistent_out=outs[k])
-        return pend
+            last_step.append((shard[pos], k, pend))
 
     def timed(step_fn, steps):
         barrier()
@@ -464,6 +533,8 @@ def main():
         clocks.start()
     ms_total, t0, t1, ms_per_rank = timed(resident_step, args.steps)
     clock_info = clocks.stop(t0, t1) if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last_step, n_out)
     launches = launches_per_image * args.steps * B
     images = world * args.steps * B
     value = images / (ms_total / 1e3)

@@ -388,6 +388,28 @@ def run_fill_case(ref, name, spec):
     print(f"{name}: fill_counts={bank.fill_counts.tolist()}")
 
 
+def run_target_feature_case(ref, name="target_features_dinov2_s", n_rows=48):
+    """The reference's `_extract_target_features` (bicubic 1024 -> 518, ImageNet normalisation, encoder, CLS dropped) on
+    the random-init DINOv2 of `sam2_builder.build_dinov2()` and a seeded image: a seeded sample of `n_rows` of its
+    [1369, C] output, and the sha256 of the whole output."""
+    import sam2_builder
+    from torchvision.transforms import Normalize
+    enc = sam2_builder.build_dinov2()
+    gen = torch.Generator().manual_seed(3)
+    img = torch.rand(3, 1024, 1024, generator=gen)
+    fake = types.SimpleNamespace(encoder=enc, encoder_img_size=518, encoder_dim=384,
+                                 encoder_transform=Normalize(mean=(0.485, 0.456, 0.406), std=(0.229, 0.224, 0.225)))
+    for fn in ("_forward_encoder", "_extract_target_features"):
+        setattr(fake, fn, types.MethodType(getattr(ref.Model, fn), fake))
+    with torch.inference_mode():
+        want = fake._extract_target_features(img, torch.device("cpu"))
+    want = (want[0] if isinstance(want, tuple) else want).reshape(-1, 384).contiguous()
+    rows = np.sort(np.random.default_rng(3).choice(want.shape[0], n_rows, replace=False))
+    np.savez_compressed(os.path.join(HERE, name + ".npz"), rows=rows, feat_rows=want[rows].numpy(),
+                        shape=np.array(want.shape), feat_sha=sha(want), image_sha=sha(img))
+    print(f"{name}: {tuple(want.shape)}, {n_rows} rows stored")
+
+
 def main():
     torch.manual_seed(0)
     ref = ref_shim.load()
@@ -406,6 +428,8 @@ def main():
             run_multimask_case(ref, name, spec)
     if not only or "rle" in only:
         run_rle_golden(ref)
+    if not only or "target_features" in only:
+        run_target_feature_case(ref)
 
 
 if __name__ == "__main__":

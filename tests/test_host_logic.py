@@ -52,12 +52,14 @@ def _fake_finalize(sums, wsum):
     return sums / w[..., None], sums.sum(1) / wall
 
 
-def _patch():
+def _patch(monkeypatch):
+    """Put the fakes in place of the fill kernels through `monkeypatch`, which undoes them after the test: later tests
+    in the same process must reach the CUDA kernels again."""
     ops = importlib.import_module("no-time-to-train_b200.ops")
-    ops.fill_pool_batch = _fake_pool_batch
-    ops.fill_pool_accumulate = _fake_pool_one
-    ops.fill_scatter = _fake_scatter
-    ops.fill_finalize = _fake_finalize
+    monkeypatch.setattr(ops, "fill_pool_batch", _fake_pool_batch)
+    monkeypatch.setattr(ops, "fill_pool_accumulate", _fake_pool_one)
+    monkeypatch.setattr(ops, "fill_scatter", _fake_scatter)
+    monkeypatch.setattr(ops, "fill_finalize", _fake_finalize)
 
 
 def _shots(n_cls, shots, c):
@@ -75,7 +77,7 @@ def _worker(rank, world, port, n_cls, shots, c, out_dir):
     os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port))
     dist.init_process_group("gloo", rank=rank, world_size=world)
     try:
-        _patch()
+        _patch(pytest.MonkeyPatch())  # a spawned worker: the patch ends with the process
         pkg = importlib.import_module("no-time-to-train_b200")
         feats, masks = _shots(n_cls, shots, c)
         bank = pkg.MemoryBank(dict(category_num=n_cls, length=shots, feat_shape=(1369, c)))
@@ -104,9 +106,9 @@ def _worker(rank, world, port, n_cls, shots, c, out_dir):
         dist.destroy_process_group()
 
 
-def _single_process_bank(n_cls, shots, c, world):
+def _single_process_bank(n_cls, shots, c, world, monkeypatch):
     """The same shots through ONE process, in the order the reference's gathered loop sees them with `world` ranks."""
-    _patch()
+    _patch(monkeypatch)
     pkg = importlib.import_module("no-time-to-train_b200")
     feats, masks = _shots(n_cls, shots, c)
     bank = pkg.MemoryBank(dict(category_num=n_cls, length=shots, feat_shape=(1369, c)))
@@ -120,7 +122,7 @@ def _single_process_bank(n_cls, shots, c, world):
 
 
 @pytest.mark.parametrize("world,n_cls,shots", [(2, 3, 2), (4, 4, 3)])
-def test_distributed_fill_matches_single_process_reference(tmp_path, world, n_cls, shots):
+def test_distributed_fill_matches_single_process_reference(tmp_path, monkeypatch, world, n_cls, shots):
     from oracle import ref_torch
     c = 16
     port = 29500 + (os.getpid() % 2000) + world
@@ -136,7 +138,7 @@ def test_distributed_fill_matches_single_process_reference(tmp_path, world, n_cl
             ref_torch.bank_fill(raw, [ci], feats[ci, li][None], masks[ci, li][None])
     want_avg, want_ins = ref_torch.bank_postprocess(raw)
     outs = [torch.load(os.path.join(tmp_path, f"rank{r}.pt")) for r in range(world)]
-    single = _single_process_bank(n_cls, shots, c, world)
+    single = _single_process_bank(n_cls, shots, c, world, monkeypatch)
     for o in outs:
         assert torch.equal(o["counts"], raw.fill_counts)
         assert torch.equal(o["sd"]["masks"], raw.masks)
@@ -147,8 +149,8 @@ def test_distributed_fill_matches_single_process_reference(tmp_path, world, n_cl
         assert torch.equal(o["ins"], single.feats_ins_avg) and torch.equal(o["avg"], single.feats_avg)
 
 
-def test_single_process_fill_and_state_dict_names():
-    _patch()
+def test_single_process_fill_and_state_dict_names(monkeypatch):
+    _patch(monkeypatch)
     pkg = importlib.import_module("no-time-to-train_b200")
     n_cls, shots, c = 2, 2, 8
     feats, masks = _shots(n_cls, shots, c)
@@ -173,13 +175,13 @@ def test_single_process_fill_and_state_dict_names():
     assert torch.equal(other.feats_ins_avg, bank.feats_ins_avg) and bool(other.postprocessed[0])
 
 
-def test_reference_fill_stage_checkpoint_is_reduced_on_load():
+def test_reference_fill_stage_checkpoint_is_reduced_on_load(monkeypatch):
     """The reference saves after `fill_memory` and post-processes FROM THAT CHECKPOINT (README.md:194-217): its state
     dict holds raw `feats [n_cls, L, E, C]` + `masks` (matching_baseline_utils.py:561-571) and none of our compact sums.
     Loading it must reduce the raw features (sum_e feats * masks) so that `postprocess()` gives what the reference's
     own postprocess gives — not silently leave zero prototypes."""
     from oracle import ref_torch
-    _patch()
+    _patch(monkeypatch)
     pkg = importlib.import_module("no-time-to-train_b200")
     n_cls, shots, c = 3, 2, 8
     feats, masks = _shots(n_cls, shots, c)
