@@ -44,8 +44,8 @@ enum {
 typedef struct nttt_ctx nttt_ctx;
 
 int nttt_version(void);
-/* 1 if the library was built with -DNTTT_ABLATE (honours NTTT_STOP_AFTER / NTTT_PACK_MODE for tools/ablate.py);
- * the product build returns 0 and contains neither switch. */
+/* 1 if the library was built with -DNTTT_ABLATE (honours NTTT_STOP_AFTER for tools/ablate.py);
+ * the product build returns 0 and does not contain the switch. */
 int nttt_build_is_ablation(void);
 const char* nttt_error_string(int code);
 /* text of the last CUDA error seen by this thread's calls ("" if none) */
@@ -56,37 +56,23 @@ const char* nttt_last_cuda_error(void);
 int nttt_ctx_create(nttt_ctx** out, int device);
 void nttt_ctx_destroy(nttt_ctx* ctx);
 
-/* Tunables of a context (defaults are the measured best on B200; results never depend on them):
- *   NTTT_TUNE_UPSAMPLE_STAGE_BYTES  shared-memory budget per CTA of the full-resolution resize for staging the logit
- *                                   tile under its row groups (0 = every tap is read from global memory; tiles that
- *                                   do not fit take that path anyway).  Default 36 KB.
- *   NTTT_TUNE_LOWRES_EXTRA_SMEM     extra dynamic shared memory per CTA of the low-res pass (fewer resident CTAs per
- *                                   SM; process-wide).  Default 0 — measured: leaving room for other kernels buys nothing.
- *   NTTT_TUNE_LOWRES_PERSISTENT     0 (default): the low-res pass runs one CTA per mask, three resident per SM; 1: persistent,
- *                                   one CTA per SM with a 7-stage TMA ring; 2: persistent, two CTAs per SM with 4 stages
- *                                   (process-wide).  Bit-identical; measured equal in throughput (92.6 / 93.8 / 92.7
- *                                   us/image): the stage is bound by L2 tag throughput, which co-residency does not create.
- *   NTTT_TUNE_AXIS_CACHE_ENTRIES    capacity of the antialias-table cache (8..1024; shrinking below the number
- *                                   held drops the cache behind a device synchronisation).  Default 1024: an image takes one table per distinct height and width.
- *   NTTT_TUNE_GEMM_BN256_MIN_M      row count from which the pooling GEMM uses 128 x 256 tiles (process-wide).
- *                                   Default 512 (measured: 32 fat CTAs beat 64 at 1024 rows, 97.9 vs 100.3 us/image).
- *   NTTT_TUNE_GEMM_SHARED_SEGMENTS  0 (default): the split-bf16 GEMMs stream all three K-segments of both operands; 1: they
- *                                   load each k-block's four distinct operand tiles (A_hi, A_lo, B_hi, B_lo) once and
- *                                   multiply them three ways (a third less L2 traffic; same products, summed in a
- *                                   different order — float results may differ in the last bit).  Measured equal in
- *                                   throughput: the kernel is bound by its SM's tensor pipe.  Process-wide.
- *   NTTT_TUNE_GEMM_BN256_STAGES     2..4 (default 3): TMA ring depth of the 128 x 256 pooling GEMM (48 KB per stage); fewer
- *                                   stages leave shared memory to co-resident CTAs of other kernels.  Process-wide.
- *   NTTT_TUNE_UPSAMPLE_CTAS_PER_SM  1..7 (default 1): persistent CTAs per SM of the full-resolution resize when many images
- *                                   are in flight (low-latency mode always uses 7).  Measured 89.8 (1) / 90.7 (2) / 91.2 (3) /
- *                                   91.9 (7) us/image.  Process-wide.
- *   NTTT_TUNE_EXPERIMENT + i        (i = 0..7) launch-shape experiment slots used by tools/ and `bench.py --tune expI=V`
- *                                   for A/B runs (grid sizes of single kernels, slot 1 = 1: pooling GEMM on unordered rows
- *                                   without k-block skipping, slot 6 = 1: programmatic dependent launch off);
- *                                   0 = the built-in default.  Results never depend on them. */
-enum { NTTT_TUNE_UPSAMPLE_STAGE_BYTES = 1, NTTT_TUNE_LOWRES_EXTRA_SMEM = 2, NTTT_TUNE_GEMM_BN256_MIN_M = 3,
-       NTTT_TUNE_AXIS_CACHE_ENTRIES = 4, NTTT_TUNE_LOWRES_PERSISTENT = 5, NTTT_TUNE_GEMM_SHARED_SEGMENTS = 6,
-       NTTT_TUNE_GEMM_BN256_STAGES = 7, NTTT_TUNE_UPSAMPLE_CTAS_PER_SM = 8, NTTT_TUNE_EXPERIMENT = 100 };
+/* Tunables (results never depend on them).  Any other `what`, or a value out of range, returns NTTT_EINVAL.
+ *   NTTT_TUNE_UPSAMPLE_STAGE_BYTES  0..160 KB: shared-memory budget per CTA of the full-resolution resize for staging the
+ *                                   logit tile under its row groups (0 = every tap is read from global memory; tiles
+ *                                   that do not fit take that path anyway).  Default 36 KB, the measured best on B200.
+ *   NTTT_TUNE_AXIS_CACHE_ENTRIES    8..1024: capacity of the context's antialias-table cache (shrinking below the number
+ *                                   held drops the cache behind a device synchronisation).  Default 1024: an image takes
+ *                                   one table per distinct height and width.
+ * The next two each choose between the two paths the library runs anyway, so that tests can force either one and
+ * compare them bit for bit:
+ *   NTTT_TUNE_LOWRES_PERSISTENT     0 or 1, process-wide.  1 (default): the low-res pass runs persistent CTAs, two per SM;
+ *                                   0: one CTA per mask, the kernel the low-latency mode always runs.
+ *   NTTT_TUNE_POOL_ORDER            0 or 1.  1 (default): with many images in flight (low_latency = 0) and more than 128
+ *                                   masks, the pooling GEMM of nttt_match_image runs on spatially ordered rows and skips
+ *                                   the k-blocks a tile of masks does not touch; 0: unordered rows without skipping, the
+ *                                   path of the low-latency mode and of 128 masks or fewer. */
+enum { NTTT_TUNE_UPSAMPLE_STAGE_BYTES = 1, NTTT_TUNE_AXIS_CACHE_ENTRIES = 4, NTTT_TUNE_LOWRES_PERSISTENT = 5,
+       NTTT_TUNE_POOL_ORDER = 9 };
 int nttt_ctx_tune(nttt_ctx* ctx, int what, long long value);
 
 /* number of kernels this library has launched in this process (bench.py's `gpu_launches`) */

@@ -47,8 +47,8 @@ def _stale(target: str, deps) -> bool:
 
 def build_library(force: bool = False, verbose: bool = False) -> str:
     os.makedirs(OBJ, exist_ok=True)
-    # NTTT_BUILD_ABLATE=1: measurement build for tools/ablate.py (-DNTTT_ABLATE compiles the NTTT_STOP_AFTER /
-    # NTTT_PACK_MODE switches in).  The flavour is recorded next to the objects so that switching it rebuilds.
+    # NTTT_BUILD_ABLATE=1: measurement build for tools/ablate.py (-DNTTT_ABLATE compiles the NTTT_STOP_AFTER switch
+    # in).  The flavour is recorded next to the objects so that switching it rebuilds.
     ablate = os.environ.get("NTTT_BUILD_ABLATE", "0") not in ("", "0")
     flavour_file = os.path.join(OBJ, "flavour")
     flavour = "ablate" if ablate else "product"

@@ -57,15 +57,9 @@ int launch_fill_scatter(const float*, const float*, const float*, const int32_t*
                         cudaStream_t);
 int launch_fill_finalize(const float*, const float*, int, int, int, float*, float*, cudaStream_t);
 
-extern int g_pack_extra_smem;  // lowres.cu
 extern int g_pack_persistent;  // lowres.cu
-extern int g_gemm_bn256_min_m;  // gemm_tc.cu
-extern int g_gemm_shared_segments;
-extern int g_gemm_bn256_stages;
-extern int g_up2_ctas_per_sm;
 static thread_local char g_cuda_err[512] = "";
 std::atomic<unsigned long long> g_launches{0};
-int g_exp[8] = {};
 thread_local bool t_low_latency = false;
 thread_local bool t_chain_break = false;
 
@@ -280,39 +274,19 @@ int nttt_ctx_tune(nttt_ctx* ctx, int what, long long value) {
       }
       ctx->max_tables = (int)value;
       return NTTT_OK;
-    case NTTT_TUNE_GEMM_BN256_MIN_M:
-      if (value < 0) return NTTT_EINVAL;
-      nttt::g_gemm_bn256_min_m = (int)value;
-      return NTTT_OK;
-    case NTTT_TUNE_GEMM_SHARED_SEGMENTS:
-      if (value < 0 || value > 1) return NTTT_EINVAL;
-      nttt::g_gemm_shared_segments = (int)value;
-      return NTTT_OK;
-    case NTTT_TUNE_GEMM_BN256_STAGES:
-      if (value < 2 || value > 4) return NTTT_EINVAL;
-      nttt::g_gemm_bn256_stages = (int)value;
-      return NTTT_OK;
-    case NTTT_TUNE_UPSAMPLE_CTAS_PER_SM:
-      if (value < 1 || value > 7) return NTTT_EINVAL;
-      nttt::g_up2_ctas_per_sm = (int)value;
-      return NTTT_OK;
     case NTTT_TUNE_LOWRES_PERSISTENT:
-      if (value < 0 || value > 49) return NTTT_EINVAL;
+      if (value < 0 || value > 1) return NTTT_EINVAL;
       nttt::g_pack_persistent = (int)value;
       return NTTT_OK;
-    case NTTT_TUNE_LOWRES_EXTRA_SMEM:
-      if (value < 0 || value > 128 * 1024) return NTTT_EINVAL;
-      nttt::g_pack_extra_smem = (int)value;
+    case NTTT_TUNE_POOL_ORDER:
+      if (value < 0 || value > 1) return NTTT_EINVAL;
+      ctx->pool_order = value != 0;
       return NTTT_OK;
     case NTTT_TUNE_UPSAMPLE_STAGE_BYTES:
       if (value < 0 || value > 160 * 1024) return NTTT_EINVAL;
       ctx->upsample_stage_floats = (int)(value / 4);
       return NTTT_OK;
     default:
-      if (what >= NTTT_TUNE_EXPERIMENT && what < NTTT_TUNE_EXPERIMENT + 8 && value >= 0 && value <= (1 << 20)) {
-        nttt::g_exp[what - NTTT_TUNE_EXPERIMENT] = (int)value;
-        return NTTT_OK;
-      }
       return NTTT_EINVAL;
   }
 }
@@ -797,6 +771,7 @@ int nttt_match_image(nttt_ctx* ctx, const nttt_match_args* a, void* stream) {
   MatchLayout L = carve(a->workspace, n, a->lr_h, a->lr_w, a->eh, a->ew, a->c, a->n_cls, a->ori_h, a->ori_w, max_sel,
                         num_out, l_neg);
   if (a->workspace_bytes < L.total) return NTTT_EWORKSPACE;
+  if (!projection_supported(a->ew, a->lr_w) || !projection_supported(a->eh, a->lr_h)) return NTTT_EUNSUPPORTED;
   float* obj_feats = a->obj_feats ? a->obj_feats : L.obj_feats;
   float* sim = a->sim ? a->sim : L.sim;
   struct LaunchMode {  // the launch shapes of this call (common.cuh: t_low_latency), restored on every return path
@@ -858,6 +833,13 @@ int nttt_match_image(nttt_ctx* ctx, const nttt_match_args* a, void* stream) {
   // low-latency mode: the two operand preparations that do not depend on the masks (features -> transposed split
   // operand, prototypes -> split operand) run on the context's side stream while the main stream reads the logits
   const bool forked = a->low_latency != 0 && ctx->side_ready();
+  // Once the side stream's work is recorded in ev_join, every return makes `s` wait for it: an early return must neither
+  // leave the side stream writing the workspace after the call nor leave a stream capture unjoined.
+  struct SideJoin {
+    cudaStream_t s;
+    cudaEvent_t ev = nullptr;  // armed while not null
+    ~SideJoin() { if (ev) cudaStreamWaitEvent(s, ev, 0); }
+  } side_join{s};
   if (forked) {
     NTTT_CUDA(cudaEventRecord(ctx->ev_fork, s));
     NTTT_CUDA(cudaStreamWaitEvent(ctx->side, ctx->ev_fork, 0));
@@ -866,16 +848,16 @@ int nttt_match_image(nttt_ctx* ctx, const nttt_match_args* a, void* stream) {
     err = launch_split_rows(a->proto, a->c, a->n_cls, a->c, pad64(a->c), 1, L.p_split, ctx->side);
     if (err) return err;
     NTTT_CUDA(cudaEventRecord(ctx->ev_join, ctx->side));
+    side_join.ev = ctx->ev_join;
   }
   // a6/a9/a15: one pass over the logits
   // (the stability counts of a15 are not read on this path, so the pipeline does not pay for them)
   NTTT_STEP(launch_lowres_pack(a->logits, n, a->lr_h, a->lr_w, 0.0f, 1.0f, L.bits_lr, L.area_lr, L.box_lr, nullptr,
                                L.flags, a->filter_iou ? pred_ious : nullptr, a->iou_thr, mask_ptr, s));
   // a6/a7: projection + pooling contraction + normalisation
-  if (!projection_supported(a->ew, a->lr_w) || !projection_supported(a->eh, a->lr_h)) return NTTT_EUNSUPPORTED;
   // Many images in flight: the pooling GEMM runs on spatially ordered rows and skips the k-blocks a tile of masks does
   // not touch (~45 % of them).  Needs the vector normalisation path (it undoes the order) and <= 32 k-blocks per segment.
-  const bool ordered = !a->low_latency && g_exp[1] != 1 && n > 128 && n <= 8192 && pad64(e) / 64 <= 32 &&
+  const bool ordered = !a->low_latency && ctx->pool_order && n > 128 && n <= 8192 && pad64(e) / 64 <= 32 &&
                        (a->c == 384 || a->c == 768 || a->c == 1024 || a->c == 1536);
   if (ordered) NTTT_STEP_QUIET(launch_pool_order(L.box_lr, n, a->lr_h, L.pool_perm, s));
   NTTT_STEP(launch_project_masks(px, py, L.bits_lr, L.box_lr, n, a->lr_h, a->lr_w, a->eh, a->ew, L.a_split, pad64(e),
@@ -883,6 +865,7 @@ int nttt_match_image(nttt_ctx* ctx, const nttt_match_args* a, void* stream) {
   int n_partials = 1;
   if (forked) {
     NTTT_CUDA(cudaStreamWaitEvent(s, ctx->ev_join, 0));
+    side_join.ev = nullptr;
     nttt::t_chain_break = true;  // the pooling GEMM depends on the side stream as well: launched the ordinary way
   }
   NTTT_STEP(pool_contract(nullptr, a->tar_feat, n, e, a->c, L.sums, L.a_split, L.b_split, &n_partials, s,
@@ -908,7 +891,7 @@ int nttt_match_image(nttt_ctx* ctx, const nttt_match_args* a, void* stream) {
   // a13
   NTTT_STEP(launch_mask_ios(L.bits_full, L.rect, L.area_full, L.box_full, L.sel, a->counts + 1, max_sel, a->ori_h,
                             a->ori_w, L.top_label, obj_feats, a->c, L.ios, nullptr, L.ios_ws, false, s,
-                            wrote_t ? L.bits_t : nullptr, /*counters_zeroed=*/wrote_t && a->low_latency != 0 && g_exp[4] != 1));  // (folding the metadata
+                            wrote_t ? L.bits_t : nullptr, /*counters_zeroed=*/wrote_t && a->low_latency != 0));  // (folding the metadata
   // kernel into the pair kernel takes 1 us off a single image's chain and costs 0.3 us/image with images in flight)
   // a14
   NTTT_STEP(launch_decay_rank(L.top_score, L.top_label, L.ios, L.sel, a->counts + 1, max_sel, num_out, L.box_full,

@@ -33,7 +33,6 @@ extern thread_local bool t_low_latency;
 // set after a cross-stream event wait: the next chain launch is an ordinary one (its predecessor in the stream is the
 // wait, not a kernel that triggers), then the flag clears itself
 extern thread_local bool t_chain_break;
-extern int g_exp[8];  // launch-shape experiments (nttt_ctx_tune ids 100..107); 0 = the built-in default
 extern std::atomic<unsigned long long> g_launches;  // (host threads of different contexts may launch concurrently)
 #define NTTT_LAUNCH_CHECK()          \
   do {                               \
@@ -46,7 +45,7 @@ extern std::atomic<unsigned long long> g_launches;  // (host threads of differen
 // still running, and its `chain_wait()` — the first statement of every chain kernel — holds it until the predecessor
 // has completed and its writes are visible.  What overlaps is the launch latency and the CTA ramp-up, 2-3 us per kernel
 // boundary of an 18-kernel chain.  Without the attribute (many images in flight: other streams fill the gaps anyway)
-// chain_wait() returns immediately.  g_exp[6] = 1 switches the attribute off (A/B).
+// chain_wait() returns immediately.
 template <typename... KArgs, typename... Args>
 inline void launch_chain(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s, Args&&... args) {
   cudaLaunchConfig_t cfg = {};
@@ -58,7 +57,7 @@ inline void launch_chain(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = (t_low_latency && g_exp[6] != 1 && !t_chain_break) ? 1 : 0;
+  cfg.numAttrs = (t_low_latency && !t_chain_break) ? 1 : 0;
   t_chain_break = false;
   (void)cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);  // (the error is picked up by NTTT_LAUNCH_CHECK)
 }
@@ -191,6 +190,9 @@ struct nttt_ctx {
   int n_tables = 0;
   // shared-memory budget of upsample_pack's logit tile, in floats (nttt_ctx_tune; 0 = read taps from global memory)
   int upsample_stage_floats = 36 * 1024 / 4;
+  // nttt_ctx_tune(NTTT_TUNE_POOL_ORDER): 0 runs the pooling GEMM of nttt_match_image on unordered rows (the path of
+  // the low-latency mode and of n <= 128), so that tests can compare it with the ordered one
+  bool pool_order = true;
   int32_t* scratch = nullptr;  // per-mask statistics scratch of the stand-alone resize entry
   size_t scratch_cap = 0;  // bytes
   // optional per-stage CUDA-event profile of nttt_match_image (off by default)

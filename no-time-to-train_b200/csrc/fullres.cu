@@ -104,9 +104,6 @@ __device__ __forceinline__ int up_ctas_needed(int n_groups) {
 // once, vertical pass per output row, one ballot per row.
 // All indices inside the loops are 32-bit (one 64-bit base per array): 64-bit index arithmetic was a third of the
 // instructions of an earlier version.
-#ifndef NTTT_UP_MINBLOCKS
-#define NTTT_UP_MINBLOCKS 5
-#endif
 // Logit tile staging: the taps of every boundary word of a CTA lie in the low-res rows [clr0, clr1) x the columns under
 // the mask's output words.  Read one by one from global memory they are chains of dependent DRAM accesses (pk_x record
 // -> logits -> pk_y record) and the kernel sat at 18 % issue utilisation; instead the CTA copies that tile into shared
@@ -120,7 +117,7 @@ __device__ __forceinline__ void cp_async16(void* smem_dst, const void* gmem_src)
 }
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
 
-__global__ void __launch_bounds__(kUpThreads, NTTT_UP_MINBLOCKS)
+__global__ void __launch_bounds__(kUpThreads, 5)
 upsample_pack_kernel(const uint32_t* __restrict__ bits_lr, const UpMeta* __restrict__ meta, int ih, int iw,
                      const int32_t* __restrict__ n_sel, int max_sel, int oh, int ow, UpTables t,
                      uint32_t* __restrict__ bits_full, int32_t* __restrict__ area_full, int32_t* __restrict__ box_full,
@@ -427,7 +424,6 @@ constexpr int kUp2Cols = 8;                          // word columns per item
 constexpr int kUp2Rows = kUp2Groups * kGrpMax;       // output rows per item (<= 128)
 constexpr int kUp2OutStride = kUp2Rows + kUp2Rows / 32;  // column-major result tile, one pad word per 32 rows
 constexpr int kUp2CtasPerSm = 7;
-int g_up2_ctas_per_sm = 1;
 
 struct alignas(16) Up2Item {  // 32 bytes, written by the plan kernel
   int k;                 // selected-mask slot
@@ -954,7 +950,9 @@ int launch_upsample_pack(const AxisTable& tx, const AxisTable& ty, const float* 
     NTTT_LAUNCH_CHECK();
     if (smem > 48 * 1024)
       NTTT_CUDA(set_dyn_smem(upsample_pack2_kernel, (int)smem));
-    const int grid = (sm_count > 0 ? sm_count : 148) * (low_latency ? kUp2CtasPerSm : g_up2_ctas_per_sm);
+    // many images in flight: one persistent CTA per SM leaves the rest of the SM to the other images' kernels (measured
+    // 89.8 / 90.7 / 91.2 / 91.9 us/image with 1 / 2 / 3 / 7 CTAs per SM); one image: kUp2CtasPerSm for the shortest kernel
+    const int grid = (sm_count > 0 ? sm_count : 148) * (low_latency ? kUp2CtasPerSm : 1);
     launch_chain(upsample_pack2_kernel, grid, kUp2Threads, smem, s, bits_lr, meta, ih, iw, oh, ow, t,
                                                           (bits_t && t_only) ? nullptr : bits_full, bits_t, area_full,
                                                           box_full, scratch, items, ctr, zero2);

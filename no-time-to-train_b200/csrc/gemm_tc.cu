@@ -262,128 +262,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
 }
 
 // ---------------------------------------------------------------------------------------------------
-// the same GEMM without the duplicated operand traffic.  Two of the three K-segments of each operand are copies
-// (A' = [hi|hi|lo], B' = [hi|lo|hi]), so per 64-wide k-block only FOUR tiles are distinct: A_lo, A_hi, B_hi, B_lo.
-// They are loaded once each and multiplied three ways (A_lo B_hi + A_hi B_hi + A_hi B_lo): a third less L2 -> shared
-// memory traffic for the same MMAs.  A tiles and B tiles live in two rings with a barrier pair per slot, so a slot
-// is handed back to the producer as soon as the last product that reads it has been issued:
-//     load order   A_lo -> a[i0]   B_hi -> b[i0]   A_hi -> a[i1]   B_lo -> b[i1]          (i0 = 2kb mod SLOTS, i1 = i0 + 1)
-//     P1 = a[i0] b[i0]  -> frees a[i0]    P2 = a[i1] b[i0]  -> frees b[i0]    P3 = a[i1] b[i1]  -> frees a[i1], b[i1]
-// a_lo_col / b_lo_col: column of the lo segment inside the operand rows (2*Kp and Kp in the [hi|hi|lo] / [hi|lo|hi] layout).
-// ---------------------------------------------------------------------------------------------------
-template <int BN, int SLOTS>
-struct Gemm3Smem {
-  alignas(1024) __nv_bfloat16 a[SLOTS][kBM * kBK];
-  alignas(1024) __nv_bfloat16 b[SLOTS][BN * kBK];
-  alignas(8) uint64_t full_a[SLOTS];
-  alignas(8) uint64_t empty_a[SLOTS];
-  alignas(8) uint64_t full_b[SLOTS];
-  alignas(8) uint64_t empty_b[SLOTS];
-  alignas(8) uint64_t acc_ready;
-  uint32_t tmem_base;
-};
-
-template <int BN>
-__device__ __forceinline__ void umma_kblock(uint32_t tmem_acc, uint32_t a_addr, uint32_t b_addr, bool first) {
-  constexpr uint32_t idesc = umma_idesc(BN);
-#pragma unroll
-  for (int k = 0; k < kBK / kUmmaK; ++k)
-    umma_f16(tmem_acc, umma_smem_desc(a_addr + k * kUmmaK * 2), umma_smem_desc(b_addr + k * kUmmaK * 2), idesc,
-             !(first && k == 0));
-}
-
-template <int BN, int SLOTS>
-__global__ void __launch_bounds__(kGemmThreads, 1)
-gemm_split3_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b,
-                   float* __restrict__ D, int ldd, int M, int N, int total_k_blocks, int kb_per_split,
-                   size_t split_stride, int a_lo_col, int b_lo_col) {
-  static_assert(SLOTS % 2 == 0, "a k-block takes two consecutive slots of each ring");
-  extern __shared__ uint8_t smem_raw[];
-  auto& sm = *reinterpret_cast<Gemm3Smem<BN, SLOTS>*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int m0 = blockIdx.y * kBM, n0 = blockIdx.x * BN;
-  const int kb0 = blockIdx.z * kb_per_split;
-  const int num_k_blocks = min(kb_per_split, total_k_blocks - kb0);
-  D += (size_t)blockIdx.z * split_stride;
-  constexpr uint32_t kABytes = kBM * kBK * sizeof(__nv_bfloat16), kBBytes = BN * kBK * sizeof(__nv_bfloat16);
-  constexpr uint32_t kTmemCols = BN < 32 ? 32 : BN;
-
-  if (warp == 0 && lane == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&map_a)) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&map_b)) : "memory");
-    for (int s = 0; s < SLOTS; ++s) {
-      mbar_init(&sm.full_a[s], 1); mbar_init(&sm.empty_a[s], 1);
-      mbar_init(&sm.full_b[s], 1); mbar_init(&sm.empty_b[s], 1);
-    }
-    mbar_init(&sm.acc_ready, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&sm.tmem_base)),
-                 "r"(kTmemCols));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::);
-  }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-  const uint32_t tmem_acc = sm.tmem_base;
-  chain_wait();  // (barriers, TMEM and tensor-map prefetch are set up while the producer of the operands drains)
-
-  if (warp == 0) {
-    if (lane == 0) {
-      for (int kb = 0; kb < num_k_blocks; ++kb) {
-        const int i0 = (2 * kb) % SLOTS, i1 = i0 + 1;
-        const uint32_t ph = ((2 * kb) / SLOTS) & 1;
-        const int col = (kb0 + kb) * kBK;
-        mbar_wait(&sm.empty_a[i0], ph ^ 1);
-        mbar_expect_tx(&sm.full_a[i0], kABytes);
-        tma_load_2d(sm.a[i0], &map_a, &sm.full_a[i0], a_lo_col + col, m0);
-        mbar_wait(&sm.empty_b[i0], ph ^ 1);
-        mbar_expect_tx(&sm.full_b[i0], kBBytes);
-        tma_load_2d(sm.b[i0], &map_b, &sm.full_b[i0], col, n0);
-        mbar_wait(&sm.empty_a[i1], ph ^ 1);
-        mbar_expect_tx(&sm.full_a[i1], kABytes);
-        tma_load_2d(sm.a[i1], &map_a, &sm.full_a[i1], col, m0);
-        mbar_wait(&sm.empty_b[i1], ph ^ 1);
-        mbar_expect_tx(&sm.full_b[i1], kBBytes);
-        tma_load_2d(sm.b[i1], &map_b, &sm.full_b[i1], b_lo_col + col, n0);
-      }
-    }
-  } else if (warp == 1) {
-    if (lane == 0) {
-      for (int kb = 0; kb < num_k_blocks; ++kb) {
-        const int i0 = (2 * kb) % SLOTS, i1 = i0 + 1;
-        const uint32_t ph = ((2 * kb) / SLOTS) & 1;
-        const uint32_t a_lo = smem_u32(sm.a[i0]), a_hi = smem_u32(sm.a[i1]);
-        const uint32_t b_hi = smem_u32(sm.b[i0]), b_lo = smem_u32(sm.b[i1]);
-        mbar_wait(&sm.full_a[i0], ph);
-        mbar_wait(&sm.full_b[i0], ph);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        umma_kblock<BN>(tmem_acc, a_lo, b_hi, kb == 0);
-        umma_commit(&sm.empty_a[i0]);
-        mbar_wait(&sm.full_a[i1], ph);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        umma_kblock<BN>(tmem_acc, a_hi, b_hi, false);
-        umma_commit(&sm.empty_b[i0]);
-        mbar_wait(&sm.full_b[i1], ph);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        umma_kblock<BN>(tmem_acc, a_hi, b_lo, false);
-        umma_commit(&sm.empty_a[i1]);
-        umma_commit(&sm.empty_b[i1]);
-      }
-      umma_commit(&sm.acc_ready);
-    }
-  } else {
-    gemm_epilogue<BN>(tmem_acc, &sm.acc_ready, warp & 3, lane, m0, n0, D, ldd, M, N);
-  }
-  __syncthreads();
-  if (warp == 1) {
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_acc), "r"(kTmemCols));
-  }
-}
-
-// ---------------------------------------------------------------------------------------------------
 // host: tensor maps + launch
 // ---------------------------------------------------------------------------------------------------
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
@@ -442,37 +320,6 @@ static int launch_tc(const __nv_bfloat16* A, int lda, const __nv_bfloat16* B, in
   return NTTT_OK;
 }
 
-// K = 3*Kp in the [hi|hi|lo] x [hi|lo|hi] layout: k-blocks run over Kp, each multiplying its four tiles three ways
-template <int BN, int SLOTS>
-static int launch_tc3(const __nv_bfloat16* A, int lda, const __nv_bfloat16* B, int ldb, float* D, int ldd, int M, int N,
-                      int K, int splits, size_t split_stride, cudaStream_t s) {
-  CUtensorMap ma, mb;
-  int err = make_map(&ma, A, M, K, lda, kBM);
-  if (err) return err;
-  err = make_map(&mb, B, N, K, ldb, BN);
-  if (err) return err;
-  const size_t smem = sizeof(Gemm3Smem<BN, SLOTS>) + 1024;
-  auto kern = gemm_split3_kernel<BN, SLOTS>;
-  NTTT_CUDA(set_dyn_smem(kern, (int)smem));
-  const int kp = K / 3;
-  const int total_kb = kp / kBK;
-  const int kb_per = ceil_div(total_kb, splits);
-  dim3 grid(ceil_div(N, BN), ceil_div(M, kBM), ceil_div(total_kb, kb_per));
-  kern<<<grid, kGemmThreads, smem, s>>>(ma, mb, D, ldd, M, N, total_kb, kb_per, split_stride, 2 * kp, kp);
-  NTTT_LAUNCH_CHECK();
-  return NTTT_OK;
-}
-
-// nttt_ctx_tune(NTTT_TUNE_GEMM_BN256_STAGES): TMA ring depth of the 128 x 256 kernel.  The kernel is tensor-pipe bound, so
-// three 48 KB stages feed it as well as four and leave 83 KB of the SM's shared memory to CTAs of the other kernels of
-// the images in flight (measured 91.8 vs 92.3 us/image; two stages: 92.0).
-int g_gemm_bn256_stages = 3;
-int g_gemm_bn256_min_m = 512;  // nttt_ctx_tune(NTTT_TUNE_GEMM_BN256_MIN_M)
-// nttt_ctx_tune(NTTT_TUNE_GEMM_SHARED_SEGMENTS): 1 = gemm_split3_kernel.  Off by default — measured equal at config 2
-// (92.5 vs 92.5 us/image) and 1.5 us/image slower at 1 203 classes: a CTA's 264 MMAs of 128 x 256 x 16 take 25 of its
-// 28 us, so the kernel is bound by its SM's tensor pipe, not by the operand traffic this variant removes.
-int g_gemm_shared_segments = 0;
-
 // A [M, K] and B [N, K] bf16, K a multiple of 64, rows 16-byte aligned (lda, ldb multiples of 8)
 // splits > 1: split-K, partial tile z is written to D + z*split_stride (the caller sums the partials in a fixed
 // order); *splits_out receives the number of partials actually produced.
@@ -482,8 +329,7 @@ int launch_gemm_tc(const void* A, int lda, const void* B, int ldb, float* D, int
   if (splits_out) *splits_out = 1;
   if (M <= 0 || N <= 0) return NTTT_OK;
   if (K <= 0 || K % kBK != 0 || lda % 8 != 0 || ldb % 8 != 0 || splits < 1) return NTTT_EINVAL;
-  const bool shared = g_gemm_shared_segments != 0 && K % (3 * kBK) == 0 && !a_active;
-  const int total_kb = shared ? K / 3 / kBK : K / kBK;
+  const int total_kb = K / kBK;
   const int kb_per = ceil_div(total_kb, splits);
   if (splits_out) *splits_out = ceil_div(total_kb, kb_per);
   const __nv_bfloat16* a = static_cast<const __nv_bfloat16*>(A);
@@ -493,22 +339,12 @@ int launch_gemm_tc(const void* A, int lda, const void* B, int ldb, float* D, int
   // 128 x 256 tiles halve the CTA count and raise the flops per operand byte by a third.  With many images in flight
   // the stage's throughput follows the SM-time a kernel consumes, not its latency: 32 CTAs x 38 us beat 64 CTAs x 25 us
   // at 1024 rows (97.9 vs 100.3 us/image), and at 4096 rows one wave of 128 CTAs beats 1.7 waves of 256 (281 vs 292).
-  // (N need not be a multiple of 256: TMA zero-fills the rows past N and the epilogue bounds its stores; g_exp[7] = 2
-  //  restores the former N % 256 == 0 rule for A/B runs)
-  const bool bn256 = !low_latency && N >= 512 && (N % 256 == 0 || g_exp[7] != 2) && M >= g_gemm_bn256_min_m;
-#ifndef NTTT_SIM_NO_BN128
+  // (N need not be a multiple of 256: TMA zero-fills the rows past N and the epilogue bounds its stores)
+  // The 128 x 256 kernel is tensor-pipe bound, so three 48 KB stages feed it as well as four and leave 83 KB of the SM's
+  // shared memory to CTAs of the other kernels of the images in flight (measured 91.8 vs 92.3 us/image; two stages: 92.0).
+  const bool bn256 = !low_latency && N >= 512 && M >= 512;
   const bool bn128 = N >= 512 || (N > 64 && N <= 128);  // 65..128 columns: ONE 128-wide tile reads the A operand once instead of twice
-#else
-  const bool bn128 = N >= 512;
-#endif
-  if (shared) {
-    if (bn256) return launch_tc3<256, 4>(a, lda, b, ldb, D, ldd, M, N, K, splits, split_stride, s);
-    if (bn128) return launch_tc3<128, 6>(a, lda, b, ldb, D, ldd, M, N, K, splits, split_stride, s);
-    return launch_tc3<64, 8>(a, lda, b, ldb, D, ldd, M, N, K, splits, split_stride, s);
-  }
-  if (bn256 && g_gemm_bn256_stages == 2) return launch_tc<256, 2>(a, lda, b, ldb, D, ldd, M, N, K, splits, split_stride, s, a_active, b_nonfinite);
-  if (bn256 && g_gemm_bn256_stages == 3) return launch_tc<256, 3>(a, lda, b, ldb, D, ldd, M, N, K, splits, split_stride, s, a_active, b_nonfinite);
-  if (bn256) return launch_tc<256, 4>(a, lda, b, ldb, D, ldd, M, N, K, splits, split_stride, s, a_active, b_nonfinite);
+  if (bn256) return launch_tc<256, 3>(a, lda, b, ldb, D, ldd, M, N, K, splits, split_stride, s, a_active, b_nonfinite);
   if (bn128) return launch_tc<128, 5>(a, lda, b, ldb, D, ldd, M, N, K, splits, split_stride, s, a_active, b_nonfinite);
   return launch_tc<64, 6>(a, lda, b, ldb, D, ldd, M, N, K, splits, split_stride, s, a_active, b_nonfinite);
 }
@@ -516,7 +352,7 @@ int launch_gemm_tc(const void* A, int lda, const void* B, int ldb, float* D, int
 // how many K splits fill the machine for an M x N output of 128 x 64 tiles (1 when the tiles already do)
 int gemm_tc_pick_splits(int M, int N, int K, int sm_count) {
   const int tiles = ceil_div(N, 64) * ceil_div(M, kBM);
-  const int total_kb = (g_gemm_shared_segments != 0 && K % (3 * kBK) == 0) ? K / 3 / kBK : K / kBK;
+  const int total_kb = K / kBK;
   int splits = sm_count / (tiles > 0 ? tiles : 1);
   if (splits < 1) splits = 1;
   if (splits > 8) splits = 8;
@@ -603,7 +439,7 @@ int launch_split_transpose(const float* X, int ld, int rows, int k, int kp, int 
   if (rows <= 0) return NTTT_OK;
   if (kp % 64 != 0) return NTTT_EINVAL;  // (callers pad K to 64: the GEMM's K block)
   const int tiles = (kp / 64) * ceil_div(rows, 32);
-  const int grid = g_exp[5] > 0 ? min(tiles, g_exp[5]) : (t_low_latency ? tiles : min(tiles, 148));
+  const int grid = t_low_latency ? tiles : min(tiles, 148);
   split_transpose_kernel<<<grid, 256, 0, s>>>(X, ld, rows, k, kp, mode, static_cast<__nv_bfloat16*>(out), nonfinite);
   NTTT_LAUNCH_CHECK();
   return NTTT_OK;

@@ -366,14 +366,8 @@ int launch_mask_ios(const uint32_t* bits_full, const int32_t* rect, const int32_
   int2* pairs = reinterpret_cast<int2*>(reinterpret_cast<char*>(label_sel) + align_up(sizeof(int32_t) * (size_t)max_sel, 256));
   const int max_pairs = (int)ios_max_pairs(max_sel);
   int32_t* n_pairs = reinterpret_cast<int32_t*>(reinterpret_cast<char*>(pairs) + align_up(sizeof(int2) * (size_t)max_pairs, 256));
-#ifdef NTTT_ABLATE
-  // ablation builds: NTTT_IOS_STOP=<k> ends this stage after its k-th kernel (marginal cost of each of the four)
-  static const int ios_stop = [] { const char* e = getenv("NTTT_IOS_STOP"); return e ? atoi(e) : 0; }();
-#else
-  constexpr int ios_stop = 0;
-#endif
-  const int pair_grid = g_exp[3] > 0 ? min(max_sel, g_exp[3]) : (t_low_latency ? max_sel : min(max_sel, 148));
-  if (counters_zeroed && ios_stop == 0) {
+  const int pair_grid = t_low_latency ? max_sel : min(max_sel, 148);
+  if (counters_zeroed) {
     launch_chain(ios_pairs_fused_kernel, pair_grid, 256, 0, s, rect, area_full, box_full, sel, n_sel, max_sel, labels, meta, ios,
                  pairs, n_pairs, max_pairs);
     NTTT_LAUNCH_CHECK();
@@ -381,14 +375,12 @@ int launch_mask_ios(const uint32_t* bits_full, const int32_t* rect, const int32_
     launch_chain(ios_meta_kernel, ceil_div(max_sel, 256), 256, 0, s, rect, area_full, box_full, sel, n_sel, max_sel, labels, meta,
                  label_sel, ios, n_pairs);
     NTTT_LAUNCH_CHECK();
-    if (ios_stop == 1) return NTTT_OK;
     launch_chain(ios_pairs_kernel, pair_grid, 256, 0, s, meta, label_sel, n_sel, max_sel, pairs, n_pairs, max_pairs);
     NTTT_LAUNCH_CHECK();
   }
-  if (ios_stop == 2) return NTTT_OK;
   // one CTA per SM when many images are in flight (measured 89.4 vs 90.0 us/image with four), four for one image alone
-  launch_chain(ios_eval_kernel, g_exp[0] > 0 ? g_exp[0] : (t_low_latency ? 148 * 4 : 148), kIosThreads, 0, s, bits_full, bits_t, meta, pairs, n_pairs, max_pairs, max_sel, oh, ow, obj_feats,
-                                                  c, ios, inter_out);
+  launch_chain(ios_eval_kernel, t_low_latency ? 148 * 4 : 148, kIosThreads, 0, s, bits_full, bits_t, meta, pairs, n_pairs,
+               max_pairs, max_sel, oh, ow, obj_feats, c, ios, inter_out);
   NTTT_LAUNCH_CHECK();
   if (finalize) {
     ios_finalize_kernel<<<ceil_div(max_sel, 256), 256, 0, s>>>(area_full, n_sel, max_sel, ios);

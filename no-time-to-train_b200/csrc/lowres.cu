@@ -60,18 +60,11 @@ __device__ __forceinline__ uint64_t pk_policy_evict_first() {
 }
 __device__ __forceinline__ void pk_bulk_load(void* smem_dst, const void* gsrc, uint32_t bytes, uint32_t bar_addr,
                                              uint64_t policy) {
-#ifdef NTTT_PACK_NO_L2_HINT
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                   pk_smem_u32(smem_dst)),
-               "l"(gsrc), "r"(bytes), "r"(bar_addr)
-               : "memory");
-#else
   asm volatile(
       "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1], %2, [%3], %4;" ::"r"(
           pk_smem_u32(smem_dst)),
       "l"(gsrc), "r"(bytes), "r"(bar_addr), "l"(policy)
       : "memory");
-#endif
 }
 
 // One CTA per mask.  A producer warp streams the 256 KB of logits through a 4-stage ring of 16 KB TMA bulk
@@ -399,29 +392,25 @@ lowres_pack_fast_kernel(const float4* __restrict__ logits, int p4 /* pixels/4 pe
   }
 }
 
-// K1c: persistent form of K1b — ONE CTA per SM, a 7-stage ring, CTA b takes masks b, b + grid, b + 2*grid, ...
+// K1c: persistent form of K1b — two CTAs per SM with a 3-stage ring each, CTA b takes masks b, b + grid, b + 2*grid, ...
 //
 // With images in flight the stage is a queue of kernels competing for SMs, and K1b (one CTA per mask, three CTAs per
 // SM to keep enough bytes in flight) owns every register and all shared memory of an SM while it runs: the other
 // kernels of the other images — which hardly touch HBM — cannot run beside the one kernel that is bound by it
 // (tools/ablate.py: the marginal costs of the stages ADD UP, 39 us of HBM time + 76 us of everything else).
-// Here one CTA per SM with a 7-stage ring (or two with 4 stages each) keeps 112 KB of bulk copies in flight (HBM needs
-// ~55 KB per SM), the producer runs ahead
-// into the next mask while the consumers finish the current one, and two thirds of the SM's registers and ~100 KB of
-// its shared memory stay free for the kernels of the other images.
+// Here two CTAs per SM keep 96 KB of bulk copies in flight (HBM needs ~55 KB per SM), the producer runs ahead into the
+// next mask while the consumers finish the current one, and what the CTAs do not occupy of the SM's registers and
+// shared memory stays free for the kernels of the other images.
 // The packed words are double-buffered so that one consumer barrier per mask is enough; the warp that finishes the
 // mask's statistics last combines and publishes them.
 // ---------------------------------------------------------------------------------------------------
 
 __device__ __forceinline__ void pk_consumer_barrier() { asm volatile("bar.sync 1, %0;" ::"n"(kPackThreads) : "memory"); }
 
-// (min-blocks 3 only caps the registers at 72 per thread: the shared-memory request admits one CTA per SM, and the
-// registers this kernel does not take are what the kernels of the other images run in)
-#ifndef NTTT_PERSIST_MINBLOCKS
-#define NTTT_PERSIST_MINBLOCKS 3
-#endif
+// (min-blocks 3 only caps the registers at 72 per thread: the grid holds two CTAs per SM, and the registers this
+// kernel does not take are what the kernels of the other images run in)
 template <int kPersistStages>
-__global__ void __launch_bounds__(kPackBlock, NTTT_PERSIST_MINBLOCKS)
+__global__ void __launch_bounds__(kPackBlock, 3)
 lowres_pack_persistent_kernel(const float4* __restrict__ logits, int n_masks, int p4 /* pixels/4 per mask */,
                               int words_per_row, uint32_t* __restrict__ bits, int32_t* __restrict__ area,
                               int32_t* __restrict__ box, int32_t* __restrict__ flags, const float* __restrict__ gate,
@@ -584,23 +573,6 @@ lowres_pack_persistent_kernel(const float4* __restrict__ logits, int n_masks, in
   }
 }
 
-// stab may be NULL: the stability counts (sam2/utils/amg.py:158-178) are not read on the noAMG path
-// gate (nullable): per-mask score; masks with !(gate[n] > gate_min) are skipped and published as empty
-// mask_ptr (nullable, device [n]): mask n is read from mask_ptr[n] (16-byte aligned) instead of logits + n*h*w
-// NTTT_PACK_MODE (ablation builds only, -DNTTT_ABLATE): 0/1 = sign-bit kernel (default), 2 = literal per-element kernel.  Requests for the
-// stability counts always take the literal kernel.
-static int pack_mode() {
-#ifdef NTTT_ABLATE
-  static const int v = [] { const char* e = getenv("NTTT_PACK_MODE"); return e ? atoi(e) : 0; }();
-  return v;
-#else
-  return 0;
-#endif
-}
-// occupancy experiment knob (nttt_ctx_tune NTTT_TUNE_LOWRES_EXTRA_SMEM): extra dynamic shared memory per CTA of the
-// fast pack kernel, i.e. fewer resident CTAs per SM, leaving room for the other images' kernels
-int g_pack_extra_smem = 0;
-
 // SM count of the current device (queried once per device)
 static int current_sm_count() {
   static int cache[64] = {};
@@ -613,12 +585,18 @@ static int current_sm_count() {
   return count;
 }
 
-// nttt_ctx_tune(NTTT_TUNE_LOWRES_PERSISTENT): 0 = one CTA per mask (3 resident per SM; always used in low-latency mode),
-// otherwise persistent CTAs that loop over masks: 10 * CTAs-per-SM + ring stages (1 and 2 = the round-2a shapes 17 / 24).
-// Measured with 16 images in flight (us/image): one CTA per mask 88.2 | 17: 90.6 | 24: 87.5 | 23: 86.7 | 22: 88.2 |
-// 33: 87.7 | 32: 89.5 | 25: 87.9 | 42: 89.1 — the thinnest shape that still covers the HBM latency wins, because what it
-// does not occupy runs the other images' kernels.
-int g_pack_persistent = 23;
+// nttt_ctx_tune(NTTT_TUNE_LOWRES_PERSISTENT), process-wide: 1 (default) = lowres_pack_persistent_kernel, two CTAs per SM
+// with a 3-stage ring each; 0 = lowres_pack_fast_kernel, one CTA per mask (3 resident per SM), which low-latency mode
+// always uses.  The two write the same bits; the switch lets tests compare them.  Shapes measured with 16 images in
+// flight (us/image, CTAs per SM x ring stages): one CTA per mask 88.2 | 1x7: 90.6 | 2x4: 87.5 | 2x3: 86.7 | 2x2: 88.2 |
+// 3x3: 87.7 | 3x2: 89.5 | 2x5: 87.9 | 4x2: 89.1 — the thinnest shape that still covers the HBM latency wins, because
+// what it does not occupy runs the other images' kernels.
+int g_pack_persistent = 1;
+
+// stab may be NULL: the stability counts (sam2/utils/amg.py:158-178) are not read on the noAMG path
+// gate (nullable): per-mask score; masks with !(gate[n] > gate_min) are skipped and published as empty
+// mask_ptr (nullable, device [n]): mask n is read from mask_ptr[n] (16-byte aligned) instead of logits + n*h*w
+// stab != NULL takes the literal per-element kernel, which also counts the stability thresholds
 int launch_lowres_pack(const float* logits, int n, int h, int w, float thr, float off, uint32_t* bits,
                        int32_t* area, int32_t* box, int32_t* stab, int32_t* flags, const float* gate, float gate_min,
                        const float* const* mask_ptr, cudaStream_t s, float* stab_score) {
@@ -632,39 +610,18 @@ int launch_lowres_pack(const float* logits, int n, int h, int w, float thr, floa
     NTTT_CUDA(set_dyn_smem(lowres_pack_kernel<true>, (int)smem));
     lowres_pack_kernel<true><<<n, kPackBlock, smem, s>>>(src, (int)(p / 4), w / 32, thr + off, thr - off, bits, area, box,
                                                         stab, stab_score, flags, gate, gate_min, mask_ptr);
-  } else if (pack_mode() <= 1 && g_pack_persistent > 0 && (!t_low_latency || g_exp[7] == 1)) {
-    const int sm_count = current_sm_count();
-    const size_t bits_bytes = 2 * (size_t)(p / 32) * sizeof(uint32_t);
-    // modes 1 and 2 are the named ones; 10 * CTAs-per-SM + stages selects any other shape (experiments)
-    const int shape = g_pack_persistent == 1 ? 17 : g_pack_persistent == 2 ? 24 : g_pack_persistent;
-    const int per_sm = shape / 10, stages = shape % 10;
-    const size_t sm = (size_t)stages * kPackStageBytes + bits_bytes;
-    const int grid = min(n, per_sm * sm_count);
-#define NTTT_PERSIST_CASE(S)                                                                                            \
-  case S:                                                                                                               \
-    NTTT_CUDA(set_dyn_smem(lowres_pack_persistent_kernel<S>, (int)sm)); \
-    lowres_pack_persistent_kernel<S><<<grid, kPackBlock, sm, s>>>(src, n, (int)(p / 4), w / 32, bits, area, box, flags, gate, \
-                                                                  gate_min, mask_ptr);                                  \
-    break;
-    switch (stages) {
-      NTTT_PERSIST_CASE(2)
-      NTTT_PERSIST_CASE(3)
-      NTTT_PERSIST_CASE(4)
-      NTTT_PERSIST_CASE(5)
-      NTTT_PERSIST_CASE(7)
-      default: return NTTT_EINVAL;
-    }
-#undef NTTT_PERSIST_CASE
-  } else if (pack_mode() <= 1) {
-    const size_t smem_fast = smem + (size_t)g_pack_extra_smem;
-    NTTT_CUDA(set_dyn_smem(lowres_pack_fast_kernel, (int)smem_fast));
-    // (first kernel of the chain, behind the fork event of the low-latency mode: an ordinary launch)
-    lowres_pack_fast_kernel<<<n, kPackBlock, smem_fast, s>>>(src, (int)(p / 4), w / 32, bits, area, box, flags, gate, gate_min,
-                                                        mask_ptr);
+  } else if (g_pack_persistent && !t_low_latency) {
+    constexpr int kCtasPerSm = 2, kStages = 3;
+    const size_t sm = (size_t)kStages * kPackStageBytes + 2 * (size_t)(p / 32) * sizeof(uint32_t);  // (words double-buffered)
+    const int grid = min(n, kCtasPerSm * current_sm_count());
+    NTTT_CUDA(set_dyn_smem(lowres_pack_persistent_kernel<kStages>, (int)sm));
+    lowres_pack_persistent_kernel<kStages><<<grid, kPackBlock, sm, s>>>(src, n, (int)(p / 4), w / 32, bits, area, box, flags,
+                                                                        gate, gate_min, mask_ptr);
   } else {
-    NTTT_CUDA(set_dyn_smem(lowres_pack_kernel<false>, (int)smem));
-    lowres_pack_kernel<false><<<n, kPackBlock, smem, s>>>(src, (int)(p / 4), w / 32, thr + off, thr - off, bits, area,
-                                                         box, stab, nullptr, flags, gate, gate_min, mask_ptr);
+    NTTT_CUDA(set_dyn_smem(lowres_pack_fast_kernel, (int)smem));
+    // (first kernel of the chain, behind the fork event of the low-latency mode: an ordinary launch)
+    lowres_pack_fast_kernel<<<n, kPackBlock, smem, s>>>(src, (int)(p / 4), w / 32, bits, area, box, flags, gate, gate_min,
+                                                        mask_ptr);
   }
   NTTT_LAUNCH_CHECK();
   return NTTT_OK;
@@ -1052,10 +1009,7 @@ int launch_project_masks(const AxisTable& tx, const AxisTable& ty, const uint32_
   ProjTables t{tx.t_lo, tx.t_len, tx.t_cum, ty.t_lo, ty.t_len, ty.t_w};
   // throughput mode: two persistent CTAs per SM walk the masks (measured 88.1 vs 89.4 us/image with one CTA per mask:
   // the span tables are staged once per CTA and 1024 CTA launches become 296); low-latency mode: one CTA per mask
-  int grid = n;
-  if (!t_low_latency) {
-    grid = min(n, g_exp[2] > 0 ? g_exp[2] : 2 * current_sm_count());
-  }
+  const int grid = t_low_latency ? n : min(n, 2 * current_sm_count());
   if (split) {
     if (smem > 48 * 1024)
       NTTT_CUDA(set_dyn_smem(project_masks_kernel<true>, (int)smem));

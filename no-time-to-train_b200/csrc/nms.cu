@@ -470,21 +470,18 @@ int launch_box_nms(const int32_t* box, const float* nms_scores, const int32_t* l
     return NTTT_OK;
   }
   // longer lists: boxes re-ordered by (label, score rank), block-diagonal matrix, the same wavefront over the non-zero
-  // words of each row; g_exp[1] = 2 keeps the score order (A/B)
-  const bool by_class = g_exp[1] != 2;
+  // words of each row
   float4* cbox = reinterpret_cast<float4*>(reinterpret_cast<char*>(nz) + align_up(sizeof(uint32_t) * (size_t)n * nz_words, 256));
   int32_t* clabel = reinterpret_cast<int32_t*>(reinterpret_cast<char*>(cbox) + align_up(sizeof(float4) * (size_t)n, 256));
   int32_t* c2s = reinterpret_cast<int32_t*>(reinterpret_cast<char*>(clabel) + align_up(sizeof(int32_t) * (size_t)n, 256));
-  if (by_class) {
-    launch_chain(nms_class_sort_kernel, 1, 1024, sizeof(uint32_t) * (size_t)n_pad, s, sorted_box, sorted_label, n, n_pad, c2s, cbox,
-                 clabel);
-    NTTT_LAUNCH_CHECK();
-  }
-  launch_chain(nms_mask_kernel<true>, grid, dim3(32, 8), 0, s, by_class ? cbox : sorted_box, by_class ? clabel : sorted_label, n,
-               thr, mask, row_words, nz, nz_words, by_class ? 1 : 0);
+  launch_chain(nms_class_sort_kernel, 1, 1024, sizeof(uint32_t) * (size_t)n_pad, s, sorted_box, sorted_label, n, n_pad, c2s, cbox,
+               clabel);
   NTTT_LAUNCH_CHECK();
-  launch_chain(nms_wave_sparse_kernel, 1, kScanThreads, 0, s, mask, nz, nz_words, row_words, order,
-               by_class ? clabel : sorted_label, top_score, n, max_keep, keep, n_keep, sel, n_sel, by_class ? c2s : nullptr);
+  launch_chain(nms_mask_kernel<true>, grid, dim3(32, 8), 0, s, cbox, clabel, n, thr, mask, row_words, nz, nz_words,
+               /*class_sorted=*/1);
+  NTTT_LAUNCH_CHECK();
+  launch_chain(nms_wave_sparse_kernel, 1, kScanThreads, 0, s, mask, nz, nz_words, row_words, order, clabel, top_score, n,
+               max_keep, keep, n_keep, sel, n_sel, c2s);
   NTTT_LAUNCH_CHECK();
   return NTTT_OK;
 }

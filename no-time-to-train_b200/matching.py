@@ -263,13 +263,14 @@ class MatchingStage:
             self._ws["pinned"] = buf
         return buf
 
-    TUNABLES = {"upsample_stage_bytes": 1, "lowres_extra_smem": 2, "gemm_bn256_min_m": 3, "axis_cache_entries": 4, "lowres_persistent": 5,
-                "gemm_shared_segments": 6, "gemm_bn256_stages": 7, "up2_ctas_per_sm": 8}  # include/nttt_b200.h: NTTT_TUNE_*
+    TUNABLES = {"upsample_stage_bytes": 1, "axis_cache_entries": 4, "lowres_persistent": 5,
+                "pool_order": 9}  # include/nttt_b200.h: NTTT_TUNE_*
 
     def tune(self, name: str, value: int) -> None:
-        """Set a performance tunable of this device's context (`nttt_ctx_tune`); results never depend on them."""
-        what = 100 + int(name[3:]) if name.startswith("exp") else self.TUNABLES[name]
-        _lib.check(self.lib.nttt_ctx_tune(self.ctx, what, int(value)), f"nttt_ctx_tune({name})")
+        """Set a tunable of this device's context (`nttt_ctx_tune`); results never depend on them."""
+        if name not in self.TUNABLES:
+            raise ValueError(f"unknown tunable {name!r}; known: {', '.join(self.TUNABLES)}")
+        _lib.check(self.lib.nttt_ctx_tune(self.ctx, self.TUNABLES[name], int(value)), f"nttt_ctx_tune({name})")
 
     def profile(self, enable: bool) -> None:
         """Per-stage CUDA-event timing of the next `match_async` calls (see nttt_ctx_profile)."""

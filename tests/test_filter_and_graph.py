@@ -132,21 +132,20 @@ def test_low_latency_chain_is_deterministic_over_many_calls():
 
 
 @pytest.mark.parametrize("n,c,ori_hw", [(300, 384, (480, 640)), (1000, 1024, (512, 512)), (130, 768, (333, 500))])
-def test_ordered_pooling_gemm_skips_only_zeros(n, c, ori_hw):
+def test_pool_order_skips_only_zeros(n, c, ori_hw):
     """Throughput mode orders the rows of the pooling GEMM spatially and skips the k-blocks a tile of masks does not
-    touch.  Skipped blocks are exact zeros: with the order switched off (experiment slot 1) every output is bit-identical
+    touch.  Skipped blocks are exact zeros: with the order switched off (`pool_order` 0) every output is bit-identical
     — pooled features and similarities included — and the low-latency mode (no order, split-K) agrees on every integer."""
     P, inp = _case(n=n, c=c, n_cls=9, seed=191, ori_hw=ori_hw)
-    ops = importlib.import_module("no-time-to-train_b200.ops")
     stage = P.MatchingStage(DEV, P.StageConfig(nms_thr=0.5, num_out_instance=40, enc_hw=(37, 37)))
     stage.set_prototypes(inp.feats_ins_avg)
     args = (inp.lr_masks.to(DEV), inp.pred_ious.to(DEV), inp.tar_feat.to(DEV), inp.ori_hw)
     a = stage.match(*args, taps=True, low_latency=False)
     try:
-        ops.tune(DEV, 101, 1)
+        stage.tune("pool_order", 0)
         b = stage.match(*args, taps=True, low_latency=False)
     finally:
-        ops.tune(DEV, 101, 0)
+        stage.tune("pool_order", 1)
     ll = stage.match(*args, taps=True, low_latency=True)
     assert a["counts"] == b["counts"] == ll["counts"] and a["counts"]["n_out"] > 0
     for key in ("binary_masks", "bboxes", "labels"):
@@ -158,11 +157,10 @@ def test_ordered_pooling_gemm_skips_only_zeros(n, c, ori_hw):
     assert torch.allclose(a["taps"]["obj_feats"], ll["taps"]["obj_feats"], rtol=0, atol=1e-6)
 
 
-def test_ordered_pooling_gemm_keeps_nonfinite_features():
+def test_pool_order_keeps_nonfinite_features():
     """0 * inf = NaN in the reference's dense product: a k-block whose features hold an inf or a NaN is multiplied even
     where the masks' projections are all zero — same NaN pattern with and without the skipping."""
     P, inp = _case(n=300, c=384, n_cls=9, seed=192, ori_hw=(256, 256))
-    ops = importlib.import_module("no-time-to-train_b200.ops")
     stage = P.MatchingStage(DEV, P.StageConfig(nms_thr=0.5, num_out_instance=40, enc_hw=(37, 37)))
     stage.set_prototypes(inp.feats_ins_avg)
     feat = inp.tar_feat.clone()
@@ -171,10 +169,10 @@ def test_ordered_pooling_gemm_keeps_nonfinite_features():
     args = (inp.lr_masks.to(DEV), inp.pred_ious.to(DEV), feat.to(DEV), inp.ori_hw)
     a = stage.match(*args, taps=True, low_latency=False)
     try:
-        ops.tune(DEV, 101, 1)
+        stage.tune("pool_order", 0)
         b = stage.match(*args, taps=True, low_latency=False)
     finally:
-        ops.tune(DEV, 101, 0)
+        stage.tune("pool_order", 1)
     fa, fb = a["taps"]["obj_feats"], b["taps"]["obj_feats"]
     assert bool(torch.isnan(fb).any())
     assert torch.equal(torch.isnan(fa), torch.isnan(fb))

@@ -113,28 +113,34 @@ def test_stability_score_value_matches_reference(ops, name):
         assert got.shape == (2, 4) and np.array_equal(got.cpu().numpy(), want.numpy(), equal_nan=True)
 
 
-@pytest.mark.parametrize("mode", [1, 2])
-def test_threshold_pack_persistent_variants_are_bit_identical(ops, synth, mode):
-    """NTTT_TUNE_LOWRES_PERSISTENT: the persistent forms of the low-res pass (one CTA per SM with a 7-stage ring, two
-    with 4 stages) give exactly the outputs of the default one-CTA-per-mask kernel, special values and gated masks
-    included (they are A/B options: measured equal in throughput, see DESIGN.md §5)."""
-    gen = torch.Generator().manual_seed(41 + mode)
-    n = 333  # more masks than CTAs in flight: every CTA loops over several masks
+@pytest.mark.parametrize("hw", [(256, 256), (64, 96)])
+def test_threshold_pack_persistent_variants_are_bit_identical(ops, synth, hw):
+    """The three low-res kernels give the same bits, areas, boxes and flags, special values and degenerate masks
+    included: the default persistent one (two CTAs per SM looping over the masks), the one-CTA-per-mask one
+    (NTTT_TUNE_LOWRES_PERSISTENT = 0, what the low-latency mode runs) and the literal one (want_stab=True).
+    64 x 96 masks end in a partial ring stage."""
+    h, w = hw
+    gen = torch.Generator().manual_seed(42)
+    n = 333  # more masks than CTAs in flight: every persistent CTA loops over several masks
     logits = synth.make_masks(n, gen)
     synth.inject_degenerate_cases(logits, torch.zeros(2, 2, 4))
     logits[9, 17, 33] = float("nan")
     logits[10, 200, 5] = float("inf")
+    logits[10, 40, 5] = float("inf")  # (inside the 64 x 96 crop as well)
     logits[11] = 0.0
-    d = logits.to(DEV)
-    want = ops.threshold_pack(d, want_stab=False)
+    d = logits[:, :h, :w].contiguous().to(DEV)
+    persistent = ops.threshold_pack(d, want_stab=False)
+    literal = ops.threshold_pack(d, want_stab=True)
     try:
-        ops.tune(DEV, 5, mode)
-        got = ops.threshold_pack(d, want_stab=False)
+        ops.tune(DEV, 5, 0)  # NTTT_TUNE_LOWRES_PERSISTENT
+        per_mask = ops.threshold_pack(d, want_stab=False)
     finally:
-        ops.tune(DEV, 5, 0)
-    for name, a, b in zip(("bits", "area", "box", "stab", "flags"), want, got):
+        ops.tune(DEV, 5, 1)
+    for name, a, b, c in zip(("bits", "area", "box", "stab", "flags"), persistent, per_mask, literal):
         if name != "stab":
             assert torch.equal(a, b), name
+            assert torch.equal(a, c), name
+    assert (persistent[4] == 0).any() and persistent[1].min() == 0
 
 
 def test_threshold_pack_empty_batch(ops):
@@ -360,27 +366,6 @@ def test_pipeline_matches_c_oracle(P, name):
                            masks=ref["binary_masks"].astype(bool), index=ref_index), what=name + " vs C oracle")
 
 
-@pytest.mark.parametrize("name", STAGE_CASES[:3])
-def test_pipeline_with_shared_segment_gemm(P, ops, name):
-    """NTTT_TUNE_GEMM_SHARED_SEGMENTS = 1 (`gemm_split3_kernel`: four operand tiles per k-block multiplied three ways
-    instead of three streamed K-segments) computes the same products in a different order: the same golden parity, and
-    every integer result of the default kernel."""
-    g, inp, cfg = load_case(name)
-    base = _run_stage(P, inp, cfg["num_out_instance"])
-    try:
-        ops.tune(DEV, 6, 1)
-        out = _run_stage(P, inp, cfg["num_out_instance"])
-    finally:
-        ops.tune(DEV, 6, 0)
-    assert_close_rel(out["taps"]["sim"].cpu().numpy(), g["sim"], what="sim")
-    assert_close_rel(out["taps"]["obj_feats"].cpu().numpy(), g["obj_feats"], what="obj_feats")
-    assert out["counts"] == base["counts"]
-    assert_rows_match(dict(scores=out["scores"], labels=out["labels"], bboxes=out["bboxes"], masks=out["binary_masks"]),
-                      dict(scores=base["scores"].cpu().numpy(), labels=base["labels"].cpu().numpy(),
-                           bboxes=base["bboxes"].cpu().numpy(), masks=base["binary_masks"].cpu().numpy()),
-                      what=name + " shared-segment GEMM vs default")
-
-
 def test_pipeline_empty_selection(P, synth):
     """All scores <= 0 -> the reference's empty early return (float32 zero boxes, :647-655)."""
     inp = synth.make_stage_inputs(n=16, c=64, n_cls=2, shots=1, ori_hw=(64, 96), seed=41)
@@ -530,3 +515,51 @@ def test_axis_table_cache_eviction(ops, synth):
         want = orc.aa_resize_threshold(logits.numpy(), hw).astype(bool)
         assert np.array_equal(got, want), hw
     ops.tune(DEV, 4, 1024)
+
+
+def test_ctx_tune_refuses_unknown_ids_and_out_of_range_values(P, ops, synth):
+    """`nttt_ctx_tune` knows four tunables and takes 0 or 1 for the two path switches: every other id or value returns
+    NTTT_EINVAL and changes nothing, so `match` gives bit for bit what it gave before the refused calls."""
+    lib = P._lib.load()
+    ctx = ops.context(DEV)
+    inp = synth.make_stage_inputs(n=300, c=384, n_cls=9, shots=2, ori_hw=(480, 640), seed=63, degenerate=True)
+    stage = P.MatchingStage(DEV, P.StageConfig(nms_thr=0.5, num_out_instance=40, enc_hw=(37, 37)))
+    stage.set_prototypes(inp.feats_ins_avg)
+    args = (inp.lr_masks.to(DEV), inp.pred_ious.to(DEV), inp.tar_feat.to(DEV), inp.ori_hw)
+    want = stage.match(*args, taps=True, low_latency=False)
+    for what, value in ((2, 0), (3, 512), (6, 1), (7, 3), (8, 2), (100, 1), (101, 1), (107, 64),
+                        (5, 2), (5, 23), (5, 49), (9, 2)):
+        assert lib.nttt_ctx_tune(ctx, what, value) == -1, (what, value)  # NTTT_EINVAL
+    with pytest.raises(ValueError, match="known: upsample_stage_bytes, axis_cache_entries"):
+        stage.tune("exp1", 1)
+    got = stage.match(*args, taps=True, low_latency=False)
+    assert got["counts"] == want["counts"] and want["counts"]["n_out"] > 0
+    for key in ("binary_masks", "bboxes", "labels", "index"):
+        assert torch.equal(got[key], want[key]), key
+    assert torch.equal(torch.nan_to_num(got["scores"]), torch.nan_to_num(want["scores"]))
+    for key in ("sim", "obj_feats"):
+        assert torch.equal(torch.nan_to_num(got["taps"][key]), torch.nan_to_num(want["taps"][key])), key
+
+
+def test_unsupported_projection_is_refused_before_any_launch(P, synth):
+    """An encoder grid too coarse for the mask size (256 / 16 pixels per cell exceeds the scatter tables) is refused
+    with NTTT_EUNSUPPORTED before the call launches anything — no table build, no side-stream work left running —
+    and the stage keeps working: the next valid call gives what the same call gave before."""
+    lib = P._lib.load()
+    inp = synth.make_stage_inputs(n=64, c=64, n_cls=3, shots=1, ori_hw=(240, 320), seed=64, e_side=16)
+    small = synth.make_masks(64, torch.Generator().manual_seed(65), lo=128)  # 128 / 16 fits
+    stage = P.MatchingStage(DEV, P.StageConfig(nms_thr=0.5, num_out_instance=10, enc_hw=(16, 16)))
+    stage.set_prototypes(inp.feats_ins_avg)
+    feat, ious = inp.tar_feat.to(DEV), inp.pred_ious.to(DEV)
+    before = stage.match(small.to(DEV), ious, feat, inp.ori_hw, low_latency=True)
+    torch.cuda.synchronize()
+    launches = lib.nttt_launch_count()
+    with pytest.raises(P._lib.NtttError) as err:
+        stage.match(inp.lr_masks.to(DEV), ious, feat, inp.ori_hw, low_latency=True)
+    assert err.value.code == -5  # NTTT_EUNSUPPORTED
+    assert lib.nttt_launch_count() == launches
+    after = stage.match(small.to(DEV), ious, feat, inp.ori_hw, low_latency=True)
+    assert after["counts"] == before["counts"] and before["counts"]["n_out"] > 0
+    for key in ("binary_masks", "bboxes", "labels", "index"):
+        assert torch.equal(after[key], before[key]), key
+    assert torch.equal(torch.nan_to_num(after["scores"]), torch.nan_to_num(before["scores"]))
