@@ -355,6 +355,18 @@ typedef struct nttt_match_args {
    * similarities may differ in the last bit (far inside the 1e-3 bound); every integer result (masks, boxes, counts,
    * keep lists) is computed identically. */
   int32_t low_latency;
+  /* more optional taps for tests (nullable), the inputs of the score decay (a13/a14); when set, the pipeline keeps these
+   * values in the caller's buffer instead of its workspace (no extra kernel), so they are what the decay and ranking read:
+   *   sel       [max_sel] i32: the selection in slot order (indices into logits), after NMS and the `score > 0` filter;
+   *             counts[1] entries are valid
+   *   ios       [max_sel] f32: the row maximum of the intersection-over-self term that the decay reads, BEFORE the
+   *             empty-mask rule: a row whose full-resolution mask is empty holds 0 here, and the decay turns it into
+   *             NaN (the reference's 0/0 on the diagonal), as it does the score of that row
+   *   ios_inter [max_sel, max_sel] i32: the integer intersection counts of same-label pairs of selected masks (0 on the
+   *             diagonal, across labels and for disjoint boxes), as nttt_mask_ios's inter_out; zeroed by the call */
+  int32_t* sel;
+  float* ios;
+  int32_t* ios_inter;
 } nttt_match_args;
 
 size_t nttt_match_workspace_bytes(int n, int lr_h, int lr_w, int eh, int ew, int c, int n_cls, int ori_h,

@@ -41,6 +41,7 @@ class MatchArgs(ctypes.Structure):
         ("rle_counts", c_void_p), ("rle_n_counts", c_void_p), ("rle_chars", c_void_p), ("rle_n_chars", c_void_p),
         ("rle_cap_counts", c_int32), ("rle_cap_chars", c_int32),
         ("low_latency", c_int32),
+        ("sel", c_void_p), ("ios", c_void_p), ("ios_inter", c_void_p),
     ]
 
 

@@ -774,6 +774,8 @@ int nttt_match_image(nttt_ctx* ctx, const nttt_match_args* a, void* stream) {
   if (!projection_supported(a->ew, a->lr_w) || !projection_supported(a->eh, a->lr_h)) return NTTT_EUNSUPPORTED;
   float* obj_feats = a->obj_feats ? a->obj_feats : L.obj_feats;
   float* sim = a->sim ? a->sim : L.sim;
+  int32_t* sel = a->sel ? a->sel : L.sel;
+  float* ios = a->ios ? a->ios : L.ios;
   struct LaunchMode {  // the launch shapes of this call (common.cuh: t_low_latency), restored on every return path
     bool prev;
     explicit LaunchMode(bool v) : prev(nttt::t_low_latency) { nttt::t_low_latency = v; }
@@ -879,22 +881,22 @@ int nttt_match_image(nttt_ctx* ctx, const nttt_match_args* a, void* stream) {
                      forked));
   // a10/a11
   NTTT_STEP(launch_box_nms(L.box_lr, pred_ious, L.top_label, L.top_score, n, a->nms_thr, max_sel, L.keep,
-                           a->counts + 0, L.sel, a->counts + 1, L.nms_ws, L.nms_ws_bytes, a->iou_thr, a->filter_iou, s));
+                           a->counts + 0, sel, a->counts + 1, L.nms_ws, L.nms_ws_bytes, a->iou_thr, a->filter_iou, s));
   // a12/a9
   bool wrote_t = false;  // the resize also left the word-column-major copy of the packed masks (v2 path only)
-  NTTT_STEP(launch_upsample_pack(ux, uy, a->logits, L.bits_lr, L.box_lr, L.flags, a->lr_h, a->lr_w, L.sel,
+  NTTT_STEP(launch_upsample_pack(ux, uy, a->logits, L.bits_lr, L.box_lr, L.flags, a->lr_h, a->lr_w, sel,
                                  a->counts + 1, max_sel, a->ori_h, a->ori_w, L.bits_full, L.rect, L.area_full,
                                  L.box_full, L.scratch, mask_ptr, s, ctx->upsample_stage_floats, ctx->sm_count, L.bits_t,
                                  &wrote_t, /*t_only=*/true, a->low_latency != 0, ios_pair_counters(L.ios_ws, max_sel)));
   // the packed full-resolution masks from here on: word-column major when the v2 resize ran, row-major otherwise
   const uint32_t* packed = wrote_t ? L.bits_t : L.bits_full;
   // a13
-  NTTT_STEP(launch_mask_ios(L.bits_full, L.rect, L.area_full, L.box_full, L.sel, a->counts + 1, max_sel, a->ori_h,
-                            a->ori_w, L.top_label, obj_feats, a->c, L.ios, nullptr, L.ios_ws, false, s,
+  NTTT_STEP(launch_mask_ios(L.bits_full, L.rect, L.area_full, L.box_full, sel, a->counts + 1, max_sel, a->ori_h,
+                            a->ori_w, L.top_label, obj_feats, a->c, ios, a->ios_inter, L.ios_ws, false, s,
                             wrote_t ? L.bits_t : nullptr, /*counters_zeroed=*/wrote_t && a->low_latency != 0));  // (folding the metadata
   // kernel into the pair kernel takes 1 us off a single image's chain and costs 0.3 us/image with images in flight)
   // a14
-  NTTT_STEP(launch_decay_rank(L.top_score, L.top_label, L.ios, L.sel, a->counts + 1, max_sel, num_out, L.box_full,
+  NTTT_STEP(launch_decay_rank(L.top_score, L.top_label, ios, sel, a->counts + 1, max_sel, num_out, L.box_full,
                               L.area_full,
                               a->out_boxes, a->out_scores, a->out_labels, a->out_index, L.out_slot, a->counts + 2,
                               nullptr, s));

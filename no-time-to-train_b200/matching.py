@@ -163,6 +163,8 @@ class MatchingStage:
         (each [testing_point_bs, m, 256, 256]; consumed in place, no `cat`) — and `pred_ious` is ignored (pass None).
         `rle=True` also emits the outputs as COCO compressed RLE (`PendingResult.rle_segmentations()`);
         with `dense_masks=False` the bool masks are not produced at all (`binary_masks` is None).
+        `taps=True` also returns the intermediate values tests compare, in `out["taps"]`: `sim`, `obj_feats` and the
+        inputs of the score decay `sel`, `ios`, `ios_inter` (nttt_match_args; the counts are [max_sel, max_sel] i32).
         `low_latency=True` shapes the kernels for the shortest duration of ONE image (a caller that synchronises after
         every image) instead of the least SM-time (many images in flight); float sums may differ in the last bit between the modes."""
         if self.proto is None:
@@ -218,6 +220,10 @@ class MatchingStage:
         if taps:
             tap_t["sim"] = torch.empty((n, self.n_cls), dtype=torch.float32, device=dev)
             tap_t["obj_feats"] = torch.empty((n, c), dtype=torch.float32, device=dev)
+            # the inputs of the score decay: selection in slot order, IoS row maxima, same-label intersection counts
+            tap_t["sel"] = torch.empty((max(max_sel, 1),), dtype=torch.int32, device=dev)
+            tap_t["ios"] = torch.empty((max(max_sel, 1),), dtype=torch.float32, device=dev)
+            tap_t["ios_inter"] = torch.empty((max(max_sel, 1), max(max_sel, 1)), dtype=torch.int32, device=dev)
         ws_bytes = self.lib.nttt_match_workspace_bytes_neg(n, lh, lw, eh, ew, c, self.n_cls, oh, ow, max_sel, self.l_neg)
         ws = self._workspace(("match", slot), ws_bytes)
         a = _lib.MatchArgs()
@@ -243,6 +249,8 @@ class MatchingStage:
         a.out_index, a.counts = index.data_ptr(), counts.data_ptr()
         a.sim = tap_t["sim"].data_ptr() if taps else None
         a.obj_feats = tap_t["obj_feats"].data_ptr() if taps else None
+        a.sel, a.ios, a.ios_inter = ((tap_t[k].data_ptr() for k in ("sel", "ios", "ios_inter")) if taps
+                                     else (None, None, None))
         a.workspace, a.workspace_bytes = ws.data_ptr(), ws.numel()
         a.proto_neg = self.proto_neg.data_ptr() if self.proto_neg is not None else None
         a.l_neg, a.sigma = self.l_neg, float(self.cfg.neg_sigma)

@@ -53,9 +53,12 @@ def test_workspace_queries_are_pure_host(lib):
     assert cdll.nttt_nms_workspace_bytes(1024) >= 1024 * 32 * 4
 
 
-def test_match_args_struct_layout(lib):
-    """The ctypes mirror must have the size of the C struct as compiled."""
-    assert ctypes.sizeof(lib.MatchArgs) == lib.load().nttt_sizeof_match_args() == 272
+def test_match_args_struct_layout_with_decay_taps(lib):
+    """The ctypes mirror must have the size of the C struct as compiled: the fields up to `low_latency` (at 264, padded
+    to 272), then the three pointer taps of the score decay (`sel`, `ios`, `ios_inter`)."""
+    assert ctypes.sizeof(lib.MatchArgs) == lib.load().nttt_sizeof_match_args() == 296
+    assert lib.MatchArgs.low_latency.offset == 264
+    assert [getattr(lib.MatchArgs, f).offset for f in ("sel", "ios", "ios_inter")] == [272, 280, 288]
 
 
 @pytest.mark.skipif(torch.cuda.is_available(), reason="checks the no-GPU failure mode")

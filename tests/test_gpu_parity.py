@@ -1,7 +1,9 @@
 """GPU parity tests: the CUDA path (through the C-ABI) against the oracle and the golden vectors.
 
-Bit-exact: thresholded masks, areas, boxes, stability counts, NMS keep indices, intersection counts.
-1e-3 relative (BASELINE.json north_star): pooled features, prototypes, similarities, IoS, scores.
+Bit-exact: thresholded masks, areas, boxes, stability counts, NMS keep indices.
+1e-3 relative (BASELINE.json north_star): pooled features, prototypes, similarities, scores.
+Intersection counts, IoS and the decayed ranking are pinned per element against exact and float64 references
+(ios_ref.py): test_mask_ios_counts_bit_exact here, every product path in test_ios_decay_accuracy.py.
 """
 import importlib
 import os
@@ -12,6 +14,7 @@ import torch
 
 from golden_util import (FILL_CASES, GOLDEN_DIR, RTOL, STAGE_CASES, assert_close_rel, assert_rows_match,
                          assert_same_ranking, load_case, sha_bool)
+from ios_ref import RESOLUTION_PX, TOL_IOS, inter_counts, ios_errors, ios_reference
 from oracle import nttt_oracle as orc
 from oracle import ref_torch
 
@@ -307,6 +310,9 @@ def test_upsample_more_selected_masks_than_one_plan_strip(ops, synth):
 
 
 def test_mask_ios_counts_bit_exact(ops, synth):
+    """`nttt_mask_ios` on 40 mixed masks (three labels, empty full-res masks) at 333 x 500: counts equal the C oracle's
+    and the exact products of the unpacked masks; IoS within TOL_IOS of each row's float64 bound (ios_ref.py), empty
+    rows NaN.  test_ios_decay_accuracy.py runs the same checks on the branches this case does not reach."""
     inp = synth.make_stage_inputs(n=48, c=64, n_cls=3, shots=2, ori_hw=(333, 500), seed=31, degenerate=True)
     d = inp.lr_masks.to(DEV)
     bits, area, box, stab, flags = ops.threshold_pack(d)
@@ -324,6 +330,15 @@ def test_mask_ios_counts_bit_exact(ops, synth):
     o_ios, o_inter = orc.semantic_ios(full, labels[:k].long().numpy(), obj_sim, want_inter=True)
     assert np.array_equal(inter.cpu().numpy(), o_inter)
     assert_close_rel(ios.cpu().numpy(), o_ios, what="ios")
+    lab = labels[:k].to(DEV)
+    want = inter_counts(ops.unpack_masks(bits_full, rect, n_sel, inp.ori_hw), lab)
+    assert torch.equal(inter.to(torch.int64), want)
+    ios64, bound, s2 = ios_reference(want, area_full, feats[:k].to(DEV), lab)
+    empty = area_full == 0
+    assert bool(empty.any()) and torch.isnan(ios[empty]).all() and not torch.isnan(ios[~empty]).any()
+    err, px = ios_errors(torch.where(empty, torch.zeros_like(ios), ios), ios64, bound, s2, "mask_ios")
+    print(f"[ios decay] mask_ios mixed_333x500 err {err:.3g} px {px:.3g}")
+    assert err <= TOL_IOS and px <= RESOLUTION_PX
 
 
 # ------------------------------------------------------------------------------------------------ pipeline
