@@ -150,9 +150,12 @@ struct AxisTable {
   // rows of one group read the same input rows, so the horizontal pass and the footprint test are shared
   int32_t* grp_of = nullptr;     // [out]  group index of each output coordinate
   int32_t* grp_start = nullptr;  // [out + 1] first coordinate of each group, grp_start[n_groups] = out
-  // one 128-bit record per output coordinate when taps <= 3 (every up-scaling): {xmin | xsize << 16, w0, w1, w2},
-  // weights beyond xsize are 0; padded with all-zero records (xsize = 0) up to a multiple of 32 coordinates
-  float4* pk = nullptr;          // [align32(out)] or nullptr
+  // two-tap records of the resize fast path, built only when every span has xsize <= 2 (up-scaling, except the sizes
+  // where fp32 rounding widens a span to three samples, see aa_spans_within_two; tests/test_resize_two_tap.py): per
+  // output coordinate the span {xmin | xsize << 16} and the weights {w0, w1} (w1 = 0 when xsize = 1), padded with
+  // all-zero records (xsize = 0) up to a multiple of 32 coordinates
+  uint32_t* pk_span = nullptr;   // [align32(out)] or nullptr
+  float2* pk_w = nullptr;        // [align32(out)] or nullptr
 };
 constexpr int kGrpMax = 4;
 constexpr int kMaxScatter = 24;

@@ -28,7 +28,8 @@ struct UpTables {
   const int32_t* x_tlo; const int32_t* x_tlen;  // input col -> output range
   const int32_t* y_tlo; const int32_t* y_tlen;  // input row -> output range
   const int32_t* y_grp_of; const int32_t* y_grp_start;  // output rows grouped by identical input span
-  const float4* pk_x; const float4* pk_y;  // packed {min | size << 16, w0, w1, w2} records (taps <= 3), else nullptr
+  // two-tap records (every span <= 2 input samples: up-scaling), else nullptr: {min | size << 16} and {w0, w1}
+  const uint32_t* pkx_span; const float2* pkx_w; const uint32_t* pky_span; const float2* pky_w;
 };
 
 // acc = s0*w0; acc = fma(s_j, w_j, acc)
@@ -110,7 +111,8 @@ __device__ __forceinline__ int up_ctas_needed(int n_groups) {
 // memory once with 16-byte cp.async (no register is held while the copies are in flight, rows are contiguous
 // segments: full sectors, each logit of the box read at most once per CTA) and the evaluation reads LDS.
 // `stage_floats` = capacity of the tile area in floats (0: staging off); tiles that do not fit (very wide / tall
-// chunks, more than 256 row groups) and the > 3-tap configurations take the direct path, which stays bit-identical.
+// chunks, more than 256 row groups) and the configurations without two-tap records take the direct path, which stays
+// bit-identical.
 __device__ __forceinline__ void cp_async16(void* smem_dst, const void* gmem_src) {
   const uint32_t d = (uint32_t)__cvta_generic_to_shared(smem_dst);
   asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(d), "l"(gmem_src) : "memory");
@@ -148,7 +150,7 @@ upsample_pack_kernel(const uint32_t* __restrict__ bits_lr, const UpMeta* __restr
   }
   const uint32_t* lr = bits_lr + ((size_t)mt.src * ih + clr0) * lr_wpr;
   const int n_lr = (clr1 - clr0) * lr_wpr;
-  const bool fast_cfg = t.pk_x != nullptr && t.pk_y != nullptr;  // <= 3 taps on both axes
+  const bool fast_cfg = t.pkx_span != nullptr && t.pky_span != nullptr;  // <= 2 taps on both axes
   const float* src = mt.logits;
   // tile = low-res rows [clr0, clr1) x columns [tc0, tc0 + tstride) (4-float aligned), behind the bits (16-byte aligned)
   float* tile = reinterpret_cast<float*>(s_lr + (((ih * lr_wpr + 1) + 3) & ~3));
@@ -214,7 +216,7 @@ upsample_pack_kernel(const uint32_t* __restrict__ bits_lr, const UpMeta* __restr
         const int nrows = yb - ya;
         int ry0, rys;
         if (fast_cfg) {
-          const int pky = __float_as_int(__ldg(t.pk_y + (uint32_t)ya).x);
+          const int pky = (int)__ldg(t.pky_span + (uint32_t)ya);
           ry0 = pky & 0xffff;
           rys = pky >> 16;
         } else {
@@ -280,33 +282,31 @@ upsample_pack_kernel(const uint32_t* __restrict__ bits_lr, const UpMeta* __restr
           const int s_rb = __shfl_sync(kFull, rb, src_lane), s_rys = __shfl_sync(kFull, rys, src_lane);
           const int x = ((wbase + (src_lane & (kUpCols - 1))) << 5) + lane;
           if (fast_cfg) {
-            // Every constant of the pixel in one 128-bit load (records past the width have size 0).  Taps beyond the
-            // span are never read; rows / taps beyond it contribute fma(0, 0, acc) = acc, so the arithmetic is exactly
+            // The pixel's span and two weights (records past the width have size 0).  Taps beyond the span are never
+            // read; rows / taps beyond it contribute fma(0, 0, acc) = acc, so the arithmetic is exactly
             // acc = s0*w0; acc = fma(s_j, w_j, acc) for j < size, horizontally and then vertically.
-            const float4 xt = __ldg(t.pk_x + (uint32_t)x);
-            const int pk = __float_as_int(xt.x);
+            const float2 xt = __ldg(t.pkx_w + (uint32_t)x);
+            const int pk = (int)__ldg(t.pkx_span + (uint32_t)x);
             const int cx = pk & 0xffff, cs = pk >> 16;
-            float T[3];
+            float T[2];
 #pragma unroll
-            for (int r = 0; r < 3; ++r) {
+            for (int r = 0; r < 2; ++r) {
               float acc = 0.0f;
               if (r < s_rys) {  // (warp-uniform)
                 // records past the image width have cs = 0, cx = 0 and zero weights: their first tap is clamped to
                 // the first column of the row (a valid address) and the lane's result is masked by `cs > 0`
                 const float* pl = tap_base + (s_rb + max(cx, tap_c0) + r * tap_stride);
-                acc = __fmul_rn(*pl, xt.y);
-                if (cs > 1) acc = __fmaf_rn(pl[1], xt.z, acc);
-                if (cs > 2) acc = __fmaf_rn(pl[2], xt.w, acc);
+                acc = __fmul_rn(*pl, xt.x);
+                if (cs > 1) acc = __fmaf_rn(pl[1], xt.y, acc);
               }
               T[r] = acc;
             }
 #pragma unroll
             for (int j = 0; j < kGrpMax; ++j) {
-              // {., w0, w1, w2} of the group's rows (rows past its last one repeat it and are dropped at the store)
-              const float4 wv = __ldg(t.pk_y + (uint32_t)min(s_ya + j, s_ya + s_nrows - 1));
-              float acc = __fmul_rn(T[0], wv.y);
-              acc = __fmaf_rn(T[1], wv.z, acc);
-              acc = __fmaf_rn(T[2], wv.w, acc);
+              // {w0, w1} of the group's rows (rows past its last one repeat it and are dropped at the store)
+              const float2 wv = __ldg(t.pky_w + (uint32_t)min(s_ya + j, s_ya + s_nrows - 1));
+              float acc = __fmul_rn(T[0], wv.x);
+              acc = __fmaf_rn(T[1], wv.y, acc);
               const uint32_t res = __ballot_sync(kFull, cs > 0 && acc > 0.0f);
               if (lane == src_lane) words[j] = res;
             }
@@ -402,7 +402,8 @@ upsample_pack_kernel(const uint32_t* __restrict__ bits_lr, const UpMeta* __restr
 }
 
 // ---------------------------------------------------------------------------------------------------
-// v2 — the path every <= 3-tap configuration takes (all up-scaling, mild down-scaling)
+// v2 — the path every two-tap configuration takes (every span of both axes <= 2 samples: up-scaling, see
+// aa_spans_within_two)
 //
 // What v1 measured as (ncu, config 2): 18-33 % issue utilisation, top stall long-scoreboard on the chain
 // pk_x record -> logits -> pk_y record, 4 800 of 6 400 CTAs exiting after two dependent global loads, ~165 warp
@@ -410,7 +411,7 @@ upsample_pack_kernel(const uint32_t* __restrict__ bits_lr, const UpMeta* __restr
 //   * a PLAN kernel turns the selected masks into a compact list of work items (mask, 32 row groups, 8 word columns)
 //     with their geometry resolved; persistent CTAs pull items from it with one atomic — no empty CTAs;
 //   * everything an item reads is copied into shared memory up front with cp.async (no register held while in flight):
-//     the logit tile under its rows/columns, the packed low-res rows, the pk_x / pk_y records, the group boundaries.
+//     the logit tile under its rows/columns, the packed low-res rows, the two-tap x / y records, the group boundaries.
 //     The evaluation loop then has no global load at all;
 //   * a warp owns a word COLUMN of the item: lane = row group for the footprint classification (32 groups at once),
 //     lane = pixel for the evaluation, so the pixel's x record is loaded once per column instead of once per word and
@@ -595,7 +596,7 @@ upsample_plan_kernel(const uint32_t* __restrict__ bits_lr, const int32_t* __rest
   if (blockIdx.x == 0 && tid == 0) { ctr[0] = base; ctr[1] = 0; }
 }
 
-// 16-byte copy that allocates in L1: the pk_x / pk_y tables are a few KB shared by every item an SM processes
+// 16-byte copy that allocates in L1: the two-tap records are a few KB shared by every item an SM processes
 __device__ __forceinline__ void cp_async16_ca(void* smem_dst, const void* gmem_src) {
   const uint32_t d = (uint32_t)__cvta_generic_to_shared(smem_dst);
   asm volatile("cp.async.ca.shared.global [%0], [%1], 16;" ::"r"(d), "l"(gmem_src) : "memory");
@@ -610,26 +611,26 @@ __device__ __forceinline__ float lds_f32(uint32_t saddr) {
   return v;
 }
 
-// taps of one input row for this lane's pixel: acc = s0*w0; acc = fma(s_j, w_j, acc) for j < cs
+// Two taps per axis.  aten's kernel runs `acc = s0*w0; acc = fma(s_j, w_j, acc)` over the table's taps; with up-scaling
+// every span has <= 2 samples, so a third term is always fma(0, 0, acc) = acc + 0.  That is acc itself for every acc
+// (inf and NaN included) except -0, which becomes +0, and a zero's sign never decides `acc > 0` (neither zero passes,
+// and a later non-zero term swamps it), so leaving those terms out keeps every thresholded bit.  A second tap beyond
+// the span (size 1) still enters as fma(0, 0, acc): its value is not read (the neighbour may be inf or NaN).
+
+// taps of one input row for this lane's pixel
 template <bool kStaged>
-__device__ __forceinline__ float up2_row(const float* __restrict__ gsrc, uint32_t saddr, int idx, const float4& xt, int cs) {
-  float a0, a1 = 0.0f, a2 = 0.0f;
+__device__ __forceinline__ float up2_row(const float* __restrict__ gsrc, uint32_t saddr, int idx, const float2& wx, int cs) {
+  float a0, a1 = 0.0f;
   if (kStaged) {
     const uint32_t p = saddr + ((uint32_t)idx << 2);
     a0 = lds_f32(p);
     if (cs > 1) a1 = lds_f32(p + 4);
-    if (cs > 2) a2 = lds_f32(p + 8);
   } else {
     const float* p = gsrc + idx;
     a0 = __ldg(p);
     if (cs > 1) a1 = __ldg(p + 1);
-    if (cs > 2) a2 = __ldg(p + 2);
   }
-  // absent taps: value 0 and weight 0 -> fma(0, 0, acc), which leaves `acc > 0` unchanged
-  float acc = __fmul_rn(a0, xt.y);
-  acc = __fmaf_rn(a1, xt.z, acc);
-  acc = __fmaf_rn(a2, xt.w, acc);
-  return acc;
+  return __fmaf_rn(a1, wx.y, __fmul_rn(a0, wx.x));
 }
 
 // per-group record of an item (shared memory): output row offset, rows, first tile row index * stride, input rows
@@ -637,33 +638,34 @@ struct alignas(16) Up2Group { int row, nrows, trow, rys; };
 
 template <bool kStaged>
 __device__ __forceinline__ void up2_evaluate(int warp, int lane, int n_list, const uint16_t* __restrict__ s_list,
-                                             const Up2Group* __restrict__ s_grp, const float4* __restrict__ s_pkx,
-                                             const float4* __restrict__ s_pky, uint32_t* __restrict__ s_out,
-                                             const float* __restrict__ gsrc, uint32_t tile_saddr, int tap_stride,
-                                             int tap_c0) {
+                                             const Up2Group* __restrict__ s_grp, const uint32_t* __restrict__ s_xspan,
+                                             const float2* __restrict__ s_xw, const float2* __restrict__ s_yw,
+                                             uint32_t* __restrict__ s_out, const float* __restrict__ gsrc,
+                                             uint32_t tile_saddr, int tap_stride, int tap_c0) {
   constexpr int kWarps = kUp2Threads / 32;
   for (int e = warp; e < n_list; e += kWarps) {
     const int ent = s_list[e];
     const int u = ent >> 5, gl = ent & 31;
     const Up2Group g = s_grp[gl];
-    const float4 xt = s_pkx[(u << 5) + lane];
-    const int pk = __float_as_int(xt.x);
+    const int px = (u << 5) + lane;
+    const int pk = (int)s_xspan[px];
+    const float2 wx = s_xw[px];
     const int cx = pk & 0xffff, cs = pk >> 16;  // records past the image width: cs = 0, cx = 0, zero weights
     const int idx = g.trow + max(cx - tap_c0, 0);
-    // horizontal pass of the group's (<= 3) input rows; rows beyond the span stay 0 and meet a zero weight
-    const float T0 = up2_row<kStaged>(gsrc, tile_saddr, idx, xt, cs);
-    float T1 = 0.0f, T2 = 0.0f;
-    if (g.rys > 1) T1 = up2_row<kStaged>(gsrc, tile_saddr, idx + tap_stride, xt, cs);
-    if (g.rys > 2) T2 = up2_row<kStaged>(gsrc, tile_saddr, idx + 2 * tap_stride, xt, cs);
-    // vertical pass of the group's rows (rows past its last one use whatever record follows and are dropped)
-    const float4* wy = s_pky + g.row;
+    // horizontal pass of the group's (<= 2) input rows.  A group with one input row (image border) reads its row twice
+    // and takes 0 for the second: no branch, and the second row's weight is 0.
+    const float T0 = up2_row<kStaged>(gsrc, tile_saddr, idx, wx, cs);
+    const float T1r = up2_row<kStaged>(gsrc, tile_saddr, idx + (g.rys > 1 ? tap_stride : 0), wx, cs);
+    const float T1 = g.rys > 1 ? T1r : 0.0f;
+    // vertical pass, all kGrpMax rows: rows past the group's last one read the records that follow and are dropped at
+    // the store.  Nearly every group is full when up-scaling (groups are runs of equal spans), and a per-row branch
+    // around the ballot costs more issue slots than the row itself.
+    const float2* wy = s_yw + g.row;
     uint32_t mine = 0;
 #pragma unroll
     for (int j = 0; j < kGrpMax; ++j) {
-      const float4 wv = wy[j];
-      float acc = __fmul_rn(T0, wv.y);
-      acc = __fmaf_rn(T1, wv.z, acc);
-      acc = __fmaf_rn(T2, wv.w, acc);
+      const float2 wv = wy[j];
+      const float acc = __fmaf_rn(T1, wv.y, __fmul_rn(T0, wv.x));
       const uint32_t res = __ballot_sync(kFull, cs > 0 && acc > 0.0f);
       if (lane == j) mine = res;
     }
@@ -671,6 +673,29 @@ __device__ __forceinline__ void up2_evaluate(int warp, int lane, int n_list, con
       const int row = g.row + lane;
       s_out[u * kUp2OutStride + row + (row >> 5)] = mine;
     }
+  }
+}
+
+// one item's area / box into its mask's scratch; the last item of the mask publishes the mask's totals
+__device__ __forceinline__ void up2_publish(int k, const int (&red)[5], int32_t* __restrict__ scratch,
+                                            int32_t* __restrict__ area_full, int32_t* __restrict__ box_full) {
+  int32_t* sc = scratch + (size_t)k * kScratchInts;
+  atomicAdd(&sc[0], red[0]);
+  atomicMax(&sc[1], red[1]);
+  atomicMax(&sc[2], red[2]);
+  atomicMax(&sc[3], red[3]);
+  atomicMax(&sc[4], red[4]);
+  __threadfence();
+  const int prev = atomicAdd(&sc[5], 1);
+  if (prev == sc[6] - 1) {  // last item of this mask
+    __threadfence();
+    const int a = atomicAdd(&sc[0], 0);
+    const int mx1 = atomicMax(&sc[1], 0), my1 = atomicMax(&sc[2], 0);
+    const int bx = atomicMax(&sc[3], 0), by = atomicMax(&sc[4], 0);
+    area_full[k] = a;
+    int4 o = make_int4(0, 0, 0, 0);
+    if (a > 0) o = make_int4(kBig - bx, kBig - by, mx1 - 1, my1 - 1);
+    reinterpret_cast<int4*>(box_full)[k] = o;
   }
 }
 
@@ -683,9 +708,12 @@ upsample_pack2_kernel(const uint32_t* __restrict__ bits_lr, const UpMeta* __rest
   // (nullable) two counters of the NEXT stage, zeroed here so that its first kernel can append to them right away
   if (zero2 && blockIdx.x == 0 && threadIdx.x == 0) { zero2[0] = 0; zero2[1] = 0; }
   extern __shared__ __align__(16) unsigned char s_raw[];
-  float4* s_pkx = reinterpret_cast<float4*>(s_raw);                       // [kUp2Cols * 32]
-  float4* s_pky = s_pkx + kUp2Cols * 32;                                  // [kUp2Rows + kGrpMax] (rows past the end are read)
-  Up2Group* s_grp = reinterpret_cast<Up2Group*>(s_pky + kUp2Rows + kGrpMax);  // [kUp2Groups]
+  // two-tap records of the item's columns and rows; the rows from ya0 rounded down to a multiple of 4 (16-byte copies)
+  float2* s_xw = reinterpret_cast<float2*>(s_raw);                        // [kUp2Cols * 32]
+  float2* s_yw = s_xw + kUp2Cols * 32;                                    // [kUp2Rows + 8] (3 rows past the end are read)
+  uint32_t* s_xspan = reinterpret_cast<uint32_t*>(s_yw + kUp2Rows + 8);   // [kUp2Cols * 32]
+  uint32_t* s_yspan = s_xspan + kUp2Cols * 32;                            // [kUp2Rows + 4]
+  Up2Group* s_grp = reinterpret_cast<Up2Group*>(s_yspan + kUp2Rows + 4);  // [kUp2Groups]
   uint32_t* s_out = reinterpret_cast<uint32_t*>(s_grp + kUp2Groups);      // [kUp2Cols * kUp2OutStride]
   int* s_gstart = reinterpret_cast<int*>(s_out + kUp2Cols * kUp2OutStride);  // [kUp2Groups + 4]
   uint16_t* s_list = reinterpret_cast<uint16_t*>(s_gstart + kUp2Groups + 4);  // [kUp2Cols * kUp2Groups] boundary words
@@ -700,13 +728,16 @@ upsample_pack2_kernel(const uint32_t* __restrict__ bits_lr, const UpMeta* __rest
   const int ow_words = (ow + 31) >> 5;
   const int total = ctr[0];
   const uint32_t tile_saddr = (uint32_t)__cvta_generic_to_shared(tile);
+  // Thread 0 claims the next item while the current one runs, and publishes an item's statistics while the next one's
+  // copies are in flight: the round trips of those atomics and of the fence no longer hold the whole CTA.
+  int next = 0, pend_k = -1, pend[5];
+  if (tid == 0) s_item = atomicAdd(&ctr[1], 1);
   for (;;) {
-    __syncthreads();  // the previous item is completely done with shared memory
-    if (tid == 0) s_item = atomicAdd(&ctr[1], 1);
-    if (tid < 5) s_red[tid] = 0;
-    __syncthreads();
+    __syncthreads();  // the previous item is completely done with shared memory; s_item is the claimed item
     const int item = s_item;
     if (item >= total) break;
+    if (tid == 0) next = atomicAdd(&ctr[1], 1);
+    if (tid < 5) s_red[tid] = 0;
     const Up2Item it = items[item];
     const int k = it.k;
     const UpMeta mt = meta[k];
@@ -739,11 +770,15 @@ upsample_pack2_kernel(const uint32_t* __restrict__ bits_lr, const UpMeta* __rest
       } else {
         for (int i = tid; i < n_lr; i += kUp2Threads) cp_async4(s_lr + i, lr + i);
       }
-      for (int i = tid; i < n_rows; i += kUp2Threads) cp_async16_ca(s_pky + i, t.pk_y + ya0 + i);
-      const float4* px = t.pk_x + (wA << 5);
-      for (int i = tid; i < (nw << 5); i += kUp2Threads) cp_async16_ca(s_pkx + i, px + i);
+      // (the tables are padded to a multiple of 32 coordinates: the rounded-up ends stay inside them)
+      const int yb = ya0 & ~3, ny = n_rows + (ya0 & 3);
+      for (int i = tid; i < ((ny + 3) >> 2); i += kUp2Threads) cp_async16_ca(s_yspan + 4 * i, t.pky_span + yb + 4 * i);
+      for (int i = tid; i < ((ny + 1) >> 1); i += kUp2Threads) cp_async16_ca(s_yw + 2 * i, t.pky_w + yb + 2 * i);
+      for (int i = tid; i < (nw << 3); i += kUp2Threads) cp_async16_ca(s_xspan + 4 * i, t.pkx_span + (wA << 5) + 4 * i);
+      for (int i = tid; i < (nw << 4); i += kUp2Threads) cp_async16_ca(s_xw + 2 * i, t.pkx_w + (wA << 5) + 2 * i);
       if (tid <= ng) s_gstart[tid] = min(max(t.y_grp_start[gA + tid], mt.r0), mt.r1);
     }
+    if (tid == 0 && pend_k >= 0) up2_publish(pend_k, pend, scratch, area_full, box_full);
     cp_async_wait_all();
     __syncthreads();
     // taps are read at index  trow + max(col - tap_c0, 0)  of the shared tile (staged) or of the global logits
@@ -756,7 +791,7 @@ upsample_pack2_kernel(const uint32_t* __restrict__ bits_lr, const UpMeta* __rest
       my_ya = s_gstart[lane];
       my_nrows = s_gstart[lane + 1] - my_ya;
       if (my_nrows > 0) {
-        const int pky = __float_as_int(s_pky[my_ya - ya0].x);
+        const int pky = (int)s_yspan[my_ya - (ya0 & ~3)];
         my_ry0 = pky & 0xffff;
         my_rys = pky >> 16;
       }
@@ -774,7 +809,7 @@ upsample_pack2_kernel(const uint32_t* __restrict__ bits_lr, const UpMeta* __rest
       const int x0 = min(wi << 5, ow - 1);
       const int x1 = min(x0 + 31, ow - 1);
       const uint32_t valid = (x1 - x0 == 31) ? 0xffffffffu : ((1u << (x1 - x0 + 1)) - 1u);
-      const int p0 = __float_as_int(s_pkx[x0 - (wA << 5)].x), p1 = __float_as_int(s_pkx[x1 - (wA << 5)].x);
+      const int p0 = (int)s_xspan[x0 - (wA << 5)], p1 = (int)s_xspan[x1 - (wA << 5)];
       const int c0 = p0 & 0xffff;
       const int c1 = (p1 & 0xffff) + (p1 >> 16);  // exclusive
       const int cw0 = c0 >> 5;
@@ -839,38 +874,54 @@ upsample_pack2_kernel(const uint32_t* __restrict__ bits_lr, const UpMeta* __rest
     __syncthreads();
     // ---- phase B: evaluation, lane = pixel of the word
     if (staged)
-      up2_evaluate<true>(warp, lane, n_list, s_list, s_grp, s_pkx, s_pky, s_out, src, tile_saddr, tap_stride, tap_c0);
+      up2_evaluate<true>(warp, lane, n_list, s_list, s_grp, s_xspan, s_xw, s_yw + (ya0 & 3), s_out, src, tile_saddr,
+                         tap_stride, tap_c0);
     else
-      up2_evaluate<false>(warp, lane, n_list, s_list, s_grp, s_pkx, s_pky, s_out, src, tile_saddr, tap_stride, tap_c0);
+      up2_evaluate<false>(warp, lane, n_list, s_list, s_grp, s_xspan, s_xw, s_yw + (ya0 & 3), s_out, src, tile_saddr,
+                          tap_stride, tap_c0);
     __syncthreads();
-    // ---- second copy, word-column major [k][word][row] (nullable): the overlap windows mask_ios walks are a few words
-    //      wide and hundreds of rows tall — 4 useful bytes per 32-byte sector in the row-major layout, contiguous here.
-    //      The result tile is column-major already: a warp writes 128 contiguous bytes per store.
-    if (bits_t) {
-      uint32_t* dt = bits_t + (size_t)k * oh * ow_words;
-      for (int c = warp; c < nw; c += kWarps)
-        for (int row = lane; row < n_rows; row += 32)
-          dt[(uint32_t)((wA + c) * oh + ya0 + row)] = s_out[c * kUp2OutStride + row + (row >> 5)];
-    }
-    // ---- epilogue: result tile -> global in 32-byte row segments; area and box from the words
+    // ---- epilogue: area and box from the result words, which leave as the word-column-major copy [k][word][row]
+    //      (nullable: the overlap windows mask_ios walks are a few words wide and hundreds of rows tall — 4 useful bytes
+    //      per 32-byte sector in the row-major layout, contiguous here; the result tile is column-major already, so a
+    //      warp writes 128 contiguous bytes per store) and/or row-major in 32-byte row segments
     {
-      uint32_t* dst = bits_full ? bits_full + (size_t)k * oh * ow_words : nullptr;  // (row-major copy: optional)
-      const int c = tid & (kUp2Cols - 1);
-      int area = 0, miny = kBig, maxy = -1;
-      uint32_t colbits = 0;
-      if (c < nw) {
-        for (int row = tid >> 3; row < n_rows; row += kUp2Threads / kUp2Cols) {
-          const uint32_t w = s_out[c * kUp2OutStride + row + (row >> 5)];
-          if (dst) dst[(uint32_t)((ya0 + row) * ow_words + wA + c)] = w;
-          area += __popc(w);
-          colbits |= w;
-          if (w) { miny = min(miny, ya0 + row); maxy = max(maxy, ya0 + row); }
+      int area = 0, minx = kBig, maxx = -1, miny = kBig, maxy = -1;
+      if (bits_t) {  // warp = word column, lane = row
+        uint32_t* dt = bits_t + (size_t)k * oh * ow_words;
+        for (int c = warp; c < nw; c += kWarps) {
+          uint32_t colbits = 0;
+          for (int row = lane; row < n_rows; row += 32) {
+            const uint32_t w = s_out[c * kUp2OutStride + row + (row >> 5)];
+            dt[(uint32_t)((wA + c) * oh + ya0 + row)] = w;
+            area += __popc(w);
+            colbits |= w;
+            if (w) { miny = min(miny, ya0 + row); maxy = max(maxy, ya0 + row); }
+          }
+          if (colbits) {
+            minx = min(minx, ((wA + c) << 5) + __ffs(colbits) - 1);
+            maxx = max(maxx, ((wA + c) << 5) + 31 - __clz(colbits));
+          }
         }
       }
-      int minx = kBig, maxx = -1;
-      if (colbits) {
-        minx = ((wA + c) << 5) + __ffs(colbits) - 1;
-        maxx = ((wA + c) << 5) + 31 - __clz(colbits);
+      if (bits_full) {  // thread = (row, word column)
+        uint32_t* dst = bits_full + (size_t)k * oh * ow_words;
+        const int c = tid & (kUp2Cols - 1);
+        uint32_t colbits = 0;
+        if (c < nw) {
+          for (int row = tid >> 3; row < n_rows; row += kUp2Threads / kUp2Cols) {
+            const uint32_t w = s_out[c * kUp2OutStride + row + (row >> 5)];
+            dst[(uint32_t)((ya0 + row) * ow_words + wA + c)] = w;
+            if (!bits_t) {
+              area += __popc(w);
+              colbits |= w;
+              if (w) { miny = min(miny, ya0 + row); maxy = max(maxy, ya0 + row); }
+            }
+          }
+        }
+        if (colbits) {
+          minx = ((wA + c) << 5) + __ffs(colbits) - 1;
+          maxx = ((wA + c) << 5) + 31 - __clz(colbits);
+        }
       }
       area = warp_sum(area);
       minx = warp_min(minx); miny = warp_min(miny); maxx = warp_max(maxx); maxy = warp_max(maxy);
@@ -884,32 +935,20 @@ upsample_pack2_kernel(const uint32_t* __restrict__ bits_lr, const UpMeta* __rest
     }
     __syncthreads();
     if (tid == 0) {
-      int32_t* sc = scratch + (size_t)k * kScratchInts;
-      atomicAdd(&sc[0], s_red[0]);
-      atomicMax(&sc[1], s_red[1]);
-      atomicMax(&sc[2], s_red[2]);
-      atomicMax(&sc[3], s_red[3]);
-      atomicMax(&sc[4], s_red[4]);
-      __threadfence();
-      const int prev = atomicAdd(&sc[5], 1);
-      if (prev == sc[6] - 1) {  // last item of this mask publishes the final statistics
-        __threadfence();
-        const int a = atomicAdd(&sc[0], 0);
-        const int mx1 = atomicMax(&sc[1], 0), my1 = atomicMax(&sc[2], 0);
-        const int bx = atomicMax(&sc[3], 0), by = atomicMax(&sc[4], 0);
-        area_full[k] = a;
-        int4 o = make_int4(0, 0, 0, 0);
-        if (a > 0) o = make_int4(kBig - bx, kBig - by, mx1 - 1, my1 - 1);
-        reinterpret_cast<int4*>(box_full)[k] = o;
-      }
+      pend_k = k;
+#pragma unroll
+      for (int q = 0; q < 5; ++q) pend[q] = s_red[q];
+      s_item = next;
     }
   }
+  if (tid == 0 && pend_k >= 0) up2_publish(pend_k, pend, scratch, area_full, box_full);
 }
 
 // shared-memory layout of upsample_pack2_kernel in bytes, without / with a logit tile of `tile_floats`
 static size_t up2_fixed_smem(int ih, int iw) {
   const size_t lr_words = (((size_t)ih * (iw / 32) + 4) + 3) & ~(size_t)3;
-  return sizeof(float4) * (kUp2Cols * 32 + kUp2Rows + kGrpMax + kUp2Groups) +
+  return (sizeof(float2) + sizeof(uint32_t)) * (kUp2Cols * 32 + kUp2Rows + 4) + sizeof(float2) * 4 +
+         sizeof(Up2Group) * kUp2Groups +
          4 * ((size_t)kUp2Cols * kUp2OutStride + kUp2Groups + 4 + lr_words) + 2 * (size_t)kUp2Cols * kUp2Groups;
 }
 // items a selection can expand to: every mask at most ceil(groups / 32) x ceil(words / 8), groups <= output rows
@@ -929,9 +968,9 @@ int launch_upsample_pack(const AxisTable& tx, const AxisTable& ty, const float* 
   if (max_sel <= 0) return NTTT_OK;
   if (iw % 32 != 0) return NTTT_EUNSUPPORTED;
   UpTables t{tx.xmin, tx.xsize, tx.w, tx.taps, ty.xmin, ty.xsize, ty.w, ty.taps, tx.t_lo, tx.t_len, ty.t_lo, ty.t_len,
-             ty.grp_of, ty.grp_start, tx.pk, ty.pk};
+             ty.grp_of, ty.grp_start, tx.pk_span, tx.pk_w, ty.pk_span, ty.pk_w};
   UpMeta* meta = reinterpret_cast<UpMeta*>(scratch + (size_t)kScratchInts * max_sel);
-  if (tx.pk && ty.pk && oh < 65536 && ow < 65536 && ih * (iw / 32) <= 16384) {
+  if (tx.pk_span && ty.pk_span && oh < 65536 && ow < 65536 && ih * (iw / 32) <= 16384) {
     // v2: plan + persistent work-list kernel
     int32_t* ctr = reinterpret_cast<int32_t*>(meta + max_sel);
     Up2Item* items = reinterpret_cast<Up2Item*>(ctr + 4);

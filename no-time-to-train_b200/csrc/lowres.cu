@@ -6,6 +6,8 @@
 #include <cuda_bf16.h>
 #include <stdlib.h>
 
+#include <algorithm>
+
 #include "common.cuh"
 
 namespace nttt {
@@ -746,21 +748,39 @@ __global__ void aa_group_kernel(int out_size, const int32_t* xmin, const int32_t
   for (int k = g + 1; k <= out_size; ++k) grp_start[k] = out_size;
 }
 
-// packed records for the resize fast path (see AxisTable::pk)
+// two-tap records for the resize fast path (see AxisTable::pk_span / pk_w)
 __global__ void aa_pack_kernel(int out_size, int out_pad, int taps, const int32_t* xmin, const int32_t* xsize,
-                               const float* w, float4* pk) {
+                               const float* w, uint32_t* pk_span, float2* pk_w) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= out_pad) return;
-  float4 e = make_float4(0.f, 0.f, 0.f, 0.f);
+  uint32_t span = 0;
+  float2 e = make_float2(0.f, 0.f);
   if (i < out_size) {
     const int cs = xsize[i];
     const float* wi = w + (size_t)i * taps;
-    e.x = __int_as_float(xmin[i] | (cs << 16));
-    e.y = cs > 0 ? wi[0] : 0.0f;
-    e.z = cs > 1 ? wi[1] : 0.0f;
-    e.w = cs > 2 ? wi[2] : 0.0f;
+    span = (uint32_t)xmin[i] | ((uint32_t)cs << 16);
+    e.x = cs > 0 ? wi[0] : 0.0f;
+    e.y = cs > 1 ? wi[1] : 0.0f;
   }
-  pk[i] = e;
+  pk_span[i] = span;
+  pk_w[i] = e;
+}
+
+// Whether every span of the axis has xsize <= 2: aa_table_kernel's spans restated on the host, the same fp32 operations
+// each rounded (the volatile intermediates keep the compiler from contracting them).  Up-scaling gives
+// int(c + 1.5) - int(c - 0.5) = 2 (1 at the borders) as long as both sums are exact; when c + 1 rounds up to the next
+// half (3 -> 37, 96 -> 608, 160 -> 736, ...) the span is three samples wide and its third weight is 0, which aten still
+// multiplies in (an inf or NaN there turns the sample into NaN).  Such axes keep the general path.
+static bool aa_spans_within_two(int in_size, int out_size) {
+  if (in_size > out_size) return false;
+  const float scale = (float)in_size / (float)out_size;
+  for (int i = 0; i < out_size; ++i) {
+    volatile float center = scale * ((float)i + 0.5f);
+    volatile float a = center - 1.0f, b = center + 1.0f;
+    const int lo = std::max((int)(a + 0.5f), 0), hi = std::min((int)(b + 0.5f), in_size);
+    if (hi - lo > 2) return false;
+  }
+  return true;
 }
 
 // All arrays of a table live in ONE device allocation (`slab`): a table costs one cudaMalloc when a new (in, out) pair is
@@ -769,7 +789,7 @@ int build_axis_table(AxisTable& t, int in_size, int out_size, cudaStream_t s) {
   t.in_size = in_size;
   t.out_size = out_size;
   t.taps = aa_max_taps(in_size, out_size);
-  const bool packed = t.taps <= 3 && in_size < 65536;
+  const bool packed = in_size < 65536 && aa_spans_within_two(in_size, out_size);
   const int out_pad = (out_size + 31) / 32 * 32;
   size_t off = 0;
   auto take = [&](size_t bytes) { const size_t o = off; off = align_up(off + bytes, 256); return o; };
@@ -779,7 +799,8 @@ int build_axis_table(AxisTable& t, int in_size, int out_size, cudaStream_t s) {
   const size_t o_tw = take(sizeof(float) * (size_t)in_size * kMaxScatter);
   const size_t o_tcum = take(sizeof(float) * (size_t)in_size * (kMaxScatter + 1));
   const size_t o_gof = take(sizeof(int32_t) * out_size), o_gst = take(sizeof(int32_t) * ((size_t)out_size + 1));
-  const size_t o_pk = packed ? take(sizeof(float4) * (size_t)out_pad) : 0;
+  const size_t o_pks = packed ? take(sizeof(uint32_t) * (size_t)out_pad) : 0;
+  const size_t o_pkw = packed ? take(sizeof(float2) * (size_t)out_pad) : 0;
   char* slab = nullptr;
   NTTT_CUDA(cudaMalloc(&slab, off));
   t.slab = slab;
@@ -792,7 +813,8 @@ int build_axis_table(AxisTable& t, int in_size, int out_size, cudaStream_t s) {
   t.t_cum = reinterpret_cast<float*>(slab + o_tcum);
   t.grp_of = reinterpret_cast<int32_t*>(slab + o_gof);
   t.grp_start = reinterpret_cast<int32_t*>(slab + o_gst);
-  t.pk = packed ? reinterpret_cast<float4*>(slab + o_pk) : nullptr;
+  t.pk_span = packed ? reinterpret_cast<uint32_t*>(slab + o_pks) : nullptr;
+  t.pk_w = packed ? reinterpret_cast<float2*>(slab + o_pkw) : nullptr;
   aa_table_kernel<<<ceil_div(out_size, 128), 128, 0, s>>>(in_size, out_size, t.taps, t.xmin, t.xsize, t.w);
   NTTT_LAUNCH_CHECK();
   aa_transpose_kernel<<<ceil_div(in_size, 128), 128, 0, s>>>(in_size, out_size, t.taps, t.xmin, t.xsize, t.w, t.t_lo,
@@ -801,7 +823,8 @@ int build_axis_table(AxisTable& t, int in_size, int out_size, cudaStream_t s) {
   aa_group_kernel<<<1, 32, 0, s>>>(out_size, t.xmin, t.xsize, t.grp_of, t.grp_start);
   NTTT_LAUNCH_CHECK();
   if (packed) {
-    aa_pack_kernel<<<ceil_div(out_pad, 128), 128, 0, s>>>(out_size, out_pad, t.taps, t.xmin, t.xsize, t.w, t.pk);
+    aa_pack_kernel<<<ceil_div(out_pad, 128), 128, 0, s>>>(out_size, out_pad, t.taps, t.xmin, t.xsize, t.w, t.pk_span,
+                                                             t.pk_w);
     NTTT_LAUNCH_CHECK();
   }
   return NTTT_OK;
