@@ -377,6 +377,33 @@ int nttt_match_image(nttt_ctx* ctx, const nttt_match_args* args, void* stream);
 /* sizeof(nttt_match_args) as compiled, so FFI mirrors can verify their layout */
 size_t nttt_sizeof_match_args(void);
 
+/* ---------------------------------------------------------------------------------------------------
+ * The whole stage for images of any output size in a range, with the size read from device memory when the kernels
+ * run: one enqueue (or one CUDA-graph capture) serves every size in [min_h, ori_h] x [min_w, ori_w].
+ *   args->ori_h / ori_w are the CAPACITY (largest size); out_masks keeps the capacity's strides
+ *   [num_out_instance, ori_h, ori_w], and the mask of output j occupies rows < h and columns < w of plane j.  With
+ *   out_prev_rect the whole buffer equals the dense masks at (h, w) embedded top-left, zeros everywhere else (also
+ *   where an earlier, larger image wrote).  Every other output is what nttt_match_image gives at ori_h = h,
+ *   ori_w = w, bit for bit, in both low_latency modes.
+ *   A size outside the range gives an empty result (counts[1] = counts[2] = 0, persistent slots cleared) and
+ *   counts[3] = 1; otherwise counts[3] = 0.  Nothing is written outside the capacity's buffers.
+ *   The first call of a range builds the resize tables of all its sizes (the context's atlas, one synchronisation);
+ *   later calls with that range allocate nothing and do not synchronise.
+ */
+typedef struct nttt_match_size_range {
+  const int32_t* ori_hw_dev; /* [2] i32, device: (h, w) of this image, read when the stage runs */
+  int32_t min_h, min_w;      /* smallest size accepted (>= 1, <= the capacity) */
+} nttt_match_size_range;
+
+/* as nttt_match_workspace_bytes_neg at the capacity; 0 for an invalid range */
+size_t nttt_match_workspace_bytes_sized(int n, int lr_h, int lr_w, int eh, int ew, int c, int n_cls, int ori_h,
+                                        int ori_w, int max_sel, int l_neg, int min_h, int min_w);
+int nttt_match_image_sized(nttt_ctx* ctx, const nttt_match_args* args, const nttt_match_size_range* range,
+                           void* stream);
+/* the context's resize-table atlases of the sized entry: returns their number, and (nullable outputs) their device
+ * bytes and the host time their builds took in total */
+int nttt_ctx_atlas_stats(nttt_ctx* ctx, size_t* bytes_host, double* build_ms_host);
+
 #ifdef __cplusplus
 }
 #endif

@@ -45,6 +45,11 @@ class MatchArgs(ctypes.Structure):
     ]
 
 
+class MatchSizeRange(ctypes.Structure):
+    """Mirror of `nttt_match_size_range` (include/nttt_b200.h)."""
+    _fields_ = [("ori_hw_dev", c_void_p), ("min_h", c_int32), ("min_w", c_int32)]
+
+
 # name -> (restype, argtypes); every symbol include/nttt_b200.h declares
 _P = c_void_p
 SIGNATURES = {
@@ -89,6 +94,9 @@ SIGNATURES = {
                                           _P]),
     "nttt_match_image": (c_int, [_P, POINTER(MatchArgs), _P]),
     "nttt_sizeof_match_args": (c_size_t, []),
+    "nttt_match_workspace_bytes_sized": (c_size_t, [c_int] * 13),
+    "nttt_match_image_sized": (c_int, [_P, POINTER(MatchArgs), POINTER(MatchSizeRange), _P]),
+    "nttt_ctx_atlas_stats": (c_int, [_P, POINTER(c_size_t), POINTER(ctypes.c_double)]),
     "nttt_launch_count": (ctypes.c_ulonglong, []),
     "nttt_profile_num_stages": (c_int, []),
     "nttt_profile_stage_name": (c_char_p, [c_int]),

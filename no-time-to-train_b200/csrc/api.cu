@@ -38,19 +38,23 @@ int launch_upsample_pack(const AxisTable&, const AxisTable&, const float*, const
                          bool* wrote_t = nullptr, bool t_only = false, bool low_latency = false, int32_t* zero2 = nullptr);
 int32_t* ios_pair_counters(void* ws, int max_sel);
 size_t upsample_scratch_bytes(int max_sel, int oh, int ow);
+int launch_upsample_pack_sized(const SizedDims&, const SizedAtlas&, const float*, const uint32_t*, const int32_t*,
+                               const int32_t*, int, int, const int32_t*, const int32_t*, int, uint32_t*, int32_t*,
+                               int32_t*, int32_t*, int32_t*, const float* const*, cudaStream_t, int, int, uint32_t*, bool,
+                               int32_t*);
 int launch_unpack_sparse(const uint32_t*, const int32_t*, const int32_t*, const int32_t*, int, int, int, uint8_t*,
-                         int32_t*, cudaStream_t, bool tr = false);
+                         int32_t*, cudaStream_t, bool tr = false, const SizedDims* sized = nullptr);
 int launch_unpack(const uint32_t*, const int32_t*, const int32_t*, const int32_t*, int, int, int, uint8_t*,
-                  cudaStream_t, bool tr = false);
+                  cudaStream_t, bool tr = false, const SizedDims* sized = nullptr);
 size_t ios_workspace_bytes(int max_sel);
 int launch_mask_ios(const uint32_t*, const int32_t*, const int32_t*, const int32_t*, const int32_t*, const int32_t*,
                     int, int, int, const int32_t*, const float*, int, float*, int32_t*, void*, bool, cudaStream_t,
-                    const uint32_t* bits_t = nullptr, bool counters_zeroed = false);
+                    const uint32_t* bits_t = nullptr, bool counters_zeroed = false, const SizedDims* sized = nullptr);
 int launch_decay_rank(const float*, const int32_t*, const float*, const int32_t*, const int32_t*, int, int,
                       const int32_t*, const int32_t*, int64_t*, float*, int64_t*, int32_t*, int32_t*, int32_t*, float*,
                       cudaStream_t);
 int launch_rle_encode(const uint32_t*, const int32_t*, const int32_t*, const int32_t*, int, int, int, int, int, uint32_t*,
-                      int32_t*, uint8_t*, int32_t*, cudaStream_t, bool tr = false);
+                      int32_t*, uint8_t*, int32_t*, cudaStream_t, bool tr = false, const SizedDims* sized = nullptr);
 int launch_rle_compact(const uint8_t*, const int32_t*, int, int, uint8_t*, long long, cudaStream_t);
 int launch_fill_pool(const float*, const float*, int, int, int, int, int, int, float*, float*, float*, int, cudaStream_t);
 int launch_fill_scatter(const float*, const float*, const float*, const int32_t*, int, int, int, float*, float*, float*,
@@ -238,6 +242,25 @@ int nttt_ctx::axis(int in_size, int out_size, cudaStream_t s, nttt::AxisTable* o
   return NTTT_OK;
 }
 
+int nttt_ctx::sized_atlas(int lr_h, int lr_w, int min_h, int min_w, int cap_h, int cap_w, cudaStream_t s,
+                          const nttt::SizedAtlas** out) {
+  for (int i = 0; i < n_atlases; ++i) {
+    const SizedAtlas& a = atlases[i];
+    if (a.lr_h == lr_h && a.lr_w == lr_w && a.min_h == min_h && a.min_w == min_w && a.cap_h == cap_h && a.cap_w == cap_w) {
+      *out = &a;
+      return NTTT_OK;
+    }
+  }
+  if (n_atlases == kMaxAtlases) return NTTT_EUNSUPPORTED;
+  SizedAtlas a;
+  a.lr_h = lr_h; a.lr_w = lr_w; a.min_h = min_h; a.min_w = min_w; a.cap_h = cap_h; a.cap_w = cap_w;
+  int err = build_sized_atlas(a, s);
+  if (err) return err;
+  atlases[n_atlases] = a;
+  *out = &atlases[n_atlases++];
+  return NTTT_OK;
+}
+
 extern "C" {
 
 int nttt_version(void) { return NTTT_VERSION; }
@@ -358,6 +381,7 @@ void nttt_ctx_destroy(nttt_ctx* ctx) {
   if (ctx->ev_join) cudaEventDestroy(ctx->ev_join);
   for (int i = 0; i < ctx->n_tables; ++i) free_axis_table(ctx->tables[i]);
   for (int i = 0; i < ctx->n_retired; ++i) free_axis_table(ctx->retired[i]);
+  for (int i = 0; i < ctx->n_atlases; ++i) cudaFree(ctx->atlases[i].slab);
   if (ctx->scratch) cudaFree(ctx->scratch);
   for (int i = 0; i <= nttt_ctx::kMaxStages; ++i)
     if (ctx->ev[i]) cudaEventDestroy(ctx->ev[i]);
@@ -745,11 +769,36 @@ size_t nttt_match_workspace_bytes_neg(int n, int lr_h, int lr_w, int eh, int ew,
   return carve(nullptr, n, lr_h, lr_w, eh, ew, c, n_cls, ori_h, ori_w, max_sel, max_sel, l_neg).total;
 }
 
-int nttt_match_image(nttt_ctx* ctx, const nttt_match_args* a, void* stream) {
+size_t nttt_match_workspace_bytes_sized(int n, int lr_h, int lr_w, int eh, int ew, int c, int n_cls, int ori_h, int ori_w,
+                                        int max_sel, int l_neg, int min_h, int min_w) {
+  if (min_h <= 0 || min_w <= 0 || min_h > ori_h || min_w > ori_w) return 0;
+  // (every buffer of the workspace grows with the output size: the capacity's layout serves the whole range)
+  return nttt_match_workspace_bytes_neg(n, lr_h, lr_w, eh, ew, c, n_cls, ori_h, ori_w, max_sel, l_neg);
+}
+
+int nttt_ctx_atlas_stats(nttt_ctx* ctx, size_t* bytes_host, double* build_ms_host) {
+  if (!ctx) return NTTT_EINVAL;
+  size_t bytes = 0;
+  double ms = 0.0;
+  for (int i = 0; i < ctx->n_atlases; ++i) {
+    bytes += ctx->atlases[i].bytes;
+    ms += ctx->atlases[i].build_ms;
+  }
+  if (bytes_host) *bytes_host = bytes;
+  if (build_ms_host) *build_ms_host = ms;
+  return ctx->n_atlases;
+}
+
+// range == nullptr: nttt_match_image (the size is a->ori_h x a->ori_w); otherwise nttt_match_image_sized
+static int match_impl(nttt_ctx* ctx, const nttt_match_args* a, const nttt_match_size_range* range, void* stream) {
   if (!ctx || !a) return NTTT_EINVAL;
   if (a->n < 0 || a->lr_h <= 0 || a->lr_w <= 0 || a->eh <= 0 || a->ew <= 0 || a->c <= 0 || a->n_cls <= 0 ||
       a->ori_h <= 0 || a->ori_w <= 0 || a->num_out_instance < 0 || a->max_sel < 0)
     return NTTT_EINVAL;
+  if (range && (!range->ori_hw_dev || range->min_h <= 0 || range->min_w <= 0 || range->min_h > a->ori_h ||
+                range->min_w > a->ori_w))
+    return NTTT_EINVAL;
+  if (range && (a->ori_h >= 65536 || a->ori_w >= 65536)) return NTTT_EUNSUPPORTED;
   if (!a->counts || !a->workspace) return NTTT_EINVAL;
   cudaStream_t s = (cudaStream_t)stream;
   const int n = a->n, max_sel = a->max_sel, num_out = a->num_out_instance;
@@ -786,8 +835,17 @@ int nttt_match_image(nttt_ctx* ctx, const nttt_match_args* a, void* stream) {
   int err = ctx->axis(a->ew, a->lr_w, s, &px);
   if (err) return err;
   if ((err = ctx->axis(a->eh, a->lr_h, s, &py))) return err;
-  if ((err = ctx->axis(a->lr_w, a->ori_w, s, &ux))) return err;
-  if ((err = ctx->axis(a->lr_h, a->ori_h, s, &uy))) return err;
+  // sized: the resize tables of every size of the range, and what the kernels read the size from
+  const SizedAtlas* atlas = nullptr;
+  SizedDims sd{};
+  if (range) {
+    if ((err = ctx->sized_atlas(a->lr_h, a->lr_w, range->min_h, range->min_w, a->ori_h, a->ori_w, s, &atlas))) return err;
+    sd = SizedDims{range->ori_hw_dev, atlas->ay, atlas->ax, a->counts, range->min_h, range->min_w, a->ori_h, a->ori_w};
+  } else {
+    if ((err = ctx->axis(a->lr_w, a->ori_w, s, &ux))) return err;
+    if ((err = ctx->axis(a->lr_h, a->ori_h, s, &uy))) return err;
+  }
+  const SizedDims* sized = range ? &sd : nullptr;
   const int e = a->eh * a->ew;
 
   ctx->n_ev = 0;
@@ -884,16 +942,25 @@ int nttt_match_image(nttt_ctx* ctx, const nttt_match_args* a, void* stream) {
                            a->counts + 0, sel, a->counts + 1, L.nms_ws, L.nms_ws_bytes, a->iou_thr, a->filter_iou, s));
   // a12/a9
   bool wrote_t = false;  // the resize also left the word-column-major copy of the packed masks (v2 path only)
-  NTTT_STEP(launch_upsample_pack(ux, uy, a->logits, L.bits_lr, L.box_lr, L.flags, a->lr_h, a->lr_w, sel,
-                                 a->counts + 1, max_sel, a->ori_h, a->ori_w, L.bits_full, L.rect, L.area_full,
-                                 L.box_full, L.scratch, mask_ptr, s, ctx->upsample_stage_floats, ctx->sm_count, L.bits_t,
-                                 &wrote_t, /*t_only=*/true, a->low_latency != 0, ios_pair_counters(L.ios_ws, max_sel)));
+  if (sized) {
+    // (a range that also takes the general resize keeps the row-major layout on both paths)
+    wrote_t = !atlas->any_general;
+    NTTT_STEP(launch_upsample_pack_sized(sd, *atlas, a->logits, L.bits_lr, L.box_lr, L.flags, a->lr_h, a->lr_w, sel,
+                                         a->counts + 1, max_sel, L.bits_full, L.rect, L.area_full, L.box_full, L.scratch,
+                                         mask_ptr, s, ctx->upsample_stage_floats, ctx->sm_count, L.bits_t,
+                                         a->low_latency != 0, wrote_t ? ios_pair_counters(L.ios_ws, max_sel) : nullptr));
+  } else {
+    NTTT_STEP(launch_upsample_pack(ux, uy, a->logits, L.bits_lr, L.box_lr, L.flags, a->lr_h, a->lr_w, sel,
+                                   a->counts + 1, max_sel, a->ori_h, a->ori_w, L.bits_full, L.rect, L.area_full,
+                                   L.box_full, L.scratch, mask_ptr, s, ctx->upsample_stage_floats, ctx->sm_count, L.bits_t,
+                                   &wrote_t, /*t_only=*/true, a->low_latency != 0, ios_pair_counters(L.ios_ws, max_sel)));
+  }
   // the packed full-resolution masks from here on: word-column major when the v2 resize ran, row-major otherwise
   const uint32_t* packed = wrote_t ? L.bits_t : L.bits_full;
   // a13
   NTTT_STEP(launch_mask_ios(L.bits_full, L.rect, L.area_full, L.box_full, sel, a->counts + 1, max_sel, a->ori_h,
                             a->ori_w, L.top_label, obj_feats, a->c, ios, a->ios_inter, L.ios_ws, false, s,
-                            wrote_t ? L.bits_t : nullptr, /*counters_zeroed=*/wrote_t && a->low_latency != 0));  // (folding the metadata
+                            wrote_t ? L.bits_t : nullptr, /*counters_zeroed=*/wrote_t && a->low_latency != 0, sized));  // (folding the metadata
   // kernel into the pair kernel takes 1 us off a single image's chain and costs 0.3 us/image with images in flight)
   // a14
   NTTT_STEP(launch_decay_rank(L.top_score, L.top_label, ios, sel, a->counts + 1, max_sel, num_out, L.box_full,
@@ -904,21 +971,28 @@ int nttt_match_image(nttt_ctx* ctx, const nttt_match_args* a, void* stream) {
     NTTT_MARK();  // RLE-only output: the dense bool masks are never produced
   else if (a->out_prev_rect)
     NTTT_STEP(launch_unpack_sparse(packed, L.rect, L.out_slot, a->counts + 2, num_out, a->ori_h, a->ori_w,
-                                   a->out_masks, a->out_prev_rect, s, wrote_t));
+                                   a->out_masks, a->out_prev_rect, s, wrote_t, sized));
   else
     NTTT_STEP(launch_unpack(packed, L.rect, L.out_slot, a->counts + 2, num_out, a->ori_h, a->ori_w, a->out_masks,
-                            s, wrote_t));
+                            s, wrote_t, sized));
   // §8f rank 1: COCO RLE of the outputs straight from the packed words
   if (want_rle)
     NTTT_STEP(launch_rle_encode(packed, L.rect, L.out_slot, a->counts + 2, num_out, a->ori_h, a->ori_w,
                                 a->rle_cap_counts, a->rle_cap_chars, a->rle_counts, a->rle_n_counts, a->rle_chars,
-                                a->rle_n_chars, s, wrote_t));
+                                a->rle_n_chars, s, wrote_t, sized));
   else
     NTTT_MARK();
 #undef NTTT_STEP
 #undef NTTT_STOP_CHECK
 #undef NTTT_MARK
   return NTTT_OK;
+}
+
+int nttt_match_image(nttt_ctx* ctx, const nttt_match_args* a, void* stream) { return match_impl(ctx, a, nullptr, stream); }
+
+int nttt_match_image_sized(nttt_ctx* ctx, const nttt_match_args* a, const nttt_match_size_range* range, void* stream) {
+  if (!range) return NTTT_EINVAL;
+  return match_impl(ctx, a, range, stream);
 }
 
 }  // extern "C"

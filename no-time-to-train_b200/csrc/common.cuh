@@ -173,6 +173,53 @@ struct ChunkTable {
 int build_axis_table(AxisTable& t, int in_size, int out_size, cudaStream_t s);
 void free_axis_table(AxisTable& t);
 
+// ---------------------------------------------------------------------------------------------------
+// Sized entry (nttt_match_image_sized): the output size is read from device memory when the kernels run, within a range
+// [min, capacity] fixed when the call is enqueued.  The resize tables of every size of the range come from an ATLAS,
+// built once per (low-res size, range) and owned by the context: one slab holding, per axis and output size, the
+// AxisTable arrays the resize reads (no scatter view), and a device index of SizedAxis records.
+// ---------------------------------------------------------------------------------------------------
+struct SizedAxis {  // one output size of one axis
+  const int32_t* xmin; const int32_t* xsize; const float* w;
+  const int32_t* t_lo; const int32_t* t_len; const int32_t* grp_of; const int32_t* grp_start;
+  const uint32_t* pk_span; const float2* pk_w;  // nullptr: the size takes the general resize path on this axis
+  int taps;
+  int budget;  // this axis's factor of the two-tap resize's logit tile budget (up2_tile_factor)
+};
+// by-value kernel argument of the sized kernels
+struct SizedDims {
+  const int32_t* hw;      // [2] (h, w), device
+  const SizedAxis* ay;    // [cap_h - min_h + 1] output heights
+  const SizedAxis* ax;    // [cap_w - min_w + 1] output widths
+  int32_t* counts;        // nttt_match_args.counts: [1] emptied and [3] (status) written by the resize
+  int min_h, min_w, cap_h, cap_w;
+};
+struct SizedAtlas {
+  int lr_h = 0, lr_w = 0, min_h = 0, min_w = 0, cap_h = 0, cap_w = 0;
+  char* slab = nullptr;
+  size_t bytes = 0;
+  double build_ms = 0.0;  // host time of the build, behind its one stream synchronisation
+  SizedAxis* ay = nullptr;  // device index (inside the slab)
+  SizedAxis* ax = nullptr;
+  bool any_two_tap = false;  // some size of the range takes the two-tap resize on both axes
+  bool any_general = false;  // some size takes the general resize
+  long max_budget = 0;       // the largest tile budget over the range (sizes the two-tap resize's shared memory)
+};
+int build_sized_atlas(SizedAtlas& a, cudaStream_t s);  // a: sizes set; fills the rest (one synchronisation)
+long up2_tile_factor(int in_size, int out_size, bool rows);
+
+#ifdef __CUDACC__
+// (h, w) of this call; a size outside the range reads as the capacity and returns false
+__device__ __forceinline__ bool sized_hw(const SizedDims& d, int& h, int& w) {
+  h = d.hw[0];
+  w = d.hw[1];
+  if (h >= d.min_h && h <= d.cap_h && w >= d.min_w && w <= d.cap_w) return true;
+  h = d.cap_h;
+  w = d.cap_w;
+  return false;
+}
+#endif
+
 }  // namespace nttt
 
 struct nttt_ctx {
@@ -220,4 +267,11 @@ struct nttt_ctx {
   }
   // returns the table BY VALUE (device pointers stay valid until evicted by a later call)
   int axis(int in_size, int out_size, cudaStream_t s, nttt::AxisTable* out);
+  // atlases of the sized entry, one per (low-res size, range); kept until the context is destroyed (graphs captured
+  // with one keep reading it)
+  static constexpr int kMaxAtlases = 16;
+  nttt::SizedAtlas atlases[kMaxAtlases];
+  int n_atlases = 0;
+  int sized_atlas(int lr_h, int lr_w, int min_h, int min_w, int cap_h, int cap_w, cudaStream_t s,
+                  const nttt::SizedAtlas** out);
 };

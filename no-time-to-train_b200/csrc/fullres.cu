@@ -56,12 +56,32 @@ struct alignas(16) UpMeta {  // 48 bytes: three 128-bit loads
   int g0, g1;           // row groups [g0, g1) covering [r0, r1)
 };
 
-__global__ void __launch_bounds__(256)
-upsample_meta_kernel(const uint32_t* __restrict__ bits_lr, const int32_t* __restrict__ box_lr,
-                     const int32_t* __restrict__ flags_lr, int ih, int iw, const int32_t* __restrict__ sel,
-                     const int32_t* __restrict__ n_sel, int max_sel, UpTables t, UpMeta* __restrict__ meta,
-                     int32_t* __restrict__ rect, int32_t* __restrict__ scratch, const float* __restrict__ logits,
-                     const float* const* __restrict__ mask_ptr) {
+// Sized entry (nttt_match_image_sized): the output size (h, w) is read from device memory when the kernel runs and the
+// tables come from the context's atlas entry of that size.  The first kernel of each resize chain also writes the status
+// (counts[3]) and, for a size outside the range, empties the selection (counts[1] = 0) so that every later kernel sees
+// no work.  A chain whose path (two-tap or general) the size does not take exits here, as does every resize kernel for a
+// size outside the range.
+__device__ __forceinline__ bool sized_tables(const SizedDims& d, bool two_tap, bool status, int& oh, int& ow,
+                                             UpTables& t) {
+  const bool in_range = sized_hw(d, oh, ow);
+  if (status && blockIdx.x == 0 && blockIdx.y == 0 && threadIdx.x == 0) {
+    d.counts[3] = in_range ? 0 : 1;
+    if (!in_range) d.counts[1] = 0;
+  }
+  if (!in_range) return false;
+  const SizedAxis y = d.ay[oh - d.min_h], x = d.ax[ow - d.min_w];
+  if ((x.pk_span != nullptr && y.pk_span != nullptr) != two_tap) return false;
+  t = UpTables{x.xmin, x.xsize, x.w, x.taps, y.xmin, y.xsize, y.w, y.taps, x.t_lo, x.t_len, y.t_lo, y.t_len,
+               y.grp_of, y.grp_start, x.pk_span, x.pk_w, y.pk_span, y.pk_w};
+  return true;
+}
+
+__device__ __forceinline__ void
+upsample_meta_body(const uint32_t* __restrict__ bits_lr, const int32_t* __restrict__ box_lr,
+                   const int32_t* __restrict__ flags_lr, int ih, int iw, const int32_t* __restrict__ sel,
+                   const int32_t* __restrict__ n_sel, int max_sel, const UpTables& t, UpMeta* __restrict__ meta,
+                   int32_t* __restrict__ rect, int32_t* __restrict__ scratch, const float* __restrict__ logits,
+                   const float* const* __restrict__ mask_ptr) {
   const int k = blockIdx.x * blockDim.x + threadIdx.x;
   if (k >= max_sel) return;
 #pragma unroll
@@ -93,6 +113,27 @@ upsample_meta_kernel(const uint32_t* __restrict__ bits_lr, const int32_t* __rest
   reinterpret_cast<int4*>(rect)[k] = make_int4(m.r0, m.r1, m.w0, m.w1);
 }
 
+__global__ void __launch_bounds__(256)
+upsample_meta_kernel(const uint32_t* __restrict__ bits_lr, const int32_t* __restrict__ box_lr,
+                     const int32_t* __restrict__ flags_lr, int ih, int iw, const int32_t* __restrict__ sel,
+                     const int32_t* __restrict__ n_sel, int max_sel, UpTables t, UpMeta* __restrict__ meta,
+                     int32_t* __restrict__ rect, int32_t* __restrict__ scratch, const float* __restrict__ logits,
+                     const float* const* __restrict__ mask_ptr) {
+  upsample_meta_body(bits_lr, box_lr, flags_lr, ih, iw, sel, n_sel, max_sel, t, meta, rect, scratch, logits, mask_ptr);
+}
+
+__global__ void __launch_bounds__(256)
+upsample_meta_sized_kernel(const uint32_t* __restrict__ bits_lr, const int32_t* __restrict__ box_lr,
+                           const int32_t* __restrict__ flags_lr, int ih, int iw, const int32_t* __restrict__ sel,
+                           const int32_t* __restrict__ n_sel, int max_sel, UpMeta* __restrict__ meta,
+                           int32_t* __restrict__ rect, int32_t* __restrict__ scratch, const float* __restrict__ logits,
+                           const float* const* __restrict__ mask_ptr, SizedDims d) {
+  int oh, ow;
+  UpTables t;
+  if (!sized_tables(d, false, true, oh, ow, t)) return;
+  upsample_meta_body(bits_lr, box_lr, flags_lr, ih, iw, sel, n_sel, max_sel, t, meta, rect, scratch, logits, mask_ptr);
+}
+
 __device__ __forceinline__ int up_ctas_needed(int n_groups) {
   return max(1, min(kUpMaxSplit, (n_groups + kUpGroupsPerCta - 1) / kUpGroupsPerCta));
 }
@@ -119,11 +160,11 @@ __device__ __forceinline__ void cp_async16(void* smem_dst, const void* gmem_src)
 }
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
 
-__global__ void __launch_bounds__(kUpThreads, 5)
-upsample_pack_kernel(const uint32_t* __restrict__ bits_lr, const UpMeta* __restrict__ meta, int ih, int iw,
-                     const int32_t* __restrict__ n_sel, int max_sel, int oh, int ow, UpTables t,
-                     uint32_t* __restrict__ bits_full, int32_t* __restrict__ area_full, int32_t* __restrict__ box_full,
-                     int32_t* __restrict__ scratch, int stage_floats) {
+__device__ __forceinline__ void
+upsample_pack_body(const uint32_t* __restrict__ bits_lr, const UpMeta* __restrict__ meta, int ih, int iw,
+                   const int32_t* __restrict__ n_sel, int max_sel, int oh, int ow, const UpTables& t,
+                   uint32_t* __restrict__ bits_full, int32_t* __restrict__ area_full, int32_t* __restrict__ box_full,
+                   int32_t* __restrict__ scratch, int stage_floats) {
   extern __shared__ __align__(16) uint32_t s_lr[];  // packed low-res bits of this mask, rows [clr0, clr1) only; then the tile
   __shared__ int s_red[5];
   const int k = blockIdx.y;
@@ -401,6 +442,27 @@ upsample_pack_kernel(const uint32_t* __restrict__ bits_lr, const UpMeta* __restr
   }
 }
 
+__global__ void __launch_bounds__(kUpThreads, 5)
+upsample_pack_kernel(const uint32_t* __restrict__ bits_lr, const UpMeta* __restrict__ meta, int ih, int iw,
+                     const int32_t* __restrict__ n_sel, int max_sel, int oh, int ow, UpTables t,
+                     uint32_t* __restrict__ bits_full, int32_t* __restrict__ area_full, int32_t* __restrict__ box_full,
+                     int32_t* __restrict__ scratch, int stage_floats) {
+  upsample_pack_body(bits_lr, meta, ih, iw, n_sel, max_sel, oh, ow, t, bits_full, area_full, box_full, scratch,
+                     stage_floats);
+}
+
+__global__ void __launch_bounds__(kUpThreads, 5)
+upsample_pack_sized_kernel(const uint32_t* __restrict__ bits_lr, const UpMeta* __restrict__ meta, int ih, int iw,
+                           const int32_t* __restrict__ n_sel, int max_sel, uint32_t* __restrict__ bits_full,
+                           int32_t* __restrict__ area_full, int32_t* __restrict__ box_full,
+                           int32_t* __restrict__ scratch, int stage_floats, SizedDims d) {
+  int oh, ow;
+  UpTables t;
+  if (!sized_tables(d, false, false, oh, ow, t)) return;
+  upsample_pack_body(bits_lr, meta, ih, iw, n_sel, max_sel, oh, ow, t, bits_full, area_full, box_full, scratch,
+                     stage_floats);
+}
+
 // ---------------------------------------------------------------------------------------------------
 // v2 — the path every two-tap configuration takes (every span of both axes <= 2 samples: up-scaling, see
 // aa_spans_within_two)
@@ -447,14 +509,13 @@ struct alignas(16) Up2Item {  // 32 bytes, written by the plan kernel
 constexpr int kPlanThreads = 256;
 constexpr int kPlanPerThread = 1024 / kPlanThreads;
 
-__global__ void __launch_bounds__(kPlanThreads)
-upsample_plan_kernel(const uint32_t* __restrict__ bits_lr, const int32_t* __restrict__ box_lr,
-                     const int32_t* __restrict__ flags_lr, int ih, int iw, const int32_t* __restrict__ sel,
-                     const int32_t* __restrict__ n_sel, int max_sel, UpTables t, UpMeta* __restrict__ meta,
-                     int32_t* __restrict__ rect, int32_t* __restrict__ scratch, const float* __restrict__ logits,
-                     const float* const* __restrict__ mask_ptr, Up2Item* __restrict__ items, int32_t* __restrict__ ctr,
-                     int32_t* __restrict__ area_full, int32_t* __restrict__ box_full, int oh, int ow, int tile_cap_floats) {
-  chain_wait();
+__device__ __forceinline__ void
+upsample_plan_body(const uint32_t* __restrict__ bits_lr, const int32_t* __restrict__ box_lr,
+                   const int32_t* __restrict__ flags_lr, int ih, int iw, const int32_t* __restrict__ sel,
+                   const int32_t* __restrict__ n_sel, int max_sel, const UpTables& t, UpMeta* __restrict__ meta,
+                   int32_t* __restrict__ rect, int32_t* __restrict__ scratch, const float* __restrict__ logits,
+                   const float* const* __restrict__ mask_ptr, Up2Item* __restrict__ items, int32_t* __restrict__ ctr,
+                   int32_t* __restrict__ area_full, int32_t* __restrict__ box_full, int oh, int ow, int tile_cap_floats) {
   __shared__ int s_warp[kPlanThreads / 32 + 1];
   __shared__ int s_off[1024];   // exclusive item offset of each mask of the strip
   __shared__ int s_ccs[1024];   // column chunks of each mask (0: no items)
@@ -596,6 +657,39 @@ upsample_plan_kernel(const uint32_t* __restrict__ bits_lr, const int32_t* __rest
   if (blockIdx.x == 0 && tid == 0) { ctr[0] = base; ctr[1] = 0; }
 }
 
+__global__ void __launch_bounds__(kPlanThreads)
+upsample_plan_kernel(const uint32_t* __restrict__ bits_lr, const int32_t* __restrict__ box_lr,
+                     const int32_t* __restrict__ flags_lr, int ih, int iw, const int32_t* __restrict__ sel,
+                     const int32_t* __restrict__ n_sel, int max_sel, UpTables t, UpMeta* __restrict__ meta,
+                     int32_t* __restrict__ rect, int32_t* __restrict__ scratch, const float* __restrict__ logits,
+                     const float* const* __restrict__ mask_ptr, Up2Item* __restrict__ items, int32_t* __restrict__ ctr,
+                     int32_t* __restrict__ area_full, int32_t* __restrict__ box_full, int oh, int ow, int tile_cap_floats) {
+  chain_wait();
+  upsample_plan_body(bits_lr, box_lr, flags_lr, ih, iw, sel, n_sel, max_sel, t, meta, rect, scratch, logits, mask_ptr,
+                     items, ctr, area_full, box_full, oh, ow, tile_cap_floats);
+}
+
+// stage_floats: the context's staging budget; the tile budget of the size is derived from it as launch_upsample_pack does
+__global__ void __launch_bounds__(kPlanThreads)
+upsample_plan_sized_kernel(const uint32_t* __restrict__ bits_lr, const int32_t* __restrict__ box_lr,
+                           const int32_t* __restrict__ flags_lr, int ih, int iw, const int32_t* __restrict__ sel,
+                           const int32_t* __restrict__ n_sel, int max_sel, UpMeta* __restrict__ meta,
+                           int32_t* __restrict__ rect, int32_t* __restrict__ scratch, const float* __restrict__ logits,
+                           const float* const* __restrict__ mask_ptr, Up2Item* __restrict__ items,
+                           int32_t* __restrict__ ctr, int32_t* __restrict__ area_full, int32_t* __restrict__ box_full,
+                           int stage_floats, bool status, SizedDims d) {
+  chain_wait();
+  int oh, ow;
+  UpTables t;
+  if (!sized_tables(d, true, status, oh, ow, t)) return;
+  const long need = (long)d.ay[oh - d.min_h].budget * (long)d.ax[ow - d.min_w].budget;
+  int tile_floats = (int)(need < stage_floats ? need : stage_floats);
+  if (tile_floats < 0) tile_floats = 0;
+  tile_floats = (tile_floats + 3) & ~3;
+  upsample_plan_body(bits_lr, box_lr, flags_lr, ih, iw, sel, n_sel, max_sel, t, meta, rect, scratch, logits, mask_ptr,
+                     items, ctr, area_full, box_full, oh, ow, tile_floats);
+}
+
 // 16-byte copy that allocates in L1: the two-tap records are a few KB shared by every item an SM processes
 __device__ __forceinline__ void cp_async16_ca(void* smem_dst, const void* gmem_src) {
   const uint32_t d = (uint32_t)__cvta_generic_to_shared(smem_dst);
@@ -699,14 +793,11 @@ __device__ __forceinline__ void up2_publish(int k, const int (&red)[5], int32_t*
   }
 }
 
-__global__ void __launch_bounds__(kUp2Threads, kUp2CtasPerSm)
-upsample_pack2_kernel(const uint32_t* __restrict__ bits_lr, const UpMeta* __restrict__ meta, int ih, int iw, int oh,
-                      int ow, UpTables t, uint32_t* __restrict__ bits_full, uint32_t* __restrict__ bits_t,
-                      int32_t* __restrict__ area_full, int32_t* __restrict__ box_full, int32_t* __restrict__ scratch,
-                      const Up2Item* __restrict__ items, int32_t* __restrict__ ctr, int32_t* __restrict__ zero2) {
-  chain_wait();
-  // (nullable) two counters of the NEXT stage, zeroed here so that its first kernel can append to them right away
-  if (zero2 && blockIdx.x == 0 && threadIdx.x == 0) { zero2[0] = 0; zero2[1] = 0; }
+__device__ __forceinline__ void
+upsample_pack2_body(const uint32_t* __restrict__ bits_lr, const UpMeta* __restrict__ meta, int ih, int iw, int oh,
+                    int ow, const UpTables& t, uint32_t* __restrict__ bits_full, uint32_t* __restrict__ bits_t,
+                    int32_t* __restrict__ area_full, int32_t* __restrict__ box_full, int32_t* __restrict__ scratch,
+                    const Up2Item* __restrict__ items, int32_t* __restrict__ ctr) {
   extern __shared__ __align__(16) unsigned char s_raw[];
   // two-tap records of the item's columns and rows; the rows from ya0 rounded down to a multiple of 4 (16-byte copies)
   float2* s_xw = reinterpret_cast<float2*>(s_raw);                        // [kUp2Cols * 32]
@@ -944,6 +1035,31 @@ upsample_pack2_kernel(const uint32_t* __restrict__ bits_lr, const UpMeta* __rest
   if (tid == 0 && pend_k >= 0) up2_publish(pend_k, pend, scratch, area_full, box_full);
 }
 
+__global__ void __launch_bounds__(kUp2Threads, kUp2CtasPerSm)
+upsample_pack2_kernel(const uint32_t* __restrict__ bits_lr, const UpMeta* __restrict__ meta, int ih, int iw, int oh,
+                      int ow, UpTables t, uint32_t* __restrict__ bits_full, uint32_t* __restrict__ bits_t,
+                      int32_t* __restrict__ area_full, int32_t* __restrict__ box_full, int32_t* __restrict__ scratch,
+                      const Up2Item* __restrict__ items, int32_t* __restrict__ ctr, int32_t* __restrict__ zero2) {
+  chain_wait();
+  // (nullable) two counters of the NEXT stage, zeroed here so that its first kernel can append to them right away
+  if (zero2 && blockIdx.x == 0 && threadIdx.x == 0) { zero2[0] = 0; zero2[1] = 0; }
+  upsample_pack2_body(bits_lr, meta, ih, iw, oh, ow, t, bits_full, bits_t, area_full, box_full, scratch, items, ctr);
+}
+
+__global__ void __launch_bounds__(kUp2Threads, kUp2CtasPerSm)
+upsample_pack2_sized_kernel(const uint32_t* __restrict__ bits_lr, const UpMeta* __restrict__ meta, int ih, int iw,
+                            uint32_t* __restrict__ bits_full, uint32_t* __restrict__ bits_t,
+                            int32_t* __restrict__ area_full, int32_t* __restrict__ box_full,
+                            int32_t* __restrict__ scratch, const Up2Item* __restrict__ items, int32_t* __restrict__ ctr,
+                            int32_t* __restrict__ zero2, SizedDims d) {
+  chain_wait();
+  if (zero2 && blockIdx.x == 0 && threadIdx.x == 0) { zero2[0] = 0; zero2[1] = 0; }  // (also for a size out of range)
+  int oh, ow;
+  UpTables t;
+  if (!sized_tables(d, true, false, oh, ow, t)) return;
+  upsample_pack2_body(bits_lr, meta, ih, iw, oh, ow, t, bits_full, bits_t, area_full, box_full, scratch, items, ctr);
+}
+
 // shared-memory layout of upsample_pack2_kernel in bytes, without / with a logit tile of `tile_floats`
 static size_t up2_fixed_smem(int ih, int iw) {
   const size_t lr_words = (((size_t)ih * (iw / 32) + 4) + 3) & ~(size_t)3;
@@ -954,6 +1070,13 @@ static size_t up2_fixed_smem(int ih, int iw) {
 // items a selection can expand to: every mask at most ceil(groups / 32) x ceil(words / 8), groups <= output rows
 static size_t up2_max_items(int max_sel, int oh, int ow) {
   return (size_t)max_sel * ((oh + kUp2Groups - 1) / kUp2Groups) * ((((ow + 31) / 32) + kUp2Cols - 1) / kUp2Cols);
+}
+
+// one axis's factor of the v2 tile budget: the input rows (columns) an item of kUp2Rows rows (kUp2Cols words) spans at
+// this scale, plus slack
+long up2_tile_factor(int in_size, int out_size, bool rows) {
+  const double sc = (double)in_size / out_size;
+  return rows ? (long)((kUp2Rows * sc + 6)) : (long)(((kUp2Cols * 32) * sc + 12));
 }
 
 int launch_upsample_pack(const AxisTable& tx, const AxisTable& ty, const float* logits, const uint32_t* bits_lr,
@@ -975,8 +1098,7 @@ int launch_upsample_pack(const AxisTable& tx, const AxisTable& ty, const float* 
     int32_t* ctr = reinterpret_cast<int32_t*>(meta + max_sel);
     Up2Item* items = reinterpret_cast<Up2Item*>(ctr + 4);
     // tile budget: what an item of 32 groups x 8 words needs at this scale (+ slack), bounded by `stage_floats`
-    const double sy = (double)ih / oh, sx = (double)iw / ow;
-    long need = (long)((kUp2Rows * sy + 6)) * (long)(((kUp2Cols * 32) * sx + 12));
+    long need = up2_tile_factor(ih, oh, true) * up2_tile_factor(iw, ow, false);
     int tile_floats = (int)(need < stage_floats ? need : stage_floats);
     if (tile_floats < 0) tile_floats = 0;
     tile_floats = (tile_floats + 3) & ~3;
@@ -1016,6 +1138,54 @@ int launch_upsample_pack(const AxisTable& tx, const AxisTable& ty, const float* 
   NTTT_LAUNCH_CHECK();
   return NTTT_OK;
 }
+// The resize of the sized entry: launch shapes and shared memory from the capacity (and the worst tile budget of the
+// range); each kernel reads the size and its tables when it runs.  Sizes of the range that take the general path
+// (an axis reaching below the low-res size, see aa_spans_within_two) enqueue its chain as well, and the chain the
+// size does not select exits at its first instruction.  With both chains the two-tap one writes the row-major words
+// too (bits_t is then nullptr): the consumers read one layout whichever chain ran.
+int launch_upsample_pack_sized(const SizedDims& d, const SizedAtlas& A, const float* logits, const uint32_t* bits_lr,
+                               const int32_t* box_lr, const int32_t* flags_lr, int ih, int iw, const int32_t* sel,
+                               const int32_t* n_sel, int max_sel, uint32_t* bits_full, int32_t* rect, int32_t* area_full,
+                               int32_t* box_full, int32_t* scratch, const float* const* mask_ptr, cudaStream_t s,
+                               int stage_floats, int sm_count, uint32_t* bits_t, bool low_latency, int32_t* zero2) {
+  if (max_sel <= 0) return NTTT_OK;
+  if (iw % 32 != 0 || d.cap_h >= 65536 || d.cap_w >= 65536) return NTTT_EUNSUPPORTED;
+  UpMeta* meta = reinterpret_cast<UpMeta*>(scratch + (size_t)kScratchInts * max_sel);
+  if (A.any_general) {
+    const size_t bits_bytes = ((((size_t)ih * (iw / 32) + 1) + 3) & ~(size_t)3) * 4;
+    if (bits_bytes > 160 * 1024) return NTTT_EUNSUPPORTED;
+    size_t stage_bytes = (size_t)(stage_floats > 0 ? stage_floats : 0) * 4;
+    if (bits_bytes + stage_bytes > 200 * 1024) stage_bytes = 0;
+    const size_t smem = bits_bytes + stage_bytes;
+    if (smem > 48 * 1024) NTTT_CUDA(set_dyn_smem(upsample_pack_sized_kernel, (int)smem));
+    upsample_meta_sized_kernel<<<ceil_div(max_sel, 256), 256, 0, s>>>(bits_lr, box_lr, flags_lr, ih, iw, sel, n_sel,
+                                                                      max_sel, meta, rect, scratch, logits, mask_ptr, d);
+    NTTT_LAUNCH_CHECK();
+    upsample_pack_sized_kernel<<<dim3(kUpMaxSplit, max_sel), kUpThreads, smem, s>>>(
+        bits_lr, meta, ih, iw, n_sel, max_sel, bits_full, area_full, box_full, scratch, (int)(stage_bytes / 4), d);
+    NTTT_LAUNCH_CHECK();
+  }
+  if (!A.any_two_tap) return NTTT_OK;
+  if (ih * (iw / 32) > 16384) return NTTT_EUNSUPPORTED;
+  int32_t* ctr = reinterpret_cast<int32_t*>(meta + max_sel);
+  Up2Item* items = reinterpret_cast<Up2Item*>(ctr + 4);
+  int tile_floats = (int)(A.max_budget < stage_floats ? A.max_budget : stage_floats);
+  if (tile_floats < 0) tile_floats = 0;
+  tile_floats = (tile_floats + 3) & ~3;
+  const size_t smem = up2_fixed_smem(ih, iw) + (size_t)tile_floats * 4;
+  if (smem > 200 * 1024) return NTTT_EUNSUPPORTED;
+  launch_chain(upsample_plan_sized_kernel, 8, kPlanThreads, 0, s, bits_lr, box_lr, flags_lr, ih, iw, sel, n_sel, max_sel,
+               meta, rect, scratch, logits, mask_ptr, items, ctr, area_full, box_full, stage_floats, !A.any_general, d);
+  NTTT_LAUNCH_CHECK();
+  if (smem > 48 * 1024) NTTT_CUDA(set_dyn_smem(upsample_pack2_sized_kernel, (int)smem));
+  const int grid = (sm_count > 0 ? sm_count : 148) * (low_latency ? kUp2CtasPerSm : 1);
+  launch_chain(upsample_pack2_sized_kernel, grid, kUp2Threads, smem, s, bits_lr, meta, ih, iw,
+               A.any_general ? bits_full : nullptr, A.any_general ? nullptr : bits_t, area_full, box_full, scratch,
+               items, ctr, zero2, d);
+  NTTT_LAUNCH_CHECK();
+  return NTTT_OK;
+}
+
 size_t upsample_scratch_bytes(int max_sel, int oh, int ow) {
   return (sizeof(int32_t) * kScratchInts + sizeof(UpMeta)) * (size_t)max_sel + 16 +
          sizeof(Up2Item) * up2_max_items(max_sel, oh, ow);
@@ -1031,20 +1201,23 @@ __device__ __forceinline__ uint32_t nibble_to_bytes(uint32_t nb) { return (nb * 
 constexpr int kUnpackRows = 32;   // output rows per CTA
 constexpr int kUnpackUnroll = 4;  // words per thread in flight
 
-__global__ void __launch_bounds__(256)
-unpack_masks_kernel(const uint32_t* __restrict__ bits_full, const int32_t* __restrict__ rect,
-                    const int32_t* __restrict__ index, const int32_t* __restrict__ count, int max_count, int oh, int ow,
-                    uint8_t* __restrict__ out, bool tr /* packed words are [word][row] instead of [row][word] */) {
+// (oh, ow): the size of the packed masks; output plane j starts at out + j * oplane, rows are ostride bytes apart and
+// bytes up to ostride may be written (the pad bits of the last word are zero).  The static entry passes
+// ostride = ow, oplane = oh * ow; the sized entry the capacity's strides, and writes the [oh, ow] corner of the plane.
+__device__ __forceinline__ void
+unpack_masks_body(const uint32_t* __restrict__ bits_full, const int32_t* __restrict__ rect,
+                  const int32_t* __restrict__ index, const int32_t* __restrict__ count, int max_count, int oh, int ow,
+                  int ostride, size_t oplane, uint8_t* __restrict__ out, bool tr) {
   const int j = blockIdx.y;
   if (j >= min(*count, max_count)) return;
   const int k = index ? index[j] : j;
   const int ow_words = (ow + 31) >> 5;
   const int4 rc = reinterpret_cast<const int4*>(rect)[k];
   const uint32_t* src = bits_full + (size_t)k * oh * ow_words;
-  uint8_t* dst = out + (size_t)j * oh * ow;
+  uint8_t* dst = out + (size_t)j * oplane;
   const int y0 = blockIdx.x * kUnpackRows;
   const int rows = min(kUnpackRows, oh - y0);
-  const bool vec = (ow & 15) == 0;  // every 16-pixel half word starts 16-byte aligned
+  const bool vec = (ostride & 15) == 0;  // every 16-pixel half word starts 16-byte aligned
   const int total = rows * ow_words;
   for (int base = 0; base < total; base += 256 * kUnpackUnroll) {
     uint32_t word[kUnpackUnroll];
@@ -1065,18 +1238,34 @@ unpack_masks_kernel(const uint32_t* __restrict__ bits_full, const int32_t* __res
       if (it >= total) continue;
       const int x = ww[u] << 5;
       const uint32_t w = word[u];
-      uint8_t* p = dst + (size_t)yy[u] * ow + x;
+      uint8_t* p = dst + (size_t)yy[u] * ostride + x;
       if (vec) {
         *reinterpret_cast<uint4*>(p) = make_uint4(nibble_to_bytes(w & 15u), nibble_to_bytes((w >> 4) & 15u),
                                                    nibble_to_bytes((w >> 8) & 15u), nibble_to_bytes((w >> 12) & 15u));
-        if (x + 16 < ow)
+        if (x + 16 < ostride)
           *reinterpret_cast<uint4*>(p + 16) = make_uint4(nibble_to_bytes((w >> 16) & 15u), nibble_to_bytes((w >> 20) & 15u),
                                                         nibble_to_bytes((w >> 24) & 15u), nibble_to_bytes(w >> 28));
       } else {
-        for (int q = 0; q < 32 && x + q < ow; ++q) p[q] = (w >> q) & 1u;
+        for (int q = 0; q < 32 && x + q < ostride; ++q) p[q] = (w >> q) & 1u;
       }
     }
   }
+}
+
+__global__ void __launch_bounds__(256)
+unpack_masks_kernel(const uint32_t* __restrict__ bits_full, const int32_t* __restrict__ rect,
+                    const int32_t* __restrict__ index, const int32_t* __restrict__ count, int max_count, int oh, int ow,
+                    uint8_t* __restrict__ out, bool tr /* packed words are [word][row] instead of [row][word] */) {
+  unpack_masks_body(bits_full, rect, index, count, max_count, oh, ow, ow, (size_t)oh * ow, out, tr);
+}
+
+__global__ void __launch_bounds__(256)
+unpack_masks_sized_kernel(const uint32_t* __restrict__ bits_full, const int32_t* __restrict__ rect,
+                          const int32_t* __restrict__ index, const int32_t* __restrict__ count, int max_count,
+                          uint8_t* __restrict__ out, bool tr, SizedDims d) {
+  int oh, ow;
+  sized_hw(d, oh, ow);  // (out of range: the count is zero)
+  unpack_masks_body(bits_full, rect, index, count, max_count, oh, ow, d.cap_w, (size_t)d.cap_h * d.cap_w, out, tr);
 }
 
 // Sparse unpack into PERSISTENT output buffers: out[j] still holds the mask the previous call wrote there, whose
@@ -1085,11 +1274,12 @@ unpack_masks_kernel(const uint32_t* __restrict__ bits_full, const int32_t* __res
 // area(old \ new) + area(new) bytes per mask whatever the distance between the two rects (never their common bounding
 // box, and never oh*ow: the dense unpack is HBM-write-bound on mostly zeros).  Every slot up to max_count is visited
 // so that slots that fall out of use are cleared.
-__global__ void __launch_bounds__(256)
-unpack_sparse_kernel(const uint32_t* __restrict__ bits_full, const int32_t* __restrict__ rect,
-                     const int32_t* __restrict__ index, const int32_t* __restrict__ count, int max_count, int oh, int ow,
-                     uint8_t* __restrict__ out, int32_t* __restrict__ prev_rect, bool tr) {
-  chain_wait();
+// (oh, ow), ostride, oplane: as in unpack_masks_body.  The sized entry's rects of earlier, larger images are cleared up
+// to the capacity's row length, so the whole buffer stays the dense result embedded top-left with zeros elsewhere.
+__device__ __forceinline__ void
+unpack_sparse_body(const uint32_t* __restrict__ bits_full, const int32_t* __restrict__ rect,
+                   const int32_t* __restrict__ index, const int32_t* __restrict__ count, int max_count, int oh, int ow,
+                   int ostride, size_t oplane, uint8_t* __restrict__ out, int32_t* __restrict__ prev_rect, bool tr) {
   const int j = blockIdx.y;
   const int ow_words = (ow + 31) >> 5;
   const bool live = j < min(*count, max_count);
@@ -1105,8 +1295,8 @@ unpack_sparse_kernel(const uint32_t* __restrict__ bits_full, const int32_t* __re
   const int n_old = has_old ? (pr.y - pr.x) * old_w : 0;
   const int total = n_old + (has_new ? (nr.y - nr.x) * new_w : 0);
   const uint32_t* src = bits_full + (size_t)k * oh * ow_words;
-  uint8_t* dst = out + (size_t)j * oh * ow;
-  const bool vec = (ow & 15) == 0;
+  uint8_t* dst = out + (size_t)j * oplane;
+  const bool vec = (ostride & 15) == 0;
   for (int it = blockIdx.x * 256 + threadIdx.x; it < total; it += gridDim.x * 256) {
     int y, wi;
     uint32_t w = 0;
@@ -1123,33 +1313,62 @@ unpack_sparse_kernel(const uint32_t* __restrict__ bits_full, const int32_t* __re
       w = __ldg(tr ? src + (size_t)wi * oh + y : src + (size_t)y * ow_words + wi);
     }
     const int x = wi << 5;
-    uint8_t* p = dst + (size_t)y * ow + x;
+    uint8_t* p = dst + (size_t)y * ostride + x;
     if (vec) {
       *reinterpret_cast<uint4*>(p) = make_uint4(nibble_to_bytes(w & 15u), nibble_to_bytes((w >> 4) & 15u),
                                                  nibble_to_bytes((w >> 8) & 15u), nibble_to_bytes((w >> 12) & 15u));
-      if (x + 16 < ow)
+      if (x + 16 < ostride)
         *reinterpret_cast<uint4*>(p + 16) = make_uint4(nibble_to_bytes((w >> 16) & 15u), nibble_to_bytes((w >> 20) & 15u),
                                                       nibble_to_bytes((w >> 24) & 15u), nibble_to_bytes(w >> 28));
     } else {
-      for (int q = 0; q < 32 && x + q < ow; ++q) p[q] = (w >> q) & 1u;
+      for (int q = 0; q < 32 && x + q < ostride; ++q) p[q] = (w >> q) & 1u;
     }
   }
 }
 
+__global__ void __launch_bounds__(256)
+unpack_sparse_kernel(const uint32_t* __restrict__ bits_full, const int32_t* __restrict__ rect,
+                     const int32_t* __restrict__ index, const int32_t* __restrict__ count, int max_count, int oh, int ow,
+                     uint8_t* __restrict__ out, int32_t* __restrict__ prev_rect, bool tr) {
+  chain_wait();
+  unpack_sparse_body(bits_full, rect, index, count, max_count, oh, ow, ow, (size_t)oh * ow, out, prev_rect, tr);
+}
+
+__global__ void __launch_bounds__(256)
+unpack_sparse_sized_kernel(const uint32_t* __restrict__ bits_full, const int32_t* __restrict__ rect,
+                           const int32_t* __restrict__ index, const int32_t* __restrict__ count, int max_count,
+                           uint8_t* __restrict__ out, int32_t* __restrict__ prev_rect, bool tr, SizedDims d) {
+  chain_wait();
+  int oh, ow;
+  sized_hw(d, oh, ow);  // (out of range: the count is zero and only the previous rects are cleared)
+  unpack_sparse_body(bits_full, rect, index, count, max_count, oh, ow, d.cap_w, (size_t)d.cap_h * d.cap_w, out,
+                     prev_rect, tr);
+}
+
+// sized (nullable): the size is read on the device; oh, ow are then the capacity
 int launch_unpack_sparse(const uint32_t* bits_full, const int32_t* rect, const int32_t* index, const int32_t* count,
-                         int max_count, int oh, int ow, uint8_t* out, int32_t* prev_rect, cudaStream_t s, bool tr) {
+                         int max_count, int oh, int ow, uint8_t* out, int32_t* prev_rect, cudaStream_t s, bool tr,
+                         const SizedDims* sized) {
   if (max_count <= 0) return NTTT_OK;
   dim3 grid(1, max_count);  // one CTA per slot: prev_rect[j] is read and rewritten by the same CTA
-  launch_chain(unpack_sparse_kernel, grid, 256, 0, s, bits_full, rect, index, count, max_count, oh, ow, out, prev_rect, tr);
+  if (sized)
+    launch_chain(unpack_sparse_sized_kernel, grid, 256, 0, s, bits_full, rect, index, count, max_count, out, prev_rect,
+                 tr, *sized);
+  else
+    launch_chain(unpack_sparse_kernel, grid, 256, 0, s, bits_full, rect, index, count, max_count, oh, ow, out, prev_rect,
+                 tr);
   NTTT_LAUNCH_CHECK();
   return NTTT_OK;
 }
 
 int launch_unpack(const uint32_t* bits_full, const int32_t* rect, const int32_t* index, const int32_t* count,
-                  int max_count, int oh, int ow, uint8_t* out, cudaStream_t s, bool tr) {
+                  int max_count, int oh, int ow, uint8_t* out, cudaStream_t s, bool tr, const SizedDims* sized) {
   if (max_count <= 0) return NTTT_OK;
   dim3 grid(ceil_div(oh, kUnpackRows), max_count);
-  unpack_masks_kernel<<<grid, 256, 0, s>>>(bits_full, rect, index, count, max_count, oh, ow, out, tr);
+  if (sized)
+    unpack_masks_sized_kernel<<<grid, 256, 0, s>>>(bits_full, rect, index, count, max_count, out, tr, *sized);
+  else
+    unpack_masks_kernel<<<grid, 256, 0, s>>>(bits_full, rect, index, count, max_count, oh, ow, out, tr);
   NTTT_LAUNCH_CHECK();
   return NTTT_OK;
 }

@@ -8,6 +8,9 @@
 
 #include <algorithm>
 
+#include <chrono>
+#include <vector>
+
 #include "common.cuh"
 
 namespace nttt {
@@ -720,6 +723,7 @@ __global__ void aa_transpose_kernel(int in_size, int out_size, int taps, const i
   const int len = lo < 0 ? 0 : hi - lo + 1;  // true length; t_w only holds the first kMaxScatter weights
   t_lo[e] = max(lo, 0);
   t_len[e] = len;
+  if (!t_w) return;  // (tables of the sized atlas: no scatter view)
   for (int t = 0; t < kMaxScatter; ++t) {
     const int x = lo + t;
     float v = 0.0f;
@@ -783,38 +787,49 @@ static bool aa_spans_within_two(int in_size, int out_size) {
   return true;
 }
 
-// All arrays of a table live in ONE device allocation (`slab`): a table costs one cudaMalloc when a new (in, out) pair is
-// first seen and one cudaFree when it is retired, instead of ten of each.
-int build_axis_table(AxisTable& t, int in_size, int out_size, cudaStream_t s) {
-  t.in_size = in_size;
-  t.out_size = out_size;
-  t.taps = aa_max_taps(in_size, out_size);
-  const bool packed = in_size < 65536 && aa_spans_within_two(in_size, out_size);
+// Byte offsets of a table's arrays inside its slab.  scatter = false leaves out the scatter weights (t_w, t_cum), which
+// only the mask projection reads.
+struct AxisLayout {
+  bool packed;
+  size_t o_xmin, o_xsize, o_w, o_tlo, o_tlen, o_tw, o_tcum, o_gof, o_gst, o_pks, o_pkw, bytes;
+};
+static AxisLayout axis_layout(int in_size, int out_size, bool scatter) {
+  AxisLayout L{};
+  L.packed = in_size < 65536 && aa_spans_within_two(in_size, out_size);
+  const int taps = aa_max_taps(in_size, out_size);
   const int out_pad = (out_size + 31) / 32 * 32;
   size_t off = 0;
   auto take = [&](size_t bytes) { const size_t o = off; off = align_up(off + bytes, 256); return o; };
-  const size_t o_xmin = take(sizeof(int32_t) * out_size), o_xsize = take(sizeof(int32_t) * out_size);
-  const size_t o_w = take(sizeof(float) * (size_t)out_size * t.taps);
-  const size_t o_tlo = take(sizeof(int32_t) * in_size), o_tlen = take(sizeof(int32_t) * in_size);
-  const size_t o_tw = take(sizeof(float) * (size_t)in_size * kMaxScatter);
-  const size_t o_tcum = take(sizeof(float) * (size_t)in_size * (kMaxScatter + 1));
-  const size_t o_gof = take(sizeof(int32_t) * out_size), o_gst = take(sizeof(int32_t) * ((size_t)out_size + 1));
-  const size_t o_pks = packed ? take(sizeof(uint32_t) * (size_t)out_pad) : 0;
-  const size_t o_pkw = packed ? take(sizeof(float2) * (size_t)out_pad) : 0;
-  char* slab = nullptr;
-  NTTT_CUDA(cudaMalloc(&slab, off));
-  t.slab = slab;
-  t.xmin = reinterpret_cast<int32_t*>(slab + o_xmin);
-  t.xsize = reinterpret_cast<int32_t*>(slab + o_xsize);
-  t.w = reinterpret_cast<float*>(slab + o_w);
-  t.t_lo = reinterpret_cast<int32_t*>(slab + o_tlo);
-  t.t_len = reinterpret_cast<int32_t*>(slab + o_tlen);
-  t.t_w = reinterpret_cast<float*>(slab + o_tw);
-  t.t_cum = reinterpret_cast<float*>(slab + o_tcum);
-  t.grp_of = reinterpret_cast<int32_t*>(slab + o_gof);
-  t.grp_start = reinterpret_cast<int32_t*>(slab + o_gst);
-  t.pk_span = packed ? reinterpret_cast<uint32_t*>(slab + o_pks) : nullptr;
-  t.pk_w = packed ? reinterpret_cast<float2*>(slab + o_pkw) : nullptr;
+  L.o_xmin = take(sizeof(int32_t) * out_size);
+  L.o_xsize = take(sizeof(int32_t) * out_size);
+  L.o_w = take(sizeof(float) * (size_t)out_size * taps);
+  L.o_tlo = take(sizeof(int32_t) * in_size);
+  L.o_tlen = take(sizeof(int32_t) * in_size);
+  L.o_tw = scatter ? take(sizeof(float) * (size_t)in_size * kMaxScatter) : 0;
+  L.o_tcum = scatter ? take(sizeof(float) * (size_t)in_size * (kMaxScatter + 1)) : 0;
+  L.o_gof = take(sizeof(int32_t) * out_size);
+  L.o_gst = take(sizeof(int32_t) * ((size_t)out_size + 1));
+  L.o_pks = L.packed ? take(sizeof(uint32_t) * (size_t)out_pad) : 0;
+  L.o_pkw = L.packed ? take(sizeof(float2) * (size_t)out_pad) : 0;
+  L.bytes = off;
+  return L;
+}
+
+// builds the table into `slab` (L.bytes, laid out by axis_layout), stream-ordered
+static int fill_axis_table(AxisTable& t, int in_size, int out_size, const AxisLayout& L, bool scatter, char* slab,
+                           cudaStream_t s) {
+  const int out_pad = (out_size + 31) / 32 * 32;
+  t.xmin = reinterpret_cast<int32_t*>(slab + L.o_xmin);
+  t.xsize = reinterpret_cast<int32_t*>(slab + L.o_xsize);
+  t.w = reinterpret_cast<float*>(slab + L.o_w);
+  t.t_lo = reinterpret_cast<int32_t*>(slab + L.o_tlo);
+  t.t_len = reinterpret_cast<int32_t*>(slab + L.o_tlen);
+  t.t_w = scatter ? reinterpret_cast<float*>(slab + L.o_tw) : nullptr;
+  t.t_cum = scatter ? reinterpret_cast<float*>(slab + L.o_tcum) : nullptr;
+  t.grp_of = reinterpret_cast<int32_t*>(slab + L.o_gof);
+  t.grp_start = reinterpret_cast<int32_t*>(slab + L.o_gst);
+  t.pk_span = L.packed ? reinterpret_cast<uint32_t*>(slab + L.o_pks) : nullptr;
+  t.pk_w = L.packed ? reinterpret_cast<float2*>(slab + L.o_pkw) : nullptr;
   aa_table_kernel<<<ceil_div(out_size, 128), 128, 0, s>>>(in_size, out_size, t.taps, t.xmin, t.xsize, t.w);
   NTTT_LAUNCH_CHECK();
   aa_transpose_kernel<<<ceil_div(in_size, 128), 128, 0, s>>>(in_size, out_size, t.taps, t.xmin, t.xsize, t.w, t.t_lo,
@@ -822,11 +837,77 @@ int build_axis_table(AxisTable& t, int in_size, int out_size, cudaStream_t s) {
   NTTT_LAUNCH_CHECK();
   aa_group_kernel<<<1, 32, 0, s>>>(out_size, t.xmin, t.xsize, t.grp_of, t.grp_start);
   NTTT_LAUNCH_CHECK();
-  if (packed) {
+  if (L.packed) {
     aa_pack_kernel<<<ceil_div(out_pad, 128), 128, 0, s>>>(out_size, out_pad, t.taps, t.xmin, t.xsize, t.w, t.pk_span,
                                                              t.pk_w);
     NTTT_LAUNCH_CHECK();
   }
+  return NTTT_OK;
+}
+
+// All arrays of a table live in ONE device allocation (`slab`): a table costs one cudaMalloc when a new (in, out) pair is
+// first seen and one cudaFree when it is retired, instead of ten of each.
+int build_axis_table(AxisTable& t, int in_size, int out_size, cudaStream_t s) {
+  t.in_size = in_size;
+  t.out_size = out_size;
+  t.taps = aa_max_taps(in_size, out_size);
+  const AxisLayout L = axis_layout(in_size, out_size, true);
+  char* slab = nullptr;
+  NTTT_CUDA(cudaMalloc(&slab, L.bytes));
+  t.slab = slab;
+  return fill_axis_table(t, in_size, out_size, L, true, slab, s);
+}
+
+// The atlas of the sized entry: the tables of every output height in [min_h, cap_h] from lr_h and of every width in
+// [min_w, cap_w] from lr_w, in one slab with the device index behind them, built with the same kernels as the tables
+// of the static entry (so a size's tables are bit for bit the ones nttt_match_image uses) behind ONE synchronisation.
+int build_sized_atlas(SizedAtlas& a, cudaStream_t s) {
+  const auto t0 = std::chrono::steady_clock::now();
+  const int ny = a.cap_h - a.min_h + 1, nx = a.cap_w - a.min_w + 1;
+  std::vector<AxisLayout> lay(ny + nx);
+  std::vector<size_t> at(ny + nx);
+  size_t off = 0;
+  for (int i = 0; i < ny + nx; ++i) {
+    const bool y = i < ny;
+    lay[i] = axis_layout(y ? a.lr_h : a.lr_w, y ? a.min_h + i : a.min_w + (i - ny), false);
+    at[i] = off;
+    off = align_up(off + lay[i].bytes, 256);
+  }
+  const size_t o_index = off;
+  off = align_up(off + sizeof(SizedAxis) * (ny + nx), 256);
+  char* slab = nullptr;
+  NTTT_CUDA(cudaMalloc(&slab, off));
+  std::vector<SizedAxis> index(ny + nx);
+  bool y_packed = false, x_packed = false, y_general = false, x_general = false;
+  long y_budget = 0, x_budget = 0;
+  for (int i = 0; i < ny + nx; ++i) {
+    const bool y = i < ny;
+    const int in_size = y ? a.lr_h : a.lr_w, out_size = y ? a.min_h + i : a.min_w + (i - ny);
+    AxisTable t{};
+    t.in_size = in_size;
+    t.out_size = out_size;
+    t.taps = aa_max_taps(in_size, out_size);
+    const int err = fill_axis_table(t, in_size, out_size, lay[i], false, slab + at[i], s);
+    if (err) { cudaStreamSynchronize(s); cudaFree(slab); return err; }
+    const long budget = up2_tile_factor(in_size, out_size, y);
+    index[i] = SizedAxis{t.xmin, t.xsize, t.w, t.t_lo, t.t_len, t.grp_of, t.grp_start, t.pk_span, t.pk_w, t.taps,
+                         (int)budget};
+    (y ? y_packed : x_packed) |= lay[i].packed;
+    (y ? y_general : x_general) |= !lay[i].packed;
+    long& mb = y ? y_budget : x_budget;
+    if (budget > mb) mb = budget;
+  }
+  cudaError_t e = cudaMemcpyAsync(slab + o_index, index.data(), sizeof(SizedAxis) * index.size(), cudaMemcpyHostToDevice, s);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(s);  // (also keeps `index` alive until the copy has run)
+  if (e != cudaSuccess) { cudaFree(slab); return cuda_fail(e, "sized atlas build"); }
+  a.slab = slab;
+  a.bytes = off;
+  a.ay = reinterpret_cast<SizedAxis*>(slab + o_index);
+  a.ax = a.ay + ny;
+  a.any_two_tap = y_packed && x_packed;
+  a.any_general = y_general || x_general;
+  a.max_budget = y_budget * x_budget;
+  a.build_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
   return NTTT_OK;
 }
 

@@ -30,7 +30,8 @@ class StageConfig:
 class PendingResult:
     """Device-side result of one image; `.get()` does the single D2H read of the counts and slices."""
 
-    def __init__(self, stage, masks, boxes, scores, labels, index, counts, taps, ori_hw, keepalive, rle=None, meta=None):
+    def __init__(self, stage, masks, boxes, scores, labels, index, counts, taps, ori_hw, keepalive, rle=None, meta=None,
+                 sized=False):
         self._stage = stage
         self.masks, self.boxes, self.scores, self.labels, self.index = masks, boxes, scores, labels, index
         self.counts = counts
@@ -40,6 +41,9 @@ class PendingResult:
         self.ori_hw = ori_hw
         self._keepalive = keepalive
         self.rle = rle  # None or (counts [K,cap] i32, n_counts [K], chars [K,cap] u8, n_chars [K])
+        # sized entry (`MatchingStage.graphed(..., min_hw=...)`): `masks` has the capacity's shape and `ori_hw` is the
+        # size of the image the buffers hold now; the stage reports a size outside its range in counts[3]
+        self._sized = sized
 
     def rle_segmentations(self) -> list:
         """The outputs as COCO `segmentation` dicts ({"size": [h, w], "counts": str}) — what
@@ -81,6 +85,9 @@ class PendingResult:
     def _host_meta(self) -> list:
         if self._meta is None:
             self._meta = self._meta_dev.cpu().tolist()  # synchronises with the producing stream
+        if self._sized and self._meta[3] != 0:
+            raise RuntimeError(f"the stage reported status {self._meta[3]}: the image size on the device lies outside "
+                               "the range the stage was enqueued for (the result is empty)")
         return self._meta
 
     def get(self) -> dict:
@@ -95,7 +102,7 @@ class PendingResult:
                        scores=torch.zeros((0,), device=dev, dtype=torch.float32),
                        labels=torch.zeros((0,), device=dev, dtype=torch.long))
         else:
-            out = dict(binary_masks=self.masks[:n_out] if self.masks is not None else None, bboxes=self.boxes[:n_out],
+            out = dict(binary_masks=self.masks[:n_out, :oh, :ow] if self.masks is not None else None, bboxes=self.boxes[:n_out],
                        scores=self.scores[:n_out], labels=self.labels[:n_out])
         out["counts"] = dict(n_keep=n_keep, n_sel=n_sel, n_out=n_out)
         out["index"] = self.index[:n_out]
@@ -153,7 +160,7 @@ class MatchingStage:
     def match_async(self, lr_masks: torch.Tensor, pred_ious: torch.Tensor, tar_feat: torch.Tensor, ori_hw,
                     taps: bool = False, slot=0, iou_thr=None, persistent_out=None, multi_ious=None,
                     multi_first: int = 1, rle: bool = False, dense_masks: bool = True,
-                    low_latency: bool = False) -> PendingResult:
+                    low_latency: bool = False, size_range=None) -> PendingResult:
         """Enqueue the whole stage for one image on the current stream.  `slot` selects which reusable
         workspace to use (callers that keep several images in flight on different streams use one slot per
         stream).  `iou_thr`, if given, fuses the reference's candidate filter (`scores_all > iou_thr`,
@@ -166,7 +173,10 @@ class MatchingStage:
         `taps=True` also returns the intermediate values tests compare, in `out["taps"]`: `sim`, `obj_feats` and the
         inputs of the score decay `sel`, `ios`, `ios_inter` (nttt_match_args; the counts are [max_sel, max_sel] i32).
         `low_latency=True` shapes the kernels for the shortest duration of ONE image (a caller that synchronises after
-        every image) instead of the least SM-time (many images in flight); float sums may differ in the last bit between the modes."""
+        every image) instead of the least SM-time (many images in flight); float sums may differ in the last bit between the modes.
+        `size_range=(hw_dev, (min_h, min_w))` enqueues the sized entry (`nttt_match_image_sized`): `ori_hw` is then the
+        capacity, and the kernels read the image's size from the device tensor `hw_dev` (int32 [2]) when they run; the
+        returned result's `ori_hw` is the capacity until the caller sets it to that size (as `GraphedMatch.replay` does)."""
         if self.proto is None:
             raise RuntimeError("Memory is not ready!")  # same text as Sam2MatchingBaseline_noAMG.py:752
         ops._need(tar_feat, torch.float32, "tar_feat")
@@ -193,6 +203,12 @@ class MatchingStage:
         if e != eh * ew:
             raise ValueError(f"tar_feat has {e} patches, expected {eh}x{ew}")
         oh, ow = int(ori_hw[0]), int(ori_hw[1])
+        if size_range is not None:
+            hw_dev, (min_h, min_w) = size_range[0], (int(size_range[1][0]), int(size_range[1][1]))
+            if hw_dev.dtype != torch.int32 or hw_dev.numel() != 2 or hw_dev.device != self.device:
+                raise ValueError("size_range needs an int32 [2] tensor on the stage's device")
+            if not (1 <= min_h <= oh and 1 <= min_w <= ow):
+                raise ValueError(f"min_hw {(min_h, min_w)} must lie between 1 and the capacity {(oh, ow)}")
         num_out = int(self.cfg.num_out_instance)
         max_sel = int(min(num_out * self.cfg.expand_ratio, n))
         dev = self.device
@@ -224,7 +240,11 @@ class MatchingStage:
             tap_t["sel"] = torch.empty((max(max_sel, 1),), dtype=torch.int32, device=dev)
             tap_t["ios"] = torch.empty((max(max_sel, 1),), dtype=torch.float32, device=dev)
             tap_t["ios_inter"] = torch.empty((max(max_sel, 1), max(max_sel, 1)), dtype=torch.int32, device=dev)
-        ws_bytes = self.lib.nttt_match_workspace_bytes_neg(n, lh, lw, eh, ew, c, self.n_cls, oh, ow, max_sel, self.l_neg)
+        if size_range is None:
+            ws_bytes = self.lib.nttt_match_workspace_bytes_neg(n, lh, lw, eh, ew, c, self.n_cls, oh, ow, max_sel, self.l_neg)
+        else:
+            ws_bytes = self.lib.nttt_match_workspace_bytes_sized(n, lh, lw, eh, ew, c, self.n_cls, oh, ow, max_sel,
+                                                                 self.l_neg, min_h, min_w)
         ws = self._workspace(("match", slot), ws_bytes)
         a = _lib.MatchArgs()
         a.logits, a.pred_ious, a.tar_feat, a.proto = (None if chunks else lr_masks.data_ptr(), ops._ptr(pred_ious),
@@ -258,10 +278,23 @@ class MatchingStage:
         a.out_prev_rect = prev_rect.data_ptr() if prev_rect is not None else None
         a.low_latency = 1 if low_latency else 0
         stream = torch.cuda.current_stream(dev).cuda_stream
-        _lib.check(self.lib.nttt_match_image(self.ctx, ctypes.byref(a), stream), "nttt_match_image")
+        if size_range is None:
+            _lib.check(self.lib.nttt_match_image(self.ctx, ctypes.byref(a), stream), "nttt_match_image")
+        else:
+            rng = _lib.MatchSizeRange(hw_dev.data_ptr(), min_h, min_w)
+            _lib.check(self.lib.nttt_match_image_sized(self.ctx, ctypes.byref(a), ctypes.byref(rng), stream),
+                       "nttt_match_image_sized")
         return PendingResult(self, masks.view(torch.bool) if masks is not None else None, boxes, scores, labels, index,
-                             counts, tap_t, (oh, ow), keepalive=(lr_masks, pred_ious, multi_ious, tar_feat, ws), rle=rle_t,
-                             meta=meta)
+                             counts, tap_t, (oh, ow), keepalive=(lr_masks, pred_ious, multi_ious, tar_feat, ws, size_range),
+                             rle=rle_t, meta=meta, sized=size_range is not None)
+
+    def atlas_stats(self) -> dict:
+        """The resize-table atlases the sized graphs of this device's context use: count, device bytes, build time."""
+        nbytes, ms = ctypes.c_size_t(0), ctypes.c_double(0.0)
+        n = self.lib.nttt_ctx_atlas_stats(self.ctx, ctypes.byref(nbytes), ctypes.byref(ms))
+        if n < 0:
+            _lib.check(n, "nttt_ctx_atlas_stats")
+        return dict(atlases=n, bytes=int(nbytes.value), build_ms=float(ms.value))
 
     def _pinned_bytes(self, nbytes: int) -> torch.Tensor:
         """Pinned host staging for result reads (grown on demand, reused call after call)."""
@@ -307,15 +340,17 @@ class MatchingStage:
 
     def graphed(self, n: int, c: int, ori_hw, iou_thr=None, key=None, n_multi: int = 0,
                 multi_first: int = 1, rle: bool = False, dense_masks: bool = True, persistent_out=None,
-                low_latency: bool = False) -> "GraphedMatch":
+                low_latency: bool = False, min_hw=None) -> "GraphedMatch":
         """A CUDA-graph capture of the whole stage at fixed shapes with static input/output buffers.
         n_multi > 1: the static mask buffer is the decoder's raw [n, n_multi, 256, 256] output (+ `multi_ious`).
         rle / dense_masks: as in `match_async`.  `key` names the workspace slot and `persistent_out` the
         (masks, prev_rect) output buffers: graphs that are replayed on the SAME stream may share both (a caller
         holding one graph per resident image passes the stream's slot).  `low_latency`: capture the launch shapes
-        for one image at a time (a caller that waits for each result) instead of many images in flight."""
+        for one image at a time (a caller that waits for each result) instead of many images in flight.
+        `min_hw=(h, w)`: one graph for every output size between `min_hw` and `ori_hw` (the capacity); the size of each
+        image is given to `replay(ori_hw=...)`, which writes it to the device, and the kernels read it when they run."""
         return GraphedMatch(self, n, c, ori_hw, iou_thr, key, n_multi, multi_first, rle, dense_masks, persistent_out,
-                            low_latency)
+                            low_latency, min_hw)
 
 
 class GraphedMatch:
@@ -325,11 +360,14 @@ class GraphedMatch:
     place of the reference's compaction, so the producer writes the decoder's masks / scores and the encoder's
     features straight into `self.lr_masks`, `self.pred_ious`, `self.tar_feat` (static device buffers) and calls
     `replay()`.  Outputs live in static buffers too: consume a result (`.get()`) before replaying the same object
-    again.  Replay costs one graph launch on the host instead of ~18 kernel launches."""
+    again.  Replay costs one graph launch on the host instead of ~18 kernel launches.
+
+    With `min_hw` the graph is SIZED: `ori_hw` is the capacity, the output masks keep its shape (image j's mask in the
+    top-left [h, w] corner of plane j, zeros elsewhere) and `replay(ori_hw=(h, w))` serves any size in between."""
 
     def __init__(self, stage: MatchingStage, n: int, c: int, ori_hw, iou_thr=None, key=None, n_multi: int = 0,
                  multi_first: int = 1, rle: bool = False, dense_masks: bool = True, persistent_out=None,
-                 low_latency: bool = False):
+                 low_latency: bool = False, min_hw=None):
         dev = stage.device
         eh, ew = stage.cfg.enc_hw
         self.stage = stage
@@ -345,6 +383,15 @@ class GraphedMatch:
         self._kw = dict(rle=rle, dense_masks=dense_masks, low_latency=low_latency)
         self.tar_feat = torch.zeros((eh * ew, c), dtype=torch.float32, device=dev)
         self.ori_hw = (int(ori_hw[0]), int(ori_hw[1]))
+        self.min_hw = None
+        self._size_range = None
+        if min_hw is not None:
+            self.min_hw = (int(min_hw[0]), int(min_hw[1]))
+            if not (1 <= self.min_hw[0] <= self.ori_hw[0] and 1 <= self.min_hw[1] <= self.ori_hw[1]):
+                raise ValueError(f"min_hw {self.min_hw} must lie between 1 and the capacity {self.ori_hw}")
+            # the size the kernels read; replay() rewrites it, stream-ordered, before each launch of the graph
+            self.hw_dev = torch.tensor(self.ori_hw, dtype=torch.int32, device=dev)
+            self._size_range = (self.hw_dev, self.min_hw)
         self.iou_thr = iou_thr
         self._slot = ("graph", id(self) if key is None else key)
         num_out = max(int(stage.cfg.num_out_instance), 1)
@@ -366,19 +413,36 @@ class GraphedMatch:
             for _ in range(2):
                 self.stage.match_async(self.lr_masks, self.pred_ious, self.tar_feat, self.ori_hw, slot=self._slot,
                                        iou_thr=self.iou_thr, persistent_out=self._out, multi_ious=self.multi_ious,
-                                       multi_first=self.multi_first, **self._kw)
+                                       multi_first=self.multi_first, size_range=self._size_range, **self._kw)
         torch.cuda.current_stream(self.stage.device).wait_stream(side)
         torch.cuda.synchronize(self.stage.device)
         self.graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(self.graph):
             self.pending = self.stage.match_async(self.lr_masks, self.pred_ious, self.tar_feat, self.ori_hw,
                                                   slot=self._slot, iou_thr=self.iou_thr, persistent_out=self._out,
-                                                  multi_ious=self.multi_ious, multi_first=self.multi_first, **self._kw)
+                                                  multi_ious=self.multi_ious, multi_first=self.multi_first,
+                                                  size_range=self._size_range, **self._kw)
         return self
 
-    def replay(self) -> PendingResult:
+    def replay(self, ori_hw=None) -> PendingResult:
+        """Launch the graph on the current stream.  A sized graph needs the image's size `ori_hw=(h, w)`."""
+        if self.min_hw is None:
+            if ori_hw is not None and (int(ori_hw[0]), int(ori_hw[1])) != self.ori_hw:
+                raise ValueError(f"this graph serves {self.ori_hw} only; capture it with min_hw to serve a range")
+            hw = self.ori_hw
+        else:
+            if ori_hw is None:
+                raise ValueError("a sized graph needs the image's size: replay(ori_hw=(h, w))")
+            hw = (int(ori_hw[0]), int(ori_hw[1]))
+            if not (self.min_hw[0] <= hw[0] <= self.ori_hw[0] and self.min_hw[1] <= hw[1] <= self.ori_hw[1]):
+                raise ValueError(f"size {hw} is outside the graph's range {self.min_hw} .. {self.ori_hw}")
         if self.graph is None:
             self.capture()
+        if self.min_hw is not None:
+            # One fill kernel on the replay's stream writes both int32 (little-endian: h is the low half): the value
+            # travels as a kernel argument, so no host buffer can be overwritten by a later replay before it is read.
+            self.hw_dev.view(torch.int64).fill_(hw[0] | (hw[1] << 32))
         self.graph.replay()
         self.pending._meta = None  # the static buffers now hold a new image's result
+        self.pending.ori_hw = hw
         return self.pending
