@@ -404,6 +404,38 @@ int nttt_match_image_sized(nttt_ctx* ctx, const nttt_match_args* args, const ntt
  * bytes and the host time their builds took in total */
 int nttt_ctx_atlas_stats(nttt_ctx* ctx, size_t* bytes_host, double* build_ms_host);
 
+/* ---------------------------------------------------------------------------------------------------
+ * The whole stage with its inputs bound when it runs: the addresses of the caller's input tensors are read from a small
+ * struct in DEVICE memory, so one enqueue (or one CUDA-graph capture) consumes whatever tensors a producer allocated for
+ * each image, in place, with no copy into static buffers.
+ *   nttt_match_bind writes the struct, stream-ordered, with one kernel that carries the values as its argument (no host
+ *   staging buffer that a later bind could overwrite before it is read).  It first checks the binding against the shapes
+ *   the stage was enqueued with (`shapes`: n, n_multi, n_chunks, chunk_prompts), and returns NTTT_EINVAL before any CUDA
+ *   call for a null pointer, a logits base that is not 16-byte aligned (TMA bulk copies read the logits), or chunks that
+ *   do not match: 1 <= n_chunks <= 64, chunk_prompts >= 1 and n_chunks * chunk_prompts >= n.
+ *   nttt_match_image_bound is nttt_match_image (range == NULL) or nttt_match_image_sized with the input pointers of
+ *   `args` (logits, pred_ious, multi_ious, tar_feat, logits_chunks_host) replaced by reads from `inputs_dev`; workspace,
+ *   outputs and prototypes still come from `args`.  With n_multi > 1 the logits are the per-batch chunks when
+ *   args->n_chunks > 0 (args->chunk_prompts prompts each), else the one buffer `logits`.  Results are those of the
+ *   unbound entries on the same tensors, bit for bit.  A sized range may point `ori_hw_dev` at inputs_dev->ori_hw: the
+ *   bind then writes the image's size as well.
+ */
+#define NTTT_MAX_CHUNKS 64
+typedef struct nttt_match_inputs {
+  const float* logits;     /* [n, lr_h, lr_w], or [n, n_multi, lr_h, lr_w] (n_multi > 1 without chunks) */
+  const float* pred_ious;  /* [n] (n_multi <= 1) */
+  const float* multi_ious; /* [n, n_multi] (n_multi > 1) */
+  const float* tar_feat;   /* [eh*ew, c] */
+  const float* chunks[NTTT_MAX_CHUNKS]; /* n_multi > 1 and n_chunks > 0: [chunk_prompts, n_multi, lr_h, lr_w] each */
+  int32_t ori_hw[2];       /* (h, w) for a sized range that reads it */
+} nttt_match_inputs;
+
+size_t nttt_sizeof_match_inputs(void);
+int nttt_match_bind(nttt_match_inputs* inputs_dev, const nttt_match_inputs* host, const nttt_match_args* shapes,
+                    void* stream);
+int nttt_match_image_bound(nttt_ctx* ctx, const nttt_match_args* args, const nttt_match_size_range* range,
+                           const nttt_match_inputs* inputs_dev, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

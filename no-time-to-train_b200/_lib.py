@@ -50,6 +50,15 @@ class MatchSizeRange(ctypes.Structure):
     _fields_ = [("ori_hw_dev", c_void_p), ("min_h", c_int32), ("min_w", c_int32)]
 
 
+MAX_CHUNKS = 64  # NTTT_MAX_CHUNKS
+
+
+class MatchInputs(ctypes.Structure):
+    """Mirror of `nttt_match_inputs` (include/nttt_b200.h): the input addresses a bound stage reads on the device."""
+    _fields_ = [("logits", c_void_p), ("pred_ious", c_void_p), ("multi_ious", c_void_p), ("tar_feat", c_void_p),
+                ("chunks", c_void_p * MAX_CHUNKS), ("ori_hw", c_int32 * 2)]
+
+
 # name -> (restype, argtypes); every symbol include/nttt_b200.h declares
 _P = c_void_p
 SIGNATURES = {
@@ -97,6 +106,9 @@ SIGNATURES = {
     "nttt_match_workspace_bytes_sized": (c_size_t, [c_int] * 13),
     "nttt_match_image_sized": (c_int, [_P, POINTER(MatchArgs), POINTER(MatchSizeRange), _P]),
     "nttt_ctx_atlas_stats": (c_int, [_P, POINTER(c_size_t), POINTER(ctypes.c_double)]),
+    "nttt_sizeof_match_inputs": (c_size_t, []),
+    "nttt_match_bind": (c_int, [_P, POINTER(MatchInputs), POINTER(MatchArgs), _P]),
+    "nttt_match_image_bound": (c_int, [_P, POINTER(MatchArgs), POINTER(MatchSizeRange), _P, _P]),
     "nttt_launch_count": (ctypes.c_ulonglong, []),
     "nttt_profile_num_stages": (c_int, []),
     "nttt_profile_stage_name": (c_char_p, [c_int]),

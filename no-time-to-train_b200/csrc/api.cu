@@ -14,6 +14,10 @@ int launch_lowres_pack(const float*, int, int, int, float, float, uint32_t*, int
                        const float*, float, const float* const*, cudaStream_t, float* stab_score = nullptr);
 int launch_multimask_select(const float*, int, int, int, const ChunkTable&, int, size_t, const float**, float*,
                             cudaStream_t);
+int launch_multimask_select_bound(const float* const*, int, int, int, const float* const*, int, size_t, const float**,
+                                  float*, cudaStream_t);
+int launch_plane_resolve(const nttt_match_inputs*, int, size_t, const float**, float*, cudaStream_t);
+int launch_match_bind(const nttt_match_inputs&, nttt_match_inputs*, cudaStream_t);
 int launch_project_masks(const AxisTable&, const AxisTable&, const uint32_t*, const int32_t*, int, int, int, int, int,
                          void*, int, bool, cudaStream_t, const int32_t* perm = nullptr, uint32_t* active = nullptr);
 int launch_pool_order(const int32_t*, int, int, int32_t*, cudaStream_t);
@@ -23,7 +27,8 @@ int launch_gemm_tc(const void*, int, const void*, int, float*, int, int, int, in
                    bool low_latency = false, const uint32_t* a_active = nullptr, const uint8_t* b_nonfinite = nullptr);
 int gemm_tc_pick_splits(int, int, int, int);
 int launch_split_rows(const float*, int, int, int, int, int, void*, cudaStream_t);
-int launch_split_transpose(const float*, int, int, int, int, int, void*, cudaStream_t, uint8_t* nonfinite = nullptr);
+int launch_split_transpose(const float*, int, int, int, int, int, void*, cudaStream_t, uint8_t* nonfinite = nullptr,
+                           const float* const* x_at = nullptr);
 int launch_normalize_rows(const float*, int, const int32_t*, int, int, float*, bool, cudaStream_t);
 int launch_proto_prepare(const float*, int, int, int, float*, cudaStream_t);
 int launch_top1(const float*, int, size_t, float*, int, int, int, float*, int32_t*, cudaStream_t);
@@ -121,13 +126,16 @@ constexpr int kPoolSplits = 1;  // measured: 2 halves the latency (25 -> 14 us) 
 // instead of 25-38 us).
 static int pool_contract(const float* proj, const float* feat, int n, int e, int c, float* sums, void* a_split,
                          void* b_split, int* n_partials, cudaStream_t s, bool low_latency = false, bool b_ready = false,
-                         const uint32_t* a_active = nullptr, uint8_t* b_nonfinite = nullptr) {
+                         const uint32_t* a_active = nullptr, uint8_t* b_nonfinite = nullptr,
+                         const float* const* feat_at = nullptr) {
   // a_active / b_nonfinite (both or neither): the A operand's rows are spatially ordered and carry their non-zero k-block
   // masks; the GEMM skips the k-blocks a tile does not touch (gemm_tc_kernel), unless the features are not finite there
+  // feat_at (nullable): the features' address is read from device memory when the kernel runs (bound inputs)
   const int ep = pad64(e);
   int err = proj ? launch_split_rows(proj, e, n, e, ep, 0, a_split, s) : NTTT_OK;
   if (err) return err;
-  err = b_ready ? NTTT_OK : launch_split_transpose(feat, c, c, e, ep, 1, b_split, s, a_active ? b_nonfinite : nullptr);  // (b_ready: done on the side stream)
+  err = b_ready ? NTTT_OK : launch_split_transpose(feat, c, c, e, ep, 1, b_split, s, a_active ? b_nonfinite : nullptr,
+                                                   feat_at);  // (b_ready: done on the side stream)
   if (err) return err;
   return launch_gemm_tc(a_split, 3 * ep, b_split, 3 * ep, sums, c, n, c, 3 * ep, low_latency ? kPoolSplitsMax : kPoolSplits,
                         (size_t)n * c, n_partials, s, low_latency, a_active, a_active ? b_nonfinite : nullptr);
@@ -274,6 +282,8 @@ int nttt_build_is_ablation(void) {
 }
 
 size_t nttt_sizeof_match_args(void) { return sizeof(nttt_match_args); }
+
+size_t nttt_sizeof_match_inputs(void) { return sizeof(nttt_match_inputs); }
 
 unsigned long long nttt_launch_count(void) { return g_launches.load(); }
 
@@ -790,7 +800,10 @@ int nttt_ctx_atlas_stats(nttt_ctx* ctx, size_t* bytes_host, double* build_ms_hos
 }
 
 // range == nullptr: nttt_match_image (the size is a->ori_h x a->ori_w); otherwise nttt_match_image_sized
-static int match_impl(nttt_ctx* ctx, const nttt_match_args* a, const nttt_match_size_range* range, void* stream) {
+// in_dev != nullptr: nttt_match_image_bound (the input pointers of `a` are ignored; the kernels that read the inputs
+// take their addresses from *in_dev)
+static int match_impl(nttt_ctx* ctx, const nttt_match_args* a, const nttt_match_size_range* range, void* stream,
+                      const nttt_match_inputs* in_dev = nullptr) {
   if (!ctx || !a) return NTTT_EINVAL;
   if (a->n < 0 || a->lr_h <= 0 || a->lr_w <= 0 || a->eh <= 0 || a->ew <= 0 || a->c <= 0 || a->n_cls <= 0 ||
       a->ori_h <= 0 || a->ori_w <= 0 || a->num_out_instance < 0 || a->max_sel < 0)
@@ -807,14 +820,18 @@ static int match_impl(nttt_ctx* ctx, const nttt_match_args* a, const nttt_match_
     return NTTT_OK;
   }
   const bool multi = a->n_multi > 1;
-  const bool chunked = multi && a->logits_chunks_host;
+  const bool bound = in_dev != nullptr;
+  const bool chunked = multi && (bound ? a->n_chunks > 0 : a->logits_chunks_host != nullptr);
   const bool want_rle = a->rle_chars != nullptr;
-  if ((!a->logits && !chunked) || (!multi && !a->pred_ious) || !a->tar_feat || !a->proto ||
+  if ((!bound && ((!a->logits && !chunked) || (!multi && !a->pred_ious) || !a->tar_feat)) || !a->proto ||
       (!a->out_masks && !want_rle) || !a->out_boxes || !a->out_scores || !a->out_labels || !a->out_index)
+    return NTTT_EINVAL;
+  if (bound && chunked &&
+      (a->n_chunks > kMaxChunks || a->chunk_prompts <= 0 || (long long)a->n_chunks * a->chunk_prompts < n))
     return NTTT_EINVAL;
   if (want_rle && (!a->rle_counts || !a->rle_n_counts || !a->rle_n_chars || a->rle_cap_counts <= 0 || a->rle_cap_chars <= 0))
     return NTTT_EINVAL;
-  if (multi && (!a->multi_ious || a->multi_first < 0 || a->multi_first >= a->n_multi)) return NTTT_EINVAL;
+  if (multi && ((!bound && !a->multi_ious) || a->multi_first < 0 || a->multi_first >= a->n_multi)) return NTTT_EINVAL;
   const int l_neg = a->proto_neg ? a->l_neg : 0;
   if (a->proto_neg && (a->l_neg <= 0 || !(a->sigma > 0.0f))) return NTTT_EINVAL;
   MatchLayout L = carve(a->workspace, n, a->lr_h, a->lr_w, a->eh, a->ew, a->c, a->n_cls, a->ori_h, a->ori_w, max_sel,
@@ -877,7 +894,20 @@ static int match_impl(nttt_ctx* ctx, const nttt_match_args* a, const nttt_match_
   // candidate selection (§8f rank 2): resolve the best decoder plane per prompt; its IoU is the score from here on
   const float* const* mask_ptr = nullptr;
   const float* pred_ious = a->pred_ious;
-  if (multi) {
+  // bound inputs: the logits are reached through mask_ptr only, and the features through feat_at
+  const float* logits = bound ? nullptr : a->logits;
+  const float* const* feat_at = bound ? &in_dev->tar_feat : nullptr;
+  if (bound) {
+    if (multi)
+      err = launch_multimask_select_bound(&in_dev->multi_ious, n, a->n_multi, a->multi_first,
+                                          chunked ? in_dev->chunks : &in_dev->logits, chunked ? a->chunk_prompts : n,
+                                          (size_t)a->lr_h * a->lr_w, L.mask_ptr, L.plane_score, s);
+    else
+      err = launch_plane_resolve(in_dev, n, (size_t)a->lr_h * a->lr_w, L.mask_ptr, L.plane_score, s);
+    if (err) return err;
+    mask_ptr = L.mask_ptr;
+    pred_ious = L.plane_score;
+  } else if (multi) {
     ChunkTable ct;
     const float* one = a->logits;
     err = chunked ? make_chunk_table(a->logits_chunks_host, a->n_chunks, a->chunk_prompts, n, &ct)
@@ -903,7 +933,7 @@ static int match_impl(nttt_ctx* ctx, const nttt_match_args* a, const nttt_match_
   if (forked) {
     NTTT_CUDA(cudaEventRecord(ctx->ev_fork, s));
     NTTT_CUDA(cudaStreamWaitEvent(ctx->side, ctx->ev_fork, 0));
-    err = launch_split_transpose(a->tar_feat, a->c, a->c, e, pad64(e), 1, L.b_split, ctx->side);
+    err = launch_split_transpose(a->tar_feat, a->c, a->c, e, pad64(e), 1, L.b_split, ctx->side, nullptr, feat_at);
     if (err) return err;
     err = launch_split_rows(a->proto, a->c, a->n_cls, a->c, pad64(a->c), 1, L.p_split, ctx->side);
     if (err) return err;
@@ -912,7 +942,7 @@ static int match_impl(nttt_ctx* ctx, const nttt_match_args* a, const nttt_match_
   }
   // a6/a9/a15: one pass over the logits
   // (the stability counts of a15 are not read on this path, so the pipeline does not pay for them)
-  NTTT_STEP(launch_lowres_pack(a->logits, n, a->lr_h, a->lr_w, 0.0f, 1.0f, L.bits_lr, L.area_lr, L.box_lr, nullptr,
+  NTTT_STEP(launch_lowres_pack(logits, n, a->lr_h, a->lr_w, 0.0f, 1.0f, L.bits_lr, L.area_lr, L.box_lr, nullptr,
                                L.flags, a->filter_iou ? pred_ious : nullptr, a->iou_thr, mask_ptr, s));
   // a6/a7: projection + pooling contraction + normalisation
   // Many images in flight: the pooling GEMM runs on spatially ordered rows and skips the k-blocks a tile of masks does
@@ -929,7 +959,7 @@ static int match_impl(nttt_ctx* ctx, const nttt_match_args* a, const nttt_match_
     nttt::t_chain_break = true;  // the pooling GEMM depends on the side stream as well: launched the ordinary way
   }
   NTTT_STEP(pool_contract(nullptr, a->tar_feat, n, e, a->c, L.sums, L.a_split, L.b_split, &n_partials, s,
-                          a->low_latency != 0, forked, ordered ? L.pool_active : nullptr, L.b_nonfinite));
+                          a->low_latency != 0, forked, ordered ? L.pool_active : nullptr, L.b_nonfinite, feat_at));
   bool a_ready = false;
   NTTT_STEP(normalize_rows(L.sums, n_partials, L.area_lr, n, a->c, obj_feats, L.a_split, &a_ready,
                            a->proto_neg != nullptr, s, ordered ? L.pool_perm : nullptr));
@@ -945,12 +975,12 @@ static int match_impl(nttt_ctx* ctx, const nttt_match_args* a, const nttt_match_
   if (sized) {
     // (a range that also takes the general resize keeps the row-major layout on both paths)
     wrote_t = !atlas->any_general;
-    NTTT_STEP(launch_upsample_pack_sized(sd, *atlas, a->logits, L.bits_lr, L.box_lr, L.flags, a->lr_h, a->lr_w, sel,
+    NTTT_STEP(launch_upsample_pack_sized(sd, *atlas, logits, L.bits_lr, L.box_lr, L.flags, a->lr_h, a->lr_w, sel,
                                          a->counts + 1, max_sel, L.bits_full, L.rect, L.area_full, L.box_full, L.scratch,
                                          mask_ptr, s, ctx->upsample_stage_floats, ctx->sm_count, L.bits_t,
                                          a->low_latency != 0, wrote_t ? ios_pair_counters(L.ios_ws, max_sel) : nullptr));
   } else {
-    NTTT_STEP(launch_upsample_pack(ux, uy, a->logits, L.bits_lr, L.box_lr, L.flags, a->lr_h, a->lr_w, sel,
+    NTTT_STEP(launch_upsample_pack(ux, uy, logits, L.bits_lr, L.box_lr, L.flags, a->lr_h, a->lr_w, sel,
                                    a->counts + 1, max_sel, a->ori_h, a->ori_w, L.bits_full, L.rect, L.area_full,
                                    L.box_full, L.scratch, mask_ptr, s, ctx->upsample_stage_floats, ctx->sm_count, L.bits_t,
                                    &wrote_t, /*t_only=*/true, a->low_latency != 0, ios_pair_counters(L.ios_ws, max_sel)));
@@ -993,6 +1023,35 @@ int nttt_match_image(nttt_ctx* ctx, const nttt_match_args* a, void* stream) { re
 int nttt_match_image_sized(nttt_ctx* ctx, const nttt_match_args* a, const nttt_match_size_range* range, void* stream) {
   if (!range) return NTTT_EINVAL;
   return match_impl(ctx, a, range, stream);
+}
+
+static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
+
+int nttt_match_bind(nttt_match_inputs* inputs_dev, const nttt_match_inputs* host, const nttt_match_args* shapes,
+                    void* stream) {
+  if (!inputs_dev || !host || !shapes || (reinterpret_cast<uintptr_t>(inputs_dev) & 7) != 0) return NTTT_EINVAL;
+  if (shapes->n < 0 || !host->tar_feat) return NTTT_EINVAL;
+  const int n = shapes->n;
+  if (shapes->n_multi > 1) {
+    if (!host->multi_ious) return NTTT_EINVAL;
+    if (shapes->n_chunks > 0) {
+      const int k = shapes->n_chunks;
+      if (k > kMaxChunks || shapes->chunk_prompts <= 0 || (long long)k * shapes->chunk_prompts < n) return NTTT_EINVAL;
+      for (int i = 0; i < k; ++i)
+        if (!host->chunks[i] || !aligned16(host->chunks[i])) return NTTT_EINVAL;
+    } else if (!host->logits || !aligned16(host->logits)) {
+      return NTTT_EINVAL;
+    }
+  } else if (!host->logits || !aligned16(host->logits) || !host->pred_ious) {
+    return NTTT_EINVAL;
+  }
+  return launch_match_bind(*host, inputs_dev, (cudaStream_t)stream);
+}
+
+int nttt_match_image_bound(nttt_ctx* ctx, const nttt_match_args* a, const nttt_match_size_range* range,
+                           const nttt_match_inputs* inputs_dev, void* stream) {
+  if (!inputs_dev) return NTTT_EINVAL;
+  return match_impl(ctx, a, range, stream, inputs_dev);
 }
 
 }  // extern "C"

@@ -165,6 +165,7 @@ int aa_max_taps(int in_size, int out_size);
 // base pointers of the decoder's per-batch output tensors, passed to multimask_select_kernel BY VALUE (stream-ordered,
 // graph-capturable, no staging copy)
 constexpr int kMaxChunks = 64;
+static_assert(kMaxChunks == NTTT_MAX_CHUNKS, "the bound inputs hold as many chunks as the by-value table");
 struct ChunkTable {
   const float* base[kMaxChunks];
 };

@@ -641,11 +641,11 @@ int launch_lowres_pack(const float* logits, int n, int h, int w, float thr, floa
 // resolved; the logits stay in the tensors the decoder returned and are read once, by lowres_pack / upsample_pack,
 // through mask_ptr[].  torch.argmax semantics: the first maximal value wins, NaN counts as maximal.
 // ---------------------------------------------------------------------------------------------------
-__global__ void multimask_select_kernel(const float* __restrict__ ious, int n, int m, int first, ChunkTable chunks,
-                                        int chunk_prompts, size_t plane_elems, const float** __restrict__ mask_ptr,
-                                        float* __restrict__ score) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
+// base_of(ch): the base address of chunk ch (a by-value table, or device memory written by nttt_match_bind)
+template <typename BaseOf>
+__device__ __forceinline__ void multimask_select_body(int i, const float* __restrict__ ious, int m, int first,
+                                                      BaseOf base_of, int chunk_prompts, size_t plane_elems,
+                                                      const float** __restrict__ mask_ptr, float* __restrict__ score) {
   const float* row = ious + (size_t)i * m;
   int best = first;
   float bv = row[first];
@@ -654,8 +654,29 @@ __global__ void multimask_select_kernel(const float* __restrict__ ious, int n, i
     if (v > bv || (v != v && bv == bv)) { bv = v; best = j; }
   }
   const int ch = i / chunk_prompts;
-  mask_ptr[i] = chunks.base[ch] + ((size_t)(i - ch * chunk_prompts) * m + best) * plane_elems;
+  mask_ptr[i] = base_of(ch) + ((size_t)(i - ch * chunk_prompts) * m + best) * plane_elems;
   score[i] = bv;
+}
+
+__global__ void multimask_select_kernel(const float* __restrict__ ious, int n, int m, int first, ChunkTable chunks,
+                                        int chunk_prompts, size_t plane_elems, const float** __restrict__ mask_ptr,
+                                        float* __restrict__ score) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  multimask_select_body(i, ious, m, first, [&](int ch) { return chunks.base[ch]; }, chunk_prompts, plane_elems, mask_ptr,
+                        score);
+}
+
+// bound twin (nttt_match_image_bound): the IoUs' address at *ious_at, chunk bases at bases[] (both inside the
+// nttt_match_inputs struct in device memory)
+__global__ void multimask_select_bound_kernel(const float* const* __restrict__ ious_at, int n, int m, int first,
+                                              const float* const* __restrict__ bases, int chunk_prompts,
+                                              size_t plane_elems, const float** __restrict__ mask_ptr,
+                                              float* __restrict__ score) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  multimask_select_body(i, *ious_at, m, first, [&](int ch) { return bases[ch]; }, chunk_prompts, plane_elems, mask_ptr,
+                        score);
 }
 
 int launch_multimask_select(const float* ious, int n, int m, int first, const ChunkTable& chunks, int chunk_prompts,
@@ -663,6 +684,54 @@ int launch_multimask_select(const float* ious, int n, int m, int first, const Ch
   if (n <= 0) return NTTT_OK;
   multimask_select_kernel<<<ceil_div(n, 256), 256, 0, s>>>(ious, n, m, first, chunks, chunk_prompts, plane_elems, mask_ptr,
                                                            score);
+  NTTT_LAUNCH_CHECK();
+  return NTTT_OK;
+}
+
+int launch_multimask_select_bound(const float* const* ious_at, int n, int m, int first, const float* const* bases,
+                                  int chunk_prompts, size_t plane_elems, const float** mask_ptr, float* score,
+                                  cudaStream_t s) {
+  if (n <= 0) return NTTT_OK;
+  multimask_select_bound_kernel<<<ceil_div(n, 256), 256, 0, s>>>(ious_at, n, m, first, bases, chunk_prompts, plane_elems,
+                                                                 mask_ptr, score);
+  NTTT_LAUNCH_CHECK();
+  return NTTT_OK;
+}
+
+// Single-plane inputs of the bound entry: mask i's address and score, in the form the multimask path leaves them, so
+// that the low-res pass, the iou_thr gate, NMS and the resize run their mask_ptr / plane_score forms unchanged.
+__global__ void __launch_bounds__(256)
+plane_resolve_kernel(const nttt_match_inputs* __restrict__ in, int n, size_t plane_elems,
+                     const float** __restrict__ mask_ptr, float* __restrict__ score) {
+  chain_wait();
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  mask_ptr[i] = in->logits + (size_t)i * plane_elems;
+  score[i] = in->pred_ious[i];
+}
+
+int launch_plane_resolve(const nttt_match_inputs* in, int n, size_t plane_elems, const float** mask_ptr, float* score,
+                         cudaStream_t s) {
+  if (n <= 0) return NTTT_OK;
+  launch_chain(plane_resolve_kernel, dim3(ceil_div(n, 256)), dim3(256), 0, s, in, n, plane_elems, mask_ptr, score);
+  NTTT_LAUNCH_CHECK();
+  return NTTT_OK;
+}
+
+// nttt_match_bind: the struct travels as the kernel's argument and is stored with static indices (one 8-byte word per
+// lane and step), so no host buffer is read when the kernel runs
+static_assert(sizeof(nttt_match_inputs) % 8 == 0, "nttt_match_inputs is copied in 8-byte words");
+__global__ void __launch_bounds__(32) match_bind_kernel(nttt_match_inputs v, nttt_match_inputs* __restrict__ dst) {
+  constexpr int kWords = sizeof(nttt_match_inputs) / 8;
+  const unsigned long long* src = reinterpret_cast<const unsigned long long*>(&v);
+  unsigned long long* out = reinterpret_cast<unsigned long long*>(dst);
+#pragma unroll
+  for (int k = 0; k < kWords; ++k)
+    if ((k & 31) == (int)threadIdx.x) out[k] = src[k];
+}
+
+int launch_match_bind(const nttt_match_inputs& v, nttt_match_inputs* dst, cudaStream_t s) {
+  match_bind_kernel<<<1, 32, 0, s>>>(v, dst);
   NTTT_LAUNCH_CHECK();
   return NTTT_OK;
 }

@@ -44,6 +44,7 @@ class PendingResult:
         # sized entry (`MatchingStage.graphed(..., min_hw=...)`): `masks` has the capacity's shape and `ori_hw` is the
         # size of the image the buffers hold now; the stage reports a size outside its range in counts[3]
         self._sized = sized
+        self._bound = None  # a bound graph's replay: the tensors it reads (GraphedMatch.replay)
 
     def rle_segmentations(self) -> list:
         """The outputs as COCO `segmentation` dicts ({"size": [h, w], "counts": str}) — what
@@ -160,7 +161,7 @@ class MatchingStage:
     def match_async(self, lr_masks: torch.Tensor, pred_ious: torch.Tensor, tar_feat: torch.Tensor, ori_hw,
                     taps: bool = False, slot=0, iou_thr=None, persistent_out=None, multi_ious=None,
                     multi_first: int = 1, rle: bool = False, dense_masks: bool = True,
-                    low_latency: bool = False, size_range=None) -> PendingResult:
+                    low_latency: bool = False, size_range=None, bound_inputs=None) -> PendingResult:
         """Enqueue the whole stage for one image on the current stream.  `slot` selects which reusable
         workspace to use (callers that keep several images in flight on different streams use one slot per
         stream).  `iou_thr`, if given, fuses the reference's candidate filter (`scores_all > iou_thr`,
@@ -176,7 +177,10 @@ class MatchingStage:
         every image) instead of the least SM-time (many images in flight); float sums may differ in the last bit between the modes.
         `size_range=(hw_dev, (min_h, min_w))` enqueues the sized entry (`nttt_match_image_sized`): `ori_hw` is then the
         capacity, and the kernels read the image's size from the device tensor `hw_dev` (int32 [2]) when they run; the
-        returned result's `ori_hw` is the capacity until the caller sets it to that size (as `GraphedMatch.replay` does)."""
+        returned result's `ori_hw` is the capacity until the caller sets it to that size (as `GraphedMatch.replay` does).
+        `bound_inputs` (a device buffer of `nttt_sizeof_match_inputs()` bytes written by `nttt_match_bind`) enqueues the
+        bound entry (`nttt_match_image_bound`): the kernels read the input addresses from it when they run, and the tensors
+        given here only fix the shapes (as `GraphedMatch` does with `bind=True`)."""
         if self.proto is None:
             raise RuntimeError("Memory is not ready!")  # same text as Sam2MatchingBaseline_noAMG.py:752
         ops._need(tar_feat, torch.float32, "tar_feat")
@@ -278,14 +282,18 @@ class MatchingStage:
         a.out_prev_rect = prev_rect.data_ptr() if prev_rect is not None else None
         a.low_latency = 1 if low_latency else 0
         stream = torch.cuda.current_stream(dev).cuda_stream
-        if size_range is None:
+        rng = _lib.MatchSizeRange(hw_dev.data_ptr(), min_h, min_w) if size_range is not None else None
+        if bound_inputs is not None:
+            _lib.check(self.lib.nttt_match_image_bound(self.ctx, ctypes.byref(a), ctypes.byref(rng) if rng else None,
+                                                       bound_inputs.data_ptr(), stream), "nttt_match_image_bound")
+        elif size_range is None:
             _lib.check(self.lib.nttt_match_image(self.ctx, ctypes.byref(a), stream), "nttt_match_image")
         else:
-            rng = _lib.MatchSizeRange(hw_dev.data_ptr(), min_h, min_w)
             _lib.check(self.lib.nttt_match_image_sized(self.ctx, ctypes.byref(a), ctypes.byref(rng), stream),
                        "nttt_match_image_sized")
         return PendingResult(self, masks.view(torch.bool) if masks is not None else None, boxes, scores, labels, index,
-                             counts, tap_t, (oh, ow), keepalive=(lr_masks, pred_ious, multi_ious, tar_feat, ws, size_range),
+                             counts, tap_t, (oh, ow), keepalive=(lr_masks, pred_ious, multi_ious, tar_feat, ws, size_range,
+                                                                bound_inputs),
                              rle=rle_t, meta=meta, sized=size_range is not None)
 
     def atlas_stats(self) -> dict:
@@ -340,7 +348,7 @@ class MatchingStage:
 
     def graphed(self, n: int, c: int, ori_hw, iou_thr=None, key=None, n_multi: int = 0,
                 multi_first: int = 1, rle: bool = False, dense_masks: bool = True, persistent_out=None,
-                low_latency: bool = False, min_hw=None) -> "GraphedMatch":
+                low_latency: bool = False, min_hw=None, bind: bool = False, chunk_prompts=None) -> "GraphedMatch":
         """A CUDA-graph capture of the whole stage at fixed shapes with static input/output buffers.
         n_multi > 1: the static mask buffer is the decoder's raw [n, n_multi, 256, 256] output (+ `multi_ious`).
         rle / dense_masks: as in `match_async`.  `key` names the workspace slot and `persistent_out` the
@@ -348,9 +356,13 @@ class MatchingStage:
         holding one graph per resident image passes the stream's slot).  `low_latency`: capture the launch shapes
         for one image at a time (a caller that waits for each result) instead of many images in flight.
         `min_hw=(h, w)`: one graph for every output size between `min_hw` and `ori_hw` (the capacity); the size of each
-        image is given to `replay(ori_hw=...)`, which writes it to the device, and the kernels read it when they run."""
+        image is given to `replay(ori_hw=...)`, which writes it to the device, and the kernels read it when they run.
+        `bind=True`: the graph reads its inputs' addresses on the device, so `replay(lr_masks=..., pred_ious=...,
+        multi_ious=..., tar_feat=...)` consumes a producer's own tensors in place (see `GraphedMatch.replay`).
+        `chunk_prompts` (with n_multi > 1): the static masks are the decoder's per-batch chunk list, `chunk_prompts`
+        prompts each (the last holds the rest), instead of one [n, n_multi, 256, 256] tensor."""
         return GraphedMatch(self, n, c, ori_hw, iou_thr, key, n_multi, multi_first, rle, dense_masks, persistent_out,
-                            low_latency, min_hw)
+                            low_latency, min_hw, bind, chunk_prompts)
 
 
 class GraphedMatch:
@@ -363,19 +375,40 @@ class GraphedMatch:
     again.  Replay costs one graph launch on the host instead of ~18 kernel launches.
 
     With `min_hw` the graph is SIZED: `ori_hw` is the capacity, the output masks keep its shape (image j's mask in the
-    top-left [h, w] corner of plane j, zeros elsewhere) and `replay(ori_hw=(h, w))` serves any size in between."""
+    top-left [h, w] corner of plane j, zeros elsewhere) and `replay(ori_hw=(h, w))` serves any size in between.
+
+    With `bind=True` the graph is BOUND: it reads the addresses of its inputs from a small device struct
+    (`nttt_match_inputs`) that `replay(lr_masks=..., ...)` rewrites with one kernel on the replay's stream, so each replay
+    consumes the producer's own tensors in place.  Until a replay binds something else, the binding points at the graph's
+    own static buffers.
+
+    The graph keeps the prototype tensors it captured alive, and re-captures on the next replay once the stage's
+    prototypes have been replaced (`set_prototypes*`)."""
 
     def __init__(self, stage: MatchingStage, n: int, c: int, ori_hw, iou_thr=None, key=None, n_multi: int = 0,
                  multi_first: int = 1, rle: bool = False, dense_masks: bool = True, persistent_out=None,
-                 low_latency: bool = False, min_hw=None):
+                 low_latency: bool = False, min_hw=None, bind: bool = False, chunk_prompts=None):
         dev = stage.device
         eh, ew = stage.cfg.enc_hw
         self.stage = stage
+        self.n, self.c = int(n), int(c)
+        self.n_multi = int(n_multi) if n_multi > 1 else 0
+        self.chunk_prompts = None
         if n_multi > 1:
-            self.lr_masks = torch.zeros((n, n_multi, 256, 256), dtype=torch.float32, device=dev)
+            full = torch.zeros((n, n_multi, 256, 256), dtype=torch.float32, device=dev)
+            if chunk_prompts is not None:
+                cp = int(chunk_prompts)
+                if cp < 1 or -(-n // cp) > _lib.MAX_CHUNKS:
+                    raise ValueError(f"chunk_prompts {chunk_prompts} must split {n} prompts into 1..{_lib.MAX_CHUNKS} chunks")
+                self.chunk_prompts = cp
+                self.lr_masks = list(full.split(cp))  # (views of one buffer: the decoder's per-batch layout)
+            else:
+                self.lr_masks = full
             self.multi_ious = torch.zeros((n, n_multi), dtype=torch.float32, device=dev)
             self.pred_ious = None
         else:
+            if chunk_prompts is not None:
+                raise ValueError("chunk_prompts needs n_multi > 1 (the decoder's raw multimask outputs)")
             self.lr_masks = torch.zeros((n, 256, 256), dtype=torch.float32, device=dev)
             self.pred_ious = torch.zeros((n,), dtype=torch.float32, device=dev)
             self.multi_ious = None
@@ -383,14 +416,31 @@ class GraphedMatch:
         self._kw = dict(rle=rle, dense_masks=dense_masks, low_latency=low_latency)
         self.tar_feat = torch.zeros((eh * ew, c), dtype=torch.float32, device=dev)
         self.ori_hw = (int(ori_hw[0]), int(ori_hw[1]))
+        self.bind = bool(bind)
+        self.inputs_dev = None
+        if self.bind:
+            lib = stage.lib
+            self.inputs_dev = torch.zeros((int(lib.nttt_sizeof_match_inputs()),), dtype=torch.uint8, device=dev)
+            # the shapes every binding is checked against (nttt_match_bind)
+            self._shapes = _lib.MatchArgs()
+            self._shapes.n, self._shapes.n_multi = self.n, self.n_multi
+            if self.n_multi:
+                k = len(self.lr_masks) if self.chunk_prompts else 1
+                self._shapes.n_chunks, self._shapes.chunk_prompts = k, self.chunk_prompts or self.n
+            self._static_bound = False  # the device struct holds the static buffers' addresses
         self.min_hw = None
         self._size_range = None
         if min_hw is not None:
             self.min_hw = (int(min_hw[0]), int(min_hw[1]))
             if not (1 <= self.min_hw[0] <= self.ori_hw[0] and 1 <= self.min_hw[1] <= self.ori_hw[1]):
                 raise ValueError(f"min_hw {self.min_hw} must lie between 1 and the capacity {self.ori_hw}")
-            # the size the kernels read; replay() rewrites it, stream-ordered, before each launch of the graph
-            self.hw_dev = torch.tensor(self.ori_hw, dtype=torch.int32, device=dev)
+            if self.bind:
+                # the size the kernels read is part of the bound struct: one bind kernel writes inputs and size
+                off = _lib.MatchInputs.ori_hw.offset
+                self.hw_dev = self.inputs_dev[off:off + 8].view(torch.int32)
+            else:
+                # the size the kernels read; replay() rewrites it, stream-ordered, before each launch of the graph
+                self.hw_dev = torch.tensor(self.ori_hw, dtype=torch.int32, device=dev)
             self._size_range = (self.hw_dev, self.min_hw)
         self.iou_thr = iou_thr
         self._slot = ("graph", id(self) if key is None else key)
@@ -404,28 +454,107 @@ class GraphedMatch:
                          torch.zeros((num_out, 4), dtype=torch.int32, device=dev)) if dense_masks else None
         self.graph = None
         self.pending = None
+        self._proto = None  # the prototype tensors the graph was captured with (its kernels read their addresses)
+
+    def _static_inputs(self) -> dict:
+        return dict(lr_masks=self.lr_masks, pred_ious=self.pred_ious, multi_ious=self.multi_ious, tar_feat=self.tar_feat)
+
+    def _bind(self, inputs: dict, hw) -> None:
+        """Write the device struct on the current stream (nttt_match_bind: one kernel, the values in its argument)."""
+        host = _lib.MatchInputs()
+        lr = inputs["lr_masks"]
+        if self.n_multi:
+            for i, t in enumerate(lr if isinstance(lr, list) else [lr]):
+                host.chunks[i] = t.data_ptr()
+            host.multi_ious = inputs["multi_ious"].data_ptr()
+        else:
+            host.logits, host.pred_ious = lr.data_ptr(), inputs["pred_ious"].data_ptr()
+        host.tar_feat = inputs["tar_feat"].data_ptr()
+        host.ori_hw[0], host.ori_hw[1] = int(hw[0]), int(hw[1])
+        stream = torch.cuda.current_stream(self.stage.device).cuda_stream
+        _lib.check(self.stage.lib.nttt_match_bind(self.inputs_dev.data_ptr(), ctypes.byref(host),
+                                                  ctypes.byref(self._shapes), stream), "nttt_match_bind")
+
+    def _check_bound(self, lr_masks, pred_ious, multi_ious, tar_feat) -> dict:
+        """The tensors a replay binds (the static buffers where one is not given), checked against the capture's shapes
+        on the host: dtype, device, contiguity, shape and the 16-byte alignment of every logits base."""
+        dev = self.stage.device
+        dev_index = dev.index if dev.index is not None else torch.cuda.current_device()
+
+        def need(t, shape, name):
+            if not isinstance(t, torch.Tensor):
+                raise TypeError(f"{name} must be a tensor")
+            if t.device.type != "cuda" or t.device.index != dev_index:
+                raise ValueError(f"{name} must be on {dev} (the graph's device), got {t.device}")
+            ops._need(t, torch.float32, name)
+            if tuple(t.shape) != tuple(shape):
+                raise ValueError(f"{name} has shape {tuple(t.shape)}, the graph was captured for {tuple(shape)}")
+            return t
+
+        def aligned(t, name):
+            if t.data_ptr() % 16:
+                raise ValueError(f"{name} must start on a 16-byte boundary (the low-res pass reads it with TMA bulk "
+                                 "copies)")
+            return t
+
+        got = self._static_inputs()
+        if tar_feat is not None:
+            got["tar_feat"] = need(tar_feat, self.tar_feat.shape, "tar_feat")
+        if self.n_multi:
+            if pred_ious is not None:
+                raise ValueError("a multimask graph takes multi_ious, not pred_ious")
+            if multi_ious is not None:
+                got["multi_ious"] = need(multi_ious, self.multi_ious.shape, "multi_ious")
+            if lr_masks is not None:
+                if self.chunk_prompts:
+                    if not isinstance(lr_masks, (list, tuple)) or len(lr_masks) != len(self.lr_masks):
+                        raise ValueError(f"lr_masks must be the decoder's list of {len(self.lr_masks)} per-batch chunks")
+                    got["lr_masks"] = [aligned(need(t, ref.shape, f"lr_masks chunk {i}"), f"lr_masks chunk {i}")
+                                       for i, (t, ref) in enumerate(zip(lr_masks, self.lr_masks))]
+                else:
+                    got["lr_masks"] = aligned(need(lr_masks, self.lr_masks.shape, "lr_masks"), "lr_masks")
+        else:
+            if multi_ious is not None:
+                raise ValueError("a single-plane graph takes pred_ious, not multi_ious")
+            if pred_ious is not None:
+                got["pred_ious"] = need(pred_ious, self.pred_ious.shape, "pred_ious")
+            if lr_masks is not None:
+                got["lr_masks"] = aligned(need(lr_masks, self.lr_masks.shape, "lr_masks"), "lr_masks")
+        return got
 
     def capture(self):
         """Warm up (workspace allocation, antialias tables) on a side stream, then capture."""
-        side = torch.cuda.Stream(self.stage.device)
-        side.wait_stream(torch.cuda.current_stream(self.stage.device))
+        st = self.stage
+        if self.bind:
+            self._bind(self._static_inputs(), self.ori_hw)
+            self._static_bound = True
+        kw = dict(slot=self._slot, iou_thr=self.iou_thr, persistent_out=self._out, multi_ious=self.multi_ious,
+                  multi_first=self.multi_first, size_range=self._size_range, bound_inputs=self.inputs_dev, **self._kw)
+        side = torch.cuda.Stream(st.device)
+        side.wait_stream(torch.cuda.current_stream(st.device))
         with torch.cuda.stream(side):
             for _ in range(2):
-                self.stage.match_async(self.lr_masks, self.pred_ious, self.tar_feat, self.ori_hw, slot=self._slot,
-                                       iou_thr=self.iou_thr, persistent_out=self._out, multi_ious=self.multi_ious,
-                                       multi_first=self.multi_first, size_range=self._size_range, **self._kw)
-        torch.cuda.current_stream(self.stage.device).wait_stream(side)
-        torch.cuda.synchronize(self.stage.device)
+                st.match_async(self.lr_masks, self.pred_ious, self.tar_feat, self.ori_hw, **kw)
+        torch.cuda.current_stream(st.device).wait_stream(side)
+        torch.cuda.synchronize(st.device)
         self.graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(self.graph):
-            self.pending = self.stage.match_async(self.lr_masks, self.pred_ious, self.tar_feat, self.ori_hw,
-                                                  slot=self._slot, iou_thr=self.iou_thr, persistent_out=self._out,
-                                                  multi_ious=self.multi_ious, multi_first=self.multi_first,
-                                                  size_range=self._size_range, **self._kw)
+            self.pending = st.match_async(self.lr_masks, self.pred_ious, self.tar_feat, self.ori_hw, **kw)
+        self._proto = (st.proto, st.proto_neg)
         return self
 
-    def replay(self, ori_hw=None) -> PendingResult:
-        """Launch the graph on the current stream.  A sized graph needs the image's size `ori_hw=(h, w)`."""
+    def replay(self, ori_hw=None, lr_masks=None, pred_ious=None, multi_ious=None, tar_feat=None) -> PendingResult:
+        """Launch the graph on the current stream.  A sized graph needs the image's size `ori_hw=(h, w)`.
+
+        A bound graph (`bind=True`) also takes the image's inputs: `lr_masks` (a tensor, or with `chunk_prompts` the
+        decoder's list of per-batch chunks), `pred_ious` or `multi_ious`, and `tar_feat`, each float32, contiguous, on the
+        graph's device and of the capture's shape; an input not given is the graph's own static buffer.  Everything is
+        checked before anything is enqueued.  The replay reads the tensors on the current stream: a producer that wrote
+        them on another stream must make this stream wait for it first (`torch.cuda.current_stream().wait_stream(p)`).
+        The result holds them until the graph's next replay."""
+        given = lr_masks is not None or pred_ious is not None or multi_ious is not None or tar_feat is not None
+        if given and not self.bind:
+            raise ValueError("this graph reads its static buffers; capture it with bind=True to pass inputs to replay()")
         if self.min_hw is None:
             if ori_hw is not None and (int(ori_hw[0]), int(ori_hw[1])) != self.ori_hw:
                 raise ValueError(f"this graph serves {self.ori_hw} only; capture it with min_hw to serve a range")
@@ -436,13 +565,20 @@ class GraphedMatch:
             hw = (int(ori_hw[0]), int(ori_hw[1]))
             if not (self.min_hw[0] <= hw[0] <= self.ori_hw[0] and self.min_hw[1] <= hw[1] <= self.ori_hw[1]):
                 raise ValueError(f"size {hw} is outside the graph's range {self.min_hw} .. {self.ori_hw}")
-        if self.graph is None:
-            self.capture()
-        if self.min_hw is not None:
+        inputs = self._check_bound(lr_masks, pred_ious, multi_ious, tar_feat) if given else None
+        st = self.stage
+        if self.graph is None or self._proto[0] is not st.proto or self._proto[1] is not st.proto_neg:
+            self.capture()  # (first replay, or the stage's prototypes were replaced since the capture)
+        if self.bind:
+            if given or self.min_hw is not None or not self._static_bound:
+                self._bind(inputs or self._static_inputs(), hw)
+                self._static_bound = not given
+        elif self.min_hw is not None:
             # One fill kernel on the replay's stream writes both int32 (little-endian: h is the low half): the value
             # travels as a kernel argument, so no host buffer can be overwritten by a later replay before it is read.
             self.hw_dev.view(torch.int64).fill_(hw[0] | (hw[1] << 32))
         self.graph.replay()
         self.pending._meta = None  # the static buffers now hold a new image's result
         self.pending.ori_hw = hw
+        self.pending._bound = inputs  # (the tensors this replay reads, held until the next one)
         return self.pending
