@@ -13,9 +13,7 @@ namespace nttt {
 int launch_lowres_pack(const float*, int, int, int, float, float, uint32_t*, int32_t*, int32_t*, int32_t*, int32_t*,
                        const float*, float, const float* const*, cudaStream_t, float* stab_score = nullptr);
 int launch_multimask_select(const float*, int, int, int, const ChunkTable&, int, size_t, const float**, float*,
-                            cudaStream_t);
-int launch_multimask_select_bound(const float* const*, int, int, int, const float* const*, int, size_t, const float**,
-                                  float*, cudaStream_t);
+                            cudaStream_t, const float* const* ious_at = nullptr, const float* const* bases = nullptr);
 int launch_plane_resolve(const nttt_match_inputs*, int, size_t, const float**, float*, cudaStream_t);
 int launch_match_bind(const nttt_match_inputs&, nttt_match_inputs*, cudaStream_t);
 int launch_project_masks(const AxisTable&, const AxisTable&, const uint32_t*, const int32_t*, int, int, int, int, int,
@@ -40,13 +38,10 @@ int launch_box_nms(const int32_t*, const float*, const int32_t*, const float*, i
 int launch_upsample_pack(const AxisTable&, const AxisTable&, const float*, const uint32_t*, const int32_t*,
                          const int32_t*, int, int, const int32_t*, const int32_t*, int, int, int, uint32_t*, int32_t*,
                          int32_t*, int32_t*, int32_t*, const float* const*, cudaStream_t, int, int, uint32_t* bits_t = nullptr,
-                         bool* wrote_t = nullptr, bool t_only = false, bool low_latency = false, int32_t* zero2 = nullptr);
+                         bool* wrote_t = nullptr, bool low_latency = false, int32_t* zero2 = nullptr,
+                         const SizedDims* sized = nullptr, const SizedAtlas* atlas = nullptr);
 int32_t* ios_pair_counters(void* ws, int max_sel);
 size_t upsample_scratch_bytes(int max_sel, int oh, int ow);
-int launch_upsample_pack_sized(const SizedDims&, const SizedAtlas&, const float*, const uint32_t*, const int32_t*,
-                               const int32_t*, int, int, const int32_t*, const int32_t*, int, uint32_t*, int32_t*,
-                               int32_t*, int32_t*, int32_t*, const float* const*, cudaStream_t, int, int, uint32_t*, bool,
-                               int32_t*);
 int launch_unpack_sparse(const uint32_t*, const int32_t*, const int32_t*, const int32_t*, int, int, int, uint8_t*,
                          int32_t*, cudaStream_t, bool tr = false, const SizedDims* sized = nullptr);
 int launch_unpack(const uint32_t*, const int32_t*, const int32_t*, const int32_t*, int, int, int, uint8_t*,
@@ -899,9 +894,9 @@ static int match_impl(nttt_ctx* ctx, const nttt_match_args* a, const nttt_match_
   const float* const* feat_at = bound ? &in_dev->tar_feat : nullptr;
   if (bound) {
     if (multi)
-      err = launch_multimask_select_bound(&in_dev->multi_ious, n, a->n_multi, a->multi_first,
-                                          chunked ? in_dev->chunks : &in_dev->logits, chunked ? a->chunk_prompts : n,
-                                          (size_t)a->lr_h * a->lr_w, L.mask_ptr, L.plane_score, s);
+      err = launch_multimask_select(nullptr, n, a->n_multi, a->multi_first, ChunkTable{}, chunked ? a->chunk_prompts : n,
+                                    (size_t)a->lr_h * a->lr_w, L.mask_ptr, L.plane_score, s, &in_dev->multi_ious,
+                                    chunked ? in_dev->chunks : &in_dev->logits);
     else
       err = launch_plane_resolve(in_dev, n, (size_t)a->lr_h * a->lr_w, L.mask_ptr, L.plane_score, s);
     if (err) return err;
@@ -970,22 +965,13 @@ static int match_impl(nttt_ctx* ctx, const nttt_match_args* a, const nttt_match_
   // a10/a11
   NTTT_STEP(launch_box_nms(L.box_lr, pred_ious, L.top_label, L.top_score, n, a->nms_thr, max_sel, L.keep,
                            a->counts + 0, sel, a->counts + 1, L.nms_ws, L.nms_ws_bytes, a->iou_thr, a->filter_iou, s));
-  // a12/a9
-  bool wrote_t = false;  // the resize also left the word-column-major copy of the packed masks (v2 path only)
-  if (sized) {
-    // (a range that also takes the general resize keeps the row-major layout on both paths)
-    wrote_t = !atlas->any_general;
-    NTTT_STEP(launch_upsample_pack_sized(sd, *atlas, logits, L.bits_lr, L.box_lr, L.flags, a->lr_h, a->lr_w, sel,
-                                         a->counts + 1, max_sel, L.bits_full, L.rect, L.area_full, L.box_full, L.scratch,
-                                         mask_ptr, s, ctx->upsample_stage_floats, ctx->sm_count, L.bits_t,
-                                         a->low_latency != 0, wrote_t ? ios_pair_counters(L.ios_ws, max_sel) : nullptr));
-  } else {
-    NTTT_STEP(launch_upsample_pack(ux, uy, logits, L.bits_lr, L.box_lr, L.flags, a->lr_h, a->lr_w, sel,
-                                   a->counts + 1, max_sel, a->ori_h, a->ori_w, L.bits_full, L.rect, L.area_full,
-                                   L.box_full, L.scratch, mask_ptr, s, ctx->upsample_stage_floats, ctx->sm_count, L.bits_t,
-                                   &wrote_t, /*t_only=*/true, a->low_latency != 0, ios_pair_counters(L.ios_ws, max_sel)));
-  }
-  // the packed full-resolution masks from here on: word-column major when the v2 resize ran, row-major otherwise
+  // a12/a9 (sized: ux, uy are empty, the tables come from the atlas)
+  bool wrote_t = false;  // the resize left the word-column-major copy of the packed masks instead of the row-major one
+  NTTT_STEP(launch_upsample_pack(ux, uy, logits, L.bits_lr, L.box_lr, L.flags, a->lr_h, a->lr_w, sel, a->counts + 1,
+                                 max_sel, a->ori_h, a->ori_w, L.bits_full, L.rect, L.area_full, L.box_full, L.scratch,
+                                 mask_ptr, s, ctx->upsample_stage_floats, ctx->sm_count, L.bits_t, &wrote_t,
+                                 a->low_latency != 0, ios_pair_counters(L.ios_ws, max_sel), sized, atlas));
+  // the packed full-resolution masks from here on: word-column major when the resize wrote that layout, row-major otherwise
   const uint32_t* packed = wrote_t ? L.bits_t : L.bits_full;
   // a13
   NTTT_STEP(launch_mask_ios(L.bits_full, L.rect, L.area_full, L.box_full, sel, a->counts + 1, max_sel, a->ori_h,

@@ -187,7 +187,8 @@ struct SizedAxis {  // one output size of one axis
   int taps;
   int budget;  // this axis's factor of the two-tap resize's logit tile budget (up2_tile_factor)
 };
-// by-value kernel argument of the sized kernels
+// by-value kernel argument that every kernel depending on the output size takes after its static parameters: read only
+// by the kernel's kSized = true instance (the static instance is passed an empty one)
 struct SizedDims {
   const int32_t* hw;      // [2] (h, w), device
   const SizedAxis* ay;    // [cap_h - min_h + 1] output heights

@@ -56,11 +56,11 @@ struct alignas(16) UpMeta {  // 48 bytes: three 128-bit loads
   int g0, g1;           // row groups [g0, g1) covering [r0, r1)
 };
 
-// Sized entry (nttt_match_image_sized): the output size (h, w) is read from device memory when the kernel runs and the
-// tables come from the context's atlas entry of that size.  The first kernel of each resize chain also writes the status
-// (counts[3]) and, for a size outside the range, empties the selection (counts[1] = 0) so that every later kernel sees
-// no work.  A chain whose path (two-tap or general) the size does not take exits here, as does every resize kernel for a
-// size outside the range.
+// Sized entry (nttt_match_image_sized): the kSized instance of each resize kernel reads the output size (h, w) from
+// device memory when it runs and takes the tables of the context's atlas entry of that size instead of the (oh, ow, t)
+// it was launched with.  The first kernel of the first resize chain also writes the status (counts[3]) and, for a size
+// outside the range, empties the selection (counts[1] = 0) so that every later kernel sees no work.  A chain whose path
+// (two-tap or general) the size does not take exits here, as does every resize kernel for a size outside the range.
 __device__ __forceinline__ bool sized_tables(const SizedDims& d, bool two_tap, bool status, int& oh, int& ow,
                                              UpTables& t) {
   const bool in_range = sized_hw(d, oh, ow);
@@ -76,6 +76,8 @@ __device__ __forceinline__ bool sized_tables(const SizedDims& d, bool two_tap, b
   return true;
 }
 
+// (A function of its own: written inside the kernel, these statements compile to different SASS; this is the one
+// measured.)
 __device__ __forceinline__ void
 upsample_meta_body(const uint32_t* __restrict__ bits_lr, const int32_t* __restrict__ box_lr,
                    const int32_t* __restrict__ flags_lr, int ih, int iw, const int32_t* __restrict__ sel,
@@ -113,24 +115,17 @@ upsample_meta_body(const uint32_t* __restrict__ bits_lr, const int32_t* __restri
   reinterpret_cast<int4*>(rect)[k] = make_int4(m.r0, m.r1, m.w0, m.w1);
 }
 
+template <bool kSized>
 __global__ void __launch_bounds__(256)
 upsample_meta_kernel(const uint32_t* __restrict__ bits_lr, const int32_t* __restrict__ box_lr,
                      const int32_t* __restrict__ flags_lr, int ih, int iw, const int32_t* __restrict__ sel,
                      const int32_t* __restrict__ n_sel, int max_sel, UpTables t, UpMeta* __restrict__ meta,
                      int32_t* __restrict__ rect, int32_t* __restrict__ scratch, const float* __restrict__ logits,
-                     const float* const* __restrict__ mask_ptr) {
-  upsample_meta_body(bits_lr, box_lr, flags_lr, ih, iw, sel, n_sel, max_sel, t, meta, rect, scratch, logits, mask_ptr);
-}
-
-__global__ void __launch_bounds__(256)
-upsample_meta_sized_kernel(const uint32_t* __restrict__ bits_lr, const int32_t* __restrict__ box_lr,
-                           const int32_t* __restrict__ flags_lr, int ih, int iw, const int32_t* __restrict__ sel,
-                           const int32_t* __restrict__ n_sel, int max_sel, UpMeta* __restrict__ meta,
-                           int32_t* __restrict__ rect, int32_t* __restrict__ scratch, const float* __restrict__ logits,
-                           const float* const* __restrict__ mask_ptr, SizedDims d) {
-  int oh, ow;
-  UpTables t;
-  if (!sized_tables(d, false, true, oh, ow, t)) return;
+                     const float* const* __restrict__ mask_ptr, SizedDims d) {
+  if constexpr (kSized) {
+    int oh, ow;
+    if (!sized_tables(d, false, true, oh, ow, t)) return;
+  }
   upsample_meta_body(bits_lr, box_lr, flags_lr, ih, iw, sel, n_sel, max_sel, t, meta, rect, scratch, logits, mask_ptr);
 }
 
@@ -160,11 +155,15 @@ __device__ __forceinline__ void cp_async16(void* smem_dst, const void* gmem_src)
 }
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
 
-__device__ __forceinline__ void
-upsample_pack_body(const uint32_t* __restrict__ bits_lr, const UpMeta* __restrict__ meta, int ih, int iw,
-                   const int32_t* __restrict__ n_sel, int max_sel, int oh, int ow, const UpTables& t,
-                   uint32_t* __restrict__ bits_full, int32_t* __restrict__ area_full, int32_t* __restrict__ box_full,
-                   int32_t* __restrict__ scratch, int stage_floats) {
+template <bool kSized>
+__global__ void __launch_bounds__(kUpThreads, 5)
+upsample_pack_kernel(const uint32_t* __restrict__ bits_lr, const UpMeta* __restrict__ meta, int ih, int iw,
+                     const int32_t* __restrict__ n_sel, int max_sel, int oh, int ow, UpTables t,
+                     uint32_t* __restrict__ bits_full, int32_t* __restrict__ area_full, int32_t* __restrict__ box_full,
+                     int32_t* __restrict__ scratch, int stage_floats, SizedDims d) {
+  if constexpr (kSized) {
+    if (!sized_tables(d, false, false, oh, ow, t)) return;
+  }
   extern __shared__ __align__(16) uint32_t s_lr[];  // packed low-res bits of this mask, rows [clr0, clr1) only; then the tile
   __shared__ int s_red[5];
   const int k = blockIdx.y;
@@ -442,27 +441,6 @@ upsample_pack_body(const uint32_t* __restrict__ bits_lr, const UpMeta* __restric
   }
 }
 
-__global__ void __launch_bounds__(kUpThreads, 5)
-upsample_pack_kernel(const uint32_t* __restrict__ bits_lr, const UpMeta* __restrict__ meta, int ih, int iw,
-                     const int32_t* __restrict__ n_sel, int max_sel, int oh, int ow, UpTables t,
-                     uint32_t* __restrict__ bits_full, int32_t* __restrict__ area_full, int32_t* __restrict__ box_full,
-                     int32_t* __restrict__ scratch, int stage_floats) {
-  upsample_pack_body(bits_lr, meta, ih, iw, n_sel, max_sel, oh, ow, t, bits_full, area_full, box_full, scratch,
-                     stage_floats);
-}
-
-__global__ void __launch_bounds__(kUpThreads, 5)
-upsample_pack_sized_kernel(const uint32_t* __restrict__ bits_lr, const UpMeta* __restrict__ meta, int ih, int iw,
-                           const int32_t* __restrict__ n_sel, int max_sel, uint32_t* __restrict__ bits_full,
-                           int32_t* __restrict__ area_full, int32_t* __restrict__ box_full,
-                           int32_t* __restrict__ scratch, int stage_floats, SizedDims d) {
-  int oh, ow;
-  UpTables t;
-  if (!sized_tables(d, false, false, oh, ow, t)) return;
-  upsample_pack_body(bits_lr, meta, ih, iw, n_sel, max_sel, oh, ow, t, bits_full, area_full, box_full, scratch,
-                     stage_floats);
-}
-
 // ---------------------------------------------------------------------------------------------------
 // v2 — the path every two-tap configuration takes (every span of both axes <= 2 samples: up-scaling, see
 // aa_spans_within_two)
@@ -509,6 +487,15 @@ struct alignas(16) Up2Item {  // 32 bytes, written by the plan kernel
 constexpr int kPlanThreads = 256;
 constexpr int kPlanPerThread = 1024 / kPlanThreads;
 
+// floats of the logit tile: what an item needs at the size (`need`, see up2_tile_factor), bounded by the staging budget
+__host__ __device__ __forceinline__ int up2_tile_floats(long need, int stage_floats) {
+  int floats = (int)(need < stage_floats ? need : stage_floats);
+  if (floats < 0) floats = 0;
+  return (floats + 3) & ~3;
+}
+
+// (A function of its own: written inside the kernel, these statements compile to different SASS; this is the one
+// measured.)
 __device__ __forceinline__ void
 upsample_plan_body(const uint32_t* __restrict__ bits_lr, const int32_t* __restrict__ box_lr,
                    const int32_t* __restrict__ flags_lr, int ih, int iw, const int32_t* __restrict__ sel,
@@ -657,37 +644,25 @@ upsample_plan_body(const uint32_t* __restrict__ bits_lr, const int32_t* __restri
   if (blockIdx.x == 0 && tid == 0) { ctr[0] = base; ctr[1] = 0; }
 }
 
+// tile_cap_floats: the tile budget of the size.  The kSized instance derives it on the device from the size's budget
+// factors, bounded by stage_floats (the context's staging budget) as launch_upsample_pack does for a static size;
+// status: this is the first kernel of the sized entry's resize.
+template <bool kSized>
 __global__ void __launch_bounds__(kPlanThreads)
 upsample_plan_kernel(const uint32_t* __restrict__ bits_lr, const int32_t* __restrict__ box_lr,
                      const int32_t* __restrict__ flags_lr, int ih, int iw, const int32_t* __restrict__ sel,
                      const int32_t* __restrict__ n_sel, int max_sel, UpTables t, UpMeta* __restrict__ meta,
                      int32_t* __restrict__ rect, int32_t* __restrict__ scratch, const float* __restrict__ logits,
                      const float* const* __restrict__ mask_ptr, Up2Item* __restrict__ items, int32_t* __restrict__ ctr,
-                     int32_t* __restrict__ area_full, int32_t* __restrict__ box_full, int oh, int ow, int tile_cap_floats) {
+                     int32_t* __restrict__ area_full, int32_t* __restrict__ box_full, int oh, int ow, int tile_cap_floats,
+                     int stage_floats, bool status, SizedDims d) {
   chain_wait();
+  if constexpr (kSized) {
+    if (!sized_tables(d, true, status, oh, ow, t)) return;
+    tile_cap_floats = up2_tile_floats((long)d.ay[oh - d.min_h].budget * (long)d.ax[ow - d.min_w].budget, stage_floats);
+  }
   upsample_plan_body(bits_lr, box_lr, flags_lr, ih, iw, sel, n_sel, max_sel, t, meta, rect, scratch, logits, mask_ptr,
                      items, ctr, area_full, box_full, oh, ow, tile_cap_floats);
-}
-
-// stage_floats: the context's staging budget; the tile budget of the size is derived from it as launch_upsample_pack does
-__global__ void __launch_bounds__(kPlanThreads)
-upsample_plan_sized_kernel(const uint32_t* __restrict__ bits_lr, const int32_t* __restrict__ box_lr,
-                           const int32_t* __restrict__ flags_lr, int ih, int iw, const int32_t* __restrict__ sel,
-                           const int32_t* __restrict__ n_sel, int max_sel, UpMeta* __restrict__ meta,
-                           int32_t* __restrict__ rect, int32_t* __restrict__ scratch, const float* __restrict__ logits,
-                           const float* const* __restrict__ mask_ptr, Up2Item* __restrict__ items,
-                           int32_t* __restrict__ ctr, int32_t* __restrict__ area_full, int32_t* __restrict__ box_full,
-                           int stage_floats, bool status, SizedDims d) {
-  chain_wait();
-  int oh, ow;
-  UpTables t;
-  if (!sized_tables(d, true, status, oh, ow, t)) return;
-  const long need = (long)d.ay[oh - d.min_h].budget * (long)d.ax[ow - d.min_w].budget;
-  int tile_floats = (int)(need < stage_floats ? need : stage_floats);
-  if (tile_floats < 0) tile_floats = 0;
-  tile_floats = (tile_floats + 3) & ~3;
-  upsample_plan_body(bits_lr, box_lr, flags_lr, ih, iw, sel, n_sel, max_sel, t, meta, rect, scratch, logits, mask_ptr,
-                     items, ctr, area_full, box_full, oh, ow, tile_floats);
 }
 
 // 16-byte copy that allocates in L1: the two-tap records are a few KB shared by every item an SM processes
@@ -793,11 +768,20 @@ __device__ __forceinline__ void up2_publish(int k, const int (&red)[5], int32_t*
   }
 }
 
-__device__ __forceinline__ void
-upsample_pack2_body(const uint32_t* __restrict__ bits_lr, const UpMeta* __restrict__ meta, int ih, int iw, int oh,
-                    int ow, const UpTables& t, uint32_t* __restrict__ bits_full, uint32_t* __restrict__ bits_t,
-                    int32_t* __restrict__ area_full, int32_t* __restrict__ box_full, int32_t* __restrict__ scratch,
-                    const Up2Item* __restrict__ items, int32_t* __restrict__ ctr) {
+template <bool kSized>
+__global__ void __launch_bounds__(kUp2Threads, kUp2CtasPerSm)
+upsample_pack2_kernel(const uint32_t* __restrict__ bits_lr, const UpMeta* __restrict__ meta, int ih, int iw, int oh,
+                      int ow, UpTables t, uint32_t* __restrict__ bits_full, uint32_t* __restrict__ bits_t,
+                      int32_t* __restrict__ area_full, int32_t* __restrict__ box_full, int32_t* __restrict__ scratch,
+                      const Up2Item* __restrict__ items, int32_t* __restrict__ ctr, int32_t* __restrict__ zero2,
+                      SizedDims d) {
+  chain_wait();
+  // (nullable) two counters of the NEXT stage, zeroed here so that its first kernel can append to them right away (also
+  // for a size out of range)
+  if (zero2 && blockIdx.x == 0 && threadIdx.x == 0) { zero2[0] = 0; zero2[1] = 0; }
+  if constexpr (kSized) {
+    if (!sized_tables(d, true, false, oh, ow, t)) return;
+  }
   extern __shared__ __align__(16) unsigned char s_raw[];
   // two-tap records of the item's columns and rows; the rows from ya0 rounded down to a multiple of 4 (16-byte copies)
   float2* s_xw = reinterpret_cast<float2*>(s_raw);                        // [kUp2Cols * 32]
@@ -1035,31 +1019,6 @@ upsample_pack2_body(const uint32_t* __restrict__ bits_lr, const UpMeta* __restri
   if (tid == 0 && pend_k >= 0) up2_publish(pend_k, pend, scratch, area_full, box_full);
 }
 
-__global__ void __launch_bounds__(kUp2Threads, kUp2CtasPerSm)
-upsample_pack2_kernel(const uint32_t* __restrict__ bits_lr, const UpMeta* __restrict__ meta, int ih, int iw, int oh,
-                      int ow, UpTables t, uint32_t* __restrict__ bits_full, uint32_t* __restrict__ bits_t,
-                      int32_t* __restrict__ area_full, int32_t* __restrict__ box_full, int32_t* __restrict__ scratch,
-                      const Up2Item* __restrict__ items, int32_t* __restrict__ ctr, int32_t* __restrict__ zero2) {
-  chain_wait();
-  // (nullable) two counters of the NEXT stage, zeroed here so that its first kernel can append to them right away
-  if (zero2 && blockIdx.x == 0 && threadIdx.x == 0) { zero2[0] = 0; zero2[1] = 0; }
-  upsample_pack2_body(bits_lr, meta, ih, iw, oh, ow, t, bits_full, bits_t, area_full, box_full, scratch, items, ctr);
-}
-
-__global__ void __launch_bounds__(kUp2Threads, kUp2CtasPerSm)
-upsample_pack2_sized_kernel(const uint32_t* __restrict__ bits_lr, const UpMeta* __restrict__ meta, int ih, int iw,
-                            uint32_t* __restrict__ bits_full, uint32_t* __restrict__ bits_t,
-                            int32_t* __restrict__ area_full, int32_t* __restrict__ box_full,
-                            int32_t* __restrict__ scratch, const Up2Item* __restrict__ items, int32_t* __restrict__ ctr,
-                            int32_t* __restrict__ zero2, SizedDims d) {
-  chain_wait();
-  if (zero2 && blockIdx.x == 0 && threadIdx.x == 0) { zero2[0] = 0; zero2[1] = 0; }  // (also for a size out of range)
-  int oh, ow;
-  UpTables t;
-  if (!sized_tables(d, true, false, oh, ow, t)) return;
-  upsample_pack2_body(bits_lr, meta, ih, iw, oh, ow, t, bits_full, bits_t, area_full, box_full, scratch, items, ctr);
-}
-
 // shared-memory layout of upsample_pack2_kernel in bytes, without / with a logit tile of `tile_floats`
 static size_t up2_fixed_smem(int ih, int iw) {
   const size_t lr_words = (((size_t)ih * (iw / 32) + 4) + 3) & ~(size_t)3;
@@ -1079,110 +1038,86 @@ long up2_tile_factor(int in_size, int out_size, bool rows) {
   return rows ? (long)((kUp2Rows * sc + 6)) : (long)(((kUp2Cols * 32) * sc + 12));
 }
 
+// The full-resolution resize: the general chain (upsample_meta + upsample_pack), the two-tap chain (upsample_plan +
+// upsample_pack2) or both.
+// Static size (sized == nullptr): the tables tx, ty of oh x ow; the two-tap chain when both axes have two-tap records
+// and the size fits its 16-bit item fields and its shared memory, the general chain otherwise.
+// Sized entry (sized, atlas; tx, ty are not read): oh x ow is the capacity, which sets the launch shapes and shared
+// memory (with the largest tile budget of the range); each kernel reads the size and its tables when it runs.  Sizes of
+// the range that take the general path (an axis reaching below the low-res size, see aa_spans_within_two) enqueue its
+// chain as well, and the chain the size does not select exits at its first instruction.
+// bits_t (nullable): the two-tap chain writes the word-column-major copy [k][word][row] instead of the row-major words
+// (every consumer of the fused pipeline reads it) unless a general chain is enqueued as well: the consumers then read
+// one layout whichever chain ran.  *wrote_t tells which layout was written; zero2 (nullable: two counters of the next
+// stage) is zeroed only when it is the transposed one.
 int launch_upsample_pack(const AxisTable& tx, const AxisTable& ty, const float* logits, const uint32_t* bits_lr,
                          const int32_t* box_lr, const int32_t* flags_lr, int ih, int iw, const int32_t* sel,
                          const int32_t* n_sel, int max_sel, int oh, int ow, uint32_t* bits_full, int32_t* rect,
                          int32_t* area_full, int32_t* box_full, int32_t* scratch, const float* const* mask_ptr,
-                         cudaStream_t s, int stage_floats, int sm_count, uint32_t* bits_t, bool* wrote_t, bool t_only,
-                         bool low_latency, int32_t* zero2) {
-  // bits_t (nullable): also write the word-column-major copy [k][word][row]; t_only: and skip the row-major one
-  // (every consumer of the fused pipeline reads the transposed layout).  *wrote_t tells whether the v2 path ran.
+                         cudaStream_t s, int stage_floats, int sm_count, uint32_t* bits_t, bool* wrote_t,
+                         bool low_latency, int32_t* zero2, const SizedDims* sized, const SizedAtlas* atlas) {
   if (wrote_t) *wrote_t = false;
   if (max_sel <= 0) return NTTT_OK;
   if (iw % 32 != 0) return NTTT_EUNSUPPORTED;
-  UpTables t{tx.xmin, tx.xsize, tx.w, tx.taps, ty.xmin, ty.xsize, ty.w, ty.taps, tx.t_lo, tx.t_len, ty.t_lo, ty.t_len,
-             ty.grp_of, ty.grp_start, tx.pk_span, tx.pk_w, ty.pk_span, ty.pk_w};
+  const bool two_tap_fits = oh < 65536 && ow < 65536 && ih * (iw / 32) <= 16384;
+  bool general, two_tap;
+  long budget;  // the two-tap chain's logit tile: what an item of 32 groups x 8 words needs at this scale (+ slack)
+  UpTables t{};
+  if (sized) {
+    general = atlas->any_general;
+    two_tap = atlas->any_two_tap;
+    if (two_tap && !two_tap_fits) return NTTT_EUNSUPPORTED;
+    budget = atlas->max_budget;
+  } else {
+    two_tap = tx.pk_span && ty.pk_span && two_tap_fits;
+    general = !two_tap;
+    budget = up2_tile_factor(ih, oh, true) * up2_tile_factor(iw, ow, false);
+    t = UpTables{tx.xmin, tx.xsize, tx.w, tx.taps, ty.xmin, ty.xsize, ty.w, ty.taps, tx.t_lo, tx.t_len, ty.t_lo,
+                 ty.t_len, ty.grp_of, ty.grp_start, tx.pk_span, tx.pk_w, ty.pk_span, ty.pk_w};
+  }
+  // general: bits (+ one spare word read and masked off by the footprint test), padded to 16 bytes, then the logit tile
+  const size_t bits_bytes = ((((size_t)ih * (iw / 32) + 1) + 3) & ~(size_t)3) * 4;
+  if (general && bits_bytes > 160 * 1024) return NTTT_EUNSUPPORTED;
+  size_t stage_bytes = (size_t)(stage_floats > 0 ? stage_floats : 0) * 4;
+  if (bits_bytes + stage_bytes > 200 * 1024) stage_bytes = 0;
+  const size_t smem1 = bits_bytes + stage_bytes;
+  // two-tap
+  const int tile_floats = up2_tile_floats(budget, stage_floats);
+  const size_t smem2 = up2_fixed_smem(ih, iw) + (size_t)tile_floats * 4;
+  if (two_tap && smem2 > 200 * 1024) return NTTT_EUNSUPPORTED;
+  const bool t_layout = two_tap && !general && bits_t;
+
+  const SizedDims d = sized ? *sized : SizedDims{};
   UpMeta* meta = reinterpret_cast<UpMeta*>(scratch + (size_t)kScratchInts * max_sel);
-  if (tx.pk_span && ty.pk_span && oh < 65536 && ow < 65536 && ih * (iw / 32) <= 16384) {
-    // v2: plan + persistent work-list kernel
+  if (general) {
+    const auto pack = sized ? upsample_pack_kernel<true> : upsample_pack_kernel<false>;
+    if (smem1 > 48 * 1024) NTTT_CUDA(set_dyn_smem(pack, (int)smem1));
+    (sized ? upsample_meta_kernel<true> : upsample_meta_kernel<false>)<<<ceil_div(max_sel, 256), 256, 0, s>>>(
+        bits_lr, box_lr, flags_lr, ih, iw, sel, n_sel, max_sel, t, meta, rect, scratch, logits, mask_ptr, d);
+    NTTT_LAUNCH_CHECK();
+    pack<<<dim3(kUpMaxSplit, max_sel), kUpThreads, smem1, s>>>(bits_lr, meta, ih, iw, n_sel, max_sel, oh, ow, t,
+                                                               bits_full, area_full, box_full, scratch,
+                                                               (int)(stage_bytes / 4), d);
+    NTTT_LAUNCH_CHECK();
+  }
+  if (two_tap) {
     int32_t* ctr = reinterpret_cast<int32_t*>(meta + max_sel);
     Up2Item* items = reinterpret_cast<Up2Item*>(ctr + 4);
-    // tile budget: what an item of 32 groups x 8 words needs at this scale (+ slack), bounded by `stage_floats`
-    long need = up2_tile_factor(ih, oh, true) * up2_tile_factor(iw, ow, false);
-    int tile_floats = (int)(need < stage_floats ? need : stage_floats);
-    if (tile_floats < 0) tile_floats = 0;
-    tile_floats = (tile_floats + 3) & ~3;
-    const size_t smem = up2_fixed_smem(ih, iw) + (size_t)tile_floats * 4;
-    if (smem > 200 * 1024) return NTTT_EUNSUPPORTED;
     // (eight CTAs: the geometry pass is redundant per CTA, the item records are shared out)
-    launch_chain(upsample_plan_kernel, 8, kPlanThreads, 0, s, bits_lr, box_lr, flags_lr, ih, iw, sel, n_sel, max_sel, t, meta, rect,
-                                                    scratch, logits, mask_ptr, items, ctr, area_full, box_full, oh, ow,
-                                                    tile_floats);
+    launch_chain(sized ? upsample_plan_kernel<true> : upsample_plan_kernel<false>, 8, kPlanThreads, 0, s, bits_lr,
+                 box_lr, flags_lr, ih, iw, sel, n_sel, max_sel, t, meta, rect, scratch, logits, mask_ptr, items, ctr,
+                 area_full, box_full, oh, ow, tile_floats, stage_floats, !general, d);
     NTTT_LAUNCH_CHECK();
-    if (smem > 48 * 1024)
-      NTTT_CUDA(set_dyn_smem(upsample_pack2_kernel, (int)smem));
+    const auto pack2 = sized ? upsample_pack2_kernel<true> : upsample_pack2_kernel<false>;
+    if (smem2 > 48 * 1024) NTTT_CUDA(set_dyn_smem(pack2, (int)smem2));
     // many images in flight: one persistent CTA per SM leaves the rest of the SM to the other images' kernels (measured
     // 89.8 / 90.7 / 91.2 / 91.9 us/image with 1 / 2 / 3 / 7 CTAs per SM); one image: kUp2CtasPerSm for the shortest kernel
     const int grid = (sm_count > 0 ? sm_count : 148) * (low_latency ? kUp2CtasPerSm : 1);
-    launch_chain(upsample_pack2_kernel, grid, kUp2Threads, smem, s, bits_lr, meta, ih, iw, oh, ow, t,
-                                                          (bits_t && t_only) ? nullptr : bits_full, bits_t, area_full,
-                                                          box_full, scratch, items, ctr, zero2);
-    NTTT_LAUNCH_CHECK();
-    if (wrote_t) *wrote_t = bits_t != nullptr;
-    return NTTT_OK;
-  }
-  // bits (+ one spare word read and masked off by the footprint test), padded to 16 bytes, then the logit tile
-  const size_t bits_bytes = ((((size_t)ih * (iw / 32) + 1) + 3) & ~(size_t)3) * 4;
-  if (bits_bytes > 160 * 1024) return NTTT_EUNSUPPORTED;
-  size_t stage_bytes = (size_t)(stage_floats > 0 ? stage_floats : 0) * 4;
-  if (bits_bytes + stage_bytes > 200 * 1024) stage_bytes = 0;
-  const size_t smem = bits_bytes + stage_bytes;
-  if (smem > 48 * 1024)
-    NTTT_CUDA(set_dyn_smem(upsample_pack_kernel, (int)smem));
-  upsample_meta_kernel<<<ceil_div(max_sel, 256), 256, 0, s>>>(bits_lr, box_lr, flags_lr, ih, iw, sel, n_sel, max_sel, t,
-                                                              meta, rect, scratch, logits, mask_ptr);
-  NTTT_LAUNCH_CHECK();
-  dim3 grid(kUpMaxSplit, max_sel);
-  upsample_pack_kernel<<<grid, kUpThreads, smem, s>>>(bits_lr, meta, ih, iw, n_sel, max_sel, oh, ow, t, bits_full,
-                                                      area_full, box_full, scratch, (int)(stage_bytes / 4));
-  NTTT_LAUNCH_CHECK();
-  return NTTT_OK;
-}
-// The resize of the sized entry: launch shapes and shared memory from the capacity (and the worst tile budget of the
-// range); each kernel reads the size and its tables when it runs.  Sizes of the range that take the general path
-// (an axis reaching below the low-res size, see aa_spans_within_two) enqueue its chain as well, and the chain the
-// size does not select exits at its first instruction.  With both chains the two-tap one writes the row-major words
-// too (bits_t is then nullptr): the consumers read one layout whichever chain ran.
-int launch_upsample_pack_sized(const SizedDims& d, const SizedAtlas& A, const float* logits, const uint32_t* bits_lr,
-                               const int32_t* box_lr, const int32_t* flags_lr, int ih, int iw, const int32_t* sel,
-                               const int32_t* n_sel, int max_sel, uint32_t* bits_full, int32_t* rect, int32_t* area_full,
-                               int32_t* box_full, int32_t* scratch, const float* const* mask_ptr, cudaStream_t s,
-                               int stage_floats, int sm_count, uint32_t* bits_t, bool low_latency, int32_t* zero2) {
-  if (max_sel <= 0) return NTTT_OK;
-  if (iw % 32 != 0 || d.cap_h >= 65536 || d.cap_w >= 65536) return NTTT_EUNSUPPORTED;
-  UpMeta* meta = reinterpret_cast<UpMeta*>(scratch + (size_t)kScratchInts * max_sel);
-  if (A.any_general) {
-    const size_t bits_bytes = ((((size_t)ih * (iw / 32) + 1) + 3) & ~(size_t)3) * 4;
-    if (bits_bytes > 160 * 1024) return NTTT_EUNSUPPORTED;
-    size_t stage_bytes = (size_t)(stage_floats > 0 ? stage_floats : 0) * 4;
-    if (bits_bytes + stage_bytes > 200 * 1024) stage_bytes = 0;
-    const size_t smem = bits_bytes + stage_bytes;
-    if (smem > 48 * 1024) NTTT_CUDA(set_dyn_smem(upsample_pack_sized_kernel, (int)smem));
-    upsample_meta_sized_kernel<<<ceil_div(max_sel, 256), 256, 0, s>>>(bits_lr, box_lr, flags_lr, ih, iw, sel, n_sel,
-                                                                      max_sel, meta, rect, scratch, logits, mask_ptr, d);
-    NTTT_LAUNCH_CHECK();
-    upsample_pack_sized_kernel<<<dim3(kUpMaxSplit, max_sel), kUpThreads, smem, s>>>(
-        bits_lr, meta, ih, iw, n_sel, max_sel, bits_full, area_full, box_full, scratch, (int)(stage_bytes / 4), d);
+    launch_chain(pack2, grid, kUp2Threads, smem2, s, bits_lr, meta, ih, iw, oh, ow, t, t_layout ? nullptr : bits_full,
+                 t_layout ? bits_t : nullptr, area_full, box_full, scratch, items, ctr, t_layout ? zero2 : nullptr, d);
     NTTT_LAUNCH_CHECK();
   }
-  if (!A.any_two_tap) return NTTT_OK;
-  if (ih * (iw / 32) > 16384) return NTTT_EUNSUPPORTED;
-  int32_t* ctr = reinterpret_cast<int32_t*>(meta + max_sel);
-  Up2Item* items = reinterpret_cast<Up2Item*>(ctr + 4);
-  int tile_floats = (int)(A.max_budget < stage_floats ? A.max_budget : stage_floats);
-  if (tile_floats < 0) tile_floats = 0;
-  tile_floats = (tile_floats + 3) & ~3;
-  const size_t smem = up2_fixed_smem(ih, iw) + (size_t)tile_floats * 4;
-  if (smem > 200 * 1024) return NTTT_EUNSUPPORTED;
-  launch_chain(upsample_plan_sized_kernel, 8, kPlanThreads, 0, s, bits_lr, box_lr, flags_lr, ih, iw, sel, n_sel, max_sel,
-               meta, rect, scratch, logits, mask_ptr, items, ctr, area_full, box_full, stage_floats, !A.any_general, d);
-  NTTT_LAUNCH_CHECK();
-  if (smem > 48 * 1024) NTTT_CUDA(set_dyn_smem(upsample_pack2_sized_kernel, (int)smem));
-  const int grid = (sm_count > 0 ? sm_count : 148) * (low_latency ? kUp2CtasPerSm : 1);
-  launch_chain(upsample_pack2_sized_kernel, grid, kUp2Threads, smem, s, bits_lr, meta, ih, iw,
-               A.any_general ? bits_full : nullptr, A.any_general ? nullptr : bits_t, area_full, box_full, scratch,
-               items, ctr, zero2, d);
-  NTTT_LAUNCH_CHECK();
+  if (wrote_t) *wrote_t = t_layout;
   return NTTT_OK;
 }
 
@@ -1202,12 +1137,18 @@ constexpr int kUnpackRows = 32;   // output rows per CTA
 constexpr int kUnpackUnroll = 4;  // words per thread in flight
 
 // (oh, ow): the size of the packed masks; output plane j starts at out + j * oplane, rows are ostride bytes apart and
-// bytes up to ostride may be written (the pad bits of the last word are zero).  The static entry passes
-// ostride = ow, oplane = oh * ow; the sized entry the capacity's strides, and writes the [oh, ow] corner of the plane.
-__device__ __forceinline__ void
-unpack_masks_body(const uint32_t* __restrict__ bits_full, const int32_t* __restrict__ rect,
-                  const int32_t* __restrict__ index, const int32_t* __restrict__ count, int max_count, int oh, int ow,
-                  int ostride, size_t oplane, uint8_t* __restrict__ out, bool tr) {
+// bytes up to ostride may be written (the pad bits of the last word are zero).  A static size has ostride = ow,
+// oplane = oh * ow; the kSized instance keeps the capacity's strides and writes the [oh, ow] corner of the plane for the
+// size read on the device (out of range: the count is zero).
+template <bool kSized>
+__global__ void __launch_bounds__(256)
+unpack_masks_kernel(const uint32_t* __restrict__ bits_full, const int32_t* __restrict__ rect,
+                    const int32_t* __restrict__ index, const int32_t* __restrict__ count, int max_count, int oh, int ow,
+                    uint8_t* __restrict__ out, bool tr /* packed words are [word][row] instead of [row][word] */,
+                    SizedDims d) {
+  const int ostride = kSized ? d.cap_w : ow;
+  const size_t oplane = kSized ? (size_t)d.cap_h * d.cap_w : (size_t)oh * ow;
+  if constexpr (kSized) sized_hw(d, oh, ow);
   const int j = blockIdx.y;
   if (j >= min(*count, max_count)) return;
   const int k = index ? index[j] : j;
@@ -1252,30 +1193,17 @@ unpack_masks_body(const uint32_t* __restrict__ bits_full, const int32_t* __restr
   }
 }
 
-__global__ void __launch_bounds__(256)
-unpack_masks_kernel(const uint32_t* __restrict__ bits_full, const int32_t* __restrict__ rect,
-                    const int32_t* __restrict__ index, const int32_t* __restrict__ count, int max_count, int oh, int ow,
-                    uint8_t* __restrict__ out, bool tr /* packed words are [word][row] instead of [row][word] */) {
-  unpack_masks_body(bits_full, rect, index, count, max_count, oh, ow, ow, (size_t)oh * ow, out, tr);
-}
-
-__global__ void __launch_bounds__(256)
-unpack_masks_sized_kernel(const uint32_t* __restrict__ bits_full, const int32_t* __restrict__ rect,
-                          const int32_t* __restrict__ index, const int32_t* __restrict__ count, int max_count,
-                          uint8_t* __restrict__ out, bool tr, SizedDims d) {
-  int oh, ow;
-  sized_hw(d, oh, ow);  // (out of range: the count is zero)
-  unpack_masks_body(bits_full, rect, index, count, max_count, oh, ow, d.cap_w, (size_t)d.cap_h * d.cap_w, out, tr);
-}
-
 // Sparse unpack into PERSISTENT output buffers: out[j] still holds the mask the previous call wrote there, whose
 // rect is remembered in prev_rect[j] (all-zero buffers and rects initially).  Two passes over one index space:
 // the OLD rect is cleared where the new rect does not cover it, then the NEW rect is written — so a call touches
 // area(old \ new) + area(new) bytes per mask whatever the distance between the two rects (never their common bounding
 // box, and never oh*ow: the dense unpack is HBM-write-bound on mostly zeros).  Every slot up to max_count is visited
 // so that slots that fall out of use are cleared.
-// (oh, ow), ostride, oplane: as in unpack_masks_body.  The sized entry's rects of earlier, larger images are cleared up
-// to the capacity's row length, so the whole buffer stays the dense result embedded top-left with zeros elsewhere.
+// (oh, ow), ostride, oplane: as in unpack_masks_kernel (out of range: the count is zero and only the previous rects are
+// cleared).  The sized entry's rects of earlier, larger images are cleared up to the capacity's row length, so the whole
+// buffer stays the dense result embedded top-left with zeros elsewhere.
+// (A function of its own: written inside the kernel, these statements compile to different SASS; this is the one
+// measured.)
 __device__ __forceinline__ void
 unpack_sparse_body(const uint32_t* __restrict__ bits_full, const int32_t* __restrict__ rect,
                    const int32_t* __restrict__ index, const int32_t* __restrict__ count, int max_count, int oh, int ow,
@@ -1326,23 +1254,16 @@ unpack_sparse_body(const uint32_t* __restrict__ bits_full, const int32_t* __rest
   }
 }
 
+template <bool kSized>
 __global__ void __launch_bounds__(256)
 unpack_sparse_kernel(const uint32_t* __restrict__ bits_full, const int32_t* __restrict__ rect,
                      const int32_t* __restrict__ index, const int32_t* __restrict__ count, int max_count, int oh, int ow,
-                     uint8_t* __restrict__ out, int32_t* __restrict__ prev_rect, bool tr) {
+                     uint8_t* __restrict__ out, int32_t* __restrict__ prev_rect, bool tr, SizedDims d) {
   chain_wait();
-  unpack_sparse_body(bits_full, rect, index, count, max_count, oh, ow, ow, (size_t)oh * ow, out, prev_rect, tr);
-}
-
-__global__ void __launch_bounds__(256)
-unpack_sparse_sized_kernel(const uint32_t* __restrict__ bits_full, const int32_t* __restrict__ rect,
-                           const int32_t* __restrict__ index, const int32_t* __restrict__ count, int max_count,
-                           uint8_t* __restrict__ out, int32_t* __restrict__ prev_rect, bool tr, SizedDims d) {
-  chain_wait();
-  int oh, ow;
-  sized_hw(d, oh, ow);  // (out of range: the count is zero and only the previous rects are cleared)
-  unpack_sparse_body(bits_full, rect, index, count, max_count, oh, ow, d.cap_w, (size_t)d.cap_h * d.cap_w, out,
-                     prev_rect, tr);
+  const int ostride = kSized ? d.cap_w : ow;
+  const size_t oplane = kSized ? (size_t)d.cap_h * d.cap_w : (size_t)oh * ow;
+  if constexpr (kSized) sized_hw(d, oh, ow);
+  unpack_sparse_body(bits_full, rect, index, count, max_count, oh, ow, ostride, oplane, out, prev_rect, tr);
 }
 
 // sized (nullable): the size is read on the device; oh, ow are then the capacity
@@ -1351,12 +1272,8 @@ int launch_unpack_sparse(const uint32_t* bits_full, const int32_t* rect, const i
                          const SizedDims* sized) {
   if (max_count <= 0) return NTTT_OK;
   dim3 grid(1, max_count);  // one CTA per slot: prev_rect[j] is read and rewritten by the same CTA
-  if (sized)
-    launch_chain(unpack_sparse_sized_kernel, grid, 256, 0, s, bits_full, rect, index, count, max_count, out, prev_rect,
-                 tr, *sized);
-  else
-    launch_chain(unpack_sparse_kernel, grid, 256, 0, s, bits_full, rect, index, count, max_count, oh, ow, out, prev_rect,
-                 tr);
+  launch_chain(sized ? unpack_sparse_kernel<true> : unpack_sparse_kernel<false>, grid, 256, 0, s, bits_full, rect, index,
+               count, max_count, oh, ow, out, prev_rect, tr, sized ? *sized : SizedDims{});
   NTTT_LAUNCH_CHECK();
   return NTTT_OK;
 }
@@ -1365,10 +1282,8 @@ int launch_unpack(const uint32_t* bits_full, const int32_t* rect, const int32_t*
                   int max_count, int oh, int ow, uint8_t* out, cudaStream_t s, bool tr, const SizedDims* sized) {
   if (max_count <= 0) return NTTT_OK;
   dim3 grid(ceil_div(oh, kUnpackRows), max_count);
-  if (sized)
-    unpack_masks_sized_kernel<<<grid, 256, 0, s>>>(bits_full, rect, index, count, max_count, out, tr, *sized);
-  else
-    unpack_masks_kernel<<<grid, 256, 0, s>>>(bits_full, rect, index, count, max_count, oh, ow, out, tr);
+  (sized ? unpack_masks_kernel<true> : unpack_masks_kernel<false>)<<<grid, 256, 0, s>>>(
+      bits_full, rect, index, count, max_count, oh, ow, out, tr, sized ? *sized : SizedDims{});
   NTTT_LAUNCH_CHECK();
   return NTTT_OK;
 }

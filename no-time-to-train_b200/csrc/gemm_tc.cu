@@ -387,6 +387,8 @@ split_rows_kernel(const float* __restrict__ X, int ld, int rows, int k, int kp, 
 // X [k, rows] (row-major, ld) -> out [rows, 3*kp]: transpose + split (for feat [E, C] -> [C, 3*Ep]).
 // 64 (k) x 32 (rows) tiles: 128-byte coalesced reads along `rows`, and every thread writes two consecutive k as one
 // bf16x2, so a warp stores 128 contiguous bytes per segment (kp is a multiple of 64).
+// (A function of its own: written inside the kernel, these statements compile to different SASS; this is the one
+// measured.)
 __device__ __forceinline__ void split_transpose_body(const float* __restrict__ X, int ld, int rows, int k, int kp, int mode,
                                                      __nv_bfloat16* __restrict__ out, uint8_t* __restrict__ nonfinite) {
   // nonfinite (nullable) [kp / 64, ceil(rows / 32)]: 1 where the tile holds an inf or a NaN — a GEMM that skips k-blocks
@@ -425,17 +427,13 @@ __device__ __forceinline__ void split_transpose_body(const float* __restrict__ X
   }
 }
 
+// kBound (nttt_match_image_bound): X's address is read from *x_at (nttt_match_inputs.tar_feat) instead
+template <bool kBound>
 __global__ void __launch_bounds__(256)
 split_transpose_kernel(const float* __restrict__ X, int ld, int rows, int k, int kp, int mode,
-                       __nv_bfloat16* __restrict__ out, uint8_t* __restrict__ nonfinite) {
-  split_transpose_body(X, ld, rows, k, kp, mode, out, nonfinite);
-}
-
-// bound twin (nttt_match_image_bound): the features' address is read from *x_at (nttt_match_inputs.tar_feat)
-__global__ void __launch_bounds__(256)
-split_transpose_bound_kernel(const float* const* __restrict__ x_at, int ld, int rows, int k, int kp, int mode,
-                             __nv_bfloat16* __restrict__ out, uint8_t* __restrict__ nonfinite) {
-  split_transpose_body(*x_at, ld, rows, k, kp, mode, out, nonfinite);
+                       __nv_bfloat16* __restrict__ out, uint8_t* __restrict__ nonfinite,
+                       const float* const* __restrict__ x_at) {
+  split_transpose_body(kBound ? *x_at : X, ld, rows, k, kp, mode, out, nonfinite);
 }
 
 int launch_split_rows(const float* X, int ld, int rows, int k, int kp, int mode, void* out, cudaStream_t s) {
@@ -453,11 +451,8 @@ int launch_split_transpose(const float* X, int ld, int rows, int k, int kp, int 
   if (kp % 64 != 0) return NTTT_EINVAL;  // (callers pad K to 64: the GEMM's K block)
   const int tiles = (kp / 64) * ceil_div(rows, 32);
   const int grid = t_low_latency ? tiles : min(tiles, 148);
-  if (x_at)
-    split_transpose_bound_kernel<<<grid, 256, 0, s>>>(x_at, ld, rows, k, kp, mode, static_cast<__nv_bfloat16*>(out),
-                                                      nonfinite);
-  else
-    split_transpose_kernel<<<grid, 256, 0, s>>>(X, ld, rows, k, kp, mode, static_cast<__nv_bfloat16*>(out), nonfinite);
+  (x_at ? split_transpose_kernel<true> : split_transpose_kernel<false>)<<<grid, 256, 0, s>>>(
+      X, ld, rows, k, kp, mode, static_cast<__nv_bfloat16*>(out), nonfinite, x_at);
   NTTT_LAUNCH_CHECK();
   return NTTT_OK;
 }

@@ -245,12 +245,16 @@ ios_eval_big_pairs(const uint32_t* __restrict__ bits_full, const uint32_t* __res
 // bits_t (nullable): the word-column-major copy [k][word][row] written by upsample_pack2_kernel.  A window is a few words
 // wide and hundreds of rows tall: in the row-major layout every word sits in its own 32-byte sector (ncu: 80 MB through L1
 // for 10 MB of words); in the column-major copy a warp reads 128 contiguous bytes per word column.
-__device__ __forceinline__ void
-ios_eval_body(const uint32_t* __restrict__ bits_full, const uint32_t* __restrict__ bits_t,
-              const IosMeta* __restrict__ meta,
-              const int2* __restrict__ pairs, const int32_t* __restrict__ n_pairs, int max_pairs, int max_sel, int oh,
-              int ow, const float* __restrict__ obj_feats, int c, float* __restrict__ ios,
-              int32_t* __restrict__ inter_out) {
+// kSized (sized entry): the packed masks have the size read on the device (out of range: the pair list is empty).
+template <bool kSized>
+__global__ void __launch_bounds__(kIosThreads)
+ios_eval_kernel(const uint32_t* __restrict__ bits_full, const uint32_t* __restrict__ bits_t,
+                const IosMeta* __restrict__ meta,
+                const int2* __restrict__ pairs, const int32_t* __restrict__ n_pairs, int max_pairs, int max_sel, int oh,
+                int ow, const float* __restrict__ obj_feats, int c, float* __restrict__ ios,
+                int32_t* __restrict__ inter_out, SizedDims d) {
+  chain_wait();
+  if constexpr (kSized) sized_hw(d, oh, ow);
   const int lane = lane_id();
   constexpr int kWarps = kIosThreads / 32;
   const int ow_words = (ow + 31) >> 5;
@@ -335,29 +339,6 @@ ios_eval_body(const uint32_t* __restrict__ bits_full, const uint32_t* __restrict
   ios_eval_big_pairs(bits_full, bits_t, meta, pairs, n_pairs, max_pairs, max_sel, oh, ow, obj_feats, c, ios, inter_out);
 }
 
-__global__ void __launch_bounds__(kIosThreads)
-ios_eval_kernel(const uint32_t* __restrict__ bits_full, const uint32_t* __restrict__ bits_t,
-                const IosMeta* __restrict__ meta,
-                const int2* __restrict__ pairs, const int32_t* __restrict__ n_pairs, int max_pairs, int max_sel, int oh,
-                int ow, const float* __restrict__ obj_feats, int c, float* __restrict__ ios,
-                int32_t* __restrict__ inter_out) {
-  chain_wait();
-  ios_eval_body(bits_full, bits_t, meta, pairs, n_pairs, max_pairs, max_sel, oh, ow, obj_feats, c, ios, inter_out);
-}
-
-// sized entry: the packed masks have the size read on the device (out of range: the pair list is empty)
-__global__ void __launch_bounds__(kIosThreads)
-ios_eval_sized_kernel(const uint32_t* __restrict__ bits_full, const uint32_t* __restrict__ bits_t,
-                      const IosMeta* __restrict__ meta,
-                      const int2* __restrict__ pairs, const int32_t* __restrict__ n_pairs, int max_pairs, int max_sel,
-                      const float* __restrict__ obj_feats, int c, float* __restrict__ ios,
-                      int32_t* __restrict__ inter_out, SizedDims d) {
-  chain_wait();
-  int oh, ow;
-  sized_hw(d, oh, ow);
-  ios_eval_body(bits_full, bits_t, meta, pairs, n_pairs, max_pairs, max_sel, oh, ow, obj_feats, c, ios, inter_out);
-}
-
 // rows of empty full-res masks: 0/0 on the diagonal -> NaN, and torch.max propagates it
 __global__ void __launch_bounds__(256)
 ios_finalize_kernel(const int32_t* __restrict__ area_full, const int32_t* __restrict__ n_sel, int max_sel,
@@ -402,12 +383,9 @@ int launch_mask_ios(const uint32_t* bits_full, const int32_t* rect, const int32_
     NTTT_LAUNCH_CHECK();
   }
   // one CTA per SM when many images are in flight (measured 89.4 vs 90.0 us/image with four), four for one image alone
-  if (sized)
-    launch_chain(ios_eval_sized_kernel, t_low_latency ? 148 * 4 : 148, kIosThreads, 0, s, bits_full, bits_t, meta, pairs,
-                 n_pairs, max_pairs, max_sel, obj_feats, c, ios, inter_out, *sized);
-  else
-    launch_chain(ios_eval_kernel, t_low_latency ? 148 * 4 : 148, kIosThreads, 0, s, bits_full, bits_t, meta, pairs,
-                 n_pairs, max_pairs, max_sel, oh, ow, obj_feats, c, ios, inter_out);
+  launch_chain(sized ? ios_eval_kernel<true> : ios_eval_kernel<false>, t_low_latency ? 148 * 4 : 148, kIosThreads, 0, s,
+               bits_full, bits_t, meta, pairs, n_pairs, max_pairs, max_sel, oh, ow, obj_feats, c, ios, inter_out,
+               sized ? *sized : SizedDims{});
   NTTT_LAUNCH_CHECK();
   if (finalize) {
     ios_finalize_kernel<<<ceil_div(max_sel, 256), 256, 0, s>>>(area_full, n_sel, max_sel, ios);

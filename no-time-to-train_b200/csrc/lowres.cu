@@ -641,11 +641,16 @@ int launch_lowres_pack(const float* logits, int n, int h, int w, float thr, floa
 // resolved; the logits stay in the tensors the decoder returned and are read once, by lowres_pack / upsample_pack,
 // through mask_ptr[].  torch.argmax semantics: the first maximal value wins, NaN counts as maximal.
 // ---------------------------------------------------------------------------------------------------
-// base_of(ch): the base address of chunk ch (a by-value table, or device memory written by nttt_match_bind)
-template <typename BaseOf>
-__device__ __forceinline__ void multimask_select_body(int i, const float* __restrict__ ious, int m, int first,
-                                                      BaseOf base_of, int chunk_prompts, size_t plane_elems,
-                                                      const float** __restrict__ mask_ptr, float* __restrict__ score) {
+// kBound (nttt_match_image_bound): the IoUs' address is read from *ious_at and the chunk bases from bases[] (both inside
+// the nttt_match_inputs struct in device memory, written by nttt_match_bind) instead of ious and the by-value table
+template <bool kBound>
+__global__ void multimask_select_kernel(const float* __restrict__ ious, int n, int m, int first, ChunkTable chunks,
+                                        int chunk_prompts, size_t plane_elems, const float** __restrict__ mask_ptr,
+                                        float* __restrict__ score, const float* const* __restrict__ ious_at,
+                                        const float* const* __restrict__ bases) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  if constexpr (kBound) ious = *ious_at;
   const float* row = ious + (size_t)i * m;
   int best = first;
   float bv = row[first];
@@ -654,46 +659,18 @@ __device__ __forceinline__ void multimask_select_body(int i, const float* __rest
     if (v > bv || (v != v && bv == bv)) { bv = v; best = j; }
   }
   const int ch = i / chunk_prompts;
-  mask_ptr[i] = base_of(ch) + ((size_t)(i - ch * chunk_prompts) * m + best) * plane_elems;
+  const float* base = kBound ? bases[ch] : chunks.base[ch];
+  mask_ptr[i] = base + ((size_t)(i - ch * chunk_prompts) * m + best) * plane_elems;
   score[i] = bv;
 }
 
-__global__ void multimask_select_kernel(const float* __restrict__ ious, int n, int m, int first, ChunkTable chunks,
-                                        int chunk_prompts, size_t plane_elems, const float** __restrict__ mask_ptr,
-                                        float* __restrict__ score) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  multimask_select_body(i, ious, m, first, [&](int ch) { return chunks.base[ch]; }, chunk_prompts, plane_elems, mask_ptr,
-                        score);
-}
-
-// bound twin (nttt_match_image_bound): the IoUs' address at *ious_at, chunk bases at bases[] (both inside the
-// nttt_match_inputs struct in device memory)
-__global__ void multimask_select_bound_kernel(const float* const* __restrict__ ious_at, int n, int m, int first,
-                                              const float* const* __restrict__ bases, int chunk_prompts,
-                                              size_t plane_elems, const float** __restrict__ mask_ptr,
-                                              float* __restrict__ score) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  multimask_select_body(i, *ious_at, m, first, [&](int ch) { return bases[ch]; }, chunk_prompts, plane_elems, mask_ptr,
-                        score);
-}
-
+// ious_at (nullable): read the IoUs' address and the chunk bases from device memory (ious and chunks are then ignored)
 int launch_multimask_select(const float* ious, int n, int m, int first, const ChunkTable& chunks, int chunk_prompts,
-                            size_t plane_elems, const float** mask_ptr, float* score, cudaStream_t s) {
+                            size_t plane_elems, const float** mask_ptr, float* score, cudaStream_t s,
+                            const float* const* ious_at, const float* const* bases) {
   if (n <= 0) return NTTT_OK;
-  multimask_select_kernel<<<ceil_div(n, 256), 256, 0, s>>>(ious, n, m, first, chunks, chunk_prompts, plane_elems, mask_ptr,
-                                                           score);
-  NTTT_LAUNCH_CHECK();
-  return NTTT_OK;
-}
-
-int launch_multimask_select_bound(const float* const* ious_at, int n, int m, int first, const float* const* bases,
-                                  int chunk_prompts, size_t plane_elems, const float** mask_ptr, float* score,
-                                  cudaStream_t s) {
-  if (n <= 0) return NTTT_OK;
-  multimask_select_bound_kernel<<<ceil_div(n, 256), 256, 0, s>>>(ious_at, n, m, first, bases, chunk_prompts, plane_elems,
-                                                                 mask_ptr, score);
+  (ious_at ? multimask_select_kernel<true> : multimask_select_kernel<false>)<<<ceil_div(n, 256), 256, 0, s>>>(
+      ious, n, m, first, chunks, chunk_prompts, plane_elems, mask_ptr, score, ious_at, bases);
   NTTT_LAUNCH_CHECK();
   return NTTT_OK;
 }

@@ -122,11 +122,16 @@ __device__ __forceinline__ uint32_t rle_wrap_edge(const RleGeom& g, int x) {
   return g.r0 > 0 ? rle_prev_column_last(g, x) : 0u;
 }
 
-__device__ __forceinline__ void
-rle_encode_body(const uint32_t* __restrict__ bits_full, const int32_t* __restrict__ rect,
-                const int32_t* __restrict__ slot, const int32_t* __restrict__ count, int max_count, int oh, int ow,
-                int cap_counts, int cap_chars, uint32_t* __restrict__ counts_out, int32_t* __restrict__ n_counts,
-                uint8_t* __restrict__ chars_out, int32_t* __restrict__ n_chars, bool tr) {
+// kSized (sized entry): the masks have the size read on the device (out of range: the count is zero, every length is
+// zeroed)
+template <bool kSized>
+__global__ void __launch_bounds__(kRleThreads)
+rle_encode_kernel(const uint32_t* __restrict__ bits_full, const int32_t* __restrict__ rect,
+                  const int32_t* __restrict__ slot, const int32_t* __restrict__ count, int max_count, int oh, int ow,
+                  int cap_counts, int cap_chars, uint32_t* __restrict__ counts_out, int32_t* __restrict__ n_counts,
+                  uint8_t* __restrict__ chars_out, int32_t* __restrict__ n_chars, bool tr, SizedDims d) {
+  chain_wait();
+  if constexpr (kSized) sized_hw(d, oh, ow);
   extern __shared__ int s_col[];  // boundaries per visited column, then their exclusive prefix
   __shared__ int s_warp[kRleWarps + 1];
   const int j = blockIdx.x;
@@ -242,29 +247,6 @@ rle_encode_body(const uint32_t* __restrict__ bits_full, const int32_t* __restric
   }
 }
 
-__global__ void __launch_bounds__(kRleThreads)
-rle_encode_kernel(const uint32_t* __restrict__ bits_full, const int32_t* __restrict__ rect,
-                  const int32_t* __restrict__ slot, const int32_t* __restrict__ count, int max_count, int oh, int ow,
-                  int cap_counts, int cap_chars, uint32_t* __restrict__ counts_out, int32_t* __restrict__ n_counts,
-                  uint8_t* __restrict__ chars_out, int32_t* __restrict__ n_chars, bool tr) {
-  chain_wait();
-  rle_encode_body(bits_full, rect, slot, count, max_count, oh, ow, cap_counts, cap_chars, counts_out, n_counts, chars_out,
-                  n_chars, tr);
-}
-
-// sized entry: the masks have the size read on the device (out of range: the count is zero, every length is zeroed)
-__global__ void __launch_bounds__(kRleThreads)
-rle_encode_sized_kernel(const uint32_t* __restrict__ bits_full, const int32_t* __restrict__ rect,
-                        const int32_t* __restrict__ slot, const int32_t* __restrict__ count, int max_count,
-                        int cap_counts, int cap_chars, uint32_t* __restrict__ counts_out, int32_t* __restrict__ n_counts,
-                        uint8_t* __restrict__ chars_out, int32_t* __restrict__ n_chars, bool tr, SizedDims d) {
-  chain_wait();
-  int oh, ow;
-  sized_hw(d, oh, ow);
-  rle_encode_body(bits_full, rect, slot, count, max_count, oh, ow, cap_counts, cap_chars, counts_out, n_counts, chars_out,
-                  n_chars, tr);
-}
-
 int launch_rle_encode(const uint32_t* bits_full, const int32_t* rect, const int32_t* slot, const int32_t* count,
                       int max_count, int oh, int ow, int cap_counts, int cap_chars, uint32_t* counts_out,
                       int32_t* n_counts, uint8_t* chars_out, int32_t* n_chars, cudaStream_t s, bool tr,
@@ -274,17 +256,10 @@ int launch_rle_encode(const uint32_t* bits_full, const int32_t* rect, const int3
   if ((unsigned long long)oh * ow > 0xffffffffull) return NTTT_EUNSUPPORTED;
   const size_t smem = sizeof(int) * (size_t)(((ow + 31) / 32 + 1) * 32);
   if (smem > 160 * 1024) return NTTT_EUNSUPPORTED;
-  if (sized) {
-    if (smem > 48 * 1024) NTTT_CUDA(set_dyn_smem(rle_encode_sized_kernel, (int)smem));
-    launch_chain(rle_encode_sized_kernel, max_count, kRleThreads, smem, s, bits_full, rect, slot, count, max_count,
-                 cap_counts, cap_chars, counts_out, n_counts, chars_out, n_chars, tr, *sized);
-    NTTT_LAUNCH_CHECK();
-    return NTTT_OK;
-  }
-  if (smem > 48 * 1024)
-    NTTT_CUDA(set_dyn_smem(rle_encode_kernel, (int)smem));
-  launch_chain(rle_encode_kernel, max_count, kRleThreads, smem, s, bits_full, rect, slot, count, max_count, oh, ow, cap_counts,
-                                                        cap_chars, counts_out, n_counts, chars_out, n_chars, tr);
+  const auto kernel = sized ? rle_encode_kernel<true> : rle_encode_kernel<false>;
+  if (smem > 48 * 1024) NTTT_CUDA(set_dyn_smem(kernel, (int)smem));
+  launch_chain(kernel, max_count, kRleThreads, smem, s, bits_full, rect, slot, count, max_count, oh, ow, cap_counts,
+               cap_chars, counts_out, n_counts, chars_out, n_chars, tr, sized ? *sized : SizedDims{});
   NTTT_LAUNCH_CHECK();
   return NTTT_OK;
 }
