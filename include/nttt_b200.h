@@ -171,7 +171,10 @@ int nttt_similarity_neg_top1(nttt_ctx* ctx, const float* obj_feats, const float*
  * (fp32 inter / (areaA + areaB - inter) > thr, areas without +1); order = score desc, index asc on ties.
  *   keep [max_keep] i32, n_keep [1] i32 : NMS survivors, truncated to max_keep (= out_num)
  *   sel  [max_keep] i32, n_sel  [1] i32 : those of `keep` whose top_score > 0, same order
+ * n <= NTTT_MAX_CANDIDATES; a longer list returns NTTT_EUNSUPPORTED before anything is enqueued.
  */
+/* candidate masks (boxes) per image that nttt_box_nms and nttt_match_image* accept: a 128 x 128 prompt grid */
+#define NTTT_MAX_CANDIDATES 16384
 size_t nttt_nms_workspace_bytes(int n);
 int nttt_box_nms(const int32_t* box, const float* nms_scores, const int32_t* labels, const float* top_score,
                  int n, float iou_thr, int max_keep, int32_t* keep, int32_t* n_keep, int32_t* sel,
@@ -373,6 +376,9 @@ size_t nttt_match_workspace_bytes(int n, int lr_h, int lr_w, int eh, int ew, int
                                   int ori_w, int max_sel);
 size_t nttt_match_workspace_bytes_neg(int n, int lr_h, int lr_w, int eh, int ew, int c, int n_cls, int ori_h,
                                       int ori_w, int max_sel, int l_neg);
+/* args->n <= NTTT_MAX_CANDIDATES (all three entries): a larger n returns NTTT_EUNSUPPORTED before anything is enqueued
+ * and leaves every output, counts included, untouched.  The chunked multimask input then needs
+ * chunk_prompts >= n / NTTT_MAX_CHUNKS (testing_point_bs 256 for a 128 x 128 grid). */
 int nttt_match_image(nttt_ctx* ctx, const nttt_match_args* args, void* stream);
 /* sizeof(nttt_match_args) as compiled, so FFI mirrors can verify their layout */
 size_t nttt_sizeof_match_args(void);

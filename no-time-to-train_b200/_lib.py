@@ -51,6 +51,7 @@ class MatchSizeRange(ctypes.Structure):
 
 
 MAX_CHUNKS = 64  # NTTT_MAX_CHUNKS
+MAX_CANDIDATES = 16384  # NTTT_MAX_CANDIDATES: candidate masks per image (points_per_side up to 128)
 
 
 class MatchInputs(ctypes.Structure):

@@ -542,6 +542,7 @@ int nttt_box_nms(const int32_t* box, const float* nms_scores, const int32_t* lab
                  void* workspace, size_t workspace_bytes, void* stream) {
   if (n < 0 || !keep || !n_keep || !sel || !n_sel) return NTTT_EINVAL;
   if (n > 0 && (!box || !nms_scores || !labels || !top_score || !workspace)) return NTTT_EINVAL;
+  if (n > NTTT_MAX_CANDIDATES) return NTTT_EUNSUPPORTED;
   return launch_box_nms(box, nms_scores, labels, top_score, n, iou_thr, max_keep, keep, n_keep, sel, n_sel, workspace,
                         workspace_bytes, 0.0f, 0, (cudaStream_t)stream);
 }
@@ -803,6 +804,7 @@ static int match_impl(nttt_ctx* ctx, const nttt_match_args* a, const nttt_match_
   if (a->n < 0 || a->lr_h <= 0 || a->lr_w <= 0 || a->eh <= 0 || a->ew <= 0 || a->c <= 0 || a->n_cls <= 0 ||
       a->ori_h <= 0 || a->ori_w <= 0 || a->num_out_instance < 0 || a->max_sel < 0)
     return NTTT_EINVAL;
+  if (a->n > NTTT_MAX_CANDIDATES) return NTTT_EUNSUPPORTED;  // (before any launch: NMS and pooling order stop there)
   if (range && (!range->ori_hw_dev || range->min_h <= 0 || range->min_w <= 0 || range->min_h > a->ori_h ||
                 range->min_w > a->ori_w))
     return NTTT_EINVAL;
@@ -942,7 +944,7 @@ static int match_impl(nttt_ctx* ctx, const nttt_match_args* a, const nttt_match_
   // a6/a7: projection + pooling contraction + normalisation
   // Many images in flight: the pooling GEMM runs on spatially ordered rows and skips the k-blocks a tile of masks does
   // not touch (~45 % of them).  Needs the vector normalisation path (it undoes the order) and <= 32 k-blocks per segment.
-  const bool ordered = !a->low_latency && ctx->pool_order && n > 128 && n <= 8192 && pad64(e) / 64 <= 32 &&
+  const bool ordered = !a->low_latency && ctx->pool_order && n > 128 && n <= NTTT_MAX_CANDIDATES && pad64(e) / 64 <= 32 &&
                        (a->c == 384 || a->c == 768 || a->c == 1024 || a->c == 1536);
   if (ordered) NTTT_STEP_QUIET(launch_pool_order(L.box_lr, n, a->lr_h, L.pool_perm, s));
   NTTT_STEP(launch_project_masks(px, py, L.bits_lr, L.box_lr, n, a->lr_h, a->lr_w, a->eh, a->ew, L.a_split, pad64(e),

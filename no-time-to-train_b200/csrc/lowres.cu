@@ -1182,7 +1182,9 @@ int launch_project_masks(const AxisTable& tx, const AxisTable& ty, const uint32_
 // (top >> 2, bottom >> 2); ranks inside a bin are handed out by an atomic, so the order inside a bin is arbitrary — the
 // row a mask lands in changes nothing in its result.  perm[n] = row of mask n.
 // ---------------------------------------------------------------------------------------------------
+// kMaxPer keys per thread: n <= 1024 * kMaxPer (8: up to 8192 masks, 16: up to 16 384)
 constexpr int kOrderBins = 64 * 64;
+template <int kMaxPer>
 __global__ void __launch_bounds__(1024)
 pool_order_kernel(const int32_t* __restrict__ box, int n, int h, int32_t* __restrict__ perm) {
   chain_wait();
@@ -1192,7 +1194,6 @@ pool_order_kernel(const int32_t* __restrict__ box, int n, int h, int32_t* __rest
   for (int i = tid; i < kOrderBins; i += 1024) s_hist[i] = 0;
   __syncthreads();
   const int shift = 32 - __clz((h - 1) >> 6);  // rows -> at most 64 bins (h = 256: >> 2)
-  constexpr int kMaxPer = 8;  // n <= 8192
   int key[kMaxPer], rank[kMaxPer];
 #pragma unroll
   for (int q = 0; q < kMaxPer; ++q) {
@@ -1248,8 +1249,12 @@ pool_order_kernel(const int32_t* __restrict__ box, int n, int h, int32_t* __rest
 
 int launch_pool_order(const int32_t* box, int n, int h, int32_t* perm, cudaStream_t s) {
   if (n <= 0) return NTTT_OK;
-  if (n > 8192) return NTTT_EUNSUPPORTED;
-  launch_chain(pool_order_kernel, 1, 1024, 0, s, box, n, h, perm);
+  if (n > NTTT_MAX_CANDIDATES) return NTTT_EUNSUPPORTED;
+  static_assert(NTTT_MAX_CANDIDATES <= 16 * 1024, "pool_order_kernel holds at most 16 keys per thread");
+  if (n <= 8 * 1024)
+    launch_chain(pool_order_kernel<8>, 1, 1024, 0, s, box, n, h, perm);
+  else
+    launch_chain(pool_order_kernel<16>, 1, 1024, 0, s, box, n, h, perm);
   NTTT_LAUNCH_CHECK();
   return NTTT_OK;
 }

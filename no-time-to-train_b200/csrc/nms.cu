@@ -73,17 +73,22 @@ nms_sort_kernel(const float* __restrict__ scores, const int32_t* __restrict__ bo
 
 // Long lists (n > 1024): a second order, by (label, score rank).  Class-aware suppression only acts inside a label, so in
 // this order the suppression matrix is block diagonal and nms_mask_kernel skips everything else.  Single CTA, bitonic sort
-// of 32-bit keys (label + bias) << 13 | score position; gathers boxes and labels into the new order and leaves the map
-// class position -> score position for the scan's epilogue.
-constexpr int kClassKeyBias = 8194;  // labels of filtered boxes go down to -2 - 8191
+// of 32-bit keys (label + bias) << kPosBits | score position; gathers boxes and labels into the new order and leaves the
+// map class position -> score position for the scan's epilogue.
+// kPosBits: the position field holds n_pad <= 2^kPosBits (13: up to 8192 boxes, 14: up to 16 384).  Filtered boxes carry
+// the labels -2 - i (i < n), so the bias 2^kPosBits + 2 keeps every label + bias >= 1; class labels stay below
+// 2^(32 - kPosBits) - 2^kPosBits - 3, so that no key reaches the padding key 0xffffffff.
+template <int kPosBits>
 __global__ void __launch_bounds__(1024)
 nms_class_sort_kernel(const float4* __restrict__ sorted_box, const int32_t* __restrict__ sorted_label, int n, int n_pad,
                       int32_t* __restrict__ c2s, float4* __restrict__ cbox, int32_t* __restrict__ clabel) {
+  constexpr int kClassKeyBias = (1 << kPosBits) + 2;
+  static_assert(-2 - ((1 << kPosBits) - 1) + kClassKeyBias >= 1, "the lowest filtered-box label must bias to >= 1");
   chain_wait();
   extern __shared__ unsigned long long s_keys[];
   uint32_t* keys = reinterpret_cast<uint32_t*>(s_keys);
   for (int i = threadIdx.x; i < n_pad; i += blockDim.x)
-    keys[i] = i < n ? (((uint32_t)(sorted_label[i] + kClassKeyBias) << 13) | (uint32_t)i) : 0xffffffffu;
+    keys[i] = i < n ? (((uint32_t)(sorted_label[i] + kClassKeyBias) << kPosBits) | (uint32_t)i) : 0xffffffffu;
   __syncthreads();
   for (int k = 2; k <= n_pad; k <<= 1) {
     for (int j = k >> 1; j > 0; j >>= 1) {
@@ -99,7 +104,7 @@ nms_class_sort_kernel(const float4* __restrict__ sorted_box, const int32_t* __re
     }
   }
   for (int i = threadIdx.x; i < n; i += blockDim.x) {
-    const int ps = (int)(keys[i] & 8191u);
+    const int ps = (int)(keys[i] & ((1u << kPosBits) - 1u));
     c2s[i] = ps;
     cbox[i] = sorted_box[ps];
     clabel[i] = sorted_label[ps];
@@ -188,7 +193,13 @@ nms_mask_kernel(const float4* __restrict__ sorted_box, const int32_t* __restrict
 // resolve + one hand-off per chunk (measured ~1 200 cycles per hop with a flag + two block fences, ~ 300 without).  All warps of the CTA are resident and a chunk only waits on lower chunks, so the spin-waits cannot deadlock.
 // Used for n <= 1024 (32 chunks = 32 warps, rows in registers); longer lists take nms_wave_sparse_kernel below.
 constexpr int kScanThreads = 1024;
-constexpr int kScanMaxN = 8192;
+constexpr int kScanMaxN = 16384;  // longest list of any scan
+constexpr int kScanMidN = 8192;   // lists up to this length keep the smaller shared arrays of the sparse scan
+static_assert(kScanMaxN == NTTT_MAX_CANDIDATES, "the scan serves every list the API accepts");
+// position fields of the class-order keys (nms_class_sort_kernel) of the two list lengths
+constexpr int kClassPosBitsMid = 13, kClassPosBitsMax = 14;
+static_assert((1 << kClassPosBitsMid) >= kScanMidN && (1 << kClassPosBitsMax) >= kScanMaxN,
+              "a class-order key's position field must hold every position of the padded list");
 
 __global__ void __launch_bounds__(kScanThreads, 1)
 nms_wave_kernel(const uint32_t* __restrict__ mt, int row_words, const int32_t* __restrict__ order,
@@ -196,9 +207,10 @@ nms_wave_kernel(const uint32_t* __restrict__ mt, int row_words, const int32_t* _
                 int32_t* __restrict__ keep, int32_t* __restrict__ n_keep, int32_t* __restrict__ sel,
                 int32_t* __restrict__ n_sel) {
   chain_wait();
-  __shared__ uint32_t s_K[kScanMaxN / 32];    // keep bits per chunk, then truncated to max_keep
-  __shared__ uint32_t s_S[kScanMaxN / 32];    // positive-score flags, then `sel` bits
-  __shared__ int s_pre[kScanMaxN / 32 + 1];   // exclusive prefix of popc over the words
+  // (n <= 1024 uses the first 32 words of each array)
+  __shared__ uint32_t s_K[kScanMidN / 32];    // keep bits per chunk, then truncated to max_keep
+  __shared__ uint32_t s_S[kScanMidN / 32];    // positive-score flags, then `sel` bits
+  __shared__ int s_pre[kScanMidN / 32 + 1];   // exclusive prefix of popc over the words
   // hand-off word of a chunk: 0 until its keep bits K are final, then (1 << 32) | K.  Flag and data travel in ONE aligned
   // 64-bit shared-memory word, so neither side needs a fence (two __threadfence_block per hop made a hop ~1 200 cycles)
   __shared__ unsigned long long s_pub[32];
@@ -293,11 +305,12 @@ nms_wave_kernel(const uint32_t* __restrict__ mt, int row_words, const int32_t* _
   if (threadIdx.x == 0) { *n_keep = total_kept; *n_sel = s_pre[row_words]; }
 }
 
-// The same wavefront for lists of up to kScanMaxN boxes (points_per_side 64: 4096 candidates).  A warp owns the chunks
-// c, c + 32, c + 64, ... and handles them in that order (a chunk only waits on lower chunks, which are either earlier
+// The same wavefront for lists of up to kMaxN boxes (points_per_side 64: 4096 candidates; 128: kScanMaxN).  A warp owns
+// the chunks c, c + 32, c + 64, ... and handles them in that order (a chunk only waits on lower chunks, which are either earlier
 // rounds or lower warps of the same round, all resident: no deadlock).  A row no longer fits in registers (128 words at
 // 4096 boxes), and almost all of it is zero, so the mask kernel leaves a per-row bitmap of its non-zero words (`nz`) and a
 // lane loads just those — the scan's work is proportional to the suppression pairs that exist, not to n^2 / 32.
+template <int kMaxN>
 __global__ void __launch_bounds__(kScanThreads, 1)
 nms_wave_sparse_kernel(const uint32_t* __restrict__ mt, const uint32_t* __restrict__ nz, int nz_words, int row_words,
                        const int32_t* __restrict__ order, const int32_t* __restrict__ sorted_label,
@@ -309,10 +322,10 @@ nms_wave_sparse_kernel(const uint32_t* __restrict__ mt, const uint32_t* __restri
   // class order (any order that keeps same-label boxes in score order gives the same greedy result), its keep bits are
   // scattered to score order before the compaction.
   chain_wait();
-  __shared__ uint32_t s_K[kScanMaxN / 32];
-  __shared__ uint32_t s_S[kScanMaxN / 32];
-  __shared__ int s_pre[kScanMaxN / 32 + 1];
-  __shared__ unsigned long long s_pub[kScanMaxN / 32];  // 0, then (1 << 32) | K: flag and keep bits in one word (no fences)
+  __shared__ uint32_t s_K[kMaxN / 32];
+  __shared__ uint32_t s_S[kMaxN / 32];
+  __shared__ int s_pre[kMaxN / 32 + 1];
+  __shared__ unsigned long long s_pub[kMaxN / 32];  // 0, then (1 << 32) | K: flag and keep bits in one word (no fences)
   volatile unsigned long long* pub = s_pub;
   const int lane = lane_id(), warp = warp_id();
   for (int i = threadIdx.x; i < row_words; i += kScanThreads) s_pub[i] = 0ull;
@@ -363,8 +376,8 @@ nms_wave_sparse_kernel(const uint32_t* __restrict__ mt, const uint32_t* __restri
   __syncthreads();
   if (c2s) {  // class order -> score order (s_pub is free now: its low and high halves take the two bit vectors)
     uint32_t* k2 = reinterpret_cast<uint32_t*>(s_pub);
-    uint32_t* s2 = k2 + kScanMaxN / 32;
-    for (int i = threadIdx.x; i < 2 * (kScanMaxN / 32); i += kScanThreads) k2[i] = 0u;
+    uint32_t* s2 = k2 + kMaxN / 32;  // (s_pub holds kMaxN / 32 64-bit words: exactly the two vectors of kMaxN bits)
+    for (int i = threadIdx.x; i < 2 * (kMaxN / 32); i += kScanThreads) k2[i] = 0u;
     __syncthreads();
     for (int j = threadIdx.x; j < n; j += kScanThreads) {
       const uint32_t kb = (s_K[j >> 5] >> (j & 31)) & 1u, sb = (s_S[j >> 5] >> (j & 31)) & 1u;
@@ -474,14 +487,23 @@ int launch_box_nms(const int32_t* box, const float* nms_scores, const int32_t* l
   float4* cbox = reinterpret_cast<float4*>(reinterpret_cast<char*>(nz) + align_up(sizeof(uint32_t) * (size_t)n * nz_words, 256));
   int32_t* clabel = reinterpret_cast<int32_t*>(reinterpret_cast<char*>(cbox) + align_up(sizeof(float4) * (size_t)n, 256));
   int32_t* c2s = reinterpret_cast<int32_t*>(reinterpret_cast<char*>(clabel) + align_up(sizeof(int32_t) * (size_t)n, 256));
-  launch_chain(nms_class_sort_kernel, 1, 1024, sizeof(uint32_t) * (size_t)n_pad, s, sorted_box, sorted_label, n, n_pad, c2s, cbox,
-               clabel);
+  const size_t class_smem = sizeof(uint32_t) * (size_t)n_pad;
+  if (n_pad <= kScanMidN) {
+    launch_chain(nms_class_sort_kernel<kClassPosBitsMid>, 1, 1024, class_smem, s, sorted_box, sorted_label, n, n_pad, c2s, cbox, clabel);
+  } else {
+    if (class_smem > 48 * 1024) NTTT_CUDA(set_dyn_smem(nms_class_sort_kernel<kClassPosBitsMax>, (int)class_smem));
+    launch_chain(nms_class_sort_kernel<kClassPosBitsMax>, 1, 1024, class_smem, s, sorted_box, sorted_label, n, n_pad, c2s, cbox, clabel);
+  }
   NTTT_LAUNCH_CHECK();
   launch_chain(nms_mask_kernel<true>, grid, dim3(32, 8), 0, s, cbox, clabel, n, thr, mask, row_words, nz, nz_words,
                /*class_sorted=*/1);
   NTTT_LAUNCH_CHECK();
-  launch_chain(nms_wave_sparse_kernel, 1, kScanThreads, 0, s, mask, nz, nz_words, row_words, order, clabel, top_score, n,
-               max_keep, keep, n_keep, sel, n_sel, c2s);
+  if (n <= kScanMidN)
+    launch_chain(nms_wave_sparse_kernel<kScanMidN>, 1, kScanThreads, 0, s, mask, nz, nz_words, row_words, order, clabel,
+                 top_score, n, max_keep, keep, n_keep, sel, n_sel, c2s);
+  else
+    launch_chain(nms_wave_sparse_kernel<kScanMaxN>, 1, kScanThreads, 0, s, mask, nz, nz_words, row_words, order, clabel,
+                 top_score, n, max_keep, keep, n_keep, sel, n_sel, c2s);
   NTTT_LAUNCH_CHECK();
   return NTTT_OK;
 }

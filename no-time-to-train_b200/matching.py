@@ -27,6 +27,14 @@ class StageConfig:
     rle_cap_chars: int = 32768
 
 
+def _check_candidates(n: int) -> None:
+    """The stage matches at most `_lib.MAX_CANDIDATES` masks per image (a 128 x 128 prompt grid); refused here, before
+    anything is allocated or enqueued."""
+    if n > _lib.MAX_CANDIDATES:
+        raise ValueError(f"{n} candidate masks exceed the stage's limit of {_lib.MAX_CANDIDATES} per image "
+                         "(points_per_side up to 128)")
+
+
 class PendingResult:
     """Device-side result of one image; `.get()` does the single D2H read of the counts and slices."""
 
@@ -202,6 +210,7 @@ class MatchingStage:
             ops._need(lr_masks, torch.float32, "lr_masks")
             ops._need(pred_ious, torch.float32, "pred_ious")
             n, lh, lw = lr_masks.shape
+        _check_candidates(n)
         eh, ew = self.cfg.enc_hw
         e, c = tar_feat.shape
         if e != eh * ew:
@@ -390,6 +399,7 @@ class GraphedMatch:
                  low_latency: bool = False, min_hw=None, bind: bool = False, chunk_prompts=None):
         dev = stage.device
         eh, ew = stage.cfg.enc_hw
+        _check_candidates(int(n))
         self.stage = stage
         self.n, self.c = int(n), int(c)
         self.n_multi = int(n_multi) if n_multi > 1 else 0

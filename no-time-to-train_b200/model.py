@@ -20,6 +20,7 @@ import torch
 import torch.nn as nn
 import torch.nn.functional as F
 
+from . import _lib
 from .matching import MatchingStage, StageConfig
 from .memory_bank import MemoryBank
 
@@ -218,7 +219,10 @@ class Sam2MatchingBaselineNoAMG(nn.Module):
             self._ensure_prototypes(with_negative)
             sam_in = _normalize(tar_img.unsqueeze(0))
             seam_overridden = type(self)._forward_sam is not Sam2MatchingBaselineNoAMG._forward_sam
-            if self.fuse_candidate_selection and not seam_overridden:
+            # the fused path hands the stage one address per decoder batch, at most _lib.MAX_CHUNKS of them: a denser
+            # grid for its batch size (points_per_side 128 with testing_point_bs 128) takes the compacting seam instead
+            if (self.fuse_candidate_selection and not seam_overridden and
+                    int(self.points_per_side) ** 2 // int(self.testing_point_bs) <= _lib.MAX_CHUNKS):
                 chunks, multi_ious, _ = self._forward_sam_raw(sam_in)
                 out = self.stage.match([c.float().contiguous() for c in chunks], None, tar_feat.float().contiguous(),
                                        ori_hw, iou_thr=float(self.iou_thr),
