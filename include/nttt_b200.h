@@ -442,6 +442,33 @@ int nttt_match_bind(nttt_match_inputs* inputs_dev, const nttt_match_inputs* host
 int nttt_match_image_bound(nttt_ctx* ctx, const nttt_match_args* args, const nttt_match_size_range* range,
                            const nttt_match_inputs* inputs_dev, void* stream);
 
+/* ---------------------------------------------------------------------------------------------------
+ * The whole stage with its memory bank bound when it runs: the prototype table's address and its live class count (and
+ * negative count) are read from a small struct in DEVICE memory, so one enqueue (or one CUDA-graph capture) scores an
+ * image against any bank of up to a class capacity fixed when the call is enqueued.
+ *   nttt_match_image_banked: args->proto and args->proto_neg are ignored; args->n_cls is the class capacity and
+ *   args->l_neg the negative capacity (0: plain cosine scoring; > 0: negative-reference scoring with args->sigma).  The
+ *   workspace is nttt_match_workspace_bytes_neg / _sized at the capacity.  `range` and `inputs_dev` (both nullable) keep
+ *   their meaning: the entry is nttt_match_image, _sized or _bound with the bank read from `bank_dev`.  The similarity
+ *   tap `sim` keeps the capacity's stride [n, capacity]; its columns below the live n_cls hold the similarities.  With
+ *   the live counts equal to the capacity, results are those of the unbanked entries on the same prototypes, bit for bit.
+ *   nttt_match_bank_bind writes the struct, stream-ordered, with one kernel that carries the values as its argument.  It
+ *   first checks the bank against the capacity and returns NTTT_EINVAL before any CUDA call for a null proto, n_cls
+ *   outside [1, capacity->n_cls], a proto_neg that is null when capacity->l_neg > 0 or set when it is 0, l_neg outside
+ *   [1, capacity->l_neg] (negative capacity only), or a bank_dev that is null or not 8-byte aligned.
+ */
+typedef struct nttt_match_bank {
+  const float* proto;     /* [n_cls, c] unit rows (nttt_proto_prepare); class-level averages when proto_neg != NULL */
+  const float* proto_neg; /* [n_cls * l_neg, c] unit rows, or NULL: plain cosine scoring */
+  int32_t n_cls, l_neg;   /* live counts of this bank */
+} nttt_match_bank;
+
+size_t nttt_sizeof_match_bank(void);
+int nttt_match_bank_bind(nttt_match_bank* bank_dev, const nttt_match_bank* host, const nttt_match_args* capacity,
+                         void* stream);
+int nttt_match_image_banked(nttt_ctx* ctx, const nttt_match_args* args, const nttt_match_size_range* range,
+                            const nttt_match_inputs* inputs_dev, const nttt_match_bank* bank_dev, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

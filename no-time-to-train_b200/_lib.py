@@ -60,6 +60,11 @@ class MatchInputs(ctypes.Structure):
                 ("chunks", c_void_p * MAX_CHUNKS), ("ori_hw", c_int32 * 2)]
 
 
+class MatchBank(ctypes.Structure):
+    """Mirror of `nttt_match_bank` (include/nttt_b200.h): the prototype table a banked stage reads on the device."""
+    _fields_ = [("proto", c_void_p), ("proto_neg", c_void_p), ("n_cls", c_int32), ("l_neg", c_int32)]
+
+
 # name -> (restype, argtypes); every symbol include/nttt_b200.h declares
 _P = c_void_p
 SIGNATURES = {
@@ -110,6 +115,9 @@ SIGNATURES = {
     "nttt_sizeof_match_inputs": (c_size_t, []),
     "nttt_match_bind": (c_int, [_P, POINTER(MatchInputs), POINTER(MatchArgs), _P]),
     "nttt_match_image_bound": (c_int, [_P, POINTER(MatchArgs), POINTER(MatchSizeRange), _P, _P]),
+    "nttt_sizeof_match_bank": (c_size_t, []),
+    "nttt_match_bank_bind": (c_int, [_P, POINTER(MatchBank), POINTER(MatchArgs), _P]),
+    "nttt_match_image_banked": (c_int, [_P, POINTER(MatchArgs), POINTER(MatchSizeRange), _P, _P, _P]),
     "nttt_launch_count": (ctypes.c_ulonglong, []),
     "nttt_profile_num_stages": (c_int, []),
     "nttt_profile_stage_name": (c_char_p, [c_int]),

@@ -15,23 +15,27 @@ int launch_lowres_pack(const float*, int, int, int, float, float, uint32_t*, int
 int launch_multimask_select(const float*, int, int, int, const ChunkTable&, int, size_t, const float**, float*,
                             cudaStream_t, const float* const* ious_at = nullptr, const float* const* bases = nullptr);
 int launch_plane_resolve(const nttt_match_inputs*, int, size_t, const float**, float*, cudaStream_t);
-int launch_match_bind(const nttt_match_inputs&, nttt_match_inputs*, cudaStream_t);
+template <typename T>
+int launch_match_bind(const T&, T*, cudaStream_t);  // T: nttt_match_inputs or nttt_match_bank
 int launch_project_masks(const AxisTable&, const AxisTable&, const uint32_t*, const int32_t*, int, int, int, int, int,
                          void*, int, bool, cudaStream_t, const int32_t* perm = nullptr, uint32_t* active = nullptr);
 int launch_pool_order(const int32_t*, int, int, int32_t*, cudaStream_t);
 int launch_normalize_split(const float*, int, const int32_t*, int, int, int, float*, void*, bool, cudaStream_t,
                            const int32_t* perm = nullptr);
 int launch_gemm_tc(const void*, int, const void*, int, float*, int, int, int, int, int, size_t, int*, cudaStream_t,
-                   bool low_latency = false, const uint32_t* a_active = nullptr, const uint8_t* b_nonfinite = nullptr);
+                   bool low_latency = false, const uint32_t* a_active = nullptr, const uint8_t* b_nonfinite = nullptr,
+                   const nttt_match_bank* bank = nullptr, int bank_neg = 0);
 int gemm_tc_pick_splits(int, int, int, int);
-int launch_split_rows(const float*, int, int, int, int, int, void*, cudaStream_t);
+int launch_split_rows(const float*, int, int, int, int, int, void*, cudaStream_t, const nttt_match_bank* bank = nullptr,
+                      int bank_neg = 0);
 int launch_split_transpose(const float*, int, int, int, int, int, void*, cudaStream_t, uint8_t* nonfinite = nullptr,
                            const float* const* x_at = nullptr);
 int launch_normalize_rows(const float*, int, const int32_t*, int, int, float*, bool, cudaStream_t);
 int launch_proto_prepare(const float*, int, int, int, float*, cudaStream_t);
-int launch_top1(const float*, int, size_t, float*, int, int, int, float*, int32_t*, cudaStream_t);
+int launch_top1(const float*, int, size_t, float*, int, int, int, float*, int32_t*, cudaStream_t,
+                const nttt_match_bank* bank = nullptr);
 int launch_neg_top1(const float*, int, size_t, const float*, int, size_t, int, int, int, float, float*, float*, int32_t*,
-                    cudaStream_t);
+                    cudaStream_t, const nttt_match_bank* bank = nullptr);
 size_t nms_workspace_bytes(int n);
 int launch_box_nms(const int32_t*, const float*, const int32_t*, const float*, int, float, int, int32_t*, int32_t*,
                    int32_t*, int32_t*, void*, size_t, float, int, cudaStream_t);
@@ -166,19 +170,20 @@ static size_t sim_partial_floats(int n, int cols, int c) {
   return (size_t)sp * n * cols;
 }
 
-// proto_neg == nullptr: plain cosine scoring.  Otherwise negative-reference scoring: proto is the normalised
-// class-level average, proto_neg [n_cls * l_neg, c] the normalised negative instance averages.
+// l_neg == 0: plain cosine scoring.  Otherwise negative-reference scoring: proto is the normalised class-level average,
+// proto_neg [n_cls * l_neg, c] the normalised negative instance averages.
 static int sim_top1(const float* obj_feats, const float* proto, const float* proto_neg, int l_neg, float sigma, int n,
                     int c, int n_cls, float* sim, float* partials, float* partials_neg, float* top_score,
                     int32_t* top_label, void* a_split, void* b_split, bool a_ready, int sm_count, cudaStream_t s,
-                    void* p_split = nullptr, bool p_ready = false) {
+                    void* p_split = nullptr, bool p_ready = false, const nttt_match_bank* bank = nullptr) {
   // p_split (nullable): a buffer of its own for the split prototypes, so that they can be prepared before b_split is free
   // (p_ready: already done, on the side stream of the low-latency mode); without it they go through b_split
+  // bank (nullable): the prototypes are the bound bank's (proto and proto_neg are ignored), n_cls and l_neg its capacity
   const int cp = pad64(c);
   int err = a_ready ? NTTT_OK : launch_split_rows(obj_feats, c, n, c, cp, 0, a_split, s);
   if (err) return err;
   void* pb = p_split ? p_split : b_split;
-  err = p_ready ? NTTT_OK : launch_split_rows(proto, c, n_cls, c, cp, 1, pb, s);
+  err = p_ready ? NTTT_OK : launch_split_rows(proto, c, n_cls, c, cp, 1, pb, s, bank, 0);
   if (err) return err;
   int want = gemm_tc_pick_splits(n, n_cls, 3 * cp, sm_count < 148 ? sm_count : 148);
   if (want > kMaxSimSplits) want = kMaxSimSplits;
@@ -187,11 +192,13 @@ static int sim_top1(const float* obj_feats, const float* proto, const float* pro
   if (!t_low_latency) want = 1;
   const size_t stride = (size_t)n * n_cls;
   int splits = 1;
-  err = launch_gemm_tc(a_split, 3 * cp, pb, 3 * cp, partials, n_cls, n, n_cls, 3 * cp, want, stride, &splits, s);
+  err = launch_gemm_tc(a_split, 3 * cp, pb, 3 * cp, partials, n_cls, n, n_cls, 3 * cp, want, stride, &splits, s, false,
+                       nullptr, nullptr, bank, 0);
   if (err) return err;
-  if (!proto_neg) return launch_top1(partials, splits, stride, sim, n_cls, n, n_cls, top_score, top_label, s);
+  if (l_neg <= 0) return launch_top1(partials, splits, stride, sim, n_cls, n, n_cls, top_score, top_label, s, bank);
   const int cols = n_cls * l_neg;
-  err = launch_split_rows(proto_neg, c, cols, c, cp, 1, b_split, s);  // stream-ordered after the GEMM that read b_split
+  // (stream-ordered after the GEMM that read b_split)
+  err = launch_split_rows(proto_neg, c, cols, c, cp, 1, b_split, s, bank, 1);
   if (err) return err;
   int want_n = gemm_tc_pick_splits(n, cols, 3 * cp, sm_count < 148 ? sm_count : 148);
   if (want_n > kMaxSimSplits) want_n = kMaxSimSplits;
@@ -199,10 +206,10 @@ static int sim_top1(const float* obj_feats, const float* proto, const float* pro
   const size_t stride_n = (size_t)n * cols;
   int splits_n = 1;
   err = launch_gemm_tc(a_split, 3 * cp, b_split, 3 * cp, partials_neg, cols, n, cols, 3 * cp, want_n, stride_n, &splits_n,
-                       s);
+                       s, false, nullptr, nullptr, bank, 1);
   if (err) return err;
   return launch_neg_top1(partials, splits, stride, partials_neg, splits_n, stride_n, n, n_cls, l_neg, sigma, sim,
-                         top_score, top_label, s);
+                         top_score, top_label, s, bank);
 }
 
 }  // namespace nttt
@@ -279,6 +286,8 @@ int nttt_build_is_ablation(void) {
 size_t nttt_sizeof_match_args(void) { return sizeof(nttt_match_args); }
 
 size_t nttt_sizeof_match_inputs(void) { return sizeof(nttt_match_inputs); }
+
+size_t nttt_sizeof_match_bank(void) { return sizeof(nttt_match_bank); }
 
 unsigned long long nttt_launch_count(void) { return g_launches.load(); }
 
@@ -798,8 +807,10 @@ int nttt_ctx_atlas_stats(nttt_ctx* ctx, size_t* bytes_host, double* build_ms_hos
 // range == nullptr: nttt_match_image (the size is a->ori_h x a->ori_w); otherwise nttt_match_image_sized
 // in_dev != nullptr: nttt_match_image_bound (the input pointers of `a` are ignored; the kernels that read the inputs
 // take their addresses from *in_dev)
+// bank != nullptr: nttt_match_image_banked (a->proto / proto_neg are ignored, a->n_cls / l_neg are the capacity; the
+// kernels that read the prototypes or the class count take them from *bank)
 static int match_impl(nttt_ctx* ctx, const nttt_match_args* a, const nttt_match_size_range* range, void* stream,
-                      const nttt_match_inputs* in_dev = nullptr) {
+                      const nttt_match_inputs* in_dev = nullptr, const nttt_match_bank* bank = nullptr) {
   if (!ctx || !a) return NTTT_EINVAL;
   if (a->n < 0 || a->lr_h <= 0 || a->lr_w <= 0 || a->eh <= 0 || a->ew <= 0 || a->c <= 0 || a->n_cls <= 0 ||
       a->ori_h <= 0 || a->ori_w <= 0 || a->num_out_instance < 0 || a->max_sel < 0)
@@ -820,7 +831,7 @@ static int match_impl(nttt_ctx* ctx, const nttt_match_args* a, const nttt_match_
   const bool bound = in_dev != nullptr;
   const bool chunked = multi && (bound ? a->n_chunks > 0 : a->logits_chunks_host != nullptr);
   const bool want_rle = a->rle_chars != nullptr;
-  if ((!bound && ((!a->logits && !chunked) || (!multi && !a->pred_ious) || !a->tar_feat)) || !a->proto ||
+  if ((!bound && ((!a->logits && !chunked) || (!multi && !a->pred_ious) || !a->tar_feat)) || (!bank && !a->proto) ||
       (!a->out_masks && !want_rle) || !a->out_boxes || !a->out_scores || !a->out_labels || !a->out_index)
     return NTTT_EINVAL;
   if (bound && chunked &&
@@ -829,8 +840,9 @@ static int match_impl(nttt_ctx* ctx, const nttt_match_args* a, const nttt_match_
   if (want_rle && (!a->rle_counts || !a->rle_n_counts || !a->rle_n_chars || a->rle_cap_counts <= 0 || a->rle_cap_chars <= 0))
     return NTTT_EINVAL;
   if (multi && ((!bound && !a->multi_ious) || a->multi_first < 0 || a->multi_first >= a->n_multi)) return NTTT_EINVAL;
-  const int l_neg = a->proto_neg ? a->l_neg : 0;
-  if (a->proto_neg && (a->l_neg <= 0 || !(a->sigma > 0.0f))) return NTTT_EINVAL;
+  const bool neg = bank ? a->l_neg > 0 : a->proto_neg != nullptr;  // negative-reference scoring
+  if ((bank && a->l_neg < 0) || (neg && (a->l_neg <= 0 || !(a->sigma > 0.0f)))) return NTTT_EINVAL;
+  const int l_neg = neg ? a->l_neg : 0;
   MatchLayout L = carve(a->workspace, n, a->lr_h, a->lr_w, a->eh, a->ew, a->c, a->n_cls, a->ori_h, a->ori_w, max_sel,
                         num_out, l_neg);
   if (a->workspace_bytes < L.total) return NTTT_EWORKSPACE;
@@ -932,7 +944,7 @@ static int match_impl(nttt_ctx* ctx, const nttt_match_args* a, const nttt_match_
     NTTT_CUDA(cudaStreamWaitEvent(ctx->side, ctx->ev_fork, 0));
     err = launch_split_transpose(a->tar_feat, a->c, a->c, e, pad64(e), 1, L.b_split, ctx->side, nullptr, feat_at);
     if (err) return err;
-    err = launch_split_rows(a->proto, a->c, a->n_cls, a->c, pad64(a->c), 1, L.p_split, ctx->side);
+    err = launch_split_rows(a->proto, a->c, a->n_cls, a->c, pad64(a->c), 1, L.p_split, ctx->side, bank, 0);
     if (err) return err;
     NTTT_CUDA(cudaEventRecord(ctx->ev_join, ctx->side));
     side_join.ev = ctx->ev_join;
@@ -958,12 +970,13 @@ static int match_impl(nttt_ctx* ctx, const nttt_match_args* a, const nttt_match_
   NTTT_STEP(pool_contract(nullptr, a->tar_feat, n, e, a->c, L.sums, L.a_split, L.b_split, &n_partials, s,
                           a->low_latency != 0, forked, ordered ? L.pool_active : nullptr, L.b_nonfinite, feat_at));
   bool a_ready = false;
-  NTTT_STEP(normalize_rows(L.sums, n_partials, L.area_lr, n, a->c, obj_feats, L.a_split, &a_ready,
-                           a->proto_neg != nullptr, s, ordered ? L.pool_perm : nullptr));
-  // a7/a8: similarity + top-1
+  NTTT_STEP(normalize_rows(L.sums, n_partials, L.area_lr, n, a->c, obj_feats, L.a_split, &a_ready, neg, s,
+                           ordered ? L.pool_perm : nullptr));
+  // a7/a8: similarity + top-1 (the last step that depends on the class count: NMS, the resize, the IoS term, the decay
+  // and the output encoding read only the top-1 labels and scores)
   NTTT_STEP(sim_top1(obj_feats, a->proto, a->proto_neg, l_neg, a->sigma, n, a->c, a->n_cls, a->sim, L.sim_part,
                      L.sim_part_neg, L.top_score, L.top_label, L.a_split, L.b_split, a_ready, ctx->sm_count, s, L.p_split,
-                     forked));
+                     forked, bank));
   // a10/a11
   NTTT_STEP(launch_box_nms(L.box_lr, pred_ious, L.top_label, L.top_score, n, a->nms_thr, max_sel, L.keep,
                            a->counts + 0, sel, a->counts + 1, L.nms_ws, L.nms_ws_bytes, a->iou_thr, a->filter_iou, s));
@@ -1040,6 +1053,22 @@ int nttt_match_image_bound(nttt_ctx* ctx, const nttt_match_args* a, const nttt_m
                            const nttt_match_inputs* inputs_dev, void* stream) {
   if (!inputs_dev) return NTTT_EINVAL;
   return match_impl(ctx, a, range, stream, inputs_dev);
+}
+
+int nttt_match_bank_bind(nttt_match_bank* bank_dev, const nttt_match_bank* host, const nttt_match_args* capacity,
+                         void* stream) {
+  if (!bank_dev || !host || !capacity || (reinterpret_cast<uintptr_t>(bank_dev) & 7) != 0) return NTTT_EINVAL;
+  if (!host->proto || host->n_cls < 1 || host->n_cls > capacity->n_cls || capacity->l_neg < 0) return NTTT_EINVAL;
+  const bool neg = capacity->l_neg > 0;
+  if (neg ? (!host->proto_neg || host->l_neg < 1 || host->l_neg > capacity->l_neg) : host->proto_neg != nullptr)
+    return NTTT_EINVAL;
+  return launch_match_bind(*host, bank_dev, (cudaStream_t)stream);
+}
+
+int nttt_match_image_banked(nttt_ctx* ctx, const nttt_match_args* a, const nttt_match_size_range* range,
+                            const nttt_match_inputs* inputs_dev, const nttt_match_bank* bank_dev, void* stream) {
+  if (!bank_dev) return NTTT_EINVAL;
+  return match_impl(ctx, a, range, stream, inputs_dev, bank_dev);
 }
 
 }  // extern "C"

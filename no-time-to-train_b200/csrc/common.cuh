@@ -211,6 +211,9 @@ int build_sized_atlas(SizedAtlas& a, cudaStream_t s);  // a: sizes set; fills th
 long up2_tile_factor(int in_size, int out_size, bool rows);
 
 #ifdef __CUDACC__
+// live rows of a bound bank's prototype table (nttt_match_image_banked): its classes, or (neg) its n_cls * l_neg negatives
+__device__ __forceinline__ int bank_rows(const nttt_match_bank* b, int neg) { return neg ? b->n_cls * b->l_neg : b->n_cls; }
+
 // (h, w) of this call; a size outside the range reads as the capacity and returns false
 __device__ __forceinline__ bool sized_hw(const SizedDims& d, int& h, int& w) {
   h = d.hw[0];

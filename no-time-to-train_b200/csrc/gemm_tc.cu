@@ -149,12 +149,14 @@ struct GemmSmem {
   uint32_t act;  // k-blocks of one operand segment that this tile has to multiply (skipping mode)
 };
 
-template <int BN, int STAGES>
+// kBank (nttt_match_image_banked, similarity launches): N is the bank's capacity; the live column count is read from
+// *bank (bank_rows), and tiles that lie wholly at or past it exit before they allocate TMEM or issue a TMA or an MMA.
+template <int BN, int STAGES, bool kBank>
 __global__ void __launch_bounds__(kGemmThreads, 1)
 gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b,
                float* __restrict__ D, int ldd, int M, int N, int total_k_blocks, int kb_per_split,
                size_t split_stride, const uint32_t* __restrict__ a_active, const uint8_t* __restrict__ b_nonfinite,
-               int nkb_seg) {
+               int nkb_seg, const nttt_match_bank* __restrict__ bank, int bank_neg) {
   // Skipping mode (a_active != nullptr; no split-K): K' is nseg = total_k_blocks / nkb_seg segments of nkb_seg k-blocks
   // (the split-bf16 layout: 3), a_active[row] has bit kb set if row `row` of A holds anything but zeros in k-block kb of a
   // segment, b_nonfinite[r-tile * nkb_seg + kb] is 1 if rows 32 r-tile .. +31 of B hold an inf / NaN there.  A k-block in
@@ -164,6 +166,11 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
   auto& sm = *reinterpret_cast<GemmSmem<BN, STAGES>*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int m0 = blockIdx.y * kBM, n0 = blockIdx.x * BN;
+  if constexpr (kBank) {
+    // (the struct is read once the predecessor has completed: this instance does not overlap its set-up with the drain)
+    chain_wait();
+    if (n0 >= bank_rows(bank, bank_neg)) return;
+  }
   // split-K: blockIdx.z owns k-blocks [kb0, kb0 + num_k_blocks) and writes its partial tile to D + z*split_stride
   const int kb0 = blockIdx.z * kb_per_split;
   const int num_k_blocks = min(kb_per_split, total_k_blocks - kb0);
@@ -300,22 +307,22 @@ static int make_map(CUtensorMap* map, const void* base, int rows, int k, int ld,
 
 template <int BN, int STAGES>
 static int launch_tc(const __nv_bfloat16* A, int lda, const __nv_bfloat16* B, int ldb, float* D, int ldd, int M, int N,
-                     int K, int splits, size_t split_stride, cudaStream_t s, const uint32_t* a_active = nullptr,
-                     const uint8_t* b_nonfinite = nullptr) {
+                     int K, int splits, size_t split_stride, cudaStream_t s, const uint32_t* a_active,
+                     const uint8_t* b_nonfinite, const nttt_match_bank* bank, int bank_neg) {
   CUtensorMap ma, mb;
   int err = make_map(&ma, A, M, K, lda, kBM);
   if (err) return err;
   err = make_map(&mb, B, N, K, ldb, BN);
   if (err) return err;
   const size_t smem = sizeof(GemmSmem<BN, STAGES>) + 1024;
-  auto kern = gemm_tc_kernel<BN, STAGES>;
+  auto kern = bank ? gemm_tc_kernel<BN, STAGES, true> : gemm_tc_kernel<BN, STAGES, false>;
   NTTT_CUDA(set_dyn_smem(kern, (int)smem));
   const int total_kb = K / kBK;
   const int kb_per = ceil_div(total_kb, splits);
   dim3 grid(ceil_div(N, BN), ceil_div(M, kBM), ceil_div(total_kb, kb_per));
   const int nkb_seg = (a_active && K % (3 * kBK) == 0) ? K / 3 / kBK : 0;
   launch_chain(kern, grid, kGemmThreads, smem, s, ma, mb, D, ldd, M, N, total_kb, kb_per, split_stride, a_active, b_nonfinite,
-               nkb_seg);
+               nkb_seg, bank, bank_neg);
   NTTT_LAUNCH_CHECK();
   return NTTT_OK;
 }
@@ -323,9 +330,11 @@ static int launch_tc(const __nv_bfloat16* A, int lda, const __nv_bfloat16* B, in
 // A [M, K] and B [N, K] bf16, K a multiple of 64, rows 16-byte aligned (lda, ldb multiples of 8)
 // splits > 1: split-K, partial tile z is written to D + z*split_stride (the caller sums the partials in a fixed
 // order); *splits_out receives the number of partials actually produced.
+// bank (nullable): B is a bound bank's split prototype table of N (the capacity) rows, of which bank_rows(bank, bank_neg)
+// are live; the tiles past them are not computed (gemm_tc_kernel<.., true>).
 int launch_gemm_tc(const void* A, int lda, const void* B, int ldb, float* D, int ldd, int M, int N, int K, int splits,
                    size_t split_stride, int* splits_out, cudaStream_t s, bool low_latency, const uint32_t* a_active,
-                   const uint8_t* b_nonfinite) {
+                   const uint8_t* b_nonfinite, const nttt_match_bank* bank, int bank_neg) {
   if (splits_out) *splits_out = 1;
   if (M <= 0 || N <= 0) return NTTT_OK;
   if (K <= 0 || K % kBK != 0 || lda % 8 != 0 || ldb % 8 != 0 || splits < 1) return NTTT_EINVAL;
@@ -344,9 +353,11 @@ int launch_gemm_tc(const void* A, int lda, const void* B, int ldb, float* D, int
   // shared memory to CTAs of the other kernels of the images in flight (measured 91.8 vs 92.3 us/image; two stages: 92.0).
   const bool bn256 = !low_latency && N >= 512 && M >= 512;
   const bool bn128 = N >= 512 || (N > 64 && N <= 128);  // 65..128 columns: ONE 128-wide tile reads the A operand once instead of twice
-  if (bn256) return launch_tc<256, 3>(a, lda, b, ldb, D, ldd, M, N, K, splits, split_stride, s, a_active, b_nonfinite);
-  if (bn128) return launch_tc<128, 5>(a, lda, b, ldb, D, ldd, M, N, K, splits, split_stride, s, a_active, b_nonfinite);
-  return launch_tc<64, 6>(a, lda, b, ldb, D, ldd, M, N, K, splits, split_stride, s, a_active, b_nonfinite);
+  if (bn256)
+    return launch_tc<256, 3>(a, lda, b, ldb, D, ldd, M, N, K, splits, split_stride, s, a_active, b_nonfinite, bank, bank_neg);
+  if (bn128)
+    return launch_tc<128, 5>(a, lda, b, ldb, D, ldd, M, N, K, splits, split_stride, s, a_active, b_nonfinite, bank, bank_neg);
+  return launch_tc<64, 6>(a, lda, b, ldb, D, ldd, M, N, K, splits, split_stride, s, a_active, b_nonfinite, bank, bank_neg);
 }
 
 // how many K splits fill the machine for an M x N output of 128 x 64 tiles (1 when the tiles already do)
@@ -369,15 +380,24 @@ __device__ __forceinline__ void split_bf16(float x, __nv_bfloat16& hi, __nv_bflo
   lo = __float2bfloat16_rn(x - __bfloat162float(hi));
 }
 
+// kBank (nttt_match_image_banked): X is the bound bank's prototype table (bank->proto, or bank->proto_neg when bank_neg)
+// and `rows` its capacity; rows from the live count (bank_rows) up to the capacity are written as zeros, so that no GEMM
+// tile reads the rows of a bank bound before
+template <bool kBank>
 __global__ void __launch_bounds__(256)
 split_rows_kernel(const float* __restrict__ X, int ld, int rows, int k, int kp, int mode,
-                  __nv_bfloat16* __restrict__ out) {
+                  __nv_bfloat16* __restrict__ out, const nttt_match_bank* __restrict__ bank, int bank_neg) {
   const int r = blockIdx.y;
+  bool live = true;
+  if constexpr (kBank) {
+    X = bank_neg ? bank->proto_neg : bank->proto;
+    live = r < bank_rows(bank, bank_neg);
+  }
   const float* src = X + (size_t)r * ld;
   __nv_bfloat16* dst = out + (size_t)r * 3 * kp;
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < kp; i += gridDim.x * blockDim.x) {
     __nv_bfloat16 hi = __float2bfloat16_rn(0.0f), lo = hi;
-    if (i < k) split_bf16(src[i], hi, lo);
+    if (i < k && live) split_bf16(src[i], hi, lo);
     dst[i] = hi;
     dst[kp + i] = mode == 0 ? hi : lo;
     dst[2 * kp + i] = mode == 0 ? lo : hi;
@@ -436,10 +456,13 @@ split_transpose_kernel(const float* __restrict__ X, int ld, int rows, int k, int
   split_transpose_body(kBound ? *x_at : X, ld, rows, k, kp, mode, out, nonfinite);
 }
 
-int launch_split_rows(const float* X, int ld, int rows, int k, int kp, int mode, void* out, cudaStream_t s) {
+// bank (nullable): split the bound bank's table (X is then ignored; rows = the capacity)
+int launch_split_rows(const float* X, int ld, int rows, int k, int kp, int mode, void* out, cudaStream_t s,
+                      const nttt_match_bank* bank, int bank_neg) {
   if (rows <= 0) return NTTT_OK;
   dim3 grid(ceil_div(kp, 256), rows);
-  split_rows_kernel<<<grid, 256, 0, s>>>(X, ld, rows, k, kp, mode, static_cast<__nv_bfloat16*>(out));
+  (bank ? split_rows_kernel<true> : split_rows_kernel<false>)<<<grid, 256, 0, s>>>(
+      X, ld, rows, k, kp, mode, static_cast<__nv_bfloat16*>(out), bank, bank_neg);
   NTTT_LAUNCH_CHECK();
   return NTTT_OK;
 }

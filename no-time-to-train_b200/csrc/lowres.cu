@@ -695,11 +695,12 @@ int launch_plane_resolve(const nttt_match_inputs* in, int n, size_t plane_elems,
   return NTTT_OK;
 }
 
-// nttt_match_bind: the struct travels as the kernel's argument and is stored with static indices (one 8-byte word per
-// lane and step), so no host buffer is read when the kernel runs
-static_assert(sizeof(nttt_match_inputs) % 8 == 0, "nttt_match_inputs is copied in 8-byte words");
-__global__ void __launch_bounds__(32) match_bind_kernel(nttt_match_inputs v, nttt_match_inputs* __restrict__ dst) {
-  constexpr int kWords = sizeof(nttt_match_inputs) / 8;
+// nttt_match_bind / nttt_match_bank_bind: the struct travels as the kernel's argument and is stored with static indices
+// (one 8-byte word per lane and step), so no host buffer is read when the kernel runs
+template <typename T>
+__global__ void __launch_bounds__(32) match_bind_kernel(T v, T* __restrict__ dst) {
+  static_assert(sizeof(T) % 8 == 0, "the bound structs are copied in 8-byte words");
+  constexpr int kWords = sizeof(T) / 8;
   const unsigned long long* src = reinterpret_cast<const unsigned long long*>(&v);
   unsigned long long* out = reinterpret_cast<unsigned long long*>(dst);
 #pragma unroll
@@ -707,11 +708,14 @@ __global__ void __launch_bounds__(32) match_bind_kernel(nttt_match_inputs v, ntt
     if ((k & 31) == (int)threadIdx.x) out[k] = src[k];
 }
 
-int launch_match_bind(const nttt_match_inputs& v, nttt_match_inputs* dst, cudaStream_t s) {
-  match_bind_kernel<<<1, 32, 0, s>>>(v, dst);
+template <typename T>
+int launch_match_bind(const T& v, T* dst, cudaStream_t s) {
+  match_bind_kernel<T><<<1, 32, 0, s>>>(v, dst);
   NTTT_LAUNCH_CHECK();
   return NTTT_OK;
 }
+template int launch_match_bind(const nttt_match_inputs&, nttt_match_inputs*, cudaStream_t);
+template int launch_match_bind(const nttt_match_bank&, nttt_match_bank*, cudaStream_t);
 
 // ---------------------------------------------------------------------------------------------------
 // Antialias weight tables.  Exact fp32 recipe (every operation individually rounded, no contraction):

@@ -175,10 +175,16 @@ __device__ __forceinline__ float clamp_min0(float x) { return x < 0.0f ? 0.0f : 
 // `k == n_cls` branch applies: score *= (score > 0.6*score)  (Sam2MatchingBaseline_noAMG.py:606-609).
 // `part` holds n_splits split-K partial similarity matrices (stride split_stride floats); they are summed here
 // in a fixed order and the sum is written to `sim` (if non-null).
+// kBank (nttt_match_image_banked): n_cls is the bank's capacity (the strides stay ld); the arg-max, the `sim` tap and the
+// one-class rule take the live class count of *bank.  The loop stops there: a padded column (similarity 0) must not beat
+// a row whose live similarities are all negative.
+template <bool kBank>
 __global__ void __launch_bounds__(256)
 top1_kernel(const float* __restrict__ part, int n_splits, size_t split_stride, float* __restrict__ sim, int ld, int n,
-            int n_cls, float* __restrict__ top_score, int32_t* __restrict__ top_label) {
+            int n_cls, float* __restrict__ top_score, int32_t* __restrict__ top_label,
+            const nttt_match_bank* __restrict__ bank) {
   chain_wait();
+  if constexpr (kBank) n_cls = bank->n_cls;
   const int row = blockIdx.x * 8 + warp_id();
   if (row >= n) return;
   const int lane = lane_id();
@@ -204,10 +210,12 @@ top1_kernel(const float* __restrict__ part, int n_splits, size_t split_stride, f
   }
 }
 
+// bank (nullable): the live class count is read from it (n_cls is then the capacity)
 int launch_top1(const float* part, int n_splits, size_t split_stride, float* sim, int ld, int n, int n_cls,
-                float* top_score, int32_t* top_label, cudaStream_t s) {
+                float* top_score, int32_t* top_label, cudaStream_t s, const nttt_match_bank* bank) {
   if (n <= 0) return NTTT_OK;
-  launch_chain(top1_kernel, ceil_div(n, 8), 256, 0, s, part, n_splits, split_stride, sim, ld, n, n_cls, top_score, top_label);
+  launch_chain(bank ? top1_kernel<true> : top1_kernel<false>, ceil_div(n, 8), 256, 0, s, part, n_splits, split_stride, sim,
+               ld, n, n_cls, top_score, top_label, bank);
   NTTT_LAUNCH_CHECK();
   return NTTT_OK;
 }
@@ -216,11 +224,20 @@ int launch_top1(const float* part, int n_splits, size_t split_stride, float* sim
 //   sim_pos = clamp(obj . proto_pos[c], 0);  sim_neg = max_l clamp(obj . proto_neg[c, l], 0)
 //   sim     = sim_pos * exp(-clamp(sim_neg - sim_pos, 0) / sigma)
 // Both similarity matrices arrive as split-K partials and are summed here in a fixed order.
+// kBank (nttt_match_image_banked): n_cls and l_neg are the capacity and fix the strides of the partials and of `sim`; the
+// loops take the live counts of *bank, whose negatives are packed live_cls x live_l (bank_rows) in the GEMM's columns.
+template <bool kBank>
 __global__ void __launch_bounds__(256)
 neg_top1_kernel(const float* __restrict__ part_pos, int splits_pos, size_t stride_pos,
                 const float* __restrict__ part_neg, int splits_neg, size_t stride_neg, int n, int n_cls, int l_neg,
-                float sigma, float* __restrict__ sim, float* __restrict__ top_score, int32_t* __restrict__ top_label) {
+                float sigma, float* __restrict__ sim, float* __restrict__ top_score, int32_t* __restrict__ top_label,
+                const nttt_match_bank* __restrict__ bank) {
   chain_wait();
+  int live_cls = n_cls, live_l = l_neg;
+  if constexpr (kBank) {
+    live_cls = bank->n_cls;
+    live_l = bank->l_neg;
+  }
   const int row = blockIdx.x * 8 + warp_id();
   if (row >= n) return;
   const int lane = lane_id();
@@ -228,14 +245,14 @@ neg_top1_kernel(const float* __restrict__ part_pos, int splits_pos, size_t strid
   const float* pn = part_neg + (size_t)row * n_cls * l_neg;
   float best = -INFINITY;
   int arg = 0x7fffffff;
-  for (int i = lane; i < n_cls; i += 32) {
+  for (int i = lane; i < live_cls; i += 32) {
     float sp = pp[i];
     for (int z = 1; z < splits_pos; ++z) sp += pp[(size_t)z * stride_pos + i];
     sp = clamp_min0(sp);
     float sn = 0.0f;  // clamp(min=0) before the max: the max of clamped values is >= 0; NaN propagates (torch.max)
-    for (int l = 0; l < l_neg; ++l) {
-      float v = pn[i * l_neg + l];
-      for (int z = 1; z < splits_neg; ++z) v += pn[(size_t)z * stride_neg + i * l_neg + l];
+    for (int l = 0; l < live_l; ++l) {
+      float v = pn[i * live_l + l];
+      for (int z = 1; z < splits_neg; ++z) v += pn[(size_t)z * stride_neg + i * live_l + l];
       if (sn == sn && (v != v || v > sn)) sn = v;
     }
     const float v = __fmul_rn(sp, expf(__fdiv_rn(__fmul_rn(-1.0f, clamp_min0(__fsub_rn(sn, sp))), sigma)));
@@ -249,7 +266,7 @@ neg_top1_kernel(const float* __restrict__ part_pos, int splits_pos, size_t strid
     if (top1_beats(ob, oa, best, arg)) { best = ob; arg = oa; }
   }
   if (lane == 0) {
-    if (n_cls == 1) best = best * (float)(best > __fmul_rn(best, 0.6f));
+    if (live_cls == 1) best = best * (float)(best > __fmul_rn(best, 0.6f));
     top_score[row] = best;
     top_label[row] = arg == 0x7fffffff ? 0 : arg;
   }
@@ -257,10 +274,10 @@ neg_top1_kernel(const float* __restrict__ part_pos, int splits_pos, size_t strid
 
 int launch_neg_top1(const float* part_pos, int splits_pos, size_t stride_pos, const float* part_neg, int splits_neg,
                     size_t stride_neg, int n, int n_cls, int l_neg, float sigma, float* sim, float* top_score,
-                    int32_t* top_label, cudaStream_t s) {
+                    int32_t* top_label, cudaStream_t s, const nttt_match_bank* bank) {
   if (n <= 0) return NTTT_OK;
-  launch_chain(neg_top1_kernel, ceil_div(n, 8), 256, 0, s, part_pos, splits_pos, stride_pos, part_neg, splits_neg, stride_neg, n,
-                                                 n_cls, l_neg, sigma, sim, top_score, top_label);
+  launch_chain(bank ? neg_top1_kernel<true> : neg_top1_kernel<false>, ceil_div(n, 8), 256, 0, s, part_pos, splits_pos,
+               stride_pos, part_neg, splits_neg, stride_neg, n, n_cls, l_neg, sigma, sim, top_score, top_label, bank);
   NTTT_LAUNCH_CHECK();
   return NTTT_OK;
 }

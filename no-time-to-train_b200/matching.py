@@ -35,11 +35,57 @@ def _check_candidates(n: int) -> None:
                          "(points_per_side up to 128)")
 
 
+@dataclass(frozen=True)
+class PreparedBank:
+    """One memory bank prepared for scoring (`MatchingStage.prepare_bank*`), once per bank: unit-row prototypes on the
+    stage's device.  `proto` [n_cls, c] (the class-level averages when `proto_neg` is set), `proto_neg`
+    [n_cls * l_neg, c] or None (plain cosine scoring)."""
+    proto: torch.Tensor
+    proto_neg: torch.Tensor | None
+    n_cls: int
+    l_neg: int
+    c: int
+
+
+def _check_bank(bank, capacity, c: int, device: torch.device) -> None:
+    """A bank against a banked stage's capacity (n_cls, l_neg) and feature width, on the host, before anything is
+    enqueued: the kernels read the prototypes' addresses and live counts from the device and check nothing."""
+    if not isinstance(bank, PreparedBank):
+        raise TypeError("bank must be a PreparedBank (MatchingStage.prepare_bank / prepare_bank_with_negatives)")
+    cap_cls, cap_neg = capacity
+    if bank.c != c:
+        raise ValueError(f"the bank's prototypes have {bank.c} channels, the stage's features {c}")
+    dev_index = device.index if device.index is not None else torch.cuda.current_device()
+    for name, t, rows in (("proto", bank.proto, bank.n_cls), ("proto_neg", bank.proto_neg, bank.n_cls * bank.l_neg)):
+        if t is None:
+            continue
+        if not isinstance(t, torch.Tensor) or t.device.type != "cuda" or t.device.index != dev_index:
+            raise ValueError(f"bank.{name} must be a tensor on {device}")
+        if t.dtype != torch.float32 or not t.is_contiguous():
+            raise ValueError(f"bank.{name} must be contiguous float32, got {t.dtype}")
+        if tuple(t.shape) != (rows, c):
+            raise ValueError(f"bank.{name} has shape {tuple(t.shape)}, expected {(rows, c)}")
+    if not 1 <= bank.n_cls <= cap_cls:
+        raise ValueError(f"the bank has {bank.n_cls} classes, the capacity is {cap_cls}")
+    if (bank.proto_neg is not None) != (cap_neg > 0):
+        raise ValueError("a negative-reference bank needs a negative capacity (bank_capacity=(n_cls, l_neg > 0)), and a "
+                         "plain bank a capacity without negatives")
+    if cap_neg > 0 and not 1 <= bank.l_neg <= cap_neg:
+        raise ValueError(f"the bank has {bank.l_neg} negatives per class, the capacity is {cap_neg}")
+
+
+def _bank_capacity(bank_capacity) -> tuple:
+    cap = (int(bank_capacity[0]), int(bank_capacity[1]))
+    if cap[0] < 1 or cap[1] < 0:
+        raise ValueError(f"bank_capacity {cap} needs n_cls >= 1 and l_neg >= 0")
+    return cap
+
+
 class PendingResult:
     """Device-side result of one image; `.get()` does the single D2H read of the counts and slices."""
 
     def __init__(self, stage, masks, boxes, scores, labels, index, counts, taps, ori_hw, keepalive, rle=None, meta=None,
-                 sized=False):
+                 sized=False, sim_cols=None):
         self._stage = stage
         self.masks, self.boxes, self.scores, self.labels, self.index = masks, boxes, scores, labels, index
         self.counts = counts
@@ -53,6 +99,8 @@ class PendingResult:
         # size of the image the buffers hold now; the stage reports a size outside its range in counts[3]
         self._sized = sized
         self._bound = None  # a bound graph's replay: the tensors it reads (GraphedMatch.replay)
+        self._bank = None  # a banked graph's replay: the bank it reads
+        self._sim_cols = sim_cols  # banked: the live columns of the [n, capacity] `sim` tap
 
     def rle_segmentations(self) -> list:
         """The outputs as COCO `segmentation` dicts ({"size": [h, w], "counts": str}) — what
@@ -116,7 +164,7 @@ class PendingResult:
         out["counts"] = dict(n_keep=n_keep, n_sel=n_sel, n_out=n_out)
         out["index"] = self.index[:n_out]
         if self.taps:
-            out["taps"] = self.taps
+            out["taps"] = self.taps if self._sim_cols is None else dict(self.taps, sim=self.taps["sim"][:, :self._sim_cols])
         return out
 
 
@@ -140,24 +188,45 @@ class MatchingStage:
         self.n_cls = 0
         self._ws = {}
 
-    def set_prototypes(self, feats_ins_avg: torch.Tensor) -> None:
+    def prepare_bank(self, feats_ins_avg: torch.Tensor) -> PreparedBank:
         """normalize(mean over all L slots) once per bank (`matching_baseline_utils.py:893-894`)."""
         f = feats_ins_avg.to(device=self.device, dtype=torch.float32).contiguous()
-        self.proto = ops.proto_prepare(f)
-        self.proto_neg, self.l_neg = None, 0
-        self.n_cls = f.shape[0]
+        return PreparedBank(ops.proto_prepare(f), None, f.shape[0], 0, f.shape[2])
 
-    def set_prototypes_with_negatives(self, feats_avg: torch.Tensor, feats_ins_avg_neg: torch.Tensor) -> None:
+    def prepare_bank_with_negatives(self, feats_avg: torch.Tensor, feats_ins_avg_neg: torch.Tensor) -> PreparedBank:
         """Negative-reference scoring (`compute_sim_global_avg_with_neg`, `matching_baseline_utils.py:906-941`):
         positive prototypes = normalize(class-level feats_avg), negatives = normalize(every negative slot)."""
         pos = feats_avg.to(device=self.device, dtype=torch.float32).contiguous()
         neg = feats_ins_avg_neg.to(device=self.device, dtype=torch.float32).contiguous()
         n_cls, l_neg, c = neg.shape
         assert pos.shape == (n_cls, c)
-        self.proto = ops.proto_prepare(pos.reshape(n_cls, 1, c))
-        self.proto_neg = ops.proto_prepare(neg.reshape(n_cls * l_neg, 1, c))
-        self.l_neg = l_neg
-        self.n_cls = n_cls
+        return PreparedBank(ops.proto_prepare(pos.reshape(n_cls, 1, c)), ops.proto_prepare(neg.reshape(n_cls * l_neg, 1, c)),
+                            n_cls, l_neg, c)
+
+    def set_prototypes(self, feats_ins_avg: torch.Tensor) -> None:
+        """Score every later call against this bank (`prepare_bank`)."""
+        self._use_bank(self.prepare_bank(feats_ins_avg))
+
+    def set_prototypes_with_negatives(self, feats_avg: torch.Tensor, feats_ins_avg_neg: torch.Tensor) -> None:
+        """Score every later call against this negative-reference bank (`prepare_bank_with_negatives`)."""
+        self._use_bank(self.prepare_bank_with_negatives(feats_avg, feats_ins_avg_neg))
+
+    def _use_bank(self, bank: PreparedBank) -> None:
+        self.proto, self.proto_neg, self.l_neg, self.n_cls = bank.proto, bank.proto_neg, bank.l_neg, bank.n_cls
+
+    def _current_bank(self) -> PreparedBank:
+        if self.proto is None:
+            raise RuntimeError("Memory is not ready!")  # same text as Sam2MatchingBaseline_noAMG.py:752
+        return PreparedBank(self.proto, self.proto_neg, self.n_cls, self.l_neg, self.proto.shape[1])
+
+    def _bind_bank(self, bank_dev: torch.Tensor, bank: PreparedBank, capacity) -> None:
+        """Write a banked stage's device struct on the current stream (nttt_match_bank_bind: one kernel, the values in
+        its argument)."""
+        host = _lib.MatchBank(bank.proto.data_ptr(), ops._ptr(bank.proto_neg), bank.n_cls, bank.l_neg)
+        cap = _lib.MatchArgs()
+        cap.n_cls, cap.l_neg = capacity
+        _lib.check(self.lib.nttt_match_bank_bind(bank_dev.data_ptr(), ctypes.byref(host), ctypes.byref(cap),
+                                                 torch.cuda.current_stream(self.device).cuda_stream), "nttt_match_bank_bind")
 
     def _workspace(self, key, nbytes: int) -> torch.Tensor:
         ws = self._ws.get(key)
@@ -169,7 +238,8 @@ class MatchingStage:
     def match_async(self, lr_masks: torch.Tensor, pred_ious: torch.Tensor, tar_feat: torch.Tensor, ori_hw,
                     taps: bool = False, slot=0, iou_thr=None, persistent_out=None, multi_ious=None,
                     multi_first: int = 1, rle: bool = False, dense_masks: bool = True,
-                    low_latency: bool = False, size_range=None, bound_inputs=None) -> PendingResult:
+                    low_latency: bool = False, size_range=None, bound_inputs=None, bank=None, bank_capacity=None,
+                    bank_dev=None) -> PendingResult:
         """Enqueue the whole stage for one image on the current stream.  `slot` selects which reusable
         workspace to use (callers that keep several images in flight on different streams use one slot per
         stream).  `iou_thr`, if given, fuses the reference's candidate filter (`scores_all > iou_thr`,
@@ -188,9 +258,24 @@ class MatchingStage:
         returned result's `ori_hw` is the capacity until the caller sets it to that size (as `GraphedMatch.replay` does).
         `bound_inputs` (a device buffer of `nttt_sizeof_match_inputs()` bytes written by `nttt_match_bind`) enqueues the
         bound entry (`nttt_match_image_bound`): the kernels read the input addresses from it when they run, and the tensors
-        given here only fix the shapes (as `GraphedMatch` does with `bind=True`)."""
-        if self.proto is None:
+        given here only fix the shapes (as `GraphedMatch` does with `bind=True`).
+        `bank_capacity=(n_cls, l_neg)` enqueues the banked entry (`nttt_match_image_banked`): the kernels read the
+        prototypes and the live class count from a device struct, so the call serves any bank of up to n_cls classes
+        (l_neg > 0: negative-reference banks of up to l_neg negatives per class).  `bank` (a `PreparedBank`; default: the
+        stage's current prototypes) is bound into a fresh struct on the current stream; `bank_dev` (a device buffer of
+        `nttt_sizeof_match_bank()` bytes) is read as it stands instead, unbound here (as `GraphedMatch` does).  The `sim`
+        tap then keeps the capacity's columns on the device; `get()` returns the live ones."""
+        banked = bank_capacity is not None
+        if not banked and (bank is not None or bank_dev is not None):
+            raise ValueError("bank= and bank_dev= need bank_capacity=(n_cls, l_neg)")
+        if banked:
+            cap = _bank_capacity(bank_capacity)
+            if bank_dev is None:
+                bank = bank if bank is not None else self._current_bank()
+                _check_bank(bank, cap, tar_feat.shape[-1], self.device)
+        elif self.proto is None:
             raise RuntimeError("Memory is not ready!")  # same text as Sam2MatchingBaseline_noAMG.py:752
+        n_cls, l_neg = cap if banked else (self.n_cls, self.l_neg)
         ops._need(tar_feat, torch.float32, "tar_feat")
         n_multi, chunks = 0, None
         if multi_ious is not None:
@@ -247,26 +332,26 @@ class MatchingStage:
         counts = meta[:4]
         tap_t = {}
         if taps:
-            tap_t["sim"] = torch.empty((n, self.n_cls), dtype=torch.float32, device=dev)
+            tap_t["sim"] = torch.empty((n, n_cls), dtype=torch.float32, device=dev)
             tap_t["obj_feats"] = torch.empty((n, c), dtype=torch.float32, device=dev)
             # the inputs of the score decay: selection in slot order, IoS row maxima, same-label intersection counts
             tap_t["sel"] = torch.empty((max(max_sel, 1),), dtype=torch.int32, device=dev)
             tap_t["ios"] = torch.empty((max(max_sel, 1),), dtype=torch.float32, device=dev)
             tap_t["ios_inter"] = torch.empty((max(max_sel, 1), max(max_sel, 1)), dtype=torch.int32, device=dev)
         if size_range is None:
-            ws_bytes = self.lib.nttt_match_workspace_bytes_neg(n, lh, lw, eh, ew, c, self.n_cls, oh, ow, max_sel, self.l_neg)
+            ws_bytes = self.lib.nttt_match_workspace_bytes_neg(n, lh, lw, eh, ew, c, n_cls, oh, ow, max_sel, l_neg)
         else:
-            ws_bytes = self.lib.nttt_match_workspace_bytes_sized(n, lh, lw, eh, ew, c, self.n_cls, oh, ow, max_sel,
-                                                                 self.l_neg, min_h, min_w)
+            ws_bytes = self.lib.nttt_match_workspace_bytes_sized(n, lh, lw, eh, ew, c, n_cls, oh, ow, max_sel, l_neg,
+                                                                 min_h, min_w)
         ws = self._workspace(("match", slot), ws_bytes)
         a = _lib.MatchArgs()
-        a.logits, a.pred_ious, a.tar_feat, a.proto = (None if chunks else lr_masks.data_ptr(), ops._ptr(pred_ious),
-                                                      tar_feat.data_ptr(), self.proto.data_ptr())
+        a.logits, a.pred_ious, a.tar_feat = None if chunks else lr_masks.data_ptr(), ops._ptr(pred_ious), tar_feat.data_ptr()
+        a.proto = None if banked else self.proto.data_ptr()
         a.multi_ious, a.n_multi, a.multi_first = ops._ptr(multi_ious), n_multi, int(multi_first)
         if chunks:
             table = ops.chunk_table(chunks)
             a.logits_chunks_host, a.n_chunks, a.chunk_prompts = table, len(chunks), int(chunks[0].shape[0])
-        a.n, a.lr_h, a.lr_w, a.eh, a.ew, a.c, a.n_cls = n, lh, lw, eh, ew, c, self.n_cls
+        a.n, a.lr_h, a.lr_w, a.eh, a.ew, a.c, a.n_cls = n, lh, lw, eh, ew, c, n_cls
         a.ori_h, a.ori_w = oh, ow
         a.nms_thr = float(self.cfg.nms_thr)
         a.num_out_instance, a.max_sel = num_out, max_sel
@@ -285,14 +370,21 @@ class MatchingStage:
         a.sel, a.ios, a.ios_inter = ((tap_t[k].data_ptr() for k in ("sel", "ios", "ios_inter")) if taps
                                      else (None, None, None))
         a.workspace, a.workspace_bytes = ws.data_ptr(), ws.numel()
-        a.proto_neg = self.proto_neg.data_ptr() if self.proto_neg is not None else None
-        a.l_neg, a.sigma = self.l_neg, float(self.cfg.neg_sigma)
+        a.proto_neg = self.proto_neg.data_ptr() if self.proto_neg is not None and not banked else None
+        a.l_neg, a.sigma = l_neg, float(self.cfg.neg_sigma)
         a.iou_thr, a.filter_iou = (float(iou_thr), 1) if iou_thr is not None else (0.0, 0)
         a.out_prev_rect = prev_rect.data_ptr() if prev_rect is not None else None
         a.low_latency = 1 if low_latency else 0
         stream = torch.cuda.current_stream(dev).cuda_stream
         rng = _lib.MatchSizeRange(hw_dev.data_ptr(), min_h, min_w) if size_range is not None else None
-        if bound_inputs is not None:
+        if banked:
+            if bank_dev is None:
+                bank_dev = torch.empty((int(self.lib.nttt_sizeof_match_bank()),), dtype=torch.uint8, device=dev)
+                self._bind_bank(bank_dev, bank, cap)
+            _lib.check(self.lib.nttt_match_image_banked(self.ctx, ctypes.byref(a), ctypes.byref(rng) if rng else None,
+                                                        ops._ptr(bound_inputs), bank_dev.data_ptr(), stream),
+                       "nttt_match_image_banked")
+        elif bound_inputs is not None:
             _lib.check(self.lib.nttt_match_image_bound(self.ctx, ctypes.byref(a), ctypes.byref(rng) if rng else None,
                                                        bound_inputs.data_ptr(), stream), "nttt_match_image_bound")
         elif size_range is None:
@@ -302,8 +394,9 @@ class MatchingStage:
                        "nttt_match_image_sized")
         return PendingResult(self, masks.view(torch.bool) if masks is not None else None, boxes, scores, labels, index,
                              counts, tap_t, (oh, ow), keepalive=(lr_masks, pred_ious, multi_ious, tar_feat, ws, size_range,
-                                                                bound_inputs),
-                             rle=rle_t, meta=meta, sized=size_range is not None)
+                                                                bound_inputs, bank, bank_dev),
+                             rle=rle_t, meta=meta, sized=size_range is not None,
+                             sim_cols=bank.n_cls if banked and bank is not None else None)
 
     def atlas_stats(self) -> dict:
         """The resize-table atlases the sized graphs of this device's context use: count, device bytes, build time."""
@@ -357,7 +450,8 @@ class MatchingStage:
 
     def graphed(self, n: int, c: int, ori_hw, iou_thr=None, key=None, n_multi: int = 0,
                 multi_first: int = 1, rle: bool = False, dense_masks: bool = True, persistent_out=None,
-                low_latency: bool = False, min_hw=None, bind: bool = False, chunk_prompts=None) -> "GraphedMatch":
+                low_latency: bool = False, min_hw=None, bind: bool = False, chunk_prompts=None,
+                bank_capacity=None) -> "GraphedMatch":
         """A CUDA-graph capture of the whole stage at fixed shapes with static input/output buffers.
         n_multi > 1: the static mask buffer is the decoder's raw [n, n_multi, 256, 256] output (+ `multi_ious`).
         rle / dense_masks: as in `match_async`.  `key` names the workspace slot and `persistent_out` the
@@ -369,9 +463,12 @@ class MatchingStage:
         `bind=True`: the graph reads its inputs' addresses on the device, so `replay(lr_masks=..., pred_ious=...,
         multi_ious=..., tar_feat=...)` consumes a producer's own tensors in place (see `GraphedMatch.replay`).
         `chunk_prompts` (with n_multi > 1): the static masks are the decoder's per-batch chunk list, `chunk_prompts`
-        prompts each (the last holds the rest), instead of one [n, n_multi, 256, 256] tensor."""
+        prompts each (the last holds the rest), instead of one [n, n_multi, 256, 256] tensor.
+        `bank_capacity=(n_cls, l_neg)`: the graph reads its memory bank on the device, so `replay(bank=...)` scores the
+        image against any `PreparedBank` of up to n_cls classes (and, with l_neg > 0, up to l_neg negatives per class)
+        without a new capture (see `GraphedMatch.replay`)."""
         return GraphedMatch(self, n, c, ori_hw, iou_thr, key, n_multi, multi_first, rle, dense_masks, persistent_out,
-                            low_latency, min_hw, bind, chunk_prompts)
+                            low_latency, min_hw, bind, chunk_prompts, bank_capacity)
 
 
 class GraphedMatch:
@@ -391,12 +488,16 @@ class GraphedMatch:
     consumes the producer's own tensors in place.  Until a replay binds something else, the binding points at the graph's
     own static buffers.
 
-    The graph keeps the prototype tensors it captured alive, and re-captures on the next replay once the stage's
+    With `bank_capacity` the graph is BANKED: it reads the prototypes' addresses and the live class count from a small
+    device struct (`nttt_match_bank`) that every replay rewrites with one kernel on the replay's stream, so one capture
+    serves every bank up to the capacity, and `set_prototypes*` never makes it re-capture.
+
+    An unbanked graph keeps the prototype tensors it captured alive, and re-captures on the next replay once the stage's
     prototypes have been replaced (`set_prototypes*`)."""
 
     def __init__(self, stage: MatchingStage, n: int, c: int, ori_hw, iou_thr=None, key=None, n_multi: int = 0,
                  multi_first: int = 1, rle: bool = False, dense_masks: bool = True, persistent_out=None,
-                 low_latency: bool = False, min_hw=None, bind: bool = False, chunk_prompts=None):
+                 low_latency: bool = False, min_hw=None, bind: bool = False, chunk_prompts=None, bank_capacity=None):
         dev = stage.device
         eh, ew = stage.cfg.enc_hw
         _check_candidates(int(n))
@@ -462,9 +563,14 @@ class GraphedMatch:
         else:
             self._out = (torch.zeros((num_out, self.ori_hw[0], self.ori_hw[1]), dtype=torch.uint8, device=dev),
                          torch.zeros((num_out, 4), dtype=torch.int32, device=dev)) if dense_masks else None
+        self.bank_capacity = None
+        self.bank_dev = None
+        if bank_capacity is not None:
+            self.bank_capacity = _bank_capacity(bank_capacity)
+            self.bank_dev = torch.zeros((int(stage.lib.nttt_sizeof_match_bank()),), dtype=torch.uint8, device=dev)
         self.graph = None
         self.pending = None
-        self._proto = None  # the prototype tensors the graph was captured with (its kernels read their addresses)
+        self._proto = None  # unbanked: the prototype tensors the graph was captured with (its kernels read their addresses)
 
     def _static_inputs(self) -> dict:
         return dict(lr_masks=self.lr_masks, pred_ious=self.pred_ious, multi_ious=self.multi_ious, tar_feat=self.tar_feat)
@@ -532,14 +638,20 @@ class GraphedMatch:
                 got["lr_masks"] = aligned(need(lr_masks, self.lr_masks.shape, "lr_masks"), "lr_masks")
         return got
 
-    def capture(self):
-        """Warm up (workspace allocation, antialias tables) on a side stream, then capture."""
+    def capture(self, bank=None):
+        """Warm up (workspace allocation, antialias tables) on a side stream, then capture.  A banked graph's warm-up
+        reads `bank` (default: the stage's current prototypes)."""
         st = self.stage
         if self.bind:
             self._bind(self._static_inputs(), self.ori_hw)
             self._static_bound = True
         kw = dict(slot=self._slot, iou_thr=self.iou_thr, persistent_out=self._out, multi_ious=self.multi_ious,
                   multi_first=self.multi_first, size_range=self._size_range, bound_inputs=self.inputs_dev, **self._kw)
+        if self.bank_capacity is not None:
+            bank = bank if bank is not None else st._current_bank()
+            _check_bank(bank, self.bank_capacity, self.c, st.device)
+            st._bind_bank(self.bank_dev, bank, self.bank_capacity)
+            kw.update(bank_capacity=self.bank_capacity, bank_dev=self.bank_dev)
         side = torch.cuda.Stream(st.device)
         side.wait_stream(torch.cuda.current_stream(st.device))
         with torch.cuda.stream(side):
@@ -553,7 +665,7 @@ class GraphedMatch:
         self._proto = (st.proto, st.proto_neg)
         return self
 
-    def replay(self, ori_hw=None, lr_masks=None, pred_ious=None, multi_ious=None, tar_feat=None) -> PendingResult:
+    def replay(self, ori_hw=None, lr_masks=None, pred_ious=None, multi_ious=None, tar_feat=None, bank=None) -> PendingResult:
         """Launch the graph on the current stream.  A sized graph needs the image's size `ori_hw=(h, w)`.
 
         A bound graph (`bind=True`) also takes the image's inputs: `lr_masks` (a tensor, or with `chunk_prompts` the
@@ -561,10 +673,19 @@ class GraphedMatch:
         graph's device and of the capture's shape; an input not given is the graph's own static buffer.  Everything is
         checked before anything is enqueued.  The replay reads the tensors on the current stream: a producer that wrote
         them on another stream must make this stream wait for it first (`torch.cuda.current_stream().wait_stream(p)`).
-        The result holds them until the graph's next replay."""
+        The result holds them until the graph's next replay.
+
+        A banked graph (`bank_capacity`) scores against `bank`, a `PreparedBank` of the graph's channel count, device
+        and kind (negative references or not) with no more classes or negatives than the capacity, or, without one,
+        against the stage's current prototypes.  It is checked before anything is enqueued, bound on the current stream
+        and held by the result until the graph's next replay."""
         given = lr_masks is not None or pred_ious is not None or multi_ious is not None or tar_feat is not None
         if given and not self.bind:
             raise ValueError("this graph reads its static buffers; capture it with bind=True to pass inputs to replay()")
+        banked = self.bank_capacity is not None
+        if bank is not None and not banked:
+            raise ValueError("this graph reads the prototypes it was captured with; capture it with bank_capacity to pass "
+                             "a bank to replay()")
         if self.min_hw is None:
             if ori_hw is not None and (int(ori_hw[0]), int(ori_hw[1])) != self.ori_hw:
                 raise ValueError(f"this graph serves {self.ori_hw} only; capture it with min_hw to serve a range")
@@ -577,8 +698,11 @@ class GraphedMatch:
                 raise ValueError(f"size {hw} is outside the graph's range {self.min_hw} .. {self.ori_hw}")
         inputs = self._check_bound(lr_masks, pred_ious, multi_ious, tar_feat) if given else None
         st = self.stage
-        if self.graph is None or self._proto[0] is not st.proto or self._proto[1] is not st.proto_neg:
-            self.capture()  # (first replay, or the stage's prototypes were replaced since the capture)
+        if banked:
+            bank = bank if bank is not None else st._current_bank()
+            _check_bank(bank, self.bank_capacity, self.c, st.device)
+        if self.graph is None or (not banked and (self._proto[0] is not st.proto or self._proto[1] is not st.proto_neg)):
+            self.capture(bank)  # (first replay, or the stage's prototypes were replaced since an unbanked capture)
         if self.bind:
             if given or self.min_hw is not None or not self._static_bound:
                 self._bind(inputs or self._static_inputs(), hw)
@@ -587,8 +711,11 @@ class GraphedMatch:
             # One fill kernel on the replay's stream writes both int32 (little-endian: h is the low half): the value
             # travels as a kernel argument, so no host buffer can be overwritten by a later replay before it is read.
             self.hw_dev.view(torch.int64).fill_(hw[0] | (hw[1] << 32))
+        if banked:
+            st._bind_bank(self.bank_dev, bank, self.bank_capacity)
         self.graph.replay()
         self.pending._meta = None  # the static buffers now hold a new image's result
         self.pending.ori_hw = hw
         self.pending._bound = inputs  # (the tensors this replay reads, held until the next one)
+        self.pending._bank = bank
         return self.pending
