@@ -372,6 +372,8 @@ typedef struct nttt_match_args {
   int32_t* ios_inter;
 } nttt_match_args;
 
+/* The workspace of n candidates also serves a counted call (nttt_match_image_counted) of capacity n at any live count:
+ * the similarity GEMM's split-K partials are sized for every row count up to n. */
 size_t nttt_match_workspace_bytes(int n, int lr_h, int lr_w, int eh, int ew, int c, int n_cls, int ori_h,
                                   int ori_w, int max_sel);
 size_t nttt_match_workspace_bytes_neg(int n, int lr_h, int lr_w, int eh, int ew, int c, int n_cls, int ori_h,
@@ -468,6 +470,30 @@ int nttt_match_bank_bind(nttt_match_bank* bank_dev, const nttt_match_bank* host,
                          void* stream);
 int nttt_match_image_banked(nttt_ctx* ctx, const nttt_match_args* args, const nttt_match_size_range* range,
                             const nttt_match_inputs* inputs_dev, const nttt_match_bank* bank_dev, void* stream);
+
+/* ---------------------------------------------------------------------------------------------------
+ * The whole stage with its candidate count read from device memory when it runs: one enqueue (or one CUDA-graph capture)
+ * serves compacted candidate lists (the reference's `masks[keep]` after `scores > iou_thr`) of any length up to a
+ * capacity fixed when the call is enqueued.
+ *   nttt_match_image_counted: args->n is the CAPACITY; it sizes the workspace (nttt_match_workspace_bytes* at the
+ *   capacity), the grids and args->max_sel (= min(8 * num_out_instance, capacity)).  The live count k = *n_dev is read
+ *   by the kernels; the inputs hold (at least) k rows and nothing at or past row k is read.  `range`, `inputs_dev` and
+ *   `bank_dev` (all nullable) keep their meaning: the entry is nttt_match_image, _sized, _bound or _banked with the count
+ *   read from `n_dev`.  Inputs must be single-plane: args->n_multi > 1 returns NTTT_EINVAL before anything is enqueued
+ *   (the fused iou_thr filter stays available).  Results are those of the same entry with args->n = k and
+ *   args->max_sel = min(args->max_sel, k), bit for bit, in both low_latency modes; the taps `sim` and `obj_feats` keep the
+ *   capacity's rows, of which the first k hold the values.  k == 0 gives an empty result (counts zero, persistent slots
+ *   cleared).  A value outside [0, capacity] written to *n_dev directly gives an empty result and sets bit 1 of counts[3]
+ *   (counts[3] = 2; a sized call keeps its own status in bit 0, so both are reported); nothing is read or written past
+ *   the capacity's buffers.  Otherwise bit 1 of counts[3] is 0.
+ *   nttt_match_count_bind writes *n_dev, stream-ordered, with one kernel that carries the value as its argument.  It
+ *   first checks 0 <= n <= capacity->n and returns NTTT_EINVAL before any CUDA call otherwise, or for an n_dev that is
+ *   null or not 4-byte aligned, or a null capacity.
+ */
+int nttt_match_count_bind(int32_t* n_dev, int32_t n, const nttt_match_args* capacity, void* stream);
+int nttt_match_image_counted(nttt_ctx* ctx, const nttt_match_args* args, const nttt_match_size_range* range,
+                             const nttt_match_inputs* inputs_dev, const nttt_match_bank* bank_dev, const int32_t* n_dev,
+                             void* stream);
 
 #ifdef __cplusplus
 }

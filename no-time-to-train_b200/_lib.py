@@ -118,6 +118,8 @@ SIGNATURES = {
     "nttt_sizeof_match_bank": (c_size_t, []),
     "nttt_match_bank_bind": (c_int, [_P, POINTER(MatchBank), POINTER(MatchArgs), _P]),
     "nttt_match_image_banked": (c_int, [_P, POINTER(MatchArgs), POINTER(MatchSizeRange), _P, _P, _P]),
+    "nttt_match_count_bind": (c_int, [_P, ctypes.c_int32, POINTER(MatchArgs), _P]),
+    "nttt_match_image_counted": (c_int, [_P, POINTER(MatchArgs), POINTER(MatchSizeRange), _P, _P, _P, _P]),
     "nttt_launch_count": (ctypes.c_ulonglong, []),
     "nttt_profile_num_stages": (c_int, []),
     "nttt_profile_stage_name": (c_char_p, [c_int]),

@@ -10,35 +10,40 @@
 namespace nttt {
 
 // launchers implemented in the kernel translation units
+// (live, every launcher that takes it: nullable; a counted call's live count, the kernels' kCounted instances)
 int launch_lowres_pack(const float*, int, int, int, float, float, uint32_t*, int32_t*, int32_t*, int32_t*, int32_t*,
-                       const float*, float, const float* const*, cudaStream_t, float* stab_score = nullptr);
+                       const float*, float, const float* const*, cudaStream_t, float* stab_score = nullptr,
+                       const LiveCount* live = nullptr);
 int launch_multimask_select(const float*, int, int, int, const ChunkTable&, int, size_t, const float**, float*,
                             cudaStream_t, const float* const* ious_at = nullptr, const float* const* bases = nullptr);
-int launch_plane_resolve(const nttt_match_inputs*, int, size_t, const float**, float*, cudaStream_t);
+int launch_plane_resolve(const nttt_match_inputs*, int, size_t, const float**, float*, cudaStream_t,
+                         const LiveCount* live = nullptr);
 template <typename T>
 int launch_match_bind(const T&, T*, cudaStream_t);  // T: nttt_match_inputs or nttt_match_bank
+int launch_count_bind(int32_t, int32_t*, cudaStream_t);
 int launch_project_masks(const AxisTable&, const AxisTable&, const uint32_t*, const int32_t*, int, int, int, int, int,
-                         void*, int, bool, cudaStream_t, const int32_t* perm = nullptr, uint32_t* active = nullptr);
-int launch_pool_order(const int32_t*, int, int, int32_t*, cudaStream_t);
+                         void*, int, bool, cudaStream_t, const int32_t* perm = nullptr, uint32_t* active = nullptr,
+                         const LiveCount* live = nullptr);
+int launch_pool_order(const int32_t*, int, int, int32_t*, cudaStream_t, const LiveCount* live = nullptr);
 int launch_normalize_split(const float*, int, const int32_t*, int, int, int, float*, void*, bool, cudaStream_t,
-                           const int32_t* perm = nullptr);
+                           const int32_t* perm = nullptr, const LiveCount* live = nullptr);
 int launch_gemm_tc(const void*, int, const void*, int, float*, int, int, int, int, int, size_t, int*, cudaStream_t,
                    bool low_latency = false, const uint32_t* a_active = nullptr, const uint8_t* b_nonfinite = nullptr,
-                   const nttt_match_bank* bank = nullptr, int bank_neg = 0);
-int gemm_tc_pick_splits(int, int, int, int);
+                   const nttt_match_bank* bank = nullptr, int bank_neg = 0, const LiveCount* live = nullptr);
 int launch_split_rows(const float*, int, int, int, int, int, void*, cudaStream_t, const nttt_match_bank* bank = nullptr,
                       int bank_neg = 0);
 int launch_split_transpose(const float*, int, int, int, int, int, void*, cudaStream_t, uint8_t* nonfinite = nullptr,
                            const float* const* x_at = nullptr);
-int launch_normalize_rows(const float*, int, const int32_t*, int, int, float*, bool, cudaStream_t);
+int launch_normalize_rows(const float*, int, const int32_t*, int, int, float*, bool, cudaStream_t,
+                          const LiveCount* live = nullptr);
 int launch_proto_prepare(const float*, int, int, int, float*, cudaStream_t);
 int launch_top1(const float*, int, size_t, float*, int, int, int, float*, int32_t*, cudaStream_t,
-                const nttt_match_bank* bank = nullptr);
+                const nttt_match_bank* bank = nullptr, const LiveCount* live = nullptr);
 int launch_neg_top1(const float*, int, size_t, const float*, int, size_t, int, int, int, float, float*, float*, int32_t*,
-                    cudaStream_t, const nttt_match_bank* bank = nullptr);
+                    cudaStream_t, const nttt_match_bank* bank = nullptr, const LiveCount* live = nullptr);
 size_t nms_workspace_bytes(int n);
 int launch_box_nms(const int32_t*, const float*, const int32_t*, const float*, int, float, int, int32_t*, int32_t*,
-                   int32_t*, int32_t*, void*, size_t, float, int, cudaStream_t);
+                   int32_t*, int32_t*, void*, size_t, float, int, cudaStream_t, const LiveCount* live = nullptr);
 int launch_upsample_pack(const AxisTable&, const AxisTable&, const float*, const uint32_t*, const int32_t*,
                          const int32_t*, int, int, const int32_t*, const int32_t*, int, int, int, uint32_t*, int32_t*,
                          int32_t*, int32_t*, int32_t*, const float* const*, cudaStream_t, int, int, uint32_t* bits_t = nullptr,
@@ -126,10 +131,11 @@ constexpr int kPoolSplits = 1;  // measured: 2 halves the latency (25 -> 14 us) 
 static int pool_contract(const float* proj, const float* feat, int n, int e, int c, float* sums, void* a_split,
                          void* b_split, int* n_partials, cudaStream_t s, bool low_latency = false, bool b_ready = false,
                          const uint32_t* a_active = nullptr, uint8_t* b_nonfinite = nullptr,
-                         const float* const* feat_at = nullptr) {
+                         const float* const* feat_at = nullptr, const LiveCount* live = nullptr) {
   // a_active / b_nonfinite (both or neither): the A operand's rows are spatially ordered and carry their non-zero k-block
   // masks; the GEMM skips the k-blocks a tile does not touch (gemm_tc_kernel), unless the features are not finite there
   // feat_at (nullable): the features' address is read from device memory when the kernel runs (bound inputs)
+  // live (nullable): n is a counted call's capacity (its split-K does not depend on the row count)
   const int ep = pad64(e);
   int err = proj ? launch_split_rows(proj, e, n, e, ep, 0, a_split, s) : NTTT_OK;
   if (err) return err;
@@ -137,7 +143,8 @@ static int pool_contract(const float* proj, const float* feat, int n, int e, int
                                                    feat_at);  // (b_ready: done on the side stream)
   if (err) return err;
   return launch_gemm_tc(a_split, 3 * ep, b_split, 3 * ep, sums, c, n, c, 3 * ep, low_latency ? kPoolSplitsMax : kPoolSplits,
-                        (size_t)n * c, n_partials, s, low_latency, a_active, a_active ? b_nonfinite : nullptr);
+                        (size_t)n * c, n_partials, s, low_latency, a_active, a_active ? b_nonfinite : nullptr, nullptr, 0,
+                        live);
 }
 
 // rows of `sums` -> /area -> L2-normalise -> obj_feats (+ split-bf16 copy when the vector path applies).
@@ -145,12 +152,13 @@ static int pool_contract(const float* proj, const float* feat, int n, int e, int
 // nan_empty: negative-reference scoring divides by the raw area (empty mask -> NaN row, as the reference does)
 // n_partials: split-K partial sums of the pooling GEMM, n*c floats apart, added in order
 static int normalize_rows(const float* sums, int n_partials, const int32_t* area, int n, int c, float* obj_feats,
-                          void* a_split, bool* split_done, bool nan_empty, cudaStream_t s, const int32_t* perm = nullptr) {
-  *split_done = a_split &&
-                launch_normalize_split(sums, n_partials, area, n, c, pad64(c), obj_feats, a_split, nan_empty, s, perm) == 1;
+                          void* a_split, bool* split_done, bool nan_empty, cudaStream_t s, const int32_t* perm = nullptr,
+                          const LiveCount* live = nullptr) {
+  *split_done = a_split && launch_normalize_split(sums, n_partials, area, n, c, pad64(c), obj_feats, a_split, nan_empty, s,
+                                                  perm, live) == 1;
   if (*split_done) return NTTT_OK;
   if (perm) return NTTT_EINVAL;  // (callers order the rows only when the vector path applies)
-  return launch_normalize_rows(sums, n_partials, area, n, c, obj_feats, nan_empty, s);
+  return launch_normalize_rows(sums, n_partials, area, n, c, obj_feats, nan_empty, s, live);
 }
 
 // the scatter tables hold kMaxScatter weights per encoder cell: enough while out/in <= ~11
@@ -162,12 +170,18 @@ static bool projection_supported(int in_size, int out_size) {
 // (a_ready: a_split already holds the split obj_feats, written by normalize_split_kernel)
 // The similarity GEMM has few output tiles (n_cls is small), so it runs split-K into `partials`
 // [splits, n, n_cls]; top1_kernel sums them in a fixed order, writes `sim` (nullable) and the row arg-max.
-constexpr int kMaxSimSplits = 8;
-// floats needed for the split-K partials of an [n, cols] similarity matrix (sized for a 148-SM part)
+// floats needed for the split-K partials of an [m, cols] similarity matrix for every m <= n (sized for a 148-SM part): the
+// partials of m rows are m * cols floats apart, and a counted call (nttt_match_image_counted) of capacity n splits at
+// its live count m, which can take more partials than n rows do
 static size_t sim_partial_floats(int n, int cols, int c) {
-  int sp = gemm_tc_pick_splits(n, cols, 3 * pad64(c), 148);
-  if (sp > kMaxSimSplits) sp = kMaxSimSplits;
-  return (size_t)sp * n * cols;
+  size_t most = 0;
+  for (int m0 = 128;; m0 += 128) {  // (the split depends on m through its 128-row tiles: the largest m of each is enough)
+    const int m = m0 < n ? m0 : n;
+    const size_t f = (size_t)sim_split_want(m, cols, 3 * pad64(c), 148) * m;
+    if (f > most) most = f;
+    if (m0 >= n) break;
+  }
+  return most * cols;
 }
 
 // l_neg == 0: plain cosine scoring.  Otherwise negative-reference scoring: proto is the normalised class-level average,
@@ -175,41 +189,43 @@ static size_t sim_partial_floats(int n, int cols, int c) {
 static int sim_top1(const float* obj_feats, const float* proto, const float* proto_neg, int l_neg, float sigma, int n,
                     int c, int n_cls, float* sim, float* partials, float* partials_neg, float* top_score,
                     int32_t* top_label, void* a_split, void* b_split, bool a_ready, int sm_count, cudaStream_t s,
-                    void* p_split = nullptr, bool p_ready = false, const nttt_match_bank* bank = nullptr) {
+                    void* p_split = nullptr, bool p_ready = false, const nttt_match_bank* bank = nullptr,
+                    const LiveCount* live = nullptr) {
   // p_split (nullable): a buffer of its own for the split prototypes, so that they can be prepared before b_split is free
   // (p_ready: already done, on the side stream of the low-latency mode); without it they go through b_split
   // bank (nullable): the prototypes are the bound bank's (proto and proto_neg are ignored), n_cls and l_neg its capacity
+  // live (nullable): n is a counted call's capacity; in low-latency mode (live->split_sm) the GEMMs' grids hold the split
+  // of one row tile, the largest, and the kernels split at the live count (gemm_tc_kernel, top1_kernel)
   const int cp = pad64(c);
+  const int m_split = live && live->split_sm > 0 ? 1 : n;
   int err = a_ready ? NTTT_OK : launch_split_rows(obj_feats, c, n, c, cp, 0, a_split, s);
   if (err) return err;
   void* pb = p_split ? p_split : b_split;
   err = p_ready ? NTTT_OK : launch_split_rows(proto, c, n_cls, c, cp, 1, pb, s, bank, 0);
   if (err) return err;
-  int want = gemm_tc_pick_splits(n, n_cls, 3 * cp, sm_count < 148 ? sm_count : 148);
-  if (want > kMaxSimSplits) want = kMaxSimSplits;
+  int want = sim_split_want(m_split, n_cls, 3 * cp, sm_count);
   // with many images in flight the partial tiles of a split-K cost more SM-time (8 x the prologues, epilogues and
   // partial sums) than the one long CTA per tile they shorten: measured 84.0 (no split) / 84.6 (2) / 85.1 (4) / 86.8 (8)
   if (!t_low_latency) want = 1;
   const size_t stride = (size_t)n * n_cls;
   int splits = 1;
   err = launch_gemm_tc(a_split, 3 * cp, pb, 3 * cp, partials, n_cls, n, n_cls, 3 * cp, want, stride, &splits, s, false,
-                       nullptr, nullptr, bank, 0);
+                       nullptr, nullptr, bank, 0, live);
   if (err) return err;
-  if (l_neg <= 0) return launch_top1(partials, splits, stride, sim, n_cls, n, n_cls, top_score, top_label, s, bank);
+  if (l_neg <= 0) return launch_top1(partials, splits, stride, sim, n_cls, n, n_cls, top_score, top_label, s, bank, live);
   const int cols = n_cls * l_neg;
   // (stream-ordered after the GEMM that read b_split)
   err = launch_split_rows(proto_neg, c, cols, c, cp, 1, b_split, s, bank, 1);
   if (err) return err;
-  int want_n = gemm_tc_pick_splits(n, cols, 3 * cp, sm_count < 148 ? sm_count : 148);
-  if (want_n > kMaxSimSplits) want_n = kMaxSimSplits;
+  int want_n = sim_split_want(m_split, cols, 3 * cp, sm_count);
   if (!t_low_latency) want_n = 1;
   const size_t stride_n = (size_t)n * cols;
   int splits_n = 1;
   err = launch_gemm_tc(a_split, 3 * cp, b_split, 3 * cp, partials_neg, cols, n, cols, 3 * cp, want_n, stride_n, &splits_n,
-                       s, false, nullptr, nullptr, bank, 1);
+                       s, false, nullptr, nullptr, bank, 1, live);
   if (err) return err;
   return launch_neg_top1(partials, splits, stride, partials_neg, splits_n, stride_n, n, n_cls, l_neg, sigma, sim,
-                         top_score, top_label, s, bank);
+                         top_score, top_label, s, bank, live);
 }
 
 }  // namespace nttt
@@ -809,9 +825,13 @@ int nttt_ctx_atlas_stats(nttt_ctx* ctx, size_t* bytes_host, double* build_ms_hos
 // take their addresses from *in_dev)
 // bank != nullptr: nttt_match_image_banked (a->proto / proto_neg are ignored, a->n_cls / l_neg are the capacity; the
 // kernels that read the prototypes or the class count take them from *bank)
+// n_dev != nullptr: nttt_match_image_counted (a->n is the capacity; the kernels that take the candidate count, up to NMS,
+// read the live count from *n_dev)
 static int match_impl(nttt_ctx* ctx, const nttt_match_args* a, const nttt_match_size_range* range, void* stream,
-                      const nttt_match_inputs* in_dev = nullptr, const nttt_match_bank* bank = nullptr) {
+                      const nttt_match_inputs* in_dev = nullptr, const nttt_match_bank* bank = nullptr,
+                      const int32_t* n_dev = nullptr) {
   if (!ctx || !a) return NTTT_EINVAL;
+  if (n_dev && a->n_multi > 1) return NTTT_EINVAL;  // (compacted candidates are single-plane)
   if (a->n < 0 || a->lr_h <= 0 || a->lr_w <= 0 || a->eh <= 0 || a->ew <= 0 || a->c <= 0 || a->n_cls <= 0 ||
       a->ori_h <= 0 || a->ori_w <= 0 || a->num_out_instance < 0 || a->max_sel < 0)
     return NTTT_EINVAL;
@@ -866,13 +886,19 @@ static int match_impl(nttt_ctx* ctx, const nttt_match_args* a, const nttt_match_
   SizedDims sd{};
   if (range) {
     if ((err = ctx->sized_atlas(a->lr_h, a->lr_w, range->min_h, range->min_w, a->ori_h, a->ori_w, s, &atlas))) return err;
-    sd = SizedDims{range->ori_hw_dev, atlas->ay, atlas->ax, a->counts, range->min_h, range->min_w, a->ori_h, a->ori_w};
+    sd = SizedDims{range->ori_hw_dev, atlas->ay, atlas->ax, a->counts, range->min_h, range->min_w, a->ori_h, a->ori_w,
+                   n_dev != nullptr};
   } else {
     if ((err = ctx->axis(a->lr_w, a->ori_w, s, &ux))) return err;
     if ((err = ctx->axis(a->lr_h, a->ori_h, s, &uy))) return err;
   }
   const SizedDims* sized = range ? &sd : nullptr;
   const int e = a->eh * a->ew;
+  // counted: the live count, and (low-latency mode) the SM count the similarity GEMM's split-K is picked for; the pooling
+  // GEMM's split does not depend on the row count
+  const LiveCount lc_sim{n_dev, n, a->low_latency ? ctx->sm_count : 0, 3 * pad64(a->c), a->counts + 3};
+  const LiveCount lc{n_dev, n, 0, 0, a->counts + 3};
+  const LiveCount* live = n_dev ? &lc : nullptr;
 
   ctx->n_ev = 0;
 #define NTTT_MARK()                                                              \
@@ -912,7 +938,7 @@ static int match_impl(nttt_ctx* ctx, const nttt_match_args* a, const nttt_match_
                                     (size_t)a->lr_h * a->lr_w, L.mask_ptr, L.plane_score, s, &in_dev->multi_ious,
                                     chunked ? in_dev->chunks : &in_dev->logits);
     else
-      err = launch_plane_resolve(in_dev, n, (size_t)a->lr_h * a->lr_w, L.mask_ptr, L.plane_score, s);
+      err = launch_plane_resolve(in_dev, n, (size_t)a->lr_h * a->lr_w, L.mask_ptr, L.plane_score, s, live);
     if (err) return err;
     mask_ptr = L.mask_ptr;
     pred_ious = L.plane_score;
@@ -952,15 +978,16 @@ static int match_impl(nttt_ctx* ctx, const nttt_match_args* a, const nttt_match_
   // a6/a9/a15: one pass over the logits
   // (the stability counts of a15 are not read on this path, so the pipeline does not pay for them)
   NTTT_STEP(launch_lowres_pack(logits, n, a->lr_h, a->lr_w, 0.0f, 1.0f, L.bits_lr, L.area_lr, L.box_lr, nullptr,
-                               L.flags, a->filter_iou ? pred_ious : nullptr, a->iou_thr, mask_ptr, s));
+                               L.flags, a->filter_iou ? pred_ious : nullptr, a->iou_thr, mask_ptr, s, nullptr, live));
   // a6/a7: projection + pooling contraction + normalisation
   // Many images in flight: the pooling GEMM runs on spatially ordered rows and skips the k-blocks a tile of masks does
   // not touch (~45 % of them).  Needs the vector normalisation path (it undoes the order) and <= 32 k-blocks per segment.
   const bool ordered = !a->low_latency && ctx->pool_order && n > 128 && n <= NTTT_MAX_CANDIDATES && pad64(e) / 64 <= 32 &&
                        (a->c == 384 || a->c == 768 || a->c == 1024 || a->c == 1536);
-  if (ordered) NTTT_STEP_QUIET(launch_pool_order(L.box_lr, n, a->lr_h, L.pool_perm, s));
+  // (counted: `ordered` and the launch shapes below follow the capacity; neither changes a result, DESIGN.md §4)
+  if (ordered) NTTT_STEP_QUIET(launch_pool_order(L.box_lr, n, a->lr_h, L.pool_perm, s, live));
   NTTT_STEP(launch_project_masks(px, py, L.bits_lr, L.box_lr, n, a->lr_h, a->lr_w, a->eh, a->ew, L.a_split, pad64(e),
-                                 true, s, ordered ? L.pool_perm : nullptr, ordered ? L.pool_active : nullptr));
+                                 true, s, ordered ? L.pool_perm : nullptr, ordered ? L.pool_active : nullptr, live));
   int n_partials = 1;
   if (forked) {
     NTTT_CUDA(cudaStreamWaitEvent(s, ctx->ev_join, 0));
@@ -968,18 +995,19 @@ static int match_impl(nttt_ctx* ctx, const nttt_match_args* a, const nttt_match_
     nttt::t_chain_break = true;  // the pooling GEMM depends on the side stream as well: launched the ordinary way
   }
   NTTT_STEP(pool_contract(nullptr, a->tar_feat, n, e, a->c, L.sums, L.a_split, L.b_split, &n_partials, s,
-                          a->low_latency != 0, forked, ordered ? L.pool_active : nullptr, L.b_nonfinite, feat_at));
+                          a->low_latency != 0, forked, ordered ? L.pool_active : nullptr, L.b_nonfinite, feat_at, live));
   bool a_ready = false;
   NTTT_STEP(normalize_rows(L.sums, n_partials, L.area_lr, n, a->c, obj_feats, L.a_split, &a_ready, neg, s,
-                           ordered ? L.pool_perm : nullptr));
+                           ordered ? L.pool_perm : nullptr, live));
   // a7/a8: similarity + top-1 (the last step that depends on the class count: NMS, the resize, the IoS term, the decay
   // and the output encoding read only the top-1 labels and scores)
   NTTT_STEP(sim_top1(obj_feats, a->proto, a->proto_neg, l_neg, a->sigma, n, a->c, a->n_cls, a->sim, L.sim_part,
                      L.sim_part_neg, L.top_score, L.top_label, L.a_split, L.b_split, a_ready, ctx->sm_count, s, L.p_split,
-                     forked, bank));
-  // a10/a11
+                     forked, bank, n_dev ? &lc_sim : nullptr));
+  // a10/a11 (counted: the last step that depends on the candidate count — everything after reads the selection, whose
+  // n_sel entries index candidates below the live count)
   NTTT_STEP(launch_box_nms(L.box_lr, pred_ious, L.top_label, L.top_score, n, a->nms_thr, max_sel, L.keep,
-                           a->counts + 0, sel, a->counts + 1, L.nms_ws, L.nms_ws_bytes, a->iou_thr, a->filter_iou, s));
+                           a->counts + 0, sel, a->counts + 1, L.nms_ws, L.nms_ws_bytes, a->iou_thr, a->filter_iou, s, live));
   // a12/a9 (sized: ux, uy are empty, the tables come from the atlas)
   bool wrote_t = false;  // the resize left the word-column-major copy of the packed masks instead of the row-major one
   NTTT_STEP(launch_upsample_pack(ux, uy, logits, L.bits_lr, L.box_lr, L.flags, a->lr_h, a->lr_w, sel, a->counts + 1,
@@ -1069,6 +1097,19 @@ int nttt_match_image_banked(nttt_ctx* ctx, const nttt_match_args* a, const nttt_
                             const nttt_match_inputs* inputs_dev, const nttt_match_bank* bank_dev, void* stream) {
   if (!bank_dev) return NTTT_EINVAL;
   return match_impl(ctx, a, range, stream, inputs_dev, bank_dev);
+}
+
+int nttt_match_count_bind(int32_t* n_dev, int32_t n, const nttt_match_args* capacity, void* stream) {
+  if (!n_dev || !capacity || (reinterpret_cast<uintptr_t>(n_dev) & 3) != 0) return NTTT_EINVAL;
+  if (n < 0 || n > capacity->n) return NTTT_EINVAL;
+  return launch_count_bind(n, n_dev, (cudaStream_t)stream);
+}
+
+int nttt_match_image_counted(nttt_ctx* ctx, const nttt_match_args* a, const nttt_match_size_range* range,
+                             const nttt_match_inputs* inputs_dev, const nttt_match_bank* bank_dev, const int32_t* n_dev,
+                             void* stream) {
+  if (!n_dev) return NTTT_EINVAL;
+  return match_impl(ctx, a, range, stream, inputs_dev, bank_dev, n_dev);
 }
 
 }  // extern "C"

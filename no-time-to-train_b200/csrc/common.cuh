@@ -195,6 +195,7 @@ struct SizedDims {
   const SizedAxis* ax;    // [cap_w - min_w + 1] output widths
   int32_t* counts;        // nttt_match_args.counts: [1] emptied and [3] (status) written by the resize
   int min_h, min_w, cap_h, cap_w;
+  int counted;            // the call is also counted: the resize keeps the count status (bit 1 of counts[3])
 };
 struct SizedAtlas {
   int lr_h = 0, lr_w = 0, min_h = 0, min_w = 0, cap_h = 0, cap_w = 0;
@@ -209,6 +210,52 @@ struct SizedAtlas {
 };
 int build_sized_atlas(SizedAtlas& a, cudaStream_t s);  // a: sizes set; fills the rest (one synchronisation)
 long up2_tile_factor(int in_size, int out_size, bool rows);
+
+// ---------------------------------------------------------------------------------------------------
+// Counted entry (nttt_match_image_counted): the candidate count is read from device memory when the kernels run, within
+// [0, capacity] where the capacity (nttt_match_args.n) sized the workspace and the grids when the call was enqueued.
+// By-value kernel argument that every kernel taking the candidate count, up to NMS, takes after its static parameters:
+// read only by the kernel's kCounted = true instance (the static instance is passed an empty one).
+// ---------------------------------------------------------------------------------------------------
+struct LiveCount {
+  const int32_t* n;  // live count, device
+  int cap;           // capacity
+  int split_sm;      // > 0: the similarity GEMM's split-K follows the live count (low-latency mode) on this many SMs
+  int split_k;       // K' of the similarity GEMM (3 * pad64(c)), with split_sm
+  int32_t* status;   // nttt_match_args.counts + 3: written by nms_sort_kernel
+};
+constexpr int kCountStatus = 2;  // counts[3] bit of a live count outside [0, capacity] (bit 0: the sized status)
+
+// how many K splits fill the machine for an M x N output of 128 x 64 tiles (1 when the tiles already do)
+__host__ __device__ inline int gemm_tc_pick_splits(int M, int N, int K, int sm_count) {
+  const int tiles = ((N + 63) / 64) * ((M + 127) / 128);
+  const int total_kb = K / 64;
+  int splits = sm_count / (tiles > 0 ? tiles : 1);
+  if (splits < 1) splits = 1;
+  if (splits > 8) splits = 8;
+  if (splits > total_kb) splits = total_kb;
+  return splits;
+}
+// the split-K the low-latency mode asks for in the similarity GEMM of an [M, N] output (K = 3 * pad64(c)) ...
+constexpr int kMaxSimSplits = 8;
+__host__ __device__ inline int sim_split_want(int M, int N, int K, int sm_count) {
+  const int want = gemm_tc_pick_splits(M, N, K, sm_count < 148 ? sm_count : 148);
+  return want > kMaxSimSplits ? kMaxSimSplits : want;
+}
+// ... and the number of partials launch_gemm_tc produces for it (k-blocks ceil(total / want) per split)
+__host__ __device__ inline int split_kb_per(int K, int want) { return (K / 64 + want - 1) / want; }
+__host__ __device__ inline int split_count(int K, int want) {
+  const int kb_per = split_kb_per(K, want);
+  return (K / 64 + kb_per - 1) / kb_per;
+}
+
+#ifdef __CUDACC__
+// the live count of a counted call; a value outside [0, capacity] reads as 0 (an empty result, nttt_match_image_counted)
+__device__ __forceinline__ int live_count(const LiveCount& c) {
+  const int k = *c.n;
+  return (k >= 0 && k <= c.cap) ? k : 0;
+}
+#endif
 
 #ifdef __CUDACC__
 // live rows of a bound bank's prototype table (nttt_match_image_banked): its classes, or (neg) its n_cls * l_neg negatives

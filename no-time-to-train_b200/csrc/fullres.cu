@@ -65,7 +65,7 @@ __device__ __forceinline__ bool sized_tables(const SizedDims& d, bool two_tap, b
                                              UpTables& t) {
   const bool in_range = sized_hw(d, oh, ow);
   if (status && blockIdx.x == 0 && blockIdx.y == 0 && threadIdx.x == 0) {
-    d.counts[3] = in_range ? 0 : 1;
+    d.counts[3] = (in_range ? 0 : 1) | (d.counted ? d.counts[3] & kCountStatus : 0);  // (counted: NMS wrote bit 1)
     if (!in_range) d.counts[1] = 0;
   }
   if (!in_range) return false;

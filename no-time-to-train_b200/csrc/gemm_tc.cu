@@ -151,12 +151,17 @@ struct GemmSmem {
 
 // kBank (nttt_match_image_banked, similarity launches): N is the bank's capacity; the live column count is read from
 // *bank (bank_rows), and tiles that lie wholly at or past it exit before they allocate TMEM or issue a TMA or an MMA.
-template <int BN, int STAGES, bool kBank>
+// kCounted (nttt_match_image_counted): M is the candidate capacity; the live row count is read from *live.n, row tiles
+// wholly at or past it exit the same way, and the epilogue (and the k-block skip mask) stop at it.  With live.split_sm
+// the split-K is the one the low-latency mode picks at the live count: the grid holds the largest split (one row tile),
+// the k-blocks per split follow the live count, the z-slices past its partials exit, and the partials are k * ldd
+// floats apart, so that top1_kernel<.., true> adds exactly the partials nttt_match_image adds at that count.
+template <int BN, int STAGES, bool kBank, bool kCounted>
 __global__ void __launch_bounds__(kGemmThreads, 1)
 gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b,
                float* __restrict__ D, int ldd, int M, int N, int total_k_blocks, int kb_per_split,
                size_t split_stride, const uint32_t* __restrict__ a_active, const uint8_t* __restrict__ b_nonfinite,
-               int nkb_seg, const nttt_match_bank* __restrict__ bank, int bank_neg) {
+               int nkb_seg, const nttt_match_bank* __restrict__ bank, int bank_neg, LiveCount live) {
   // Skipping mode (a_active != nullptr; no split-K): K' is nseg = total_k_blocks / nkb_seg segments of nkb_seg k-blocks
   // (the split-bf16 layout: 3), a_active[row] has bit kb set if row `row` of A holds anything but zeros in k-block kb of a
   // segment, b_nonfinite[r-tile * nkb_seg + kb] is 1 if rows 32 r-tile .. +31 of B hold an inf / NaN there.  A k-block in
@@ -170,6 +175,23 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
     // (the struct is read once the predecessor has completed: this instance does not overlap its set-up with the drain)
     chain_wait();
     if (n0 >= bank_rows(bank, bank_neg)) return;
+  }
+  if constexpr (kCounted) {
+    // (read without waiting for the predecessor: the count is written before the stage's first kernel, an ordinary
+    // launch, so this instance still sets up its barriers and TMEM while the producer of the operands drains.  A CTA
+    // that exits still waits first: chain_wait is on every path, so the kernels after this one stay ordered behind all
+    // earlier ones.)
+    M = live_count(live);
+    bool idle = m0 >= M;
+    if (!idle && live.split_sm > 0) {
+      kb_per_split = split_kb_per(live.split_k, sim_split_want(M, N, live.split_k, live.split_sm));
+      idle = (int)blockIdx.z * kb_per_split >= total_k_blocks;
+      split_stride = (size_t)M * ldd;
+    }
+    if (idle) {
+      chain_wait();
+      return;
+    }
   }
   // split-K: blockIdx.z owns k-blocks [kb0, kb0 + num_k_blocks) and writes its partial tile to D + z*split_stride
   const int kb0 = blockIdx.z * kb_per_split;
@@ -308,21 +330,22 @@ static int make_map(CUtensorMap* map, const void* base, int rows, int k, int ld,
 template <int BN, int STAGES>
 static int launch_tc(const __nv_bfloat16* A, int lda, const __nv_bfloat16* B, int ldb, float* D, int ldd, int M, int N,
                      int K, int splits, size_t split_stride, cudaStream_t s, const uint32_t* a_active,
-                     const uint8_t* b_nonfinite, const nttt_match_bank* bank, int bank_neg) {
+                     const uint8_t* b_nonfinite, const nttt_match_bank* bank, int bank_neg, const LiveCount* live) {
   CUtensorMap ma, mb;
   int err = make_map(&ma, A, M, K, lda, kBM);
   if (err) return err;
   err = make_map(&mb, B, N, K, ldb, BN);
   if (err) return err;
   const size_t smem = sizeof(GemmSmem<BN, STAGES>) + 1024;
-  auto kern = bank ? gemm_tc_kernel<BN, STAGES, true> : gemm_tc_kernel<BN, STAGES, false>;
+  auto kern = live ? (bank ? gemm_tc_kernel<BN, STAGES, true, true> : gemm_tc_kernel<BN, STAGES, false, true>)
+                   : (bank ? gemm_tc_kernel<BN, STAGES, true, false> : gemm_tc_kernel<BN, STAGES, false, false>);
   NTTT_CUDA(set_dyn_smem(kern, (int)smem));
   const int total_kb = K / kBK;
   const int kb_per = ceil_div(total_kb, splits);
   dim3 grid(ceil_div(N, BN), ceil_div(M, kBM), ceil_div(total_kb, kb_per));
   const int nkb_seg = (a_active && K % (3 * kBK) == 0) ? K / 3 / kBK : 0;
   launch_chain(kern, grid, kGemmThreads, smem, s, ma, mb, D, ldd, M, N, total_kb, kb_per, split_stride, a_active, b_nonfinite,
-               nkb_seg, bank, bank_neg);
+               nkb_seg, bank, bank_neg, live ? *live : LiveCount{});
   NTTT_LAUNCH_CHECK();
   return NTTT_OK;
 }
@@ -331,10 +354,12 @@ static int launch_tc(const __nv_bfloat16* A, int lda, const __nv_bfloat16* B, in
 // splits > 1: split-K, partial tile z is written to D + z*split_stride (the caller sums the partials in a fixed
 // order); *splits_out receives the number of partials actually produced.
 // bank (nullable): B is a bound bank's split prototype table of N (the capacity) rows, of which bank_rows(bank, bank_neg)
-// are live; the tiles past them are not computed (gemm_tc_kernel<.., true>).
+// are live; the tiles past them are not computed (gemm_tc_kernel<.., true, ..>).
+// live (nullable): M is the capacity of a counted call, the live row count is read on the device (gemm_tc_kernel<.., true>);
+// with live->split_sm, `splits` is the largest split the live count can take and *splits_out is not meaningful.
 int launch_gemm_tc(const void* A, int lda, const void* B, int ldb, float* D, int ldd, int M, int N, int K, int splits,
                    size_t split_stride, int* splits_out, cudaStream_t s, bool low_latency, const uint32_t* a_active,
-                   const uint8_t* b_nonfinite, const nttt_match_bank* bank, int bank_neg) {
+                   const uint8_t* b_nonfinite, const nttt_match_bank* bank, int bank_neg, const LiveCount* live) {
   if (splits_out) *splits_out = 1;
   if (M <= 0 || N <= 0) return NTTT_OK;
   if (K <= 0 || K % kBK != 0 || lda % 8 != 0 || ldb % 8 != 0 || splits < 1) return NTTT_EINVAL;
@@ -354,21 +379,13 @@ int launch_gemm_tc(const void* A, int lda, const void* B, int ldb, float* D, int
   const bool bn256 = !low_latency && N >= 512 && M >= 512;
   const bool bn128 = N >= 512 || (N > 64 && N <= 128);  // 65..128 columns: ONE 128-wide tile reads the A operand once instead of twice
   if (bn256)
-    return launch_tc<256, 3>(a, lda, b, ldb, D, ldd, M, N, K, splits, split_stride, s, a_active, b_nonfinite, bank, bank_neg);
+    return launch_tc<256, 3>(a, lda, b, ldb, D, ldd, M, N, K, splits, split_stride, s, a_active, b_nonfinite, bank, bank_neg,
+                                  live);
   if (bn128)
-    return launch_tc<128, 5>(a, lda, b, ldb, D, ldd, M, N, K, splits, split_stride, s, a_active, b_nonfinite, bank, bank_neg);
-  return launch_tc<64, 6>(a, lda, b, ldb, D, ldd, M, N, K, splits, split_stride, s, a_active, b_nonfinite, bank, bank_neg);
-}
-
-// how many K splits fill the machine for an M x N output of 128 x 64 tiles (1 when the tiles already do)
-int gemm_tc_pick_splits(int M, int N, int K, int sm_count) {
-  const int tiles = ceil_div(N, 64) * ceil_div(M, kBM);
-  const int total_kb = K / kBK;
-  int splits = sm_count / (tiles > 0 ? tiles : 1);
-  if (splits < 1) splits = 1;
-  if (splits > 8) splits = 8;
-  if (splits > total_kb) splits = total_kb;
-  return splits;
+    return launch_tc<128, 5>(a, lda, b, ldb, D, ldd, M, N, K, splits, split_stride, s, a_active, b_nonfinite, bank, bank_neg,
+                                  live);
+  return launch_tc<64, 6>(a, lda, b, ldb, D, ldd, M, N, K, splits, split_stride, s, a_active, b_nonfinite, bank, bank_neg,
+                                  live);
 }
 
 // ---------------------------------------------------------------------------------------------------

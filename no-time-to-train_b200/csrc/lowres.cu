@@ -253,12 +253,18 @@ __device__ __forceinline__ uint32_t pk_sign_chain(uint32_t acc, const uint4& v) 
   return acc;
 }
 
+// kCounted (nttt_match_image_counted, this kernel and the persistent one): the grid covers the capacity, the masks stop
+// at the live count (nothing at or past it is read or written)
+template <bool kCounted>
 __global__ void __launch_bounds__(kPackBlock, 3)
 lowres_pack_fast_kernel(const float4* __restrict__ logits, int p4 /* pixels/4 per mask */, int words_per_row,
                         uint32_t* __restrict__ bits, int32_t* __restrict__ area, int32_t* __restrict__ box,
                         int32_t* __restrict__ flags, const float* __restrict__ gate, float gate_min,
-                        const float* const* __restrict__ mask_ptr) {
+                        const float* const* __restrict__ mask_ptr, LiveCount live) {
   chain_wait();
+  if constexpr (kCounted) {
+    if ((int)blockIdx.x >= live_count(live)) return;
+  }
   extern __shared__ __align__(128) unsigned char s_raw[];
   if (gate && !(gate[blockIdx.x] > gate_min)) {
     const int nw = p4 >> 3;
@@ -414,12 +420,13 @@ __device__ __forceinline__ void pk_consumer_barrier() { asm volatile("bar.sync 1
 
 // (min-blocks 3 only caps the registers at 72 per thread: the grid holds two CTAs per SM, and the registers this
 // kernel does not take are what the kernels of the other images run in)
-template <int kPersistStages>
+template <int kPersistStages, bool kCounted>
 __global__ void __launch_bounds__(kPackBlock, 3)
 lowres_pack_persistent_kernel(const float4* __restrict__ logits, int n_masks, int p4 /* pixels/4 per mask */,
                               int words_per_row, uint32_t* __restrict__ bits, int32_t* __restrict__ area,
                               int32_t* __restrict__ box, int32_t* __restrict__ flags, const float* __restrict__ gate,
-                              float gate_min, const float* const* __restrict__ mask_ptr) {
+                              float gate_min, const float* const* __restrict__ mask_ptr, LiveCount live) {
+  if constexpr (kCounted) n_masks = live_count(live);
   extern __shared__ __align__(128) unsigned char s_raw[];
   uint4* s_stage = reinterpret_cast<uint4*>(s_raw);
   const int n_words = p4 >> 3;
@@ -602,11 +609,14 @@ int g_pack_persistent = 1;
 // gate (nullable): per-mask score; masks with !(gate[n] > gate_min) are skipped and published as empty
 // mask_ptr (nullable, device [n]): mask n is read from mask_ptr[n] (16-byte aligned) instead of logits + n*h*w
 // stab != NULL takes the literal per-element kernel, which also counts the stability thresholds
+// live (nullable): n is a counted call's capacity, the masks stop at the live count (not with stab: the literal kernel
+// is not on the counted path)
 int launch_lowres_pack(const float* logits, int n, int h, int w, float thr, float off, uint32_t* bits,
                        int32_t* area, int32_t* box, int32_t* stab, int32_t* flags, const float* gate, float gate_min,
-                       const float* const* mask_ptr, cudaStream_t s, float* stab_score) {
+                       const float* const* mask_ptr, cudaStream_t s, float* stab_score, const LiveCount* live) {
   const long p = (long)h * w;
   if (n <= 0) return NTTT_OK;
+  if (live && stab) return NTTT_EINVAL;
   if (w % 32 != 0 || p % 128 != 0 || p / 32 * 4 > 32 * 1024) return NTTT_EUNSUPPORTED;
   if (!mask_ptr && (reinterpret_cast<uintptr_t>(logits) & 15) != 0) return NTTT_EINVAL;  // TMA bulk copies need 16-byte alignment
   const size_t smem = (size_t)kPackStages * kPackStageBytes + (size_t)(p / 32) * sizeof(uint32_t);
@@ -619,14 +629,16 @@ int launch_lowres_pack(const float* logits, int n, int h, int w, float thr, floa
     constexpr int kCtasPerSm = 2, kStages = 3;
     const size_t sm = (size_t)kStages * kPackStageBytes + 2 * (size_t)(p / 32) * sizeof(uint32_t);  // (words double-buffered)
     const int grid = min(n, kCtasPerSm * current_sm_count());
-    NTTT_CUDA(set_dyn_smem(lowres_pack_persistent_kernel<kStages>, (int)sm));
-    lowres_pack_persistent_kernel<kStages><<<grid, kPackBlock, sm, s>>>(src, n, (int)(p / 4), w / 32, bits, area, box, flags,
-                                                                        gate, gate_min, mask_ptr);
+    auto kern = live ? lowres_pack_persistent_kernel<kStages, true> : lowres_pack_persistent_kernel<kStages, false>;
+    NTTT_CUDA(set_dyn_smem(kern, (int)sm));
+    kern<<<grid, kPackBlock, sm, s>>>(src, n, (int)(p / 4), w / 32, bits, area, box, flags, gate, gate_min, mask_ptr,
+                                      live ? *live : LiveCount{});
   } else {
-    NTTT_CUDA(set_dyn_smem(lowres_pack_fast_kernel, (int)smem));
+    auto kern = live ? lowres_pack_fast_kernel<true> : lowres_pack_fast_kernel<false>;
+    NTTT_CUDA(set_dyn_smem(kern, (int)smem));
     // (first kernel of the chain, behind the fork event of the low-latency mode: an ordinary launch)
-    lowres_pack_fast_kernel<<<n, kPackBlock, smem, s>>>(src, (int)(p / 4), w / 32, bits, area, box, flags, gate, gate_min,
-                                                        mask_ptr);
+    kern<<<n, kPackBlock, smem, s>>>(src, (int)(p / 4), w / 32, bits, area, box, flags, gate, gate_min, mask_ptr,
+                                     live ? *live : LiveCount{});
   }
   NTTT_LAUNCH_CHECK();
   return NTTT_OK;
@@ -677,10 +689,13 @@ int launch_multimask_select(const float* ious, int n, int m, int first, const Ch
 
 // Single-plane inputs of the bound entry: mask i's address and score, in the form the multimask path leaves them, so
 // that the low-res pass, the iou_thr gate, NMS and the resize run their mask_ptr / plane_score forms unchanged.
+// kCounted: the bound tensors hold the live count's rows; nothing at or past it is read.
+template <bool kCounted>
 __global__ void __launch_bounds__(256)
 plane_resolve_kernel(const nttt_match_inputs* __restrict__ in, int n, size_t plane_elems,
-                     const float** __restrict__ mask_ptr, float* __restrict__ score) {
+                     const float** __restrict__ mask_ptr, float* __restrict__ score, LiveCount live) {
   chain_wait();
+  if constexpr (kCounted) n = live_count(live);
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   mask_ptr[i] = in->logits + (size_t)i * plane_elems;
@@ -688,9 +703,10 @@ plane_resolve_kernel(const nttt_match_inputs* __restrict__ in, int n, size_t pla
 }
 
 int launch_plane_resolve(const nttt_match_inputs* in, int n, size_t plane_elems, const float** mask_ptr, float* score,
-                         cudaStream_t s) {
+                         cudaStream_t s, const LiveCount* live) {
   if (n <= 0) return NTTT_OK;
-  launch_chain(plane_resolve_kernel, dim3(ceil_div(n, 256)), dim3(256), 0, s, in, n, plane_elems, mask_ptr, score);
+  launch_chain(live ? plane_resolve_kernel<true> : plane_resolve_kernel<false>, dim3(ceil_div(n, 256)), dim3(256), 0, s, in,
+               n, plane_elems, mask_ptr, score, live ? *live : LiveCount{});
   NTTT_LAUNCH_CHECK();
   return NTTT_OK;
 }
@@ -716,6 +732,17 @@ int launch_match_bind(const T& v, T* dst, cudaStream_t s) {
 }
 template int launch_match_bind(const nttt_match_inputs&, nttt_match_inputs*, cudaStream_t);
 template int launch_match_bind(const nttt_match_bank&, nttt_match_bank*, cudaStream_t);
+
+// nttt_match_count_bind: the count travels as the kernel's argument
+__global__ void __launch_bounds__(32) count_bind_kernel(int32_t n, int32_t* __restrict__ dst) {
+  if (threadIdx.x == 0) *dst = n;
+}
+
+int launch_count_bind(int32_t n, int32_t* dst, cudaStream_t s) {
+  count_bind_kernel<<<1, 32, 0, s>>>(n, dst);
+  NTTT_LAUNCH_CHECK();
+  return NTTT_OK;
+}
 
 // ---------------------------------------------------------------------------------------------------
 // Antialias weight tables.  Exact fp32 recipe (every operation individually rounded, no contraction):
@@ -1008,12 +1035,14 @@ __device__ __forceinline__ void warp_range(int n, F flag, int& lo, int& hi) {
   hi = b1 ? 63 - __clz(b1) : (b0 ? 31 - __clz(b0) : 0);
 }
 
-template <bool kSplit>
+// kCounted (nttt_match_image_counted): n_masks is the capacity; the masks stop at the live count
+template <bool kSplit, bool kCounted>
 __global__ void __launch_bounds__(kProjThreads)
 project_masks_kernel(const uint32_t* __restrict__ bits, const int32_t* __restrict__ box, int n_masks, int h,
                      int words_per_row, int eh, int ew, ProjTables t, void* __restrict__ out, int stride_or_kp,
-                     const int32_t* __restrict__ perm, uint32_t* __restrict__ active) {
+                     const int32_t* __restrict__ perm, uint32_t* __restrict__ active, LiveCount live) {
   chain_wait();
+  if constexpr (kCounted) n_masks = live_count(live);
   extern __shared__ uint32_t smem[];
   // layout: x_lo[ew] x_len[ew] y_lo[eh] y_len[eh] | bits[rc*wpr] | row[rc*ew] | acc[eh*ew]     (rc = min(h, kProjRows))
   // (the weight tables — running column sums, row weights — are the same for every mask and are read through L1
@@ -1153,10 +1182,12 @@ static size_t project_smem_bytes(int h, int w, int eh, int ew) {
 }
 
 // split=false: out = float [n, out_stride];  split=true: out = bf16 [n, 3*out_stride] with out_stride = kp
+// live (nullable, split only): n is a counted call's capacity
 int launch_project_masks(const AxisTable& tx, const AxisTable& ty, const uint32_t* bits, const int32_t* box, int n,
                          int h, int w, int eh, int ew, void* out, int out_stride, bool split, cudaStream_t s,
-                         const int32_t* perm, uint32_t* active) {
+                         const int32_t* perm, uint32_t* active, const LiveCount* live) {
   if (n <= 0) return NTTT_OK;
+  if (live && !split) return NTTT_EINVAL;
   if (w % 32 != 0 || eh > 64 || ew > 64) return NTTT_EUNSUPPORTED;
   const size_t smem = project_smem_bytes(h, w, eh, ew);
   if (smem > 200 * 1024) return NTTT_EUNSUPPORTED;
@@ -1165,14 +1196,16 @@ int launch_project_masks(const AxisTable& tx, const AxisTable& ty, const uint32_
   // the span tables are staged once per CTA and 1024 CTA launches become 296); low-latency mode: one CTA per mask
   const int grid = t_low_latency ? n : min(n, 2 * current_sm_count());
   if (split) {
+    auto kern = live ? project_masks_kernel<true, true> : project_masks_kernel<true, false>;
     if (smem > 48 * 1024)
-      NTTT_CUDA(set_dyn_smem(project_masks_kernel<true>, (int)smem));
-    launch_chain(project_masks_kernel<true>, grid, kProjThreads, smem, s, bits, box, n, h, w / 32, eh, ew, t, out, out_stride, perm,
-                 active);
+      NTTT_CUDA(set_dyn_smem(kern, (int)smem));
+    launch_chain(kern, grid, kProjThreads, smem, s, bits, box, n, h, w / 32, eh, ew, t, out, out_stride, perm,
+                 active, live ? *live : LiveCount{});
   } else {
     if (smem > 48 * 1024)
-      NTTT_CUDA(set_dyn_smem(project_masks_kernel<false>, (int)smem));
-    project_masks_kernel<false><<<grid, kProjThreads, smem, s>>>(bits, box, n, h, w / 32, eh, ew, t, out, out_stride, perm, active);
+      NTTT_CUDA(set_dyn_smem(project_masks_kernel<false, false>, (int)smem));
+    project_masks_kernel<false, false><<<grid, kProjThreads, smem, s>>>(bits, box, n, h, w / 32, eh, ew, t, out, out_stride,
+                                                                        perm, active, LiveCount{});
   }
   NTTT_LAUNCH_CHECK();
   return NTTT_OK;
@@ -1188,10 +1221,13 @@ int launch_project_masks(const AxisTable& tx, const AxisTable& ty, const uint32_
 // ---------------------------------------------------------------------------------------------------
 // kMaxPer keys per thread: n <= 1024 * kMaxPer (8: up to 8192 masks, 16: up to 16 384)
 constexpr int kOrderBins = 64 * 64;
-template <int kMaxPer>
+// kCounted (nttt_match_image_counted): n is the capacity; the order covers the live count's masks, so that their rows are
+// [0, live count) as nttt_match_image at that count makes them
+template <int kMaxPer, bool kCounted>
 __global__ void __launch_bounds__(1024)
-pool_order_kernel(const int32_t* __restrict__ box, int n, int h, int32_t* __restrict__ perm) {
+pool_order_kernel(const int32_t* __restrict__ box, int n, int h, int32_t* __restrict__ perm, LiveCount live) {
   chain_wait();
+  if constexpr (kCounted) n = live_count(live);
   __shared__ int s_hist[kOrderBins];
   __shared__ int s_warp[33];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -1251,14 +1287,16 @@ pool_order_kernel(const int32_t* __restrict__ box, int n, int h, int32_t* __rest
   }
 }
 
-int launch_pool_order(const int32_t* box, int n, int h, int32_t* perm, cudaStream_t s) {
+// live (nullable): n is a counted call's capacity
+int launch_pool_order(const int32_t* box, int n, int h, int32_t* perm, cudaStream_t s, const LiveCount* live) {
   if (n <= 0) return NTTT_OK;
   if (n > NTTT_MAX_CANDIDATES) return NTTT_EUNSUPPORTED;
   static_assert(NTTT_MAX_CANDIDATES <= 16 * 1024, "pool_order_kernel holds at most 16 keys per thread");
+  const LiveCount lc = live ? *live : LiveCount{};
   if (n <= 8 * 1024)
-    launch_chain(pool_order_kernel<8>, 1, 1024, 0, s, box, n, h, perm);
+    launch_chain(live ? pool_order_kernel<8, true> : pool_order_kernel<8, false>, 1, 1024, 0, s, box, n, h, perm, lc);
   else
-    launch_chain(pool_order_kernel<16>, 1, 1024, 0, s, box, n, h, perm);
+    launch_chain(live ? pool_order_kernel<16, true> : pool_order_kernel<16, false>, 1, 1024, 0, s, box, n, h, perm, lc);
   NTTT_LAUNCH_CHECK();
   return NTTT_OK;
 }

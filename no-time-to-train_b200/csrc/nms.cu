@@ -9,6 +9,8 @@
 
 namespace nttt {
 
+__device__ __forceinline__ int ceil_div_dev(int a, int b) { return (a + b - 1) / b; }
+
 // float -> uint key whose ascending order is the float's DESCENDING order (positive NaN first, like torch)
 __device__ __forceinline__ uint32_t desc_key(float f) {
   uint32_t u = __float_as_uint(f);
@@ -19,13 +21,32 @@ __device__ __forceinline__ uint32_t desc_key(float f) {
 // single-CTA bitonic sort of (score desc, index asc); also gathers the boxes / labels into sorted order so the
 // matrix kernel reads them coalesced instead of chasing order[] -> box[] pointers.
 // kReg: n_pad <= 1024, one key per thread in registers (warp shuffles for the short exchanges)
-template <bool kReg>
+// Counted (nttt_match_image_counted), every kernel of this file: the launch fixes the capacity's instance, grid and
+// shared memory; the kCounted instance reads the live count k and works on the list of k boxes — the padded length
+// (next power of two at or above k), the matrix's row words and the nz words all follow k, so the matrix and nz are laid
+// out for k inside the capacity's buffers.  nms_sort_kernel also writes the count status (live.status).
+__device__ __forceinline__ int nms_pow2(int n) {
+  int p = 1;
+  while (p < n) p <<= 1;
+  return p;
+}
+
+template <bool kReg, bool kCounted>
 __global__ void __launch_bounds__(1024)
 nms_sort_kernel(const float* __restrict__ scores, const int32_t* __restrict__ box, const int32_t* __restrict__ labels,
                 int n, int n_pad, float min_score, int filter, int32_t* __restrict__ order,
                 float4* __restrict__ sorted_box, int32_t* __restrict__ sorted_label, uint32_t* __restrict__ nz,
-                int nz_total) {
+                int nz_total, LiveCount live) {
   chain_wait();
+  if constexpr (kCounted) {
+    n = live_count(live);
+    if (!kReg) n_pad = nms_pow2(n);
+    if (nz) nz_total = n * ((ceil_div_dev(n, 32) + 31) / 32);
+    if (threadIdx.x == 0 && live.status) {
+      const int raw = *live.n;
+      *live.status = (raw >= 0 && raw <= live.cap) ? 0 : kCountStatus;
+    }
+  }
   extern __shared__ unsigned long long s_keys[];
   // (lists above 1024 boxes) clear the per-row summary of non-zero matrix words that nms_mask_kernel ORs into
   for (int i = threadIdx.x; i < nz_total; i += blockDim.x) nz[i] = 0u;
@@ -78,13 +99,17 @@ nms_sort_kernel(const float* __restrict__ scores, const int32_t* __restrict__ bo
 // kPosBits: the position field holds n_pad <= 2^kPosBits (13: up to 8192 boxes, 14: up to 16 384).  Filtered boxes carry
 // the labels -2 - i (i < n), so the bias 2^kPosBits + 2 keeps every label + bias >= 1; class labels stay below
 // 2^(32 - kPosBits) - 2^kPosBits - 3, so that no key reaches the padding key 0xffffffff.
-template <int kPosBits>
+template <int kPosBits, bool kCounted>
 __global__ void __launch_bounds__(1024)
 nms_class_sort_kernel(const float4* __restrict__ sorted_box, const int32_t* __restrict__ sorted_label, int n, int n_pad,
-                      int32_t* __restrict__ c2s, float4* __restrict__ cbox, int32_t* __restrict__ clabel) {
+                      int32_t* __restrict__ c2s, float4* __restrict__ cbox, int32_t* __restrict__ clabel, LiveCount live) {
   constexpr int kClassKeyBias = (1 << kPosBits) + 2;
   static_assert(-2 - ((1 << kPosBits) - 1) + kClassKeyBias >= 1, "the lowest filtered-box label must bias to >= 1");
   chain_wait();
+  if constexpr (kCounted) {
+    n = live_count(live);
+    n_pad = nms_pow2(n);
+  }
   extern __shared__ unsigned long long s_keys[];
   uint32_t* keys = reinterpret_cast<uint32_t*>(s_keys);
   for (int i = threadIdx.x; i < n_pad; i += blockDim.x)
@@ -114,11 +139,17 @@ nms_class_sort_kernel(const float4* __restrict__ sorted_box, const int32_t* __re
 // suppression bit matrix in sorted order.  kByVictim: bit i of row j set iff i < j, same label, IoU(i,j) > thr — row j
 // lists the earlier boxes that would suppress j if they are kept (wavefront scan).  Otherwise by suppressor: bit j of
 // row i set iff j > i (serial scan).  The IoU arithmetic is symmetric in its two boxes (float additions commute exactly).
-template <bool kByVictim>
+template <bool kByVictim, bool kCounted>
 __global__ void __launch_bounds__(256)
 nms_mask_kernel(const float4* __restrict__ sorted_box, const int32_t* __restrict__ sorted_label, int n, float thr,
-                uint32_t* __restrict__ mask, int row_words, uint32_t* __restrict__ nz, int nz_words, int class_sorted) {
+                uint32_t* __restrict__ mask, int row_words, uint32_t* __restrict__ nz, int nz_words, int class_sorted,
+                LiveCount live) {
   chain_wait();
+  if constexpr (kCounted) {
+    n = live_count(live);
+    row_words = ceil_div_dev(n, 32);
+    nz_words = (row_words + 31) / 32;
+  }
   // class_sorted (by-victim form with the nz summary only): the boxes are ordered by (label, score) and the labels
   // ascend, so a block whose last column box has a smaller label than its first row box holds no same-label pair at all.
   // It writes nothing — the scan only reads the words flagged in `nz` — and with 80 classes that is all but the two or
@@ -201,12 +232,17 @@ constexpr int kClassPosBitsMid = 13, kClassPosBitsMax = 14;
 static_assert((1 << kClassPosBitsMid) >= kScanMidN && (1 << kClassPosBitsMax) >= kScanMaxN,
               "a class-order key's position field must hold every position of the padded list");
 
+template <bool kCounted>
 __global__ void __launch_bounds__(kScanThreads, 1)
 nms_wave_kernel(const uint32_t* __restrict__ mt, int row_words, const int32_t* __restrict__ order,
                 const int32_t* __restrict__ sorted_label, const float* __restrict__ top_score, int n, int max_keep,
                 int32_t* __restrict__ keep, int32_t* __restrict__ n_keep, int32_t* __restrict__ sel,
-                int32_t* __restrict__ n_sel) {
+                int32_t* __restrict__ n_sel, LiveCount live) {
   chain_wait();
+  if constexpr (kCounted) {
+    n = live_count(live);
+    row_words = ceil_div_dev(n, 32);
+  }
   // (n <= 1024 uses the first 32 words of each array)
   __shared__ uint32_t s_K[kScanMidN / 32];    // keep bits per chunk, then truncated to max_keep
   __shared__ uint32_t s_S[kScanMidN / 32];    // positive-score flags, then `sel` bits
@@ -310,18 +346,23 @@ nms_wave_kernel(const uint32_t* __restrict__ mt, int row_words, const int32_t* _
 // rounds or lower warps of the same round, all resident: no deadlock).  A row no longer fits in registers (128 words at
 // 4096 boxes), and almost all of it is zero, so the mask kernel leaves a per-row bitmap of its non-zero words (`nz`) and a
 // lane loads just those — the scan's work is proportional to the suppression pairs that exist, not to n^2 / 32.
-template <int kMaxN>
+template <int kMaxN, bool kCounted>
 __global__ void __launch_bounds__(kScanThreads, 1)
 nms_wave_sparse_kernel(const uint32_t* __restrict__ mt, const uint32_t* __restrict__ nz, int nz_words, int row_words,
                        const int32_t* __restrict__ order, const int32_t* __restrict__ sorted_label,
                        const float* __restrict__ top_score, int n, int max_keep, int32_t* __restrict__ keep,
                        int32_t* __restrict__ n_keep, int32_t* __restrict__ sel, int32_t* __restrict__ n_sel,
-                       const int32_t* __restrict__ c2s) {
+                       const int32_t* __restrict__ c2s, LiveCount live) {
   // c2s (nullable): the matrix, `nz` and `sorted_label` are in CLASS order (nms_class_sort_kernel) and c2s maps a position
   // there to the box's position in score order, which is what `order` and the output lists are in: the wavefront runs in
   // class order (any order that keeps same-label boxes in score order gives the same greedy result), its keep bits are
   // scattered to score order before the compaction.
   chain_wait();
+  if constexpr (kCounted) {
+    n = live_count(live);
+    row_words = ceil_div_dev(n, 32);
+    nz_words = (row_words + 31) / 32;
+  }
   __shared__ uint32_t s_K[kMaxN / 32];
   __shared__ uint32_t s_S[kMaxN / 32];
   __shared__ int s_pre[kMaxN / 32 + 1];
@@ -440,9 +481,10 @@ size_t nms_workspace_bytes(int n) {
          align_up(sizeof(float4) * (size_t)n, 256) + 2 * align_up(sizeof(int32_t) * (size_t)n, 256);
 }
 
+// live (nullable): n is a counted call's capacity; the kernels take the live count (see nms_sort_kernel)
 int launch_box_nms(const int32_t* box, const float* nms_scores, const int32_t* labels, const float* top_score, int n,
                    float thr, int max_keep, int32_t* keep, int32_t* n_keep, int32_t* sel, int32_t* n_sel, void* ws,
-                   size_t ws_bytes, float min_score, int filter, cudaStream_t s) {
+                   size_t ws_bytes, float min_score, int filter, cudaStream_t s, const LiveCount* live) {
   if (n <= 0 || max_keep <= 0) {
     NTTT_CUDA(cudaMemsetAsync(n_keep, 0, sizeof(int32_t), s));
     NTTT_CUDA(cudaMemsetAsync(n_sel, 0, sizeof(int32_t), s));
@@ -462,23 +504,27 @@ int launch_box_nms(const int32_t* box, const float* nms_scores, const int32_t* l
   uint32_t* nz = reinterpret_cast<uint32_t*>(reinterpret_cast<char*>(sorted_label) + align_up(sizeof(int32_t) * (size_t)n, 256));
   int n_pad = 1;
   while (n_pad < n) n_pad <<= 1;
+  const LiveCount lc = live ? *live : LiveCount{};
+  const bool cn = live != nullptr;
   if (n_pad <= 1024) {
-    launch_chain(nms_sort_kernel<true>, 1, 1024, sizeof(unsigned long long) * 1024, s, nms_scores, box, labels, n, 1024, min_score, filter, order,
-                                                                             sorted_box, sorted_label, nullptr, 0);
+    launch_chain(cn ? nms_sort_kernel<true, true> : nms_sort_kernel<true, false>, 1, 1024, sizeof(unsigned long long) * 1024, s,
+                 nms_scores, box, labels, n, 1024, min_score, filter, order, sorted_box, sorted_label, nullptr, 0, lc);
   } else {
     const size_t smem = sizeof(unsigned long long) * (size_t)n_pad;
+    auto kern = cn ? nms_sort_kernel<false, true> : nms_sort_kernel<false, false>;
     if (smem > 48 * 1024)
-      NTTT_CUDA(set_dyn_smem(nms_sort_kernel<false>, (int)smem));
-    launch_chain(nms_sort_kernel<false>, 1, 1024, smem, s, nms_scores, box, labels, n, n_pad, min_score, filter, order, sorted_box,
-                                                 sorted_label, nz, n * nz_words);
+      NTTT_CUDA(set_dyn_smem(kern, (int)smem));
+    launch_chain(kern, 1, 1024, smem, s, nms_scores, box, labels, n, n_pad, min_score, filter, order, sorted_box,
+                 sorted_label, nz, n * nz_words, lc);
   }
   NTTT_LAUNCH_CHECK();
   dim3 grid(ceil_div(row_words, 8), ceil_div(n, 32));
+  auto mask_kern = cn ? nms_mask_kernel<true, true> : nms_mask_kernel<true, false>;
   if (n <= 1024) {
-    launch_chain(nms_mask_kernel<true>, grid, dim3(32, 8), 0, s, sorted_box, sorted_label, n, thr, mask, row_words, nullptr, 0, 0);
+    launch_chain(mask_kern, grid, dim3(32, 8), 0, s, sorted_box, sorted_label, n, thr, mask, row_words, nullptr, 0, 0, lc);
     NTTT_LAUNCH_CHECK();
-    launch_chain(nms_wave_kernel, 1, kScanThreads, 0, s, mask, row_words, order, sorted_label, top_score, n, max_keep, keep, n_keep, sel,
-                                               n_sel);
+    launch_chain(cn ? nms_wave_kernel<true> : nms_wave_kernel<false>, 1, kScanThreads, 0, s, mask, row_words, order,
+                 sorted_label, top_score, n, max_keep, keep, n_keep, sel, n_sel, lc);
     NTTT_LAUNCH_CHECK();
     return NTTT_OK;
   }
@@ -489,21 +535,23 @@ int launch_box_nms(const int32_t* box, const float* nms_scores, const int32_t* l
   int32_t* c2s = reinterpret_cast<int32_t*>(reinterpret_cast<char*>(clabel) + align_up(sizeof(int32_t) * (size_t)n, 256));
   const size_t class_smem = sizeof(uint32_t) * (size_t)n_pad;
   if (n_pad <= kScanMidN) {
-    launch_chain(nms_class_sort_kernel<kClassPosBitsMid>, 1, 1024, class_smem, s, sorted_box, sorted_label, n, n_pad, c2s, cbox, clabel);
+    launch_chain(cn ? nms_class_sort_kernel<kClassPosBitsMid, true> : nms_class_sort_kernel<kClassPosBitsMid, false>, 1, 1024,
+                 class_smem, s, sorted_box, sorted_label, n, n_pad, c2s, cbox, clabel, lc);
   } else {
-    if (class_smem > 48 * 1024) NTTT_CUDA(set_dyn_smem(nms_class_sort_kernel<kClassPosBitsMax>, (int)class_smem));
-    launch_chain(nms_class_sort_kernel<kClassPosBitsMax>, 1, 1024, class_smem, s, sorted_box, sorted_label, n, n_pad, c2s, cbox, clabel);
+    auto kern = cn ? nms_class_sort_kernel<kClassPosBitsMax, true> : nms_class_sort_kernel<kClassPosBitsMax, false>;
+    if (class_smem > 48 * 1024) NTTT_CUDA(set_dyn_smem(kern, (int)class_smem));
+    launch_chain(kern, 1, 1024, class_smem, s, sorted_box, sorted_label, n, n_pad, c2s, cbox, clabel, lc);
   }
   NTTT_LAUNCH_CHECK();
-  launch_chain(nms_mask_kernel<true>, grid, dim3(32, 8), 0, s, cbox, clabel, n, thr, mask, row_words, nz, nz_words,
-               /*class_sorted=*/1);
+  launch_chain(mask_kern, grid, dim3(32, 8), 0, s, cbox, clabel, n, thr, mask, row_words, nz, nz_words,
+               /*class_sorted=*/1, lc);
   NTTT_LAUNCH_CHECK();
   if (n <= kScanMidN)
-    launch_chain(nms_wave_sparse_kernel<kScanMidN>, 1, kScanThreads, 0, s, mask, nz, nz_words, row_words, order, clabel,
-                 top_score, n, max_keep, keep, n_keep, sel, n_sel, c2s);
+    launch_chain(cn ? nms_wave_sparse_kernel<kScanMidN, true> : nms_wave_sparse_kernel<kScanMidN, false>, 1, kScanThreads, 0,
+                 s, mask, nz, nz_words, row_words, order, clabel, top_score, n, max_keep, keep, n_keep, sel, n_sel, c2s, lc);
   else
-    launch_chain(nms_wave_sparse_kernel<kScanMaxN>, 1, kScanThreads, 0, s, mask, nz, nz_words, row_words, order, clabel,
-                 top_score, n, max_keep, keep, n_keep, sel, n_sel, c2s);
+    launch_chain(cn ? nms_wave_sparse_kernel<kScanMaxN, true> : nms_wave_sparse_kernel<kScanMaxN, false>, 1, kScanThreads, 0,
+                 s, mask, nz, nz_words, row_words, order, clabel, top_score, n, max_keep, keep, n_keep, sel, n_sel, c2s, lc);
   NTTT_LAUNCH_CHECK();
   return NTTT_OK;
 }

@@ -13,11 +13,14 @@ namespace nttt {
 // one warp per row.  nan_empty: the negative-reference variant has NO zero guard (matching_baseline_utils.py:925,
 // Sam2MatchingBaseline_noAMG.py:598-600): an empty mask divides 0 by 0 and its whole row is NaN, as in the reference.
 // ---------------------------------------------------------------------------------------------------
+// kCounted (nttt_match_image_counted, both kernels): n is the capacity and keeps the partials' stride; the rows stop at
+// the live count
+template <bool kCounted>
 __global__ void __launch_bounds__(256)
 normalize_rows_kernel(const float* __restrict__ sums, int n_partials, const int32_t* __restrict__ area, int n, int c,
-                      float* __restrict__ out, bool nan_empty) {
+                      float* __restrict__ out, bool nan_empty, LiveCount live) {
   const int row = blockIdx.x * 8 + warp_id();
-  if (row >= n) return;
+  if (row >= (kCounted ? live_count(live) : n)) return;
   const int lane = lane_id();
   float denom = 1.0f;
   if (area) { const int a = area[row]; denom = (a == 0 && !nan_empty) ? 1.0f : (float)a; }
@@ -41,15 +44,15 @@ normalize_rows_kernel(const float* __restrict__ sums, int n_partials, const int3
 // Vector path for encoder widths that are multiples of 128 (384, 768, 1024, 1536): one warp per row keeps the
 // whole row in registers (one pass over HBM), and also emits the split-bf16 A operand [hi | hi | lo] of the
 // similarity GEMM so no separate conversion pass is needed.
-template <int kVec>  // float4 per lane, c = 128 * kVec
+template <int kVec, bool kCounted>  // float4 per lane, c = 128 * kVec
 __global__ void __launch_bounds__(256)
 normalize_split_kernel(const float* __restrict__ sums, int n_partials, const int32_t* __restrict__ area, int n, int cp,
                        float* __restrict__ out, __nv_bfloat16* __restrict__ split, bool nan_empty,
-                       const int32_t* __restrict__ perm) {
+                       const int32_t* __restrict__ perm, LiveCount live) {
   chain_wait();
   constexpr int c = 128 * kVec;
   const int row = blockIdx.x * 8 + warp_id();
-  if (row >= n) return;
+  if (row >= (kCounted ? live_count(live) : n)) return;
   const int lane = lane_id();
   float denom = 1.0f;
   if (area) { const int a = area[row]; denom = (a == 0 && !nan_empty) ? 1.0f : (float)a; }
@@ -105,17 +108,30 @@ normalize_split_kernel(const float* __restrict__ sums, int n_partials, const int
 }
 
 // returns 1 if the fused vector path ran (split written), 0 if the caller must use the generic kernels
+// live (nullable, both launchers): n is a counted call's capacity, the rows stop at the live count
+template <int kVec>
+static void launch_normalize_split_vec(int grid, cudaStream_t s, const float* sums, int n_partials, const int32_t* area,
+                                       int n, int cp, float* out, __nv_bfloat16* sp, bool nan_empty, const int32_t* perm,
+                                       const LiveCount* live) {
+  if (live)
+    launch_chain(normalize_split_kernel<kVec, true>, grid, 256, 0, s, sums, n_partials, area, n, cp, out, sp, nan_empty,
+                 perm, *live);
+  else
+    launch_chain(normalize_split_kernel<kVec, false>, grid, 256, 0, s, sums, n_partials, area, n, cp, out, sp, nan_empty,
+                 perm, LiveCount{});
+}
+
 int launch_normalize_split(const float* sums, int n_partials, const int32_t* area, int n, int c, int cp, float* out,
-                           void* split, bool nan_empty, cudaStream_t s, const int32_t* perm) {
+                           void* split, bool nan_empty, cudaStream_t s, const int32_t* perm, const LiveCount* live) {
   if (n <= 0) return 1;
   if (c % 128 != 0 || cp != c) return 0;
   const int grid = ceil_div(n, 8);
   __nv_bfloat16* sp = static_cast<__nv_bfloat16*>(split);
   switch (c / 128) {
-    case 3: launch_chain(normalize_split_kernel<3>, grid, 256, 0, s, sums, n_partials, area, n, cp, out, sp, nan_empty, perm); break;
-    case 6: launch_chain(normalize_split_kernel<6>, grid, 256, 0, s, sums, n_partials, area, n, cp, out, sp, nan_empty, perm); break;
-    case 8: launch_chain(normalize_split_kernel<8>, grid, 256, 0, s, sums, n_partials, area, n, cp, out, sp, nan_empty, perm); break;
-    case 12: launch_chain(normalize_split_kernel<12>, grid, 256, 0, s, sums, n_partials, area, n, cp, out, sp, nan_empty, perm); break;
+    case 3: launch_normalize_split_vec<3>(grid, s, sums, n_partials, area, n, cp, out, sp, nan_empty, perm, live); break;
+    case 6: launch_normalize_split_vec<6>(grid, s, sums, n_partials, area, n, cp, out, sp, nan_empty, perm, live); break;
+    case 8: launch_normalize_split_vec<8>(grid, s, sums, n_partials, area, n, cp, out, sp, nan_empty, perm, live); break;
+    case 12: launch_normalize_split_vec<12>(grid, s, sums, n_partials, area, n, cp, out, sp, nan_empty, perm, live); break;
     default: return 0;
   }
   ++g_launches;
@@ -124,9 +140,10 @@ int launch_normalize_split(const float* sums, int n_partials, const int32_t* are
 }
 
 int launch_normalize_rows(const float* sums, int n_partials, const int32_t* area, int n, int c, float* out,
-                          bool nan_empty, cudaStream_t s) {
+                          bool nan_empty, cudaStream_t s, const LiveCount* live) {
   if (n <= 0) return NTTT_OK;
-  normalize_rows_kernel<<<ceil_div(n, 8), 256, 0, s>>>(sums, n_partials, area, n, c, out, nan_empty);
+  (live ? normalize_rows_kernel<true> : normalize_rows_kernel<false>)<<<ceil_div(n, 8), 256, 0, s>>>(
+      sums, n_partials, area, n, c, out, nan_empty, live ? *live : LiveCount{});
   NTTT_LAUNCH_CHECK();
   return NTTT_OK;
 }
@@ -178,12 +195,22 @@ __device__ __forceinline__ float clamp_min0(float x) { return x < 0.0f ? 0.0f : 
 // kBank (nttt_match_image_banked): n_cls is the bank's capacity (the strides stay ld); the arg-max, the `sim` tap and the
 // one-class rule take the live class count of *bank.  The loop stops there: a padded column (similarity 0) must not beat
 // a row whose live similarities are all negative.
-template <bool kBank>
+// kCounted (nttt_match_image_counted): n is the candidate capacity; the rows stop at the live count, and with
+// live.split_sm the partials are those gemm_tc_kernel<.., true> left at that count: as many as nttt_match_image adds at
+// it, live-count * ld floats apart.
+template <bool kBank, bool kCounted>
 __global__ void __launch_bounds__(256)
 top1_kernel(const float* __restrict__ part, int n_splits, size_t split_stride, float* __restrict__ sim, int ld, int n,
             int n_cls, float* __restrict__ top_score, int32_t* __restrict__ top_label,
-            const nttt_match_bank* __restrict__ bank) {
+            const nttt_match_bank* __restrict__ bank, LiveCount live) {
   chain_wait();
+  if constexpr (kCounted) {
+    n = live_count(live);
+    if (live.split_sm > 0) {
+      n_splits = split_count(live.split_k, sim_split_want(n, ld, live.split_k, live.split_sm));
+      split_stride = (size_t)n * ld;
+    }
+  }
   if constexpr (kBank) n_cls = bank->n_cls;
   const int row = blockIdx.x * 8 + warp_id();
   if (row >= n) return;
@@ -211,11 +238,14 @@ top1_kernel(const float* __restrict__ part, int n_splits, size_t split_stride, f
 }
 
 // bank (nullable): the live class count is read from it (n_cls is then the capacity)
+// live (nullable): n is a counted call's capacity (top1_kernel<.., true>)
 int launch_top1(const float* part, int n_splits, size_t split_stride, float* sim, int ld, int n, int n_cls,
-                float* top_score, int32_t* top_label, cudaStream_t s, const nttt_match_bank* bank) {
+                float* top_score, int32_t* top_label, cudaStream_t s, const nttt_match_bank* bank, const LiveCount* live) {
   if (n <= 0) return NTTT_OK;
-  launch_chain(bank ? top1_kernel<true> : top1_kernel<false>, ceil_div(n, 8), 256, 0, s, part, n_splits, split_stride, sim,
-               ld, n, n_cls, top_score, top_label, bank);
+  auto kern = live ? (bank ? top1_kernel<true, true> : top1_kernel<false, true>)
+                   : (bank ? top1_kernel<true, false> : top1_kernel<false, false>);
+  launch_chain(kern, ceil_div(n, 8), 256, 0, s, part, n_splits, split_stride, sim, ld, n, n_cls, top_score, top_label, bank,
+               live ? *live : LiveCount{});
   NTTT_LAUNCH_CHECK();
   return NTTT_OK;
 }
@@ -226,13 +256,23 @@ int launch_top1(const float* part, int n_splits, size_t split_stride, float* sim
 // Both similarity matrices arrive as split-K partials and are summed here in a fixed order.
 // kBank (nttt_match_image_banked): n_cls and l_neg are the capacity and fix the strides of the partials and of `sim`; the
 // loops take the live counts of *bank, whose negatives are packed live_cls x live_l (bank_rows) in the GEMM's columns.
-template <bool kBank>
+// kCounted: as top1_kernel, for both similarity matrices.
+template <bool kBank, bool kCounted>
 __global__ void __launch_bounds__(256)
 neg_top1_kernel(const float* __restrict__ part_pos, int splits_pos, size_t stride_pos,
                 const float* __restrict__ part_neg, int splits_neg, size_t stride_neg, int n, int n_cls, int l_neg,
                 float sigma, float* __restrict__ sim, float* __restrict__ top_score, int32_t* __restrict__ top_label,
-                const nttt_match_bank* __restrict__ bank) {
+                const nttt_match_bank* __restrict__ bank, LiveCount live) {
   chain_wait();
+  if constexpr (kCounted) {
+    n = live_count(live);
+    if (live.split_sm > 0) {
+      splits_pos = split_count(live.split_k, sim_split_want(n, n_cls, live.split_k, live.split_sm));
+      splits_neg = split_count(live.split_k, sim_split_want(n, n_cls * l_neg, live.split_k, live.split_sm));
+      stride_pos = (size_t)n * n_cls;
+      stride_neg = (size_t)n * n_cls * l_neg;
+    }
+  }
   int live_cls = n_cls, live_l = l_neg;
   if constexpr (kBank) {
     live_cls = bank->n_cls;
@@ -274,10 +314,12 @@ neg_top1_kernel(const float* __restrict__ part_pos, int splits_pos, size_t strid
 
 int launch_neg_top1(const float* part_pos, int splits_pos, size_t stride_pos, const float* part_neg, int splits_neg,
                     size_t stride_neg, int n, int n_cls, int l_neg, float sigma, float* sim, float* top_score,
-                    int32_t* top_label, cudaStream_t s, const nttt_match_bank* bank) {
+                    int32_t* top_label, cudaStream_t s, const nttt_match_bank* bank, const LiveCount* live) {
   if (n <= 0) return NTTT_OK;
-  launch_chain(bank ? neg_top1_kernel<true> : neg_top1_kernel<false>, ceil_div(n, 8), 256, 0, s, part_pos, splits_pos,
-               stride_pos, part_neg, splits_neg, stride_neg, n, n_cls, l_neg, sigma, sim, top_score, top_label, bank);
+  auto kern = live ? (bank ? neg_top1_kernel<true, true> : neg_top1_kernel<false, true>)
+                   : (bank ? neg_top1_kernel<true, false> : neg_top1_kernel<false, false>);
+  launch_chain(kern, ceil_div(n, 8), 256, 0, s, part_pos, splits_pos, stride_pos, part_neg, splits_neg, stride_neg, n, n_cls,
+               l_neg, sigma, sim, top_score, top_label, bank, live ? *live : LiveCount{});
   NTTT_LAUNCH_CHECK();
   return NTTT_OK;
 }

@@ -85,7 +85,7 @@ class PendingResult:
     """Device-side result of one image; `.get()` does the single D2H read of the counts and slices."""
 
     def __init__(self, stage, masks, boxes, scores, labels, index, counts, taps, ori_hw, keepalive, rle=None, meta=None,
-                 sized=False, sim_cols=None):
+                 sized=False, sim_cols=None, counted=False, rows=None):
         self._stage = stage
         self.masks, self.boxes, self.scores, self.labels, self.index = masks, boxes, scores, labels, index
         self.counts = counts
@@ -101,6 +101,10 @@ class PendingResult:
         self._bound = None  # a bound graph's replay: the tensors it reads (GraphedMatch.replay)
         self._bank = None  # a banked graph's replay: the bank it reads
         self._sim_cols = sim_cols  # banked: the live columns of the [n, capacity] `sim` tap
+        # counted entry (`match_async(..., count_capacity=...)`, `graphed(..., counted=True)`): the taps keep the capacity's
+        # rows, of which the first `rows` are this image's; the stage reports a count outside its capacity in counts[3]
+        self._counted = counted
+        self.rows = rows
 
     def rle_segmentations(self) -> list:
         """The outputs as COCO `segmentation` dicts ({"size": [h, w], "counts": str}) — what
@@ -142,9 +146,12 @@ class PendingResult:
     def _host_meta(self) -> list:
         if self._meta is None:
             self._meta = self._meta_dev.cpu().tolist()  # synchronises with the producing stream
-        if self._sized and self._meta[3] != 0:
+        if self._sized and self._meta[3] & 1:
             raise RuntimeError(f"the stage reported status {self._meta[3]}: the image size on the device lies outside "
                                "the range the stage was enqueued for (the result is empty)")
+        if self._counted and self._meta[3] & 2:
+            raise RuntimeError(f"the stage reported status {self._meta[3]}: the candidate count on the device lies outside "
+                               "the capacity the stage was enqueued for (the result is empty)")
         return self._meta
 
     def get(self) -> dict:
@@ -164,7 +171,12 @@ class PendingResult:
         out["counts"] = dict(n_keep=n_keep, n_sel=n_sel, n_out=n_out)
         out["index"] = self.index[:n_out]
         if self.taps:
-            out["taps"] = self.taps if self._sim_cols is None else dict(self.taps, sim=self.taps["sim"][:, :self._sim_cols])
+            taps = dict(self.taps)
+            if self._sim_cols is not None:
+                taps["sim"] = taps["sim"][:, :self._sim_cols]
+            if self._counted:
+                taps["sim"], taps["obj_feats"] = taps["sim"][:self.rows], taps["obj_feats"][:self.rows]
+            out["taps"] = taps
         return out
 
 
@@ -239,7 +251,7 @@ class MatchingStage:
                     taps: bool = False, slot=0, iou_thr=None, persistent_out=None, multi_ious=None,
                     multi_first: int = 1, rle: bool = False, dense_masks: bool = True,
                     low_latency: bool = False, size_range=None, bound_inputs=None, bank=None, bank_capacity=None,
-                    bank_dev=None) -> PendingResult:
+                    bank_dev=None, count_capacity=None, count_dev=None) -> PendingResult:
         """Enqueue the whole stage for one image on the current stream.  `slot` selects which reusable
         workspace to use (callers that keep several images in flight on different streams use one slot per
         stream).  `iou_thr`, if given, fuses the reference's candidate filter (`scores_all > iou_thr`,
@@ -264,7 +276,13 @@ class MatchingStage:
         (l_neg > 0: negative-reference banks of up to l_neg negatives per class).  `bank` (a `PreparedBank`; default: the
         stage's current prototypes) is bound into a fresh struct on the current stream; `bank_dev` (a device buffer of
         `nttt_sizeof_match_bank()` bytes) is read as it stands instead, unbound here (as `GraphedMatch` does).  The `sim`
-        tap then keeps the capacity's columns on the device; `get()` returns the live ones."""
+        tap then keeps the capacity's columns on the device; `get()` returns the live ones.
+        `count_capacity=N` enqueues the counted entry (`nttt_match_image_counted`): the workspace, the grids and the
+        selection are sized for N candidates, and the kernels read the live count from a device int32 when they run, so
+        the call serves a compacted candidate list of any length k <= N (single-plane inputs only).  The count is the
+        tensors' rows, written into a fresh device int32 on the current stream; `count_dev` (a device int32 [1]) is read as
+        it stands instead, unwritten here (as `GraphedMatch` does with `counted=True`).  The `sim` and `obj_feats` taps
+        then keep N rows on the device; `get()` returns the first k."""
         banked = bank_capacity is not None
         if not banked and (bank is not None or bank_dev is not None):
             raise ValueError("bank= and bank_dev= need bank_capacity=(n_cls, l_neg)")
@@ -296,6 +314,17 @@ class MatchingStage:
             ops._need(pred_ious, torch.float32, "pred_ious")
             n, lh, lw = lr_masks.shape
         _check_candidates(n)
+        counted = count_capacity is not None
+        rows = n  # the candidates this call's tensors hold (counted: the live count k)
+        if counted:
+            if n_multi:
+                raise ValueError("the counted entry takes single-plane candidates (compacted lists), not multi_ious")
+            n = int(count_capacity)
+            _check_candidates(n)
+            if not 0 <= rows <= n:
+                raise ValueError(f"{rows} candidates exceed the count capacity {n}")
+        elif count_dev is not None:
+            raise ValueError("count_dev= needs count_capacity=N")
         eh, ew = self.cfg.enc_hw
         e, c = tar_feat.shape
         if e != eh * ew:
@@ -346,6 +375,12 @@ class MatchingStage:
         ws = self._workspace(("match", slot), ws_bytes)
         a = _lib.MatchArgs()
         a.logits, a.pred_ious, a.tar_feat = None if chunks else lr_masks.data_ptr(), ops._ptr(pred_ious), tar_feat.data_ptr()
+        empty_rows = None
+        if counted and rows == 0:
+            # an empty compacted list (`masks[keep]` with nothing kept) may have no address at all; the stage reads no
+            # row of it, so any valid 16-byte-aligned buffer stands in
+            empty_rows = torch.empty((4,), dtype=torch.float32, device=dev)
+            a.logits = a.pred_ious = empty_rows.data_ptr()
         a.proto = None if banked else self.proto.data_ptr()
         a.multi_ious, a.n_multi, a.multi_first = ops._ptr(multi_ious), n_multi, int(multi_first)
         if chunks:
@@ -377,10 +412,19 @@ class MatchingStage:
         a.low_latency = 1 if low_latency else 0
         stream = torch.cuda.current_stream(dev).cuda_stream
         rng = _lib.MatchSizeRange(hw_dev.data_ptr(), min_h, min_w) if size_range is not None else None
-        if banked:
-            if bank_dev is None:
-                bank_dev = torch.empty((int(self.lib.nttt_sizeof_match_bank()),), dtype=torch.uint8, device=dev)
-                self._bind_bank(bank_dev, bank, cap)
+        if banked and bank_dev is None:
+            bank_dev = torch.empty((int(self.lib.nttt_sizeof_match_bank()),), dtype=torch.uint8, device=dev)
+            self._bind_bank(bank_dev, bank, cap)
+        if counted:
+            if count_dev is None:
+                count_dev = torch.empty((1,), dtype=torch.int32, device=dev)
+                self._bind_count(count_dev, rows, n)
+            elif count_dev.dtype != torch.int32 or count_dev.numel() != 1 or count_dev.device != dev:
+                raise ValueError("count_dev must be an int32 [1] tensor on the stage's device")
+            _lib.check(self.lib.nttt_match_image_counted(self.ctx, ctypes.byref(a), ctypes.byref(rng) if rng else None,
+                                                         ops._ptr(bound_inputs), ops._ptr(bank_dev), count_dev.data_ptr(),
+                                                         stream), "nttt_match_image_counted")
+        elif banked:
             _lib.check(self.lib.nttt_match_image_banked(self.ctx, ctypes.byref(a), ctypes.byref(rng) if rng else None,
                                                         ops._ptr(bound_inputs), bank_dev.data_ptr(), stream),
                        "nttt_match_image_banked")
@@ -393,10 +437,19 @@ class MatchingStage:
             _lib.check(self.lib.nttt_match_image_sized(self.ctx, ctypes.byref(a), ctypes.byref(rng), stream),
                        "nttt_match_image_sized")
         return PendingResult(self, masks.view(torch.bool) if masks is not None else None, boxes, scores, labels, index,
-                             counts, tap_t, (oh, ow), keepalive=(lr_masks, pred_ious, multi_ious, tar_feat, ws, size_range,
-                                                                bound_inputs, bank, bank_dev),
+                             counts, tap_t, (oh, ow), keepalive=(lr_masks, pred_ious, multi_ious, tar_feat, ws, size_range, empty_rows,
+                                                                bound_inputs, bank, bank_dev, count_dev),
                              rle=rle_t, meta=meta, sized=size_range is not None,
-                             sim_cols=bank.n_cls if banked and bank is not None else None)
+                             sim_cols=bank.n_cls if banked and bank is not None else None, counted=counted, rows=rows)
+
+    def _bind_count(self, count_dev: torch.Tensor, k: int, capacity: int) -> None:
+        """Write a counted stage's live count on the current stream (nttt_match_count_bind: one kernel, the value in its
+        argument)."""
+        cap = _lib.MatchArgs()
+        cap.n = int(capacity)
+        _lib.check(self.lib.nttt_match_count_bind(count_dev.data_ptr(), int(k), ctypes.byref(cap),
+                                                  torch.cuda.current_stream(self.device).cuda_stream),
+                   "nttt_match_count_bind")
 
     def atlas_stats(self) -> dict:
         """The resize-table atlases the sized graphs of this device's context use: count, device bytes, build time."""
@@ -451,7 +504,7 @@ class MatchingStage:
     def graphed(self, n: int, c: int, ori_hw, iou_thr=None, key=None, n_multi: int = 0,
                 multi_first: int = 1, rle: bool = False, dense_masks: bool = True, persistent_out=None,
                 low_latency: bool = False, min_hw=None, bind: bool = False, chunk_prompts=None,
-                bank_capacity=None) -> "GraphedMatch":
+                bank_capacity=None, counted: bool = False) -> "GraphedMatch":
         """A CUDA-graph capture of the whole stage at fixed shapes with static input/output buffers.
         n_multi > 1: the static mask buffer is the decoder's raw [n, n_multi, 256, 256] output (+ `multi_ious`).
         rle / dense_masks: as in `match_async`.  `key` names the workspace slot and `persistent_out` the
@@ -466,9 +519,12 @@ class MatchingStage:
         prompts each (the last holds the rest), instead of one [n, n_multi, 256, 256] tensor.
         `bank_capacity=(n_cls, l_neg)`: the graph reads its memory bank on the device, so `replay(bank=...)` scores the
         image against any `PreparedBank` of up to n_cls classes (and, with l_neg > 0, up to l_neg negatives per class)
-        without a new capture (see `GraphedMatch.replay`)."""
+        without a new capture (see `GraphedMatch.replay`).
+        `counted=True`: `n` is a capacity; the graph reads the live candidate count on the device, so `replay(n=k)` (or,
+        bound, `replay(lr_masks=[k, 256, 256], pred_ious=[k])`) serves a compacted candidate list of any length
+        0 <= k <= n without a new capture (single-plane inputs only)."""
         return GraphedMatch(self, n, c, ori_hw, iou_thr, key, n_multi, multi_first, rle, dense_masks, persistent_out,
-                            low_latency, min_hw, bind, chunk_prompts, bank_capacity)
+                            low_latency, min_hw, bind, chunk_prompts, bank_capacity, counted)
 
 
 class GraphedMatch:
@@ -492,15 +548,23 @@ class GraphedMatch:
     device struct (`nttt_match_bank`) that every replay rewrites with one kernel on the replay's stream, so one capture
     serves every bank up to the capacity, and `set_prototypes*` never makes it re-capture.
 
+    With `counted=True` the graph is COUNTED: `n` is a capacity, and every replay writes the live candidate count k to a
+    device int32 with one kernel on the replay's stream; the kernels read it and touch no candidate at or past it.
+
     An unbanked graph keeps the prototype tensors it captured alive, and re-captures on the next replay once the stage's
     prototypes have been replaced (`set_prototypes*`)."""
 
     def __init__(self, stage: MatchingStage, n: int, c: int, ori_hw, iou_thr=None, key=None, n_multi: int = 0,
                  multi_first: int = 1, rle: bool = False, dense_masks: bool = True, persistent_out=None,
-                 low_latency: bool = False, min_hw=None, bind: bool = False, chunk_prompts=None, bank_capacity=None):
+                 low_latency: bool = False, min_hw=None, bind: bool = False, chunk_prompts=None, bank_capacity=None,
+                 counted: bool = False):
         dev = stage.device
         eh, ew = stage.cfg.enc_hw
         _check_candidates(int(n))
+        if counted and n_multi > 1:
+            raise ValueError("a counted graph takes single-plane candidates (compacted lists): n_multi must be <= 1")
+        self.counted = bool(counted)
+        self.count_dev = torch.zeros((1,), dtype=torch.int32, device=dev) if self.counted else None
         self.stage = stage
         self.n, self.c = int(n), int(c)
         self.n_multi = int(n_multi) if n_multi > 1 else 0
@@ -591,9 +655,10 @@ class GraphedMatch:
         _lib.check(self.stage.lib.nttt_match_bind(self.inputs_dev.data_ptr(), ctypes.byref(host),
                                                   ctypes.byref(self._shapes), stream), "nttt_match_bind")
 
-    def _check_bound(self, lr_masks, pred_ious, multi_ious, tar_feat) -> dict:
+    def _check_bound(self, lr_masks, pred_ious, multi_ious, tar_feat, k=None) -> dict:
         """The tensors a replay binds (the static buffers where one is not given), checked against the capture's shapes
-        on the host: dtype, device, contiguity, shape and the 16-byte alignment of every logits base."""
+        on the host: dtype, device, contiguity, shape and the 16-byte alignment of every logits base.  A counted graph
+        takes k candidate rows (its static buffers' first k where no tensor is given)."""
         dev = self.stage.device
         dev_index = dev.index if dev.index is not None else torch.cuda.current_device()
 
@@ -614,6 +679,8 @@ class GraphedMatch:
             return t
 
         got = self._static_inputs()
+        if k is not None:
+            got["lr_masks"], got["pred_ious"] = got["lr_masks"][:k], got["pred_ious"][:k]
         if tar_feat is not None:
             got["tar_feat"] = need(tar_feat, self.tar_feat.shape, "tar_feat")
         if self.n_multi:
@@ -633,9 +700,9 @@ class GraphedMatch:
             if multi_ious is not None:
                 raise ValueError("a single-plane graph takes pred_ious, not multi_ious")
             if pred_ious is not None:
-                got["pred_ious"] = need(pred_ious, self.pred_ious.shape, "pred_ious")
+                got["pred_ious"] = need(pred_ious, got["pred_ious"].shape, "pred_ious")
             if lr_masks is not None:
-                got["lr_masks"] = aligned(need(lr_masks, self.lr_masks.shape, "lr_masks"), "lr_masks")
+                got["lr_masks"] = aligned(need(lr_masks, got["lr_masks"].shape, "lr_masks"), "lr_masks")
         return got
 
     def capture(self, bank=None):
@@ -652,6 +719,9 @@ class GraphedMatch:
             _check_bank(bank, self.bank_capacity, self.c, st.device)
             st._bind_bank(self.bank_dev, bank, self.bank_capacity)
             kw.update(bank_capacity=self.bank_capacity, bank_dev=self.bank_dev)
+        if self.counted:
+            st._bind_count(self.count_dev, self.n, self.n)  # (the warm-up and the capture read the static buffers)
+            kw.update(count_capacity=self.n, count_dev=self.count_dev)
         side = torch.cuda.Stream(st.device)
         side.wait_stream(torch.cuda.current_stream(st.device))
         with torch.cuda.stream(side):
@@ -665,7 +735,8 @@ class GraphedMatch:
         self._proto = (st.proto, st.proto_neg)
         return self
 
-    def replay(self, ori_hw=None, lr_masks=None, pred_ious=None, multi_ious=None, tar_feat=None, bank=None) -> PendingResult:
+    def replay(self, ori_hw=None, lr_masks=None, pred_ious=None, multi_ious=None, tar_feat=None, bank=None,
+               n=None) -> PendingResult:
         """Launch the graph on the current stream.  A sized graph needs the image's size `ori_hw=(h, w)`.
 
         A bound graph (`bind=True`) also takes the image's inputs: `lr_masks` (a tensor, or with `chunk_prompts` the
@@ -678,8 +749,31 @@ class GraphedMatch:
         A banked graph (`bank_capacity`) scores against `bank`, a `PreparedBank` of the graph's channel count, device
         and kind (negative references or not) with no more classes or negatives than the capacity, or, without one,
         against the stage's current prototypes.  It is checked before anything is enqueued, bound on the current stream
-        and held by the result until the graph's next replay."""
+        and held by the result until the graph's next replay.
+
+        A counted graph (`counted=True`) matches k candidates, 0 <= k <= the capacity `n` of the capture: bound, the
+        given `lr_masks` [k, 256, 256] and `pred_ious` [k] (both, with the same k); otherwise `n=k` of its inputs' rows
+        (the static buffers' first k), by default all of them.  k is checked before anything is enqueued and written to
+        the device on the current stream; `get()` slices the `sim` / `obj_feats` taps to k rows."""
         given = lr_masks is not None or pred_ious is not None or multi_ious is not None or tar_feat is not None
+        k = None
+        if self.counted:
+            if (lr_masks is None) != (pred_ious is None):
+                raise ValueError("a counted graph takes lr_masks and pred_ious together (their rows are the count)")
+            if lr_masks is not None:
+                if not isinstance(lr_masks, torch.Tensor) or not isinstance(pred_ious, torch.Tensor):
+                    raise TypeError("lr_masks and pred_ious must be tensors")
+                k = int(lr_masks.shape[0])
+                if pred_ious.dim() != 1 or int(pred_ious.shape[0]) != k:
+                    raise ValueError(f"pred_ious has shape {tuple(pred_ious.shape)}, lr_masks {k} rows")
+                if n is not None and int(n) != k:
+                    raise ValueError(f"n={n} does not match the {k} rows of lr_masks")
+            else:
+                k = self.n if n is None else int(n)
+            if not 0 <= k <= self.n:
+                raise ValueError(f"{k} candidates are outside the graph's count capacity 0 .. {self.n}")
+        elif n is not None:
+            raise ValueError("this graph serves its capture's candidate count only; capture it with counted=True")
         if given and not self.bind:
             raise ValueError("this graph reads its static buffers; capture it with bind=True to pass inputs to replay()")
         banked = self.bank_capacity is not None
@@ -696,7 +790,10 @@ class GraphedMatch:
             hw = (int(ori_hw[0]), int(ori_hw[1]))
             if not (self.min_hw[0] <= hw[0] <= self.ori_hw[0] and self.min_hw[1] <= hw[1] <= self.ori_hw[1]):
                 raise ValueError(f"size {hw} is outside the graph's range {self.min_hw} .. {self.ori_hw}")
-        inputs = self._check_bound(lr_masks, pred_ious, multi_ious, tar_feat) if given else None
+        # (without tensors a bound graph reads its static buffers, whose first k rows start where all of them do)
+        inputs = self._check_bound(lr_masks, pred_ious, multi_ious, tar_feat, k) if given else None
+        if inputs is not None and k == 0:  # (an empty list has no address to bind; no row of the static ones is read)
+            inputs.update(lr_masks=self.lr_masks, pred_ious=self.pred_ious)
         st = self.stage
         if banked:
             bank = bank if bank is not None else st._current_bank()
@@ -713,9 +810,12 @@ class GraphedMatch:
             self.hw_dev.view(torch.int64).fill_(hw[0] | (hw[1] << 32))
         if banked:
             st._bind_bank(self.bank_dev, bank, self.bank_capacity)
+        if self.counted:
+            st._bind_count(self.count_dev, k, self.n)
         self.graph.replay()
         self.pending._meta = None  # the static buffers now hold a new image's result
         self.pending.ori_hw = hw
         self.pending._bound = inputs  # (the tensors this replay reads, held until the next one)
         self.pending._bank = bank
+        self.pending.rows = k if self.counted else self.pending.rows
         return self.pending
